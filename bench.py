@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR      (+ the matrices of the last timed step)
 
 A step = one pass of both hot paths over one library:
   basefc on config C3 (10k cells, 300M reads, ~60k features: hg38 genes + seeded nested intervals)
@@ -44,6 +45,33 @@ def matrix_checksum(row, col, val):
         x = (x ^ (x >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
         x ^= x >> np.uint64(31)
         return int((x * (np.asarray(val).astype(np.uint64) * np.uint64(2) + np.uint64(1))).sum(dtype=np.uint64))
+
+
+DUMP_LIMIT = 64 * 10 ** 6         # bytes of all --dump-outputs files together
+DUMP_ENTRIES = {"basefc": 1 << 21, "baf_ad": 1 << 17, "baf_dp": 1 << 17, "baf_oth": 1 << 17}
+
+
+def dump_outputs(out_dir, mats):
+    """mats = {name: (row, col, val, shape)}, entries sorted by (row, col).  Writes out_dir/<name>_row.npy, _col.npy,
+    _val.npy (every entry, or an evenly spaced sample of DUMP_ENTRIES[name] entries when there are more),
+    <name>_row_sum.npy (the total of every row, float64) and <name>_shape.npy (rows, cols, nnz): with the same
+    arguments two builds can be compared output for output."""
+    arrays = {}
+    for name, (row, col, val, shape) in mats.items():
+        row, col, val = (np.asarray(a) for a in (row, col, val))
+        nnz, cap = len(val), DUMP_ENTRIES[name]
+        arrays[name + "_shape"] = np.array([shape[0], shape[1], nnz], dtype=np.float64)
+        arrays[name + "_row_sum"] = np.bincount(row, weights=val, minlength=shape[0]).astype(np.float64)
+        idx = np.arange(nnz) if nnz <= cap else np.arange(cap, dtype=np.int64) * nnz // cap
+        exact = max(shape[0], shape[1], int(val.max()) + 1 if nnz else 0) <= 1 << 24     # float32 holds them exactly
+        for k, a in (("row", row), ("col", col), ("val", val)):
+            arrays["%s_%s" % (name, k)] = a[idx].astype(np.float32 if exact else np.float64)
+    total = sum(a.nbytes + 128 for a in arrays.values())      # + the .npy header
+    if total > DUMP_LIMIT:
+        raise RuntimeError("--dump-outputs: %d bytes, more than %d" % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def peaks():
@@ -200,7 +228,8 @@ class Batch(object):
 
     # SNP filter of the baf half: min_count = 1, min_maf = 0 (the values xcltk baf passes, baf/pipeline.py:355)
 
-    def step_device(self, checksum=False):
+    def step_device(self, checksum=False, keep=False):
+        """keep: the result also carries what the two calls returned ("outputs")."""
         ctx, fc, bf = self.ctx, self.fc, self.baf
         launches = 0
         w0 = time.perf_counter()
@@ -229,9 +258,12 @@ class Batch(object):
             for k, m in enumerate((ad, dp, oth)):
                 chk = (chk + matrix_checksum(bf.feat_index[m[0]] + (k + 1) * (1 << 24), m[1], m[2])) % (1 << 64)
         w4 = time.perf_counter()
-        return dict(nnz=seg.nnz, checksum=chk, wall_ms=[1e3 * (w1 - w0), 1e3 * w_baf, 1e3 * (w2 - w0), 1e3 * (w4 - w2)],
-                    launches=launches, t_fc=t_fc, t_pileup=t_p, t_count=t_c, baf_nnz=len(ad[2]) + len(dp[2]) + len(oth[2]),
-                    out_bytes=2 * seg.nnz + 16 * len(seg.over[0]) + 8 * (len(ad[2]) + len(dp[2]) + len(oth[2])))
+        res = dict(nnz=seg.nnz, checksum=chk, wall_ms=[1e3 * (w1 - w0), 1e3 * w_baf, 1e3 * (w2 - w0), 1e3 * (w4 - w2)],
+                   launches=launches, t_fc=t_fc, t_pileup=t_p, t_count=t_c, baf_nnz=len(ad[2]) + len(dp[2]) + len(oth[2]),
+                   out_bytes=2 * seg.nnz + 16 * len(seg.over[0]) + 8 * (len(ad[2]) + len(dp[2]) + len(oth[2])))
+        if keep:
+            res["outputs"] = (seg, (ad, dp, oth))
+        return res
 
     def make_host(self):
         self.h_fc = self.fc.dreads.download()         # pinned host record arrays
@@ -510,12 +542,16 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--scaling", default="strong", choices=["strong", "weak"],
                     help="N > 1: strong = one library cut into N genomic chunks; weak = one library per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the matrices of the last timed step to DIR/<name>.npy (one GPU; large ones sampled)")
     args = ap.parse_args()
     args.reads, args.baf_reads, args.cpu_sample = int(args.reads), int(args.baf_reads), int(args.cpu_sample)
     args.file_reads = int(args.file_reads)
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank, world, local, dist = dist_setup(args.gpus)
+    if args.dump_outputs and (world > 1 or args.impl != "ours"):
+        ap.error("--dump-outputs: the GPU path on one GPU only")
     from xcltk_b200 import engine
     strong = args.scaling == "strong"
     workload_name = ("basefc C3 (%d cells, %.0fM reads, %d features: hg38 genes + nested) + baf fc C2 "
@@ -565,10 +601,16 @@ def main():
     barrier_sync(dist, local)
     sampler.start()
     t0 = time.perf_counter()
-    infos = [batch.step_device() for _ in range(args.steps)]
+    infos = [batch.step_device(keep=bool(args.dump_outputs) and k == args.steps - 1) for k in range(args.steps)]
     barrier_sync(dist, local)
     dt = time.perf_counter() - t0
     clocks = sampler.stop()
+    if args.dump_outputs:            # the results hold library buffers: let them go before the e2e steps are timed
+        seg, baf_out = infos[-1].pop("outputs")
+        mats = {"basefc": seg.to_sorted() + (seg.shape,)}
+        mats.update(zip(("baf_ad", "baf_dp", "baf_oth"), baf_out))
+        dump_outputs(args.dump_outputs, mats)
+        del seg, baf_out, mats
     dt = max_over_ranks(dist, local, dt)
     # reads counted per step: the library once (strong: halo reads are not counted twice), or one library per GPU
     total_reads = float(args.reads + args.baf_reads) * (1 if strong else world)
