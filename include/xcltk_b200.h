@@ -132,15 +132,15 @@ const char *xg_host_last_error(void);
 int xg_write_mtx(const char *path, int32_t n_rows_in, const int64_t *row_ptr, const int32_t *out_row,
                  int32_t n_rows_out, int32_t n_cols, const int32_t *col, const int32_t *val,
                  int32_t n_threads);
-/* Same text from rows located by (row_beg, row_cnt) -- the "row_order" 0 layout of xg_coo.   */
+/* Same text from rows located by (row_beg, row_cnt) -- the XG_LAYOUT_ROWS layout of xg_coo.  */
 int xg_write_mtx_rows(const char *path, int32_t n_rows_in, const int64_t *row_beg, const int32_t *row_cnt,
                       const int32_t *out_row, int32_t n_rows_out, int32_t n_cols, const int32_t *col,
                       const int32_t *val, int32_t n_threads);
-/* ... and from the "narrow_rows" layout (colval16 + side list of large counts).                */
+/* ... and from the XG_LAYOUT_ROWS_NARROW layout (colval16 + side list of large counts).       */
 int xg_write_mtx_rows16(const char *path, int32_t n_rows_in, const int64_t *row_beg, const int32_t *row_cnt,
                         const int32_t *out_row, int32_t n_rows_out, int32_t n_cols, const uint32_t *colval16,
                         int64_t n_over, const int64_t *over_idx, const int32_t *over_val, int32_t n_threads);
-/* ... and from the 16-bit layout ("narrow_rows" 2: coldelta16 + side list, see xg_coo).          */
+/* ... and from the XG_LAYOUT_ROWS_TINY layout (coldelta16 + side list, see xg_coo).           */
 int xg_write_mtx_rows_tiny(const char *path, int32_t n_rows_in, const int64_t *row_beg, const int32_t *row_cnt,
                            const int32_t *out_row, int32_t n_rows_out, int32_t n_cols, const uint16_t *coldelta16,
                            int64_t n_over, const int64_t *over_idx, const int32_t *over_col, const int32_t *over_val,
@@ -153,12 +153,8 @@ typedef struct xg_dreads xg_dreads;      /* read records resident in HBM */
 int xg_create(int32_t device, xg_ctx **out);
 void xg_destroy(xg_ctx *ctx);
 const char *xg_last_error(xg_ctx *ctx);
-/* Options: "coo_rows" (default 1): 0 = results are CSR only (row == NULL; row_ptr, col, val),
- * which saves a third of the device->host result copy.  "row_order" (default 1): 0 = basefc
- * results keep the device's completion order of the rows (see xg_coo), which lets the result
- * copy overlap the counting.  "narrow_rows" (default 0; 2 = the 16-bit layout, see xg_coo.coldelta16): 1 = with "row_order" 0, entries are packed
- * into 32 bits (see xg_coo).  "stream_priority" 1: the context's stream is recreated with the device's
- * greatest priority (a context whose short kernels run beside another context's long ones).    */
+/* Options: "stream_priority" 1: the context's stream is recreated with the device's greatest
+ * priority (a context whose short kernels run beside another context's long ones).            */
 int xg_set_option(xg_ctx *ctx, const char *name, int64_t value);
 
 /* Host -> HBM copy of a decoded batch (the only cross-device traffic of the path).      */
@@ -249,28 +245,32 @@ typedef struct {
 } xg_barcodes;
 
 /* Sparse result, 0-based; library-owned pinned host memory, valid until xg_coo_free() (which
- * must be called before the context is destroyed).  Default layout: sorted by (row, col) with
- * CSR offsets.  With the context option "row_order" = 0 (xg_basefc / xg_basefc_host only) the
- * rows are stored in the order the device completed them -- each row still contiguous and
- * sorted by col -- and located by row_beg / row_cnt; this layout is copied to the host while
- * the later reads are still being counted, and xg_write_mtx_rows writes it directly.        */
+ * must be called before the context is destroyed).  The layout is chosen by the `layout` argument
+ * of xg_basefc / xg_basefc_host; every other entry point returns XG_LAYOUT_CSR.              */
+#define XG_LAYOUT_CSR 0         /* sorted by (row, col): row_ptr, col, val                             */
+#define XG_LAYOUT_ROWS 1        /* rows in the order the device completed them -- each row contiguous and
+                                 * sorted by col -- located by row_beg / row_cnt, entries in col / val;
+                                 * copied to the host while the later reads are still being counted   */
+#define XG_LAYOUT_ROWS_NARROW 2 /* the same, entries in colval16; with more than 65536 columns, or too
+                                 * many large counts for the side list, the call returns XG_LAYOUT_ROWS */
+#define XG_LAYOUT_ROWS_TINY 3   /* the same, entries in coldelta16; with too many entries for the side
+                                 * list the call returns XG_LAYOUT_ROWS                                */
 typedef struct {
     int64_t nnz;
     int32_t n_rows, n_cols;
-    const int32_t *row;       /* NULL when the context option "coo_rows" is 0, or "row_order" is 0 */
-    const int32_t *col;
+    const int32_t *col;       /* NULL in the packed layouts */
     const int32_t *val;
-    const int64_t *row_ptr;   /* CSR offsets, n_rows + 1; NULL when "row_order" is 0 */
-    const int64_t *row_beg;   /* "row_order" 0: first entry of every row, n_rows; else NULL */
-    const int32_t *row_cnt;   /* "row_order" 0: entries of every row, n_rows; else NULL */
-    /* "narrow_rows" 1 (with "row_order" 0 and n_cols <= 65536): col and val are NULL and entry k is
-     * colval16[k] = column | count << 16; a count field of 65535 means "look entry k up in the side
-     * list" (over_idx ascending is not guaranteed; n_over entries).  Half the bytes per entry.   */
+    const int64_t *row_ptr;   /* XG_LAYOUT_CSR: CSR offsets, n_rows + 1; else NULL */
+    const int64_t *row_beg;   /* rows layouts: first entry of every row, n_rows; else NULL */
+    const int32_t *row_cnt;   /* rows layouts: entries of every row, n_rows; else NULL */
+    /* XG_LAYOUT_ROWS_NARROW: entry k is colval16[k] = column | count << 16; a count field of 65535 means
+     * "look entry k up in the side list" (over_idx ascending is not guaranteed; n_over entries).  Half the
+     * bytes per entry.                                                                                  */
     const uint32_t *colval16;
     int64_t n_over;
     const int64_t *over_idx;
     const int32_t *over_val;
-    /* "narrow_rows" 2 (with "row_order" 0): col, val and colval16 are NULL and entry k is the 16-bit word
+    /* XG_LAYOUT_ROWS_TINY: entry k is the 16-bit word
      * coldelta16[k] = (column - previous column of the row - 1) << 4 | count  (count 1..15, gap <= 4095 columns);
      * the word 0 means "look entry k up in the side list": over_idx / over_col / over_val, n_over entries in no
      * particular order -- always the first entry of a row, else entries whose gap or count does not fit.
@@ -282,18 +282,19 @@ void xg_coo_free(xg_coo *m);
 
 /* basefc (needs a batch from xg_upload_reads, not xg_map_reads): replaces the per-feature loop fc_features()/fc_fet1() (rdr/fc/core.py:96-124,151-178)
  * and MCount/SCount (rdr/fc/mcount.py): out[row f, col c] = number of distinct UMI keys among
- * the reads of cell c that overlap feature f and pass check_read + the include test.     */
+ * the reads of cell c that overlap feature f and pass check_read + the include test.
+ * layout: one of XG_LAYOUT_*, the layout of *out (see xg_coo).                              */
 int xg_basefc(xg_ctx *ctx, const xg_dreads *reads, const xg_features *feats,
-              const xg_barcodes *cells, const xg_params *par, xg_coo **out);
+              const xg_barcodes *cells, const xg_params *par, int32_t layout, xg_coo **out);
 
 /* Same from a pinned host batch (xg_decode_bams output): the records are copied to HBM epoch
  * by epoch on a copy stream while the previous epochs are being counted, so that the call
  * costs about max(H2D, kernels) instead of their sum.  This is the end-to-end entry point. */
 int xg_basefc_host(xg_ctx *ctx, const xg_reads *host, const xg_features *feats,
-                   const xg_barcodes *cells, const xg_params *par, xg_coo **out);
-/* Matrix-Market text written on the device (SURVEY.md 8f N2; replaces merge_mtx, rdr/fc/utils.py:54-94): the rows of the LAST xg_basefc call of this context with "row_order" 0
- * are still in its staging area; they are formatted there (one warp per row, rows placed in input order by a scan)
- * and the text leaves through pinned buffers that writer threads pwrite() in parallel.  The same bytes as the
+                   const xg_barcodes *cells, const xg_params *par, int32_t layout, xg_coo **out);
+/* Matrix-Market text written on the device (SURVEY.md 8f N2; replaces merge_mtx, rdr/fc/utils.py:54-94): when the LAST
+ * xg_basefc call of this context produced a rows layout, its rows are still in its staging area; they are formatted
+ * there (one warp per row, rows placed in input order by a scan) and the text leaves through pinned buffers that writer threads pwrite() in parallel.  The same bytes as the
  * writers above (out_row[r]: 1-based output row of input row r, 0 = not emitted; n_rows_in = rows of that call). */
 int xg_basefc_write_mtx_device(xg_ctx *ctx, const char *path, int32_t n_rows_in, const int32_t *out_row,
                                int32_t n_rows_out, int32_t n_threads);

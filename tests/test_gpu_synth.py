@@ -56,7 +56,6 @@ def test_basefc_matches_oracle(gpu_ctx, fc_batch, kw):
     {"XG_SEG_MAX": "1000"},                             # light features in segments, the rest in sets
     {"XG_SEG_MAX": "100000000", "XG_EPOCH_TILES": "97"},     # every feature a segment; heavy ones split by hash
     {"XG_HIST_COLS": "700"},                            # three column ranges per row
-    {"XG_CNT_CTAS": "3"},
 ])
 def test_basefc_counting_modes_match_oracle(gpu_ctx, fc_batch, monkeypatch, env):
     """Every way the counting kernel can route a (feature, cell, UMI) triple gives the oracle's matrix."""
@@ -110,17 +109,16 @@ def test_basefc_umi_keys_that_do_not_fit_a_pair_word(gpu_ctx):
     host.close()
 
 
-def test_basefc_epoch_size_and_overlap_invariance(gpu_ctx, fc_batch, monkeypatch):
+def test_basefc_epoch_size_invariance(gpu_ctx, fc_batch, monkeypatch):
     w, conf = fc_batch, Conf()
     ref = None
-    for tiles, ov in (("100000", "1"), ("64", "1"), ("64", "0"), ("7", "1"), ("1", "1")):
+    for tiles in ("100000", "64", "7", "1"):
         monkeypatch.setenv("XG_EPOCH_TILES", tiles)
-        monkeypatch.setenv("XG_OVERLAP", ov)
         out = gpu_ctx.basefc(w.dreads, w.gid, w.beg, w.end, w.cell_keys, 2000, gpu_params(conf))[:3]
         out = [np.array(x) for x in out]
         if ref is None:
             ref = out
-        assert all(np.array_equal(a, b) for a, b in zip(ref, out)), (tiles, ov)
+        assert all(np.array_equal(a, b) for a, b in zip(ref, out)), tiles
 
 
 def test_basefc_feature_rows_are_independent(gpu_ctx, fc_batch):
@@ -287,7 +285,7 @@ def test_basefc_full_size_properties(gpu_ctx):
 
 
 def test_basefc_row_segments_equal_sorted_result(gpu_ctx, fc_batch, tmp_path):
-    """context option row_order = 0: rows in completion order, copied out under the kernels --
+    """the rows layouts: rows in completion order, copied out under the kernels --
     the same matrix as the sorted result, from HBM and streamed from the host, on the first call
     (no size hint: one copy at the end) and on repeated ones (per-epoch copies); and the
     Matrix-Market text written from it is the one written from the sorted CSR."""

@@ -155,7 +155,7 @@ def test_write_mtx_format(tmp_path):
 
 def test_write_mtx_rows_equals_csr_writer(tmp_path):
     """rows stored out of order and located by (row_beg, row_cnt) -- the layout basefc returns
-    with row_order = 0 -- give the text of the sorted CSR"""
+    with XG_LAYOUT_ROWS -- give the text of the sorted CSR"""
     import numpy as np
     from xcltk_b200 import engine, lib
     rng = np.random.RandomState(4)

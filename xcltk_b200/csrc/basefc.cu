@@ -33,7 +33,7 @@
 // XG_DEBUG_SYNC=1: synchronise and report after every launch (locates a faulting / hanging kernel)
 #define XG_DBG(name)                                                                          \
     do {                                                                                      \
-        if (dbg_sync) {                                                                       \
+        if (c.dbg_sync) {                                                                     \
             cudaError_t e_ = cudaDeviceSynchronize();                                         \
             fprintf(stderr, "[xg] %s: %s\n", name, cudaGetErrorString(e_));                   \
         }                                                                                     \
@@ -1058,7 +1058,7 @@ __global__ void k_pack_rows(const int32_t *col, const int32_t *val, uint32_t *pa
     packed[i] = c | (v16 << 16);
 }
 
-// "tiny" result entries (narrow_rows = 2): 16 bits each -- (column - previous column of the row - 1) << 4 | count.
+// "tiny" result entries (XG_LAYOUT_ROWS_TINY): 16 bits each -- (column - previous column of the row - 1) << 4 | count.
 // An entry that does not fit (the first of its row, a gap of more than 4095 columns, a count above 15) is the word
 // 0 and goes to the side list with its column and count.  A quarter of the bytes of (col, val) pairs.
 __global__ void k_mark_row_starts(const int64_t *seg_base, const int32_t *seg_nnz, int32_t n_rows, uint32_t *bits) {
@@ -1636,37 +1636,46 @@ static int upload_vec(xg_ctx *ctx, const std::vector<T> &v, const char *name, co
     return XG_OK;
 }
 
-// `src` != nullptr: the records of `rd` are not in HBM yet -- its device arrays are allocated
-// but empty, and every epoch's slice is copied from the pinned host batch `src` on a copy
-// stream just ahead of the epoch that counts it (H2D overlaps the kernels).
-static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, const xg_features *feats,
-                      const xg_barcodes *cells, const xg_params *par, xg_coo **out, bool force_sets = false) {
-    if (!ctx || !ctx->stream) return ctx ? ctx->fail(XG_E_CUDA, "context has no device") : XG_E_ARG;
-    if (!rd || !feats || !cells || !par || !out) return ctx->fail(XG_E_ARG, "xg_basefc: null argument");
-    if (feats->n < 0 || cells->n_samples <= 0) return ctx->fail(XG_E_ARG, "xg_basefc: empty sample list");
-    if (par->use_cell_tag && cells->n != cells->n_samples)
-        return ctx->fail(XG_E_ARG, "xg_basefc: barcode mode needs one key per column");
-    if (rd->mapped) return ctx->fail(XG_E_ARG, "xg_basefc: needs an uploaded batch (xg_upload_reads), not xg_map_reads");
-    XG_CUDA(cudaSetDevice(ctx->device));
-    ctx->fx_res_valid = false;
-    for (double &t : ctx->timing) t = 0;
+static double ms_since(std::chrono::steady_clock::time_point a) {
+    return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - a).count();
+}
+
+// One basefc call: what its phases (windows -> plan -> epochs -> result) hand on to one another.
+struct BasefcCall {
+    xg_ctx *ctx = nullptr;
+    const xg_dreads *rd = nullptr;
+    // != nullptr: the records of `rd` are not in HBM yet -- its device arrays are allocated but empty, and every
+    // epoch's slice is copied from this pinned host batch on a copy stream just ahead of the epoch that counts it
+    const xg_reads *src = nullptr;
+    int32_t n_rows = 0, n_cols = 0;
+    bool dbg_sync = false;
     int launches = 0;
-    const bool dbg_sync = getenv("XG_DEBUG_SYNC") && atoi(getenv("XG_DEBUG_SYNC")) != 0;
-    const int32_t n_rows = feats->n, n_cols = cells->n_samples;
+    FeatCache *fc = nullptr;          // interval index, windows and epoch plan (kept by the context)
+    size_t m = 0;                     // sorted features of the interval index
+    BasefcDev P;
+    const int32_t *d_sf_row = nullptr;
+    TileDesc *d_tdesc = nullptr;
+    bool seg_mode = false;
+    const int32_t *d_fin_feat = nullptr, *d_fin_set = nullptr, *d_fin_big = nullptr;
+    const uint64_t *d_zoff = nullptr, *d_zpre = nullptr;
+    int64_t *seg_base = nullptr;      // staging area: first entry and entries of every row, the entries
+    int32_t *seg_nnz = nullptr, *st_col = nullptr, *st_val = nullptr;
+    unsigned long long *cursor = nullptr;
+    unsigned int *fin_work = nullptr;
+    uint32_t *seg_cur = nullptr;
+    unsigned long long *h_cur = nullptr;    // rows layouts: the staging cursor after every epoch (mapped host memory)
+    int64_t h2d_bytes = 0;
+    double ms_index = 0, ms_windows = 0, ms_plan = 0, ms_upload = 0;
+    // per-epoch events: 0 count start, 1 count end, 2 epoch end, 3 H2D, 4 big finalize end
+    cudaEvent_t ev(int kind, int32_t e) const { return ctx->ev_pool[(size_t)5 * e + kind]; }
+    cudaEvent_t ev_init() const { return ctx->ev_pool[(size_t)5 * fc->plan.n_epochs]; }
+};
 
-    int32_t n_gid = 0;
-    for (auto &r : rd->h_runs) n_gid = std::max(n_gid, r.gid + 1);
-    if (!par->use_cell_tag)
-        for (auto &r : rd->h_runs)
-            if (r.bam_idx >= n_cols) return ctx->fail(XG_E_ARG, "more BAMs than sample columns");
-
-    // ---- interval index and per-feature tile windows (host), exact candidate counts (device)
-    auto now = [] { return std::chrono::steady_clock::now(); };
-    auto ms_since = [](std::chrono::steady_clock::time_point a) {
-        return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - a).count();
-    };
-    const auto t_call = now();
-    auto t_ph = now();
+// Interval index of the features (host) and every feature's tile window and exact candidate count (device).
+static int basefc_windows(BasefcCall &c, const xg_features *feats, int32_t n_gid) {
+    xg_ctx *ctx = c.ctx;
+    const xg_dreads *rd = c.rd;
+    auto t_ph = std::chrono::steady_clock::now();
     // the interval index depends on the features only: reuse it (host copy and the uploaded
     // device arrays, which live in named scratch buffers) while the caller passes the same set
     uint64_t fh = 1469598103934665603ull;
@@ -1682,6 +1691,7 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
         ctx->fx_cache = fc;
         ctx->fx_cache_free = [](void *p) { delete (FeatCache *)p; };
     }
+    c.fc = fc;
     const bool index_cached = fc->valid && fc->hash == fh;
     int rc = XG_OK;
     if (!index_cached) {
@@ -1691,11 +1701,10 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
         fc->hash = fh;
     }
     const FeatIndexHost &ix = fc->ix;
-    const size_t m = ix.sf_beg.size();
-    const double ms_index = ms_since(t_ph);
-    t_ph = now();
-    BasefcDev P;
-    memset(&P, 0, sizeof(P));
+    const size_t m = c.m = ix.sf_beg.size();
+    c.ms_index = ms_since(t_ph);
+    t_ph = std::chrono::steady_clock::now();
+    BasefcDev &P = c.P;
     P.pos_end = rd->pos_end;
     P.fmq = rd->fmq;
     P.cig_off = rd->cig_off;
@@ -1704,8 +1713,6 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
     if (((uintptr_t)rd->pos_end | (uintptr_t)rd->fmq | (uintptr_t)rd->cig_off | (uintptr_t)rd->keys |
          (uintptr_t)rd->cigar) & 15)
         return ctx->fail(XG_E_ARG, "xg_basefc: record arrays must be 16-byte aligned");
-    const int32_t *d_sf_row = nullptr;
-    const int32_t *d_sf_beg = nullptr;
     if (!index_cached) {
         std::vector<int4> stab4(ix.stab.size());
         for (size_t k = 0; k < ix.stab.size(); k++) {
@@ -1728,9 +1735,9 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
     }
     // the named scratch buffers keep their addresses between calls
     const int32_t *d_sf_goff = (const int32_t *)ctx->scratch["fx_sf_goff"].p;
-    d_sf_beg = (const int32_t *)ctx->scratch["fx_sf_beg"].p;
+    const int32_t *d_sf_beg = (const int32_t *)ctx->scratch["fx_sf_beg"].p;
     P.sf_end = (const int32_t *)ctx->scratch["fx_sf_end"].p;
-    d_sf_row = (const int32_t *)ctx->scratch["fx_sf_row"].p;
+    c.d_sf_row = (const int32_t *)ctx->scratch["fx_sf_row"].p;
     const int32_t *d_bnd_goff = (const int32_t *)ctx->scratch["fx_bnd_goff"].p;
     P.bnd = (const int32_t *)ctx->scratch["fx_bnd"].p;
     P.stab_off = (const int32_t *)ctx->scratch["fx_stab_off"].p;
@@ -1760,7 +1767,7 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
     XG_GET(d_tlo, int32_t, "fx_tlo", m + 1);
     XG_GET(d_thi, int32_t, "fx_thi", m + 1);
     XG_GET(d_tdesc, TileDesc, "fx_tdesc", rd->n_tiles + 1);
-    P.tdesc = d_tdesc;
+    P.tdesc = c.d_tdesc = d_tdesc;
     cudaEventRecord(ctx->ev[0], ctx->stream);
     XG_CUDA(cudaMemsetAsync(d_cand, 0, sizeof(unsigned long long) * (m + 1), ctx->stream));
     XG_CUDA(cudaMemsetAsync(d_tlo, 0x7f, sizeof(int32_t) * (m + 1), ctx->stream));
@@ -1772,17 +1779,17 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
     thi.assign(m, -1);
     if (n_warps > 0) {
         k_feature_windows<<<(unsigned)((n_warps + 7) / 8), 256, 0, ctx->stream>>>(
-            d_jobs, (int32_t)jobs.size(), n_warps, rd->tiles, rd->tile_pmax, rd->pos_end, src ? 0 : 1, d_sf_beg,
+            d_jobs, (int32_t)jobs.size(), n_warps, rd->tiles, rd->tile_pmax, rd->pos_end, c.src ? 0 : 1, d_sf_beg,
             P.sf_end, d_cand, d_tlo, d_thi);
-        launches++;
+        c.launches++;
         XG_DBG("k_feature_windows");
     }
     if (rd->n_tiles > 0) {
         // streaming call: the records (and with them the tiles' CIGAR ranges) arrive epoch by epoch
         k_tile_desc<<<(rd->n_tiles + 255) / 256, 256, 0, ctx->stream>>>(
             rd->tiles, rd->runs, rd->n_tiles, n_gid, d_sf_goff, d_bnd_goff, P.bnd, P.stab_off, P.stab4, P.fb,
-            src ? nullptr : rd->cig_off, d_tdesc);
-        launches++;
+            c.src ? nullptr : rd->cig_off, d_tdesc);
+        c.launches++;
         XG_DBG("k_tile_desc");
     }
     if (m) {
@@ -1791,13 +1798,24 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
         XG_CUDA(cudaMemcpyAsync(thi.data(), d_thi, sizeof(int32_t) * m, cudaMemcpyDeviceToHost, ctx->stream));
     }
     XG_CUDA(cudaStreamSynchronize(ctx->stream));
-    const double ms_windows = ms_since(t_ph);
+    c.ms_windows = ms_since(t_ph);
+    return XG_OK;
+}
 
-    // ---- pool layout over epochs
-    int32_t epoch_tiles = src ? 8192 : 65536;     // streaming: finer epochs = finer H2D / kernel overlap
-    if (const char *e = getenv(src ? "XG_EPOCH_TILES_HOST" : "XG_EPOCH_TILES")) {
+// The epoch plan (host) -- pool layout, which features each epoch zeroes and finalizes -- and its upload with the
+// filters and the buffers of the call.
+static int basefc_plan(BasefcCall &c, const xg_barcodes *cells, const xg_params *par, bool force_sets) {
+    xg_ctx *ctx = c.ctx;
+    const xg_dreads *rd = c.rd;
+    FeatCache *fc = c.fc;
+    const FeatIndexHost &ix = fc->ix;
+    const size_t m = c.m;
+    const int32_t n_cols = c.n_cols;
+    BasefcDev &P = c.P;
+    int32_t epoch_tiles = c.src ? 8192 : 65536;     // streaming: finer epochs = finer H2D / kernel overlap
+    if (const char *e = getenv(c.src ? "XG_EPOCH_TILES_HOST" : "XG_EPOCH_TILES")) {
         epoch_tiles = std::max(1, atoi(e));
-    } else if (!src && rd->n_tiles > 0) {
+    } else if (!c.src && rd->n_tiles > 0) {
         // equal epochs: a short last epoch costs its launches, its drain and its finalize like a full one
         const int32_t n_ep = (rd->n_tiles + epoch_tiles - 1) / epoch_tiles;
         epoch_tiles = (rd->n_tiles + n_ep - 1) / n_ep;
@@ -1808,11 +1826,12 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
     // flag and the call is redone with a set per feature (and the batch remembers it).
     bool seg_mode = !force_sets && n_cols <= (1 << 19) && rd->umi_compact != 0;      // cell bitmap + ranks in shared memory
     if (const char *e = getenv("XG_SEG_MODE")) seg_mode = seg_mode && atoi(e) != 0;
+    c.seg_mode = seg_mode;
     uint64_t seg_max = 1ull << 22;             // heavier features keep a set in global memory
     if (const char *e = getenv("XG_SEG_MAX")) seg_max = (uint64_t)atoll(e);
     EpochPlan &pl = fc->plan;
     pl.reset();
-    t_ph = now();
+    auto t_ph = std::chrono::steady_clock::now();
     // The reduction of a feature is one CTA's work and its passes are bound by the loads that CTA keeps in flight:
     // the few features with very many reads (a long tail in expression data) would be the critical path of their
     // epoch.  They get CTAs of 1024 threads, launched beside the ordinary ones.
@@ -1820,11 +1839,12 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
     if (const char *e = getenv("XG_SEG_BIG")) seg_big = (uint64_t)atoll(e);
     if (((size_t)10 << FS_BIG_TBL_LOG2) + (size_t)(2 * ((n_cols + 31) / 32) + 1) * 4 + sizeof(FsShared) + 1280 > 200 * 1024)
         seg_big = ~0ull;                      // so many cells that the big CTA's shared memory does not fit: no big CTAs
-    if ((rc = make_plan(ctx, cand, tlo, thi, rd->n_tiles, n_cols, epoch_tiles, seg_mode ? seg_max : 0, seg_big, pl))) return rc;
-    const double ms_plan = ms_since(t_ph);
-    t_ph = now();
-    const int32_t *d_fin_feat = nullptr, *d_fin_set = nullptr, *d_fin_big = nullptr;
-    const uint64_t *d_zoff = nullptr, *d_zpre = nullptr;
+    int rc = XG_OK;
+    if ((rc = make_plan(ctx, fc->cand, fc->tlo, fc->thi, rd->n_tiles, n_cols, epoch_tiles, seg_mode ? seg_max : 0,
+                        seg_big, pl)))
+        return rc;
+    c.ms_plan = ms_since(t_ph);
+    t_ph = std::chrono::steady_clock::now();
     std::vector<FeatDesc> &fdesc = fc->fdesc;
     std::vector<uint32_t> &segoff16 = fc->segoff16;
     fdesc.resize(m);
@@ -1838,14 +1858,14 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
     if (!ix.stab.empty()) {
         k_patch_stab<<<(unsigned)((ix.stab.size() + 255) / 256), 256, 0, ctx->stream>>>(
             (int4 *)ctx->scratch["fx_stab4"].p, (int32_t)ix.stab.size(), P.segoff16);
-        launches++;
+        c.launches++;
         XG_DBG("k_patch_stab");
     }
-    if ((rc = upload_vec(ctx, pl.fin_feat, "fx_fin_feat", &d_fin_feat))) return rc;
-    if ((rc = upload_vec(ctx, pl.fin_set, "fx_fin_set", &d_fin_set))) return rc;
-    if ((rc = upload_vec(ctx, pl.fin_big, "fx_fin_big", &d_fin_big))) return rc;
-    if ((rc = upload_vec(ctx, pl.zseg_off, "fx_zseg_off", &d_zoff))) return rc;
-    if ((rc = upload_vec(ctx, pl.zseg_pre, "fx_zseg_pre", &d_zpre))) return rc;
+    if ((rc = upload_vec(ctx, pl.fin_feat, "fx_fin_feat", &c.d_fin_feat))) return rc;
+    if ((rc = upload_vec(ctx, pl.fin_set, "fx_fin_set", &c.d_fin_set))) return rc;
+    if ((rc = upload_vec(ctx, pl.fin_big, "fx_fin_big", &c.d_fin_big))) return rc;
+    if ((rc = upload_vec(ctx, pl.zseg_off, "fx_zseg_off", &c.d_zoff))) return rc;
+    if ((rc = upload_vec(ctx, pl.zseg_pre, "fx_zseg_pre", &c.d_zpre))) return rc;
     if (par->min_incl_tab) {
         if (par->min_incl_tab_len <= rd->max_aln_len)
             return ctx->fail(XG_E_ARG, "min_incl_tab shorter than max aligned length + 1");
@@ -1869,23 +1889,39 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
         if ((rc = xg_build_barcode_table(ctx, cells, &P.bc))) return rc;
     }
     XG_GET(pool, uint8_t, "fx_pool", pl.pool_bytes + 16);
-    XG_GET(seg_base, int64_t, "fx_seg_base", n_rows + 1);
-    XG_GET(seg_nnz, int32_t, "fx_seg_nnz", n_rows + 1);
+    XG_GET(seg_base, int64_t, "fx_seg_base", c.n_rows + 1);
+    XG_GET(seg_nnz, int32_t, "fx_seg_nnz", c.n_rows + 1);
     XG_GET(st_col, int32_t, "fx_st_col", pl.staging_cap + 1);
     XG_GET(st_val, int32_t, "fx_st_val", pl.staging_cap + 1);
     XG_GET(cursor, unsigned long long, "fx_cursor", 2);
+    // per epoch: work counters of the ordinary finalize, counting, set finalize and big finalize launches; flags
     XG_GET(fin_work, unsigned int, "fx_fin_work", 4 * (pl.n_epochs + 1) + 4);
-    unsigned int *cnt_work = fin_work + pl.n_epochs + 1;          // tile counters of the counting launches
-    unsigned int *set_work = fin_work + 2 * (pl.n_epochs + 1);    // work counters of the set finalize launches
-    unsigned int *big_work = fin_work + 3 * (pl.n_epochs + 1);    // ... of the big-segment finalize launches
-    unsigned int *d_flags = fin_work + 4 * (pl.n_epochs + 1);
     XG_GET(seg_cur, uint32_t, "fx_seg_cur", m + 1);
+    c.seg_base = seg_base;
+    c.seg_nnz = seg_nnz;
+    c.st_col = st_col;
+    c.st_val = st_val;
+    c.cursor = cursor;
+    c.fin_work = fin_work;
+    c.seg_cur = seg_cur;
     P.pool = pool;
     P.seg_cur = seg_cur;
-    P.flags = d_flags;
+    P.flags = fin_work + 4 * (pl.n_epochs + 1);
     XG_CUDA(cudaStreamSynchronize(ctx->stream));   // host vectors above are about to die
-    const double ms_upload = ms_since(t_ph);
+    c.ms_upload = ms_since(t_ph);
+    return XG_OK;
+}
 
+// The epochs on the device: zero(e) -> count(e) -> finalize(e), one after another on the context's stream.  The
+// counting kernel is persistent and fills the GPU by itself; only the big-segment finalize runs beside the
+// ordinary one, and (xg_basefc_host) the copy of the next epoch's records beside the kernels.
+static int basefc_epochs(BasefcCall &c, bool rows) {
+    xg_ctx *ctx = c.ctx;
+    const xg_dreads *rd = c.rd;
+    const EpochPlan &pl = c.fc->plan;
+    const int32_t n_rows = c.n_rows, n_cols = c.n_cols;
+    const size_t m = c.m;
+    BasefcDev &P = c.P;
     // shared memory of the finalize kernels.  Segments: dedup table, rank counters, bitmap over the cells and
     // its prefix popcounts.  Sets: histogram (+ bitmap) over the cells -- all cells if they fit.
     const int bm_words = (n_cols + 31) / 32;
@@ -1906,69 +1942,49 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
     const size_t hist_bytes = (size_t)hist_cols * 4 + (size_t)((hist_cols + 31) / 32) * 4;
     XG_CUDA(cudaFuncSetAttribute(k_basefc_finalize_sets, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hist_bytes));
     const int fin_ctas_per_sm = std::max(1, std::min(4, (int)(220 * 1024 / (hist_bytes + 2048))));
-    int cnt_ctas_per_sm = 4;
-    if (const char *e = getenv("XG_CNT_CTAS")) cnt_ctas_per_sm = atoi(e) == 3 ? 3 : 4;
-    void (*count_kernel)(const BasefcDev) = cnt_ctas_per_sm == 3 ? k_basefc_count<3> : k_basefc_count<4>;
-    XG_CUDA(cudaFuncSetAttribute(count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CountSmem)));
+    XG_CUDA(cudaFuncSetAttribute(k_basefc_count<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CountSmem)));
 
-    // ---- device: epochs.  zero(e) -> count(e) -> finalize(e) per epoch:
-    //   zero(e)     after finalize(e-2)           (the arena of epoch e is free again)
-    //   count(e)    after zero(e)
-    //   finalize(e) after count(e)
-    // XG_OVERLAP=1: zero / finalize kernels on their own streams next to the counting kernel.  The counting
-    // kernel is persistent and fills the GPU by itself, so by default the kernels of the epochs follow one
-    // another on one stream and only the result copy runs beside them.
-    bool overlap = false;
-    if (const char *e = getenv("XG_OVERLAP")) overlap = pl.n_epochs > 1 && atoi(e) != 0;
-    const bool fork_big = !pl.fin_big.empty();
-    if ((overlap || src || fork_big) && !ctx->aux[0])
-        for (auto &st : ctx->aux) XG_CUDA(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-    if (src && !ctx->copy_stream) XG_CUDA(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-    while ((int32_t)ctx->ev_pool.size() < 6 * pl.n_epochs + 1) {
+    if (!pl.fin_big.empty() && !ctx->big_stream)
+        XG_CUDA(cudaStreamCreateWithFlags(&ctx->big_stream, cudaStreamNonBlocking));
+    if (c.src && !ctx->copy_stream) XG_CUDA(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+    while ((int32_t)ctx->ev_pool.size() < 5 * pl.n_epochs + 1) {
         cudaEvent_t ev;
         XG_CUDA(cudaEventCreate(&ev));
         ctx->ev_pool.push_back(ev);
     }
-    auto EV = [&](int kind, int32_t e) { return ctx->ev_pool[(size_t)6 * e + kind]; };   // 0 Z, 1 S, 2 C, 3 F, 4 H2D, 5 big F
-    cudaEvent_t ev_init = ctx->ev_pool[(size_t)6 * pl.n_epochs];
-    XG_CUDA(cudaMemsetAsync(seg_nnz, 0, sizeof(int32_t) * (size_t)(n_rows + 1), ctx->stream));
-    XG_CUDA(cudaMemsetAsync(seg_base, 0, sizeof(int64_t) * (size_t)(n_rows + 1), ctx->stream));
-    XG_CUDA(cudaMemsetAsync(cursor, 0, 16, ctx->stream));
-    XG_CUDA(cudaMemsetAsync(fin_work, 0, sizeof(unsigned int) * (size_t)(4 * (pl.n_epochs + 1) + 4), ctx->stream));
-    XG_CUDA(cudaMemsetAsync(seg_cur, 0, sizeof(uint32_t) * (m + 1), ctx->stream));
-    launches += 6;
-    cudaEventRecord(ev_init, ctx->stream);
-    cudaStream_t st_z = overlap ? ctx->aux[0] : ctx->stream, st_f = overlap ? ctx->aux[1] : ctx->stream;
-    if (overlap) {
-        cudaStreamWaitEvent(st_z, ev_init, 0);
-        cudaStreamWaitEvent(st_f, ev_init, 0);
-        cudaStreamWaitEvent(ctx->aux[2], ev_init, 0);
-    }
-    if (src) cudaStreamWaitEvent(ctx->copy_stream, ev_init, 0);
-    // "row_order" 0: the rows stay in the order they were completed; after every epoch the
-    // staging cursor is snapshotted so that the host can copy that epoch's rows out while the
-    // later epochs are still being counted
-    const bool staged_out = !ctx->row_order;
-    unsigned long long *h_cur = nullptr, *d_cur = nullptr;
-    if (staged_out) {
+    unsigned int *cnt_work = c.fin_work + pl.n_epochs + 1;          // tile counters of the counting launches
+    unsigned int *set_work = c.fin_work + 2 * (pl.n_epochs + 1);    // work counters of the set finalize launches
+    unsigned int *big_work = c.fin_work + 3 * (pl.n_epochs + 1);    // ... of the big-segment finalize launches
+    cudaStream_t st = ctx->stream;
+    XG_CUDA(cudaMemsetAsync(c.seg_nnz, 0, sizeof(int32_t) * (size_t)(n_rows + 1), st));
+    XG_CUDA(cudaMemsetAsync(c.seg_base, 0, sizeof(int64_t) * (size_t)(n_rows + 1), st));
+    XG_CUDA(cudaMemsetAsync(c.cursor, 0, 16, st));
+    XG_CUDA(cudaMemsetAsync(c.fin_work, 0, sizeof(unsigned int) * (size_t)(4 * (pl.n_epochs + 1) + 4), st));
+    XG_CUDA(cudaMemsetAsync(c.seg_cur, 0, sizeof(uint32_t) * (m + 1), st));
+    c.launches += 6;
+    cudaEventRecord(c.ev_init(), st);
+    if (c.src) cudaStreamWaitEvent(ctx->copy_stream, c.ev_init(), 0);
+    // rows layouts: the rows stay in the order they were completed; after every epoch the staging cursor is
+    // snapshotted so that the host can copy that epoch's rows out while the later epochs are still being counted
+    unsigned long long *d_cur = nullptr;
+    if (rows) {
         if (!ctx->d2h_stream) XG_CUDA(cudaStreamCreateWithFlags(&ctx->d2h_stream, cudaStreamNonBlocking));
-        h_cur = (unsigned long long *)ctx->pinned_get(sizeof(unsigned long long) * (size_t)(pl.n_epochs + 1));
-        if (!h_cur) return ctx->fail(XG_E_NOMEM, "out of pinned host memory");
-        if (cudaHostGetDevicePointer((void **)&d_cur, h_cur, 0) != cudaSuccess) {
+        c.h_cur = (unsigned long long *)ctx->pinned_get(sizeof(unsigned long long) * (size_t)(pl.n_epochs + 1));
+        if (!c.h_cur) return ctx->fail(XG_E_NOMEM, "out of pinned host memory");
+        if (cudaHostGetDevicePointer((void **)&d_cur, c.h_cur, 0) != cudaSuccess) {
             cudaGetLastError();
-            ctx->pinned_put(h_cur);
+            ctx->pinned_put(c.h_cur);
+            c.h_cur = nullptr;
             return ctx->fail(XG_E_CUDA, "pinned host memory is not mapped for the device");
         }
     }
-    int64_t h2d_bytes = 0;
     for (int32_t e = 0; e < pl.n_epochs; e++) {
-        // the counting kernels are persistent (they fill the GPU on their own): one stream for all of them
-        cudaStream_t st_c = ctx->stream;
-        if (src) {      // this epoch's records: host -> HBM on the copy stream
-            const int32_t ta = e * pl.epoch_tiles, tb_ = std::min(rd->n_tiles, ta + pl.epoch_tiles);
-            if (tb_ > ta) {
-                const int64_t ra = rd->h_tiles[(size_t)ta].rec_beg;
-                const int64_t rb = rd->h_tiles[(size_t)tb_ - 1].rec_beg + rd->h_tiles[(size_t)tb_ - 1].n_rec;
+        const int32_t t0 = e * pl.epoch_tiles, t1 = std::min(rd->n_tiles, t0 + pl.epoch_tiles);
+        if (c.src) {      // this epoch's records: host -> HBM on the copy stream
+            const xg_reads *src = c.src;
+            if (t1 > t0) {
+                const int64_t ra = rd->h_tiles[(size_t)t0].rec_beg;
+                const int64_t rb = rd->h_tiles[(size_t)t1 - 1].rec_beg + rd->h_tiles[(size_t)t1 - 1].n_rec;
                 const size_t nr = (size_t)(rb - ra);
                 const uint32_t ca = src->cig_off[ra], cb = src->cig_off[rb];
                 cudaStream_t cs = ctx->copy_stream;
@@ -1979,319 +1995,353 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
                 const uint32_t ca1 = ca ? ca - 1 : 0;      // one word back: a >=255-op count word
                 if (cb > ca1)
                     cudaMemcpyAsync(rd->cigar + ca1, src->cigar + ca1, (size_t)(cb - ca1) * 4, cudaMemcpyHostToDevice, cs);
-                h2d_bytes += (int64_t)(nr * 32 + 4 + (size_t)(cb - ca1) * 4);
+                c.h2d_bytes += (int64_t)(nr * 32 + 4 + (size_t)(cb - ca1) * 4);
             }
-            cudaEventRecord(EV(4, e), ctx->copy_stream);
-            cudaStreamWaitEvent(st_c, EV(4, e), 0);
+            cudaEventRecord(c.ev(3, e), ctx->copy_stream);
+            cudaStreamWaitEvent(st, c.ev(3, e), 0);
         }
         const int32_t z0 = pl.zero_ptr[(size_t)e], z1 = pl.zero_ptr[(size_t)e + 1];
         const int32_t n_seg = z1 - z0 - 1;
-        if (overlap && e >= 2) cudaStreamWaitEvent(st_z, EV(3, e - 2), 0);
         if (n_seg > 0) {
             const uint64_t total = pl.zseg_pre[(size_t)z1 - 1];
-            k_zero_segments<<<(unsigned)((total + ZERO_CHUNK - 1) / ZERO_CHUNK), 256, 0, st_z>>>(
-                pool, d_zoff + z0, d_zpre + z0, n_seg);
-            launches++;
+            k_zero_segments<<<(unsigned)((total + ZERO_CHUNK - 1) / ZERO_CHUNK), 256, 0, st>>>(
+                P.pool, c.d_zoff + z0, c.d_zpre + z0, n_seg);
+            c.launches++;
             XG_DBG("k_zero_segments");
         }
-        cudaEventRecord(EV(0, e), st_z);
-        if (overlap) cudaStreamWaitEvent(st_c, EV(0, e), 0);
-        const int32_t t0 = e * pl.epoch_tiles, t1 = std::min(rd->n_tiles, t0 + pl.epoch_tiles);
-        if (src && t1 > t0) {      // the CIGAR ranges of the tiles whose records have just arrived
-            k_tile_cig<<<(t1 - t0 + 255) / 256, 256, 0, st_c>>>(rd->tiles, t0, t1, rd->cig_off, d_tdesc);
-            launches++;
+        if (c.src && t1 > t0) {      // the CIGAR ranges of the tiles whose records have just arrived
+            k_tile_cig<<<(t1 - t0 + 255) / 256, 256, 0, st>>>(rd->tiles, t0, t1, rd->cig_off, c.d_tdesc);
+            c.launches++;
             XG_DBG("k_tile_cig");
         }
-        cudaEventRecord(EV(1, e), st_c);
+        cudaEventRecord(c.ev(0, e), st);
         if (t1 > t0 && m > 0) {
             P.tile0 = t0;
             P.tile1 = t1;
             P.work = cnt_work + e;
-            count_kernel<<<std::min(t1 - t0, 148 * cnt_ctas_per_sm), CNT_THREADS, sizeof(CountSmem), st_c>>>(P);
-            launches++;
+            k_basefc_count<4><<<std::min(t1 - t0, 148 * 4), CNT_THREADS, sizeof(CountSmem), st>>>(P);
+            c.launches++;
             XG_DBG("k_basefc_count");
         }
-        cudaEventRecord(EV(2, e), st_c);
+        cudaEventRecord(c.ev(1, e), st);
         const int32_t n_fin = pl.fin_ptr[(size_t)e + 1] - pl.fin_ptr[(size_t)e];
         const int32_t n_fin_set = pl.fin_set_ptr[(size_t)e + 1] - pl.fin_set_ptr[(size_t)e];
-        if (overlap) {
-            cudaStreamWaitEvent(st_f, EV(2, e), 0);
-            if (e > 0) cudaStreamWaitEvent(st_f, EV(2, e - 1), 0);
-        }
         // big segments first, on a stream of their own: their few large CTAs take their SMs before the ordinary
         // finalize CTAs fill the rest, and both kernels run side by side
         const int32_t n_big = pl.fin_big_ptr[(size_t)e + 1] - pl.fin_big_ptr[(size_t)e];
         if (n_big > 0) {
-            cudaStream_t st_b = overlap ? st_f : ctx->aux[1];
-            if (!overlap) cudaStreamWaitEvent(st_b, EV(2, e), 0);
-            k_basefc_finalize_segs<FS_BIG_THREADS, FS_BIG_TBL_LOG2><<<std::min(n_big, 148), FS_BIG_THREADS, big_bytes, st_b>>>(
-                pool, P.fdesc, seg_cur, d_sf_row, d_fin_big + pl.fin_big_ptr[(size_t)e], n_big, n_cols, big_work + e,
-                cursor, seg_base, seg_nnz, st_col, st_val);
-            launches++;
+            cudaStreamWaitEvent(ctx->big_stream, c.ev(1, e), 0);
+            k_basefc_finalize_segs<FS_BIG_THREADS, FS_BIG_TBL_LOG2><<<std::min(n_big, 148), FS_BIG_THREADS, big_bytes,
+                                                                     ctx->big_stream>>>(
+                P.pool, P.fdesc, c.seg_cur, c.d_sf_row, c.d_fin_big + pl.fin_big_ptr[(size_t)e], n_big, n_cols,
+                big_work + e, c.cursor, c.seg_base, c.seg_nnz, c.st_col, c.st_val);
+            c.launches++;
             XG_DBG("k_basefc_finalize_segs<big>");
-            if (!overlap) cudaEventRecord(EV(5, e), st_b);
+            cudaEventRecord(c.ev(4, e), ctx->big_stream);
         }
         if (n_fin > 0) {
             const int grid = std::min(n_fin, 148 * segs_ctas_per_sm);
-            k_basefc_finalize_segs<FS_THREADS, FS_TBL_LOG2><<<grid, FS_THREADS, segs_bytes, st_f>>>(
-                pool, P.fdesc, seg_cur, d_sf_row, d_fin_feat + pl.fin_ptr[(size_t)e], n_fin, n_cols, fin_work + e,
-                cursor, seg_base, seg_nnz, st_col, st_val);
-            launches++;
+            k_basefc_finalize_segs<FS_THREADS, FS_TBL_LOG2><<<grid, FS_THREADS, segs_bytes, st>>>(
+                P.pool, P.fdesc, c.seg_cur, c.d_sf_row, c.d_fin_feat + pl.fin_ptr[(size_t)e], n_fin, n_cols,
+                c.fin_work + e, c.cursor, c.seg_base, c.seg_nnz, c.st_col, c.st_val);
+            c.launches++;
             XG_DBG("k_basefc_finalize_segs");
         }
         if (n_fin_set > 0) {
             const int grid = std::min(n_fin_set, 148 * fin_ctas_per_sm);
-            k_basefc_finalize_sets<<<grid, FIN_THREADS, hist_bytes, st_f>>>(
-                pool, P.fdesc, d_sf_row, d_fin_set + pl.fin_set_ptr[(size_t)e], n_fin_set, n_cols, hist_cols,
-                set_work + e, cursor, seg_base, seg_nnz, st_col, st_val);
-            launches++;
+            k_basefc_finalize_sets<<<grid, FIN_THREADS, hist_bytes, st>>>(
+                P.pool, P.fdesc, c.d_sf_row, c.d_fin_set + pl.fin_set_ptr[(size_t)e], n_fin_set, n_cols, hist_cols,
+                set_work + e, c.cursor, c.seg_base, c.seg_nnz, c.st_col, c.st_val);
+            c.launches++;
             XG_DBG("k_basefc_finalize_sets");
         }
         // the snapshot is a store into mapped host memory, not a copy: a D2H of 8 bytes would queue
         // behind the result copies on the copy engine and stall the finalize stream with them
-        if (n_big > 0 && !overlap) cudaStreamWaitEvent(st_f, EV(5, e), 0);      // join: the epoch's rows are all reserved
-        if (h_cur) k_snapshot_cursor<<<1, 1, 0, st_f>>>(cursor, d_cur + e);
-        cudaEventRecord(EV(3, e), st_f);
-    }
-    if (overlap) {
-        cudaStreamWaitEvent(ctx->stream, EV(3, pl.n_epochs - 1), 0);
-        cudaStreamWaitEvent(ctx->stream, EV(2, pl.n_epochs - 1), 0);
-        if (pl.n_epochs > 1) cudaStreamWaitEvent(ctx->stream, EV(2, pl.n_epochs - 2), 0);
+        if (n_big > 0) cudaStreamWaitEvent(st, c.ev(4, e), 0);      // join: the epoch's rows are all reserved
+        if (d_cur) k_snapshot_cursor<<<1, 1, 0, st>>>(c.cursor, d_cur + e);
+        cudaEventRecord(c.ev(2, e), st);
     }
     XG_CUDA(cudaGetLastError());
-    if (staged_out) {
-        const auto t_tail = std::chrono::steady_clock::now();
-        xg_coo_owner *o = new xg_coo_owner();
-        memset(&o->m, 0, sizeof(o->m));
-        o->ctx = ctx;
-        auto give_up = [&](int code, const std::string &msg) {
-            cudaStreamSynchronize(ctx->d2h_stream);
-            cudaStreamSynchronize(ctx->stream);
-            for (void *q : o->bufs) ctx->pinned_put(q);
-            ctx->pinned_put(h_cur);
-            delete o;
-            return ctx->fail(code, msg);
-        };
-        int64_t cap = ctx->fx_nnz_hint > 0 ? ctx->fx_nnz_hint + ctx->fx_nnz_hint / 8 + 1024 : 0;
-        cap = std::min<int64_t>(cap, pl.staging_cap + 1);
-        // "narrow" results: column and count of an entry in one 32-bit word (16 bits each; counts of
-        // 65535 and more go to a side list).  Halves the bytes of the result copy, which is what a
-        // host shared by several GPUs runs out of first.
-        bool narrow = ctx->narrow_rows == 1 && n_cols <= 65536;
-        // "tiny" results: 16 bits per entry (column delta | small count), the rest in a side list
-        bool tiny = ctx->narrow_rows == 2;
-        const int64_t OVER_CAP = tiny ? (1 << 23) : (1 << 20);
-        uint32_t *d_packed = nullptr;
-        uint16_t *d_tiny = nullptr;
-        uint32_t *d_row_start = nullptr;
-        long long *d_over_idx = nullptr;
-        int32_t *d_over_val = nullptr, *d_over_col = nullptr;
-        unsigned int *d_over_n = nullptr;
-        const size_t row_start_words = (size_t)(pl.staging_cap + 32) / 32 + 1;
-        if (narrow || tiny) {
-            if (narrow) d_packed = (uint32_t *)ctx->get("fx_packed", sizeof(uint32_t) * (size_t)(pl.staging_cap + 1));
-            if (tiny) {
-                d_tiny = (uint16_t *)ctx->get("fx_tiny", sizeof(uint16_t) * (size_t)(pl.staging_cap + 2));
-                d_row_start = (uint32_t *)ctx->get("fx_row_start", sizeof(uint32_t) * row_start_words);
-                d_over_col = (int32_t *)ctx->get("fx_over_col", sizeof(int32_t) * (size_t)OVER_CAP);
-            }
-            d_over_idx = (long long *)ctx->get("fx_over_idx", sizeof(long long) * (size_t)OVER_CAP);
-            d_over_val = (int32_t *)ctx->get("fx_over_val", sizeof(int32_t) * (size_t)OVER_CAP);
-            d_over_n = (unsigned int *)ctx->get("fx_over_n", 16);
-            if ((narrow && !d_packed) || (tiny && (!d_tiny || !d_row_start || !d_over_col)) || !d_over_idx || !d_over_val ||
-                !d_over_n)
-                return give_up(XG_E_CUDA, ctx->err);
-            cudaMemsetAsync(d_over_n, 0, 4, ctx->d2h_stream);
-            if (tiny) cudaMemsetAsync(d_row_start, 0, sizeof(uint32_t) * row_start_words, ctx->d2h_stream);
+    return XG_OK;
+}
+
+// Rows layouts: every epoch's rows go to pinned host memory as soon as the epoch has finished, while the later
+// epochs are counted -- as they are, or packed on the way (16-bit column | 16-bit count, or the 16-bit words of
+// XG_LAYOUT_ROWS_TINY) with a side list for the entries that do not fit.  The first call has no size hint and
+// copies everything at the end.
+static int basefc_collect_rows(BasefcCall &c, int32_t layout, xg_coo **out) {
+    xg_ctx *ctx = c.ctx;
+    const EpochPlan &pl = c.fc->plan;
+    const int32_t n_rows = c.n_rows, n_cols = c.n_cols;
+    const int32_t *st_col = c.st_col, *st_val = c.st_val;
+    const auto t_tail = std::chrono::steady_clock::now();
+    xg_coo_owner *o = new xg_coo_owner();
+    memset(&o->m, 0, sizeof(o->m));
+    o->ctx = ctx;
+    auto give_up = [&](int code, const std::string &msg) {
+        cudaStreamSynchronize(ctx->d2h_stream);
+        cudaStreamSynchronize(ctx->stream);
+        for (void *q : o->bufs) ctx->pinned_put(q);
+        ctx->pinned_put(c.h_cur);
+        delete o;
+        return ctx->fail(code, msg);
+    };
+    int64_t cap = ctx->fx_nnz_hint > 0 ? ctx->fx_nnz_hint + ctx->fx_nnz_hint / 8 + 1024 : 0;
+    cap = std::min<int64_t>(cap, pl.staging_cap + 1);
+    // The entry format: narrow entries need 16-bit columns, and a packed format whose side list overflows falls
+    // back to plain entries (below) -- the only two places it is chosen.
+    int32_t fmt = layout == XG_LAYOUT_ROWS_NARROW && n_cols > 65536 ? XG_LAYOUT_ROWS : layout;
+    const bool narrow = fmt == XG_LAYOUT_ROWS_NARROW, tiny = fmt == XG_LAYOUT_ROWS_TINY;    // device buffers
+    const int64_t OVER_CAP = tiny ? (1 << 23) : (1 << 20);
+    uint32_t *d_packed = nullptr;
+    uint16_t *d_tiny = nullptr;
+    uint32_t *d_row_start = nullptr;
+    long long *d_over_idx = nullptr;
+    int32_t *d_over_val = nullptr, *d_over_col = nullptr;
+    unsigned int *d_over_n = nullptr;
+    const size_t row_start_words = (size_t)(pl.staging_cap + 32) / 32 + 1;
+    if (narrow || tiny) {
+        if (narrow) d_packed = (uint32_t *)ctx->get("fx_packed", sizeof(uint32_t) * (size_t)(pl.staging_cap + 1));
+        if (tiny) {
+            d_tiny = (uint16_t *)ctx->get("fx_tiny", sizeof(uint16_t) * (size_t)(pl.staging_cap + 2));
+            d_row_start = (uint32_t *)ctx->get("fx_row_start", sizeof(uint32_t) * row_start_words);
+            d_over_col = (int32_t *)ctx->get("fx_over_col", sizeof(int32_t) * (size_t)OVER_CAP);
         }
-        int32_t *h_col = nullptr, *h_val = nullptr;
-        uint32_t *h_packed = nullptr;
-        uint16_t *h_tiny = nullptr;
-        auto host_buffers = [&](int64_t n_cap) {
-            for (void *q : o->bufs) ctx->pinned_put(q);
-            o->bufs.clear();
-            h_col = h_val = nullptr;
-            h_packed = nullptr;
-            h_tiny = nullptr;
-            if (tiny) {
-                h_tiny = (uint16_t *)ctx->pinned_get((size_t)n_cap * 2 + 16);
-                if (h_tiny) o->bufs.push_back(h_tiny);
-                return h_tiny != nullptr;
-            }
-            if (narrow) {
-                h_packed = (uint32_t *)ctx->pinned_get((size_t)n_cap * 4);
-                if (h_packed) o->bufs.push_back(h_packed);
-                return h_packed != nullptr;
-            }
-            h_col = (int32_t *)ctx->pinned_get((size_t)n_cap * 4);
-            h_val = (int32_t *)ctx->pinned_get((size_t)n_cap * 4);
-            if (h_col) o->bufs.push_back(h_col);
-            if (h_val) o->bufs.push_back(h_val);
+        d_over_idx = (long long *)ctx->get("fx_over_idx", sizeof(long long) * (size_t)OVER_CAP);
+        d_over_val = (int32_t *)ctx->get("fx_over_val", sizeof(int32_t) * (size_t)OVER_CAP);
+        d_over_n = (unsigned int *)ctx->get("fx_over_n", 16);
+        if ((narrow && !d_packed) || (tiny && (!d_tiny || !d_row_start || !d_over_col)) || !d_over_idx || !d_over_val ||
+            !d_over_n)
+            return give_up(XG_E_CUDA, ctx->err);
+        cudaMemsetAsync(d_over_n, 0, 4, ctx->d2h_stream);
+        if (tiny) cudaMemsetAsync(d_row_start, 0, sizeof(uint32_t) * row_start_words, ctx->d2h_stream);
+    }
+    int32_t *h_col = nullptr, *h_val = nullptr;
+    uint32_t *h_packed = nullptr;
+    uint16_t *h_tiny = nullptr;
+    auto host_buffers = [&](int64_t n_cap) {
+        for (void *q : o->bufs) ctx->pinned_put(q);
+        o->bufs.clear();
+        h_col = h_val = nullptr;
+        h_packed = nullptr;
+        h_tiny = nullptr;
+        switch (fmt) {
+        case XG_LAYOUT_ROWS_TINY:
+            if ((h_tiny = (uint16_t *)ctx->pinned_get((size_t)n_cap * 2 + 16))) o->bufs.push_back(h_tiny);
+            return h_tiny != nullptr;
+        case XG_LAYOUT_ROWS_NARROW:
+            if ((h_packed = (uint32_t *)ctx->pinned_get((size_t)n_cap * 4))) o->bufs.push_back(h_packed);
+            return h_packed != nullptr;
+        default:
+            if ((h_col = (int32_t *)ctx->pinned_get((size_t)n_cap * 4))) o->bufs.push_back(h_col);
+            if ((h_val = (int32_t *)ctx->pinned_get((size_t)n_cap * 4))) o->bufs.push_back(h_val);
             return h_col && h_val;
-        };
-        auto queue_rows = [&](int64_t from, int64_t to) {       // staging entries [from, to) -> host
-            const size_t n = (size_t)(to - from);
-            if (tiny) {
-                // the rows finished so far have their places (seg_base / seg_nnz): mark their first entries
-                k_mark_row_starts<<<(n_rows + 255) / 256, 256, 0, ctx->d2h_stream>>>(seg_base, seg_nnz, n_rows, d_row_start);
-                k_pack_rows_tiny<<<(unsigned)((n + 255) / 256), 256, 0, ctx->d2h_stream>>>(
-                    st_col, st_val, d_row_start, d_tiny, from, to, d_over_idx, d_over_col, d_over_val, d_over_n,
-                    (unsigned int)OVER_CAP);
-                cudaMemcpyAsync(h_tiny + from, d_tiny + from, n * 2, cudaMemcpyDeviceToHost, ctx->d2h_stream);
-            } else if (narrow) {
-                k_pack_rows<<<(unsigned)((n + 255) / 256), 256, 0, ctx->d2h_stream>>>(st_col, st_val, d_packed, from, to, d_over_idx,
-                                                                                    d_over_val, d_over_n, (unsigned int)OVER_CAP);
-                cudaMemcpyAsync(h_packed + from, d_packed + from, n * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
-            } else {
-                cudaMemcpyAsync(h_col + from, st_col + from, n * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
-                cudaMemcpyAsync(h_val + from, st_val + from, n * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
-            }
-        };
-        if (cap > 0 && !host_buffers(cap)) return give_up(XG_E_NOMEM, "out of pinned host memory for the result");
-        int64_t done = 0;            // entries already queued for the host
-        bool fits = cap > 0;
-        for (int32_t e = 0; e < pl.n_epochs && fits; e++) {
-            cudaError_t ce = cudaEventSynchronize(EV(3, e));
-            if (ce != cudaSuccess) return give_up(XG_E_CUDA, std::string("basefc: ") + cudaGetErrorString(ce));
-            const int64_t cur = (int64_t)h_cur[e];
-            if (cur > cap) {
-                fits = false;        // more rows than the last call: finish with one copy at the end
-                break;
-            }
-            if (cur > done) {
-                queue_rows(done, cur);
-                done = cur;
-            }
         }
-        cudaError_t ce = cudaStreamSynchronize(ctx->stream);      // every epoch has finished
+    };
+    auto queue_rows = [&](int64_t from, int64_t to) {       // staging entries [from, to) -> host
+        const size_t n = (size_t)(to - from);
+        switch (fmt) {
+        case XG_LAYOUT_ROWS_TINY:
+            // the rows finished so far have their places (seg_base / seg_nnz): mark their first entries
+            k_mark_row_starts<<<(n_rows + 255) / 256, 256, 0, ctx->d2h_stream>>>(c.seg_base, c.seg_nnz, n_rows, d_row_start);
+            k_pack_rows_tiny<<<(unsigned)((n + 255) / 256), 256, 0, ctx->d2h_stream>>>(
+                st_col, st_val, d_row_start, d_tiny, from, to, d_over_idx, d_over_col, d_over_val, d_over_n,
+                (unsigned int)OVER_CAP);
+            cudaMemcpyAsync(h_tiny + from, d_tiny + from, n * 2, cudaMemcpyDeviceToHost, ctx->d2h_stream);
+            break;
+        case XG_LAYOUT_ROWS_NARROW:
+            k_pack_rows<<<(unsigned)((n + 255) / 256), 256, 0, ctx->d2h_stream>>>(st_col, st_val, d_packed, from, to, d_over_idx,
+                                                                                d_over_val, d_over_n, (unsigned int)OVER_CAP);
+            cudaMemcpyAsync(h_packed + from, d_packed + from, n * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
+            break;
+        default:
+            cudaMemcpyAsync(h_col + from, st_col + from, n * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
+            cudaMemcpyAsync(h_val + from, st_val + from, n * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
+        }
+    };
+    if (cap > 0 && !host_buffers(cap)) return give_up(XG_E_NOMEM, "out of pinned host memory for the result");
+    int64_t done = 0;            // entries already queued for the host
+    bool fits = cap > 0;
+    for (int32_t e = 0; e < pl.n_epochs && fits; e++) {
+        cudaError_t ce = cudaEventSynchronize(c.ev(2, e));
         if (ce != cudaSuccess) return give_up(XG_E_CUDA, std::string("basefc: ") + cudaGetErrorString(ce));
-        unsigned long long nnz_u = 0;
-        XG_CUDA(cudaMemcpy(&nnz_u, cursor, 8, cudaMemcpyDeviceToHost));
-        const int64_t nnz = (int64_t)nnz_u;
-        if (!fits || nnz > cap) {
-            cudaStreamSynchronize(ctx->d2h_stream);
-            cap = nnz + nnz / 8 + 1024;
-            if (!host_buffers(cap)) return give_up(XG_E_NOMEM, "out of pinned host memory for the result");
-            if (narrow || tiny) cudaMemsetAsync(d_over_n, 0, 4, ctx->d2h_stream);
-            done = 0;
+        const int64_t cur = (int64_t)c.h_cur[e];
+        if (cur > cap) {
+            fits = false;        // more rows than the last call: finish with one copy at the end
+            break;
         }
-        if (nnz > done) queue_rows(done, nnz);
-        unsigned int n_over = 0;
-        if (narrow || tiny) {
-            cudaMemcpyAsync(&n_over, d_over_n, 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
-            ce = cudaStreamSynchronize(ctx->d2h_stream);
-            if (ce != cudaSuccess) return give_up(XG_E_CUDA, std::string("result D2H: ") + cudaGetErrorString(ce));
-            if ((int64_t)n_over > OVER_CAP) {       // too many entries for the side list: plain 32-bit columns
-                narrow = tiny = false;
-                if (!host_buffers(cap)) return give_up(XG_E_NOMEM, "out of pinned host memory for the result");
-                if (nnz > 0) queue_rows(0, nnz);
-                n_over = 0;
-            }
+        if (cur > done) {
+            queue_rows(done, cur);
+            done = cur;
         }
-        long long *h_over_idx = nullptr;
-        int32_t *h_over_val = nullptr, *h_over_col = nullptr;
-        if (narrow || tiny) {
-            h_over_idx = (long long *)ctx->pinned_get(((size_t)n_over + 1) * 8);
-            h_over_val = (int32_t *)ctx->pinned_get(((size_t)n_over + 1) * 4);
-            if (h_over_idx) o->bufs.push_back(h_over_idx);
-            if (h_over_val) o->bufs.push_back(h_over_val);
-            if (tiny) {
-                h_over_col = (int32_t *)ctx->pinned_get(((size_t)n_over + 1) * 4);
-                if (h_over_col) o->bufs.push_back(h_over_col);
-            }
-            if (!h_over_idx || !h_over_val || (tiny && !h_over_col))
-                return give_up(XG_E_NOMEM, "out of pinned host memory for the result");
-            if (n_over) {
-                cudaMemcpyAsync(h_over_idx, d_over_idx, (size_t)n_over * 8, cudaMemcpyDeviceToHost, ctx->d2h_stream);
-                cudaMemcpyAsync(h_over_val, d_over_val, (size_t)n_over * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
-                if (tiny) cudaMemcpyAsync(h_over_col, d_over_col, (size_t)n_over * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
-            }
-        }
-        int64_t *h_beg = (int64_t *)ctx->pinned_get((size_t)(n_rows + 1) * 8);
-        int32_t *h_cnt = (int32_t *)ctx->pinned_get((size_t)(n_rows + 1) * 4);
-        if (h_beg) o->bufs.push_back(h_beg);
-        if (h_cnt) o->bufs.push_back(h_cnt);
-        if (!h_beg || !h_cnt) return give_up(XG_E_NOMEM, "out of pinned host memory for the result");
-        cudaMemcpyAsync(h_beg, seg_base, (size_t)n_rows * 8, cudaMemcpyDeviceToHost, ctx->d2h_stream);
-        cudaMemcpyAsync(h_cnt, seg_nnz, (size_t)n_rows * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
-        cudaEventRecord(ctx->ev[3], ctx->stream);
+    }
+    cudaError_t ce = cudaStreamSynchronize(ctx->stream);      // every epoch has finished
+    if (ce != cudaSuccess) return give_up(XG_E_CUDA, std::string("basefc: ") + cudaGetErrorString(ce));
+    unsigned long long nnz_u = 0;
+    XG_CUDA(cudaMemcpy(&nnz_u, c.cursor, 8, cudaMemcpyDeviceToHost));
+    const int64_t nnz = (int64_t)nnz_u;
+    if (!fits || nnz > cap) {
+        cudaStreamSynchronize(ctx->d2h_stream);
+        cap = nnz + nnz / 8 + 1024;
+        if (!host_buffers(cap)) return give_up(XG_E_NOMEM, "out of pinned host memory for the result");
+        if (fmt != XG_LAYOUT_ROWS) cudaMemsetAsync(d_over_n, 0, 4, ctx->d2h_stream);
+        done = 0;
+    }
+    if (nnz > done) queue_rows(done, nnz);
+    unsigned int n_over = 0;
+    if (fmt != XG_LAYOUT_ROWS) {
+        cudaMemcpyAsync(&n_over, d_over_n, 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
         ce = cudaStreamSynchronize(ctx->d2h_stream);
         if (ce != cudaSuccess) return give_up(XG_E_CUDA, std::string("result D2H: ") + cudaGetErrorString(ce));
-        cudaEventSynchronize(ctx->ev[3]);
-        ctx->pinned_put(h_cur);
-        ctx->fx_nnz_hint = nnz;
-        ctx->fx_res_valid = true;
-        ctx->fx_res_nnz = nnz;
-        ctx->fx_res_rows = n_rows;
-        ctx->fx_res_cols = n_cols;
-        ctx->timing[4] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_tail).count();
-        o->m.nnz = nnz;
-        o->m.n_rows = n_rows;
-        o->m.n_cols = n_cols;
-        o->m.col = h_col;
-        o->m.val = h_val;
-        o->m.colval16 = h_packed;
-        o->m.n_over = (narrow || tiny) ? (int64_t)n_over : 0;
-        o->m.over_idx = (const int64_t *)h_over_idx;
-        o->m.over_val = h_over_val;
-        o->m.coldelta16 = h_tiny;
-        o->m.over_col = h_over_col;
-        o->m.row_beg = h_beg;
-        o->m.row_cnt = h_cnt;
-        *out = &o->m;
-    } else if ((rc = xg_staging_to_coo(ctx, "fx", n_rows, n_cols, seg_base, seg_nnz, st_col, st_val, out, &launches))) {
-        return rc;
+        if ((int64_t)n_over > OVER_CAP) {       // too many entries for the side list: plain 32-bit columns
+            fmt = XG_LAYOUT_ROWS;
+            if (!host_buffers(cap)) return give_up(XG_E_NOMEM, "out of pinned host memory for the result");
+            if (nnz > 0) queue_rows(0, nnz);
+            n_over = 0;
+        }
     }
+    long long *h_over_idx = nullptr;
+    int32_t *h_over_val = nullptr, *h_over_col = nullptr;
+    if (fmt != XG_LAYOUT_ROWS) {
+        h_over_idx = (long long *)ctx->pinned_get(((size_t)n_over + 1) * 8);
+        h_over_val = (int32_t *)ctx->pinned_get(((size_t)n_over + 1) * 4);
+        if (h_over_idx) o->bufs.push_back(h_over_idx);
+        if (h_over_val) o->bufs.push_back(h_over_val);
+        if (fmt == XG_LAYOUT_ROWS_TINY) {
+            h_over_col = (int32_t *)ctx->pinned_get(((size_t)n_over + 1) * 4);
+            if (h_over_col) o->bufs.push_back(h_over_col);
+        }
+        if (!h_over_idx || !h_over_val || (fmt == XG_LAYOUT_ROWS_TINY && !h_over_col))
+            return give_up(XG_E_NOMEM, "out of pinned host memory for the result");
+        if (n_over) {
+            cudaMemcpyAsync(h_over_idx, d_over_idx, (size_t)n_over * 8, cudaMemcpyDeviceToHost, ctx->d2h_stream);
+            cudaMemcpyAsync(h_over_val, d_over_val, (size_t)n_over * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
+            if (h_over_col) cudaMemcpyAsync(h_over_col, d_over_col, (size_t)n_over * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
+        }
+    }
+    int64_t *h_beg = (int64_t *)ctx->pinned_get((size_t)(n_rows + 1) * 8);
+    int32_t *h_cnt = (int32_t *)ctx->pinned_get((size_t)(n_rows + 1) * 4);
+    if (h_beg) o->bufs.push_back(h_beg);
+    if (h_cnt) o->bufs.push_back(h_cnt);
+    if (!h_beg || !h_cnt) return give_up(XG_E_NOMEM, "out of pinned host memory for the result");
+    cudaMemcpyAsync(h_beg, c.seg_base, (size_t)n_rows * 8, cudaMemcpyDeviceToHost, ctx->d2h_stream);
+    cudaMemcpyAsync(h_cnt, c.seg_nnz, (size_t)n_rows * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream);
+    cudaEventRecord(ctx->ev[3], ctx->stream);
+    ce = cudaStreamSynchronize(ctx->d2h_stream);
+    if (ce != cudaSuccess) return give_up(XG_E_CUDA, std::string("result D2H: ") + cudaGetErrorString(ce));
+    cudaEventSynchronize(ctx->ev[3]);
+    ctx->pinned_put(c.h_cur);
+    ctx->fx_nnz_hint = nnz;
+    ctx->fx_res_valid = true;
+    ctx->fx_res_nnz = nnz;
+    ctx->fx_res_rows = n_rows;
+    ctx->fx_res_cols = n_cols;
+    ctx->timing[4] = ms_since(t_tail);
+    o->m.nnz = nnz;
+    o->m.n_rows = n_rows;
+    o->m.n_cols = n_cols;
+    o->m.col = h_col;
+    o->m.val = h_val;
+    o->m.colval16 = h_packed;
+    o->m.n_over = (int64_t)n_over;
+    o->m.over_idx = (const int64_t *)h_over_idx;
+    o->m.over_val = h_over_val;
+    o->m.coldelta16 = h_tiny;
+    o->m.over_col = h_over_col;
+    o->m.row_beg = h_beg;
+    o->m.row_cnt = h_cnt;
+    *out = &o->m;
+    return XG_OK;
+}
 
-    float t_all = 0;
-    const double t_d2h = ctx->timing[4];
+// xg_last_timing of the call (include/xcltk_b200.h); [4], the result copy, is set by the result phase.
+static void basefc_timing(const BasefcCall &c, std::chrono::steady_clock::time_point t_call) {
+    xg_ctx *ctx = c.ctx;
+    const EpochPlan &pl = c.fc->plan;
+    float t_all = 0, t_span = 0;
     double t_cnt = 0;
     cudaEventElapsedTime(&t_all, ctx->ev[0], ctx->ev[3]);
-    int n_cnt = 0;
     for (int32_t e = 0; e < pl.n_epochs; e++) {
         float t = 0;
-        cudaEventElapsedTime(&t, EV(1, e), EV(2, e));     // per-launch duration on its own stream
+        cudaEventElapsedTime(&t, c.ev(0, e), c.ev(1, e));
         t_cnt += t;
-        n_cnt++;
     }
-    float t_span = 0;
-    cudaEventElapsedTime(&t_span, ev_init, ctx->ev[3]);
+    cudaEventElapsedTime(&t_span, c.ev_init(), ctx->ev[3]);
     ctx->timing[0] = t_all;      // device time of the call: planning kernels, zero, count, finalize, gather
     ctx->timing[1] = t_cnt;      // sum over epochs of the counting kernel
-    ctx->timing[2] = launches;
+    ctx->timing[2] = c.launches;
     ctx->timing[3] = t_span;     // epochs + scan + gather (no host planning in between)
-    ctx->timing[4] = t_d2h;
     ctx->timing[5] = pl.n_epochs;
     ctx->timing[6] = (double)pl.pool_bytes;
     ctx->timing[7] = (double)pl.staging_cap;
-    ctx->timing[8] = ms_index;
-    ctx->timing[9] = ms_windows;
-    ctx->timing[10] = ms_plan;
-    ctx->timing[11] = ms_upload;
+    ctx->timing[8] = c.ms_index;
+    ctx->timing[9] = c.ms_windows;
+    ctx->timing[10] = c.ms_plan;
+    ctx->timing[11] = c.ms_upload;
     ctx->timing[12] = ms_since(t_call);
-    ctx->timing[13] = (double)h2d_bytes;
+    ctx->timing[13] = (double)c.h2d_bytes;
     ctx->timing[14] = (double)pl.n_seg_feat;
     ctx->timing[15] = (double)pl.n_set_feat;
-    if (seg_mode) {               // did every UMI key fit the pair word?
+}
+
+// `src` != nullptr: the records of `rd` are copied from the pinned host batch `src` epoch by epoch (BasefcCall).
+static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, const xg_features *feats,
+                      const xg_barcodes *cells, const xg_params *par, int32_t layout, xg_coo **out,
+                      bool force_sets = false) {
+    if (!ctx || !ctx->stream) return ctx ? ctx->fail(XG_E_CUDA, "context has no device") : XG_E_ARG;
+    if (!rd || !feats || !cells || !par || !out) return ctx->fail(XG_E_ARG, "xg_basefc: null argument");
+    if (layout < XG_LAYOUT_CSR || layout > XG_LAYOUT_ROWS_TINY) return ctx->fail(XG_E_ARG, "xg_basefc: unknown layout");
+    if (feats->n < 0 || cells->n_samples <= 0) return ctx->fail(XG_E_ARG, "xg_basefc: empty sample list");
+    if (par->use_cell_tag && cells->n != cells->n_samples)
+        return ctx->fail(XG_E_ARG, "xg_basefc: barcode mode needs one key per column");
+    if (rd->mapped) return ctx->fail(XG_E_ARG, "xg_basefc: needs an uploaded batch (xg_upload_reads), not xg_map_reads");
+    XG_CUDA(cudaSetDevice(ctx->device));
+    ctx->fx_res_valid = false;
+    for (double &t : ctx->timing) t = 0;
+    BasefcCall c;
+    memset(&c.P, 0, sizeof(c.P));
+    c.ctx = ctx;
+    c.rd = rd;
+    c.src = src;
+    c.n_rows = feats->n;
+    c.n_cols = cells->n_samples;
+    c.dbg_sync = getenv("XG_DEBUG_SYNC") && atoi(getenv("XG_DEBUG_SYNC")) != 0;
+    int32_t n_gid = 0;
+    for (auto &r : rd->h_runs) n_gid = std::max(n_gid, r.gid + 1);
+    if (!par->use_cell_tag)
+        for (auto &r : rd->h_runs)
+            if (r.bam_idx >= c.n_cols) return ctx->fail(XG_E_ARG, "more BAMs than sample columns");
+    const auto t_call = std::chrono::steady_clock::now();
+    int rc = XG_OK;
+    if ((rc = basefc_windows(c, feats, n_gid)) || (rc = basefc_plan(c, cells, par, force_sets)) ||
+        (rc = basefc_epochs(c, layout != XG_LAYOUT_CSR)))
+        return rc;
+    if (layout != XG_LAYOUT_CSR)
+        rc = basefc_collect_rows(c, layout, out);
+    else
+        rc = xg_staging_to_coo(ctx, "fx", c.n_rows, c.n_cols, c.seg_base, c.seg_nnz, c.st_col, c.st_val, out, &c.launches);
+    if (rc) return rc;
+    basefc_timing(c, t_call);
+    if (c.seg_mode) {             // did every UMI key fit the pair word?
         unsigned int h_flags = 0;
-        XG_CUDA(cudaMemcpy(&h_flags, d_flags, sizeof(h_flags), cudaMemcpyDeviceToHost));
+        XG_CUDA(cudaMemcpy(&h_flags, c.P.flags, sizeof(h_flags), cudaMemcpyDeviceToHost));
         if (h_flags & 1u) {
             xg_coo_free(*out);
             *out = nullptr;
             const_cast<xg_dreads *>(rd)->umi_compact = 0;
-            return basefc_run(ctx, rd, src, feats, cells, par, out, true);
+            return basefc_run(ctx, rd, src, feats, cells, par, layout, out, true);
         }
     }
     return XG_OK;
 }
 
 extern "C" int xg_basefc(xg_ctx *ctx, const xg_dreads *rd, const xg_features *feats,
-                         const xg_barcodes *cells, const xg_params *par, xg_coo **out) {
-    return basefc_run(ctx, rd, nullptr, feats, cells, par, out);
+                         const xg_barcodes *cells, const xg_params *par, int32_t layout, xg_coo **out) {
+    return basefc_run(ctx, rd, nullptr, feats, cells, par, layout, out);
 }
 
 extern "C" int xg_basefc_host(xg_ctx *ctx, const xg_reads *h, const xg_features *feats,
-                              const xg_barcodes *cells, const xg_params *par, xg_coo **out) {
+                              const xg_barcodes *cells, const xg_params *par, int32_t layout, xg_coo **out) {
     if (!ctx || !ctx->stream) return ctx ? ctx->fail(XG_E_CUDA, "context has no device") : XG_E_ARG;
     if (!h) return ctx->fail(XG_E_ARG, "xg_basefc_host: null argument");
     XG_CUDA(cudaSetDevice(ctx->device));
@@ -2300,16 +2350,7 @@ extern "C" int xg_basefc_host(xg_ctx *ctx, const xg_reads *h, const xg_features 
         cudaGetLastError();
         return ctx->fail(XG_E_ARG, "xg_basefc_host: record arrays must be pinned host memory");
     }
-    xg_dreads *d = new xg_dreads();
-    d->n_reads = h->n_reads;
-    d->n_cigar = h->n_cigar;
-    d->n_runs = h->n_runs;
-    d->n_tiles = h->n_tiles;
-    d->max_aln_len = h->max_aln_len;
-    d->max_span = h->max_span;
-    d->h_runs.assign(h->runs, h->runs + h->n_runs);
-    d->h_tiles.assign(h->tiles, h->tiles + h->n_tiles);
-    d->pooled = true;
+    xg_dreads *d = xg_dreads_new(h);
     const size_t n = (size_t)h->n_reads;
     d->pos_end = (int2 *)ctx->dev_get(n * 8 + 64);
     d->fmq = (uint32_t *)ctx->dev_get(n * 4 + 64);
@@ -2325,7 +2366,7 @@ extern "C" int xg_basefc_host(xg_ctx *ctx, const xg_reads *h, const xg_features 
         cudaMemcpyAsync(d->runs, h->runs, (size_t)h->n_runs * sizeof(xg_run), cudaMemcpyHostToDevice, ctx->stream);
         cudaMemcpyAsync(d->tiles, h->tiles, (size_t)h->n_tiles * sizeof(xg_tile), cudaMemcpyHostToDevice, ctx->stream);
         rc = xg_make_tile_pmax(ctx, d);
-        if (!rc) rc = basefc_run(ctx, d, h, feats, cells, par, out);
+        if (!rc) rc = basefc_run(ctx, d, h, feats, cells, par, layout, out);
     }
     cudaStreamSynchronize(ctx->stream);
     xg_dreads_free(ctx, d);
@@ -2333,7 +2374,7 @@ extern "C" int xg_basefc_host(xg_ctx *ctx, const xg_reads *h, const xg_features 
 }
 
 // ---- Matrix-Market text on the device (SURVEY.md 8f N2) ----------------------------------------------------------
-// Replaces merge_mtx (rdr/fc/utils.py:54-94) for the rows of the last xg_basefc call with "row_order" 0, which are
+// Replaces merge_mtx (rdr/fc/utils.py:54-94) for the rows of the last xg_basefc call with a rows layout, which are
 // still in the staging area: one warp per row sizes its lines ("<output row>\t<column + 1>\t<count>\n"), a scan
 // places the rows in input order, one warp per row writes its lines, and the text leaves through a ring of pinned
 // buffers that writer threads pwrite() at their offsets (several at a time: the page cache takes them in parallel).
@@ -2407,7 +2448,7 @@ extern "C" int xg_basefc_write_mtx_device(xg_ctx *ctx, const char *path, int32_t
     if (!ctx || !ctx->stream) return ctx ? ctx->fail(XG_E_CUDA, "context has no device") : XG_E_ARG;
     if (!path || !out_row || n_rows_in < 0) return ctx->fail(XG_E_ARG, "xg_basefc_write_mtx_device: bad argument");
     if (!ctx->fx_res_valid || ctx->fx_res_rows != n_rows_in)
-        return ctx->fail(XG_E_ARG, "xg_basefc_write_mtx_device: no basefc result with \"row_order\" 0 of that many rows on this context");
+        return ctx->fail(XG_E_ARG, "xg_basefc_write_mtx_device: the last basefc call of this context did not produce a rows layout of that many rows");
     XG_CUDA(cudaSetDevice(ctx->device));
     const int32_t n_rows = n_rows_in;
     const int64_t *seg_base = (const int64_t *)ctx->scratch["fx_seg_base"].p;

@@ -71,22 +71,19 @@ struct xg_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
     cudaStream_t copy_stream = nullptr;    // xg_basefc_host: H2D of the next epoch
-    cudaStream_t d2h_stream = nullptr;     // "row_order" 0: result rows copied out while later epochs run
+    cudaStream_t d2h_stream = nullptr;     // basefc rows layouts: result rows copied out while later epochs run
     int64_t fx_nnz_hint = 0;               // nnz of the last basefc call (sizes the pinned result up front)
-    // the rows of the last basefc call with "row_order" 0 are still in the staging area (scratch "fx_st_col" /
+    // the rows of the last basefc call with a rows layout are still in the staging area (scratch "fx_st_col" /
     // "fx_st_val", places in "fx_seg_base" / "fx_seg_nnz") until the next call: xg_basefc_write_mtx_device formats them
     bool fx_res_valid = false;
     int64_t fx_res_nnz = 0;
     int32_t fx_res_rows = 0, fx_res_cols = 0;
-    cudaStream_t aux[3] = {};              // overlapped epochs: zero, finalize, second count stream
+    cudaStream_t big_stream = nullptr;     // basefc: big-segment finalize beside the ordinary one
+    cudaStream_t inflate_stream = nullptr; // device decoder: second inflate stream
     cudaEvent_t ev[8] = {};
     std::vector<cudaEvent_t> ev_pool;     // per-epoch timing events
     std::string err;
     double timing[16] = {};
-    bool coo_rows = true;                  // results carry the row array (else CSR: row_ptr only)
-    int narrow_rows = 0;                   // ... and, with row_order 0: 1 = 16-bit column | 16-bit count per entry,
-                                           // 2 = 16 bits per entry (column delta | small count) + side list
-    bool row_order = true;                 // basefc results sorted by row (else rows as completed + row_beg/row_cnt)
     // growable named scratch buffers (avoid cudaMalloc/cudaFree on every call)
     struct Buf {
         void *p = nullptr;
@@ -336,3 +333,5 @@ __device__ __forceinline__ bool read_passes_flags(const FilterParams &f, uint32_
 
 int xg_build_barcode_table(xg_ctx *ctx, const xg_barcodes *cells, BarcodeTable *out);
 int xg_make_tile_pmax(xg_ctx *ctx, xg_dreads *d);
+// A pooled batch with the counts and the host run / tile index of `h`, and no device arrays yet.
+xg_dreads *xg_dreads_new(const xg_reads *h);

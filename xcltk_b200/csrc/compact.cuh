@@ -1,4 +1,4 @@
-// compact.cuh -- per-row staging segments -> (row, col)-sorted sparse output (CSR / COO).
+// compact.cuh -- per-row staging segments -> (row, col)-sorted sparse output (CSR).
 //
 // Tail of the emit loops `for i, smp in enumerate(conf.samples): if nu > 0: "%d\t%d\t%d"`
 // (xcltk/rdr/fc/core.py:109-124, xcltk/baf/fc/core.py:84-113): the finalize kernels write every
@@ -49,19 +49,18 @@ static __global__ void __launch_bounds__(1024) k_exclusive_scan(const int32_t *i
 static __global__ void __launch_bounds__(256) k_gather_rows(int32_t n_rows, const int64_t *seg_base,
                                                             const int32_t *seg_nnz, const int64_t *row_ptr,
                                                             const int32_t *st_col, const int32_t *st_val,
-                                                            int32_t *o_row, int32_t *o_col, int32_t *o_val) {
+                                                            int32_t *o_col, int32_t *o_val) {
     for (int row = blockIdx.x; row < n_rows; row += gridDim.x) {
         const int n = seg_nnz[row];
         const int64_t src = seg_base[row], dst = row_ptr[row];
         for (int k = threadIdx.x; k < n; k += blockDim.x) {
-            if (o_row) o_row[dst + k] = row;
             o_col[dst + k] = st_col[src + k];
             o_val[dst + k] = st_val[src + k];
         }
     }
 }
 
-// seg_nnz -> row_ptr (scan), staging -> (row, col)-sorted device COO (gather), -> pinned host.
+// seg_nnz -> row_ptr (scan), staging -> (row, col)-sorted device CSR (gather), -> pinned host.
 // One host synchronisation for nnz.  `tag` names the scratch buffers.
 static int xg_staging_to_coo(xg_ctx *ctx, const char *tag, int32_t n_rows, int32_t n_cols,
                              const int64_t *seg_base, const int32_t *seg_nnz, const int32_t *st_col,
@@ -72,42 +71,34 @@ static int xg_staging_to_coo(xg_ctx *ctx, const char *tag, int32_t n_rows, int32
     int64_t nnz = 0;
     XG_CUDA(cudaMemcpyAsync(&nnz, row_ptr + n_rows, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
     XG_CUDA(cudaStreamSynchronize(ctx->stream));
-    const bool want_rows = ctx->coo_rows;      // CSR only: a third less D2H (xg_set_option "coo_rows")
-    int32_t *d_row = nullptr;
-    if (want_rows) {
-        d_row = (int32_t *)ctx->get((t + "_coo_row").c_str(), sizeof(int32_t) * (size_t)(nnz + 1));
-        if (!d_row) return XG_E_CUDA;
-    }
     XG_GET(d_col, int32_t, (t + "_coo_col").c_str(), nnz + 1);
     XG_GET(d_val, int32_t, (t + "_coo_val").c_str(), nnz + 1);
     *n_launches += 1;
     if (nnz > 0) {
         k_gather_rows<<<n_rows < 148 * 32 ? n_rows : 148 * 32, 256, 0, ctx->stream>>>(
-            n_rows, seg_base, seg_nnz, row_ptr, st_col, st_val, d_row, d_col, d_val);
+            n_rows, seg_base, seg_nnz, row_ptr, st_col, st_val, d_col, d_val);
         *n_launches += 1;
     }
     cudaEventRecord(ctx->ev[3], ctx->stream);
     XG_CUDA(cudaGetLastError());
     xg_coo_owner *o = new xg_coo_owner();
     memset(&o->m, 0, sizeof(o->m));
-    void *hp[4] = {nullptr, nullptr, nullptr, nullptr};
-    size_t hs[4] = {want_rows ? (size_t)(nnz + 1) * 4 : 16, (size_t)(nnz + 1) * 4, (size_t)(nnz + 1) * 4,
-                    (size_t)(n_rows + 1) * 8};
-    for (int k = 0; k < 4; k++)
+    void *hp[3] = {nullptr, nullptr, nullptr};
+    size_t hs[3] = {(size_t)(nnz + 1) * 4, (size_t)(nnz + 1) * 4, (size_t)(n_rows + 1) * 8};
+    for (int k = 0; k < 3; k++)
         if (!(hp[k] = ctx->pinned_get(hs[k]))) {
             for (int q = 0; q < k; q++) ctx->pinned_put(hp[q]);
             delete o;
             return ctx->fail(XG_E_NOMEM, "out of pinned host memory for the result");
         }
-    o->bufs = {hp[0], hp[1], hp[2], hp[3]};
+    o->bufs = {hp[0], hp[1], hp[2]};
     o->ctx = ctx;
     cudaEventRecord(ctx->ev[4], ctx->stream);
     if (nnz > 0) {
-        if (want_rows) cudaMemcpyAsync(hp[0], d_row, (size_t)nnz * 4, cudaMemcpyDeviceToHost, ctx->stream);
-        cudaMemcpyAsync(hp[1], d_col, (size_t)nnz * 4, cudaMemcpyDeviceToHost, ctx->stream);
-        cudaMemcpyAsync(hp[2], d_val, (size_t)nnz * 4, cudaMemcpyDeviceToHost, ctx->stream);
+        cudaMemcpyAsync(hp[0], d_col, (size_t)nnz * 4, cudaMemcpyDeviceToHost, ctx->stream);
+        cudaMemcpyAsync(hp[1], d_val, (size_t)nnz * 4, cudaMemcpyDeviceToHost, ctx->stream);
     }
-    cudaMemcpyAsync(hp[3], row_ptr, (size_t)(n_rows + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream);
+    cudaMemcpyAsync(hp[2], row_ptr, (size_t)(n_rows + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream);
     cudaEventRecord(ctx->ev[5], ctx->stream);
     cudaError_t ce = cudaStreamSynchronize(ctx->stream);
     if (ce != cudaSuccess) {
@@ -121,10 +112,9 @@ static int xg_staging_to_coo(xg_ctx *ctx, const char *tag, int32_t n_rows, int32
     o->m.nnz = nnz;
     o->m.n_rows = n_rows;
     o->m.n_cols = n_cols;
-    o->m.row = want_rows ? (const int32_t *)hp[0] : nullptr;
-    o->m.col = (const int32_t *)hp[1];
-    o->m.val = (const int32_t *)hp[2];
-    o->m.row_ptr = (const int64_t *)hp[3];
+    o->m.col = (const int32_t *)hp[0];
+    o->m.val = (const int32_t *)hp[1];
+    o->m.row_ptr = (const int64_t *)hp[2];
     *out = &o->m;
     return XG_OK;
 }
@@ -136,8 +126,7 @@ static int xg_staging_to_coo(xg_ctx *ctx, const char *tag, int32_t n_rows, int32
 static __global__ void __launch_bounds__(256) k_gather_rows3(int32_t n_rows, int64_t st_stride, const int64_t *seg_base,
                                                              const int32_t *seg_nnz, const int64_t *row_ptr,
                                                              const int32_t *st_col, const int32_t *st_val,
-                                                             int32_t *o_row, int32_t *o_col, int32_t *o_val,
-                                                             int64_t *o_ptr) {
+                                                             int32_t *o_col, int32_t *o_val, int64_t *o_ptr) {
     for (int g = blockIdx.x; g < 3 * n_rows; g += gridDim.x) {
         const int wh = g / n_rows, row = g - wh * n_rows;
         const int n = seg_nnz[g];
@@ -148,7 +137,6 @@ static __global__ void __launch_bounds__(256) k_gather_rows3(int32_t n_rows, int
             if (row == n_rows - 1) o_ptr[(int64_t)wh * (n_rows + 1) + n_rows] = dst + n - first;
         }
         for (int k = threadIdx.x; k < n; k += blockDim.x) {
-            if (o_row) o_row[dst + k] = row;
             o_col[dst + k] = st_col[src + k];
             o_val[dst + k] = st_val[src + k];
         }
@@ -168,17 +156,11 @@ static int xg_staging_to_coo3(xg_ctx *ctx, const char *tag, int32_t n_rows, int3
         XG_CUDA(cudaMemcpyAsync(&edge[k], row_ptr + (size_t)k * n_rows, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
     XG_CUDA(cudaStreamSynchronize(ctx->stream));
     const int64_t total = edge[3];
-    const bool want_rows = ctx->coo_rows;
-    int32_t *d_row = nullptr;
-    if (want_rows) {
-        d_row = (int32_t *)ctx->get((t + "_coo_row").c_str(), sizeof(int32_t) * (size_t)(total + 1));
-        if (!d_row) return XG_E_CUDA;
-    }
     XG_GET(d_col, int32_t, (t + "_coo_col").c_str(), total + 1);
     XG_GET(d_val, int32_t, (t + "_coo_val").c_str(), total + 1);
     if (n_rows > 0) {
         k_gather_rows3<<<3 * n_rows < 148 * 32 ? 3 * n_rows : 148 * 32, 256, 0, ctx->stream>>>(
-            n_rows, st_stride, seg_base, seg_nnz, row_ptr, st_col, st_val, d_row, d_col, d_val, o_ptr);
+            n_rows, st_stride, seg_base, seg_nnz, row_ptr, st_col, st_val, d_col, d_val, o_ptr);
         *n_launches += 1;
     } else {
         XG_CUDA(cudaMemsetAsync(o_ptr, 0, sizeof(int64_t) * 4, ctx->stream));
@@ -199,10 +181,9 @@ static int xg_staging_to_coo3(xg_ctx *ctx, const char *tag, int32_t n_rows, int3
         xg_coo_owner *o = own[k] = new xg_coo_owner();
         memset(&o->m, 0, sizeof(o->m));
         o->ctx = ctx;
-        size_t hs[4] = {want_rows ? (size_t)(nnz + 1) * 4 : 16, (size_t)(nnz + 1) * 4, (size_t)(nnz + 1) * 4,
-                        (size_t)(n_rows + 1) * 8};
-        void *hp[4];
-        for (int q = 0; q < 4; q++) {
+        size_t hs[3] = {(size_t)(nnz + 1) * 4, (size_t)(nnz + 1) * 4, (size_t)(n_rows + 1) * 8};
+        void *hp[3];
+        for (int q = 0; q < 3; q++) {
             if (!(hp[q] = ctx->pinned_get(hs[q]))) {
                 drop();
                 return ctx->fail(XG_E_NOMEM, "out of pinned host memory for the result");
@@ -210,19 +191,17 @@ static int xg_staging_to_coo3(xg_ctx *ctx, const char *tag, int32_t n_rows, int3
             o->bufs.push_back(hp[q]);
         }
         if (nnz > 0) {
-            if (want_rows) cudaMemcpyAsync(hp[0], d_row + edge[k], (size_t)nnz * 4, cudaMemcpyDeviceToHost, ctx->stream);
-            cudaMemcpyAsync(hp[1], d_col + edge[k], (size_t)nnz * 4, cudaMemcpyDeviceToHost, ctx->stream);
-            cudaMemcpyAsync(hp[2], d_val + edge[k], (size_t)nnz * 4, cudaMemcpyDeviceToHost, ctx->stream);
+            cudaMemcpyAsync(hp[0], d_col + edge[k], (size_t)nnz * 4, cudaMemcpyDeviceToHost, ctx->stream);
+            cudaMemcpyAsync(hp[1], d_val + edge[k], (size_t)nnz * 4, cudaMemcpyDeviceToHost, ctx->stream);
         }
-        cudaMemcpyAsync(hp[3], o_ptr + (size_t)k * ((size_t)n_rows + 1), (size_t)(n_rows + 1) * 8, cudaMemcpyDeviceToHost,
+        cudaMemcpyAsync(hp[2], o_ptr + (size_t)k * ((size_t)n_rows + 1), (size_t)(n_rows + 1) * 8, cudaMemcpyDeviceToHost,
                         ctx->stream);
         o->m.nnz = nnz;
         o->m.n_rows = n_rows;
         o->m.n_cols = n_cols;
-        o->m.row = want_rows ? (const int32_t *)hp[0] : nullptr;
-        o->m.col = (const int32_t *)hp[1];
-        o->m.val = (const int32_t *)hp[2];
-        o->m.row_ptr = (const int64_t *)hp[3];
+        o->m.col = (const int32_t *)hp[0];
+        o->m.val = (const int32_t *)hp[1];
+        o->m.row_ptr = (const int64_t *)hp[2];
     }
     cudaEventRecord(ctx->ev[5], ctx->stream);
     const cudaError_t ce = cudaStreamSynchronize(ctx->stream);

@@ -56,10 +56,8 @@ void xg_destroy(xg_ctx *ctx) {
         for (auto &ev : ctx->ev)
             if (ev) cudaEventDestroy(ev);
         for (auto &ev : ctx->ev_pool) cudaEventDestroy(ev);
-        for (auto &st : ctx->aux)
+        for (cudaStream_t st : {ctx->big_stream, ctx->inflate_stream, ctx->copy_stream, ctx->d2h_stream})
             if (st) cudaStreamDestroy(st);
-        if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
-        if (ctx->d2h_stream) cudaStreamDestroy(ctx->d2h_stream);
         for (auto &b : ctx->pinned) cudaFreeHost(b.p);
         for (auto &b : ctx->devbufs) cudaFree(b.p);
         if (ctx->fx_cache && ctx->fx_cache_free) ctx->fx_cache_free(ctx->fx_cache);
@@ -70,18 +68,6 @@ void xg_destroy(xg_ctx *ctx) {
 
 int xg_set_option(xg_ctx *ctx, const char *name, int64_t value) {
     if (!ctx || !name) return XG_E_ARG;
-    if (std::string(name) == "coo_rows") {
-        ctx->coo_rows = value != 0;
-        return XG_OK;
-    }
-    if (std::string(name) == "narrow_rows") {
-        ctx->narrow_rows = value == 2 ? 2 : value != 0 ? 1 : 0;
-        return XG_OK;
-    }
-    if (std::string(name) == "row_order") {
-        ctx->row_order = value != 0;
-        return XG_OK;
-    }
     if (std::string(name) == "stream_priority") {
         // 1: the context's stream gets the device's greatest priority -- for a context whose short kernels run
         // beside another context's long ones on the same GPU (their CTAs are scheduled first whenever both wait)
@@ -139,16 +125,7 @@ int xg_upload_reads(xg_ctx *ctx, const xg_reads *h, xg_dreads **out) {
     if (!ctx || !ctx->stream) return ctx ? ctx->fail(XG_E_CUDA, "context has no device") : XG_E_ARG;
     if (!h || !out) return ctx->fail(XG_E_ARG, "xg_upload_reads: null argument");
     XG_CUDA(cudaSetDevice(ctx->device));
-    xg_dreads *d = new xg_dreads();
-    d->n_reads = h->n_reads;
-    d->n_cigar = h->n_cigar;
-    d->n_seq_words = h->n_seq_words;
-    d->n_runs = h->n_runs;
-    d->n_tiles = h->n_tiles;
-    d->max_aln_len = h->max_aln_len;
-    d->max_span = h->max_span;
-    d->h_runs.assign(h->runs, h->runs + h->n_runs);
-    d->h_tiles.assign(h->tiles, h->tiles + h->n_tiles);
+    xg_dreads *d = xg_dreads_new(h);
     size_t n = (size_t)h->n_reads;
     bool seq = h->seq_off != nullptr && h->seq != nullptr;
     struct Cp {
@@ -166,7 +143,6 @@ int xg_upload_reads(xg_ctx *ctx, const xg_reads *h, xg_dreads **out) {
         {(void **)&d->runs, h->runs, (size_t)h->n_runs * sizeof(xg_run)},
         {(void **)&d->tiles, h->tiles, (size_t)h->n_tiles * sizeof(xg_tile)},
     };
-    d->pooled = true;
     for (auto &c : cps) {
         if (!c.src) continue;
         *c.dst = ctx->dev_get(c.bytes + 64);      // slack: the kernels load records in aligned pairs / quads
@@ -222,17 +198,7 @@ int xg_map_reads(xg_ctx *ctx, const xg_reads *h, xg_dreads **out) {
                                        "(xg_decode_bams output after xg_create, or cudaHostRegister)");
         }
     }
-    xg_dreads *d = new xg_dreads();
-    d->n_reads = h->n_reads;
-    d->n_cigar = h->n_cigar;
-    d->n_seq_words = h->n_seq_words;
-    d->n_runs = h->n_runs;
-    d->n_tiles = h->n_tiles;
-    d->max_aln_len = h->max_aln_len;
-    d->max_span = h->max_span;
-    d->h_runs.assign(h->runs, h->runs + h->n_runs);
-    d->h_tiles.assign(h->tiles, h->tiles + h->n_tiles);
-    d->pooled = true;
+    xg_dreads *d = xg_dreads_new(h);
     d->mapped = true;
     size_t n = (size_t)h->n_reads;
     d->pos_end = (int2 *)ctx->dev_get(n * 8 + 16);
@@ -338,6 +304,21 @@ void xg_coo_free(xg_coo *m) {
 }
 
 }  // extern "C"
+
+xg_dreads *xg_dreads_new(const xg_reads *h) {
+    xg_dreads *d = new xg_dreads();
+    d->n_reads = h->n_reads;
+    d->n_cigar = h->n_cigar;
+    d->n_seq_words = h->n_seq_words;
+    d->n_runs = h->n_runs;
+    d->n_tiles = h->n_tiles;
+    d->max_aln_len = h->max_aln_len;
+    d->max_span = h->max_span;
+    d->h_runs.assign(h->runs, h->runs + h->n_runs);
+    d->h_tiles.assign(h->tiles, h->tiles + h->n_tiles);
+    d->pooled = true;
+    return d;
+}
 
 // Prefix max (restarting at every run) of the tiles' max_end: with it "first tile whose records
 // can still reach position x" is a binary search.  Built once per batch from the host tile index.

@@ -855,7 +855,7 @@ extern "C" int xg_write_mtx_rows16(const char *path, int32_t n_rows_in, const in
     }
 }
 
-// ... and from the 16-bit layout ("narrow_rows" 2): entry k = (column - previous column of the row - 1) << 4 | count,
+// ... and from the 16-bit layout (XG_LAYOUT_ROWS_TINY): entry k = (column - previous column of the row - 1) << 4 | count,
 // the word 0 = look the entry up in the side list (every row's first entry is there).  The side list is sorted by
 // entry index once; a reader walks a row with a cursor into it.
 namespace {

@@ -1435,10 +1435,9 @@ static int decode_bams_device_impl(xg_ctx *ctx, int32_t n_bams, const char *cons
     if (cudaEventCreateWithFlags(&D.ev_win, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&D.ev_i2, cudaEventDisableTiming) != cudaSuccess)
         return bail(XG_E_CUDA, "cudaEventCreate");
-    if (!ctx->aux[2])
-        for (auto &s2 : ctx->aux)
-            if (!s2 && cudaStreamCreateWithFlags(&s2, cudaStreamNonBlocking) != cudaSuccess) return bail(XG_E_CUDA, "cudaStreamCreate");
-    if (!getenv("XG_INFLATE_ONE_STREAM")) D.ist2 = ctx->aux[2];
+    if (!ctx->inflate_stream && cudaStreamCreateWithFlags(&ctx->inflate_stream, cudaStreamNonBlocking) != cudaSuccess)
+        return bail(XG_E_CUDA, "cudaStreamCreate");
+    if (!getenv("XG_INFLATE_ONE_STREAM")) D.ist2 = ctx->inflate_stream;
     cudaStream_t st = ctx->stream;
     cudaMemsetAsync(D.cnt, 0, 8 * sizeof(int), st);
     cudaEventRecord(ctx->ev[2], st);

@@ -26,6 +26,9 @@ c_u8p = C.POINTER(C.c_uint8)
 
 XG_E_UNSUPPORTED = -7
 
+# result layouts of xg_basefc (include/xcltk_b200.h), by Context.basefc's `segments`
+XG_LAYOUT_CSR, XG_LAYOUT_ROWS, XG_LAYOUT_ROWS_NARROW, XG_LAYOUT_ROWS_TINY = 0, 1, 2, 3
+
 
 class XgError(RuntimeError):
     def __init__(self, code, msg):
@@ -68,7 +71,7 @@ class Barcodes(C.Structure):
 
 class Coo(C.Structure):
     _fields_ = [("nnz", C.c_int64), ("n_rows", C.c_int32), ("n_cols", C.c_int32),
-                ("row", c_i32p), ("col", c_i32p), ("val", c_i32p), ("row_ptr", c_i64p),
+                ("col", c_i32p), ("val", c_i32p), ("row_ptr", c_i64p),
                 ("row_beg", c_i64p), ("row_cnt", c_i32p),
                 ("colval16", c_u32p), ("n_over", C.c_int64), ("over_idx", c_i64p), ("over_val", c_i32p),
                 ("coldelta16", c_u16p), ("over_col", c_i32p)]
@@ -132,10 +135,10 @@ SYMBOLS = {
                                         C.c_char_p, C.c_char_p, C.c_int32, _P, C.POINTER(_P), c_i64p]),
     "xg_bgzf_inflate_device": (C.c_int, [_P, C.c_char_p, c_u8p, C.c_int64, c_i64p]),
     "xg_coo_free": (None, [C.POINTER(Coo)]),
-    "xg_basefc": (C.c_int, [_P, _P, C.POINTER(Features), C.POINTER(Barcodes), C.POINTER(Params),
+    "xg_basefc": (C.c_int, [_P, _P, C.POINTER(Features), C.POINTER(Barcodes), C.POINTER(Params), C.c_int32,
                             C.POINTER(C.POINTER(Coo))]),
     "xg_basefc_host": (C.c_int, [_P, C.POINTER(Reads), C.POINTER(Features), C.POINTER(Barcodes), C.POINTER(Params),
-                                 C.POINTER(C.POINTER(Coo))]),
+                                 C.c_int32, C.POINTER(C.POINTER(Coo))]),
     "xg_baf_pileup": (C.c_int, [_P, _P, C.POINTER(Snps), C.POINTER(Barcodes), C.POINTER(Params),
                                 c_i64p, C.POINTER(_P)]),
     "xg_baf_count": (C.c_int, [_P, _P, C.c_int32, c_i64p, c_i32p, c_u8p, c_u8p, C.c_int32,
@@ -384,15 +387,15 @@ class LazyRows(object):
 
 
 class RowSegments(object):
-    """basefc result with the rows in the order the device completed them (context option
-    row_order = 0): row r is entries [row_beg[r], row_beg[r] + row_cnt[r]), sorted by col.  The
-    entries are either `col` / `val` (int32 each) or, with the narrow_rows option, `cv16` (uint32:
+    """basefc result with the rows in the order the device completed them (the rows layouts of
+    xg_basefc): row r is entries [row_beg[r], row_beg[r] + row_cnt[r]), sorted by col.  The
+    entries are either `col` / `val` (int32 each) or, in the narrow layout, `cv16` (uint32:
     column | count << 16, counts >= 65535 in the side list `over`); `.col` / `.val` unpack on
     demand.  This is what the Matrix-Market writer consumes (write_mtx_rows); to_sorted() gives
     (row, col, val) sorted by (row, col) for everything else."""
 
     def __init__(self, row_beg, row_cnt, col, val, shape, cv16=None, over=None, tiny=None):
-        """tiny: the 16-bit layout (narrow_rows = 2): (column - previous column of the row - 1) << 4 | count per entry,
+        """tiny: the 16-bit layout (XG_LAYOUT_ROWS_TINY): (column - previous column of the row - 1) << 4 | count per entry,
         0 = the entry is in the side list `over` = (idx, val, col) -- every row's first entry is."""
         self.row_beg, self.row_cnt, self.shape = row_beg, row_cnt, shape
         self._col, self._val, self.cv16, self.over, self.tiny = col, val, cv16, over, tiny
@@ -477,67 +480,45 @@ def write_mtx_rows(path, seg, out_row, n_rows_out, n_threads=0):
         raise XgError(rc, lib.xg_host_last_error().decode())
 
 
+def _take(lib, pcoo, ctx_obj, views, copy):
+    """Copies of `views` with the result freed at once, or views that keep it alive (a _CooOwner)."""
+    if copy:
+        out = [v.copy() for v in views]
+        lib.xg_coo_free(pcoo)
+        return out
+    owner = _CooOwner(lib, pcoo, ctx_obj)
+    out = [v.view(_View) for v in views]
+    for v in out:
+        v._owner = owner
+    return out
+
+
 def coo_to_numpy(lib, pcoo, copy_below=1 << 16, ctx_obj=None):
-    """(row, col, val, shape).  Large results are zero-copy views of the library's pinned
-    buffers (released when the last view dies); small ones are copied and freed at once.
-    With the context option coo_rows = 0 `row` is a LazyRows (expanded from row_ptr on use)."""
+    """(row, col, val, shape) with `row` a LazyRows (expanded from row_ptr on use), or a RowSegments for the rows
+    layouts.  Large results are zero-copy views of the library's pinned buffers (released when the last view dies);
+    small ones are copied and freed at once."""
     m = pcoo.contents
     nnz = int(m.nnz)
     shape = (int(m.n_rows), int(m.n_cols))
-    if bool(m.row_beg):                       # rows in completion order
-        row_beg = np_view(m.row_beg, shape[0], np.int64).copy()
-        row_cnt = np_view(m.row_cnt, shape[0], np.int32).copy()
-        if bool(m.coldelta16):                # 16-bit entries
-            n_over = int(m.n_over)
-            views = [np_view(m.coldelta16, nnz, np.uint16), np_view(m.over_idx, n_over, np.int64),
-                     np_view(m.over_val, n_over, np.int32), np_view(m.over_col, n_over, np.int32)]
-            if nnz <= copy_below:
-                views = [v.copy() for v in views]
-                lib.xg_coo_free(pcoo)
-            else:                             # the side list holds about one entry per row: views, not copies
-                owner = _CooOwner(lib, pcoo, ctx_obj)
-                for k, v in enumerate(views):
-                    views[k] = v.view(_View)
-                    views[k]._owner = owner
-            return RowSegments(row_beg, row_cnt, None, None, shape, over=(views[1], views[2], views[3]), tiny=views[0])
-        if bool(m.colval16):                  # narrow entries
-            n_over = int(m.n_over)
-            over = (np_view(m.over_idx, n_over, np.int64).copy(), np_view(m.over_val, n_over, np.int32).copy())
-            v = np_view(m.colval16, nnz, np.uint32)
-            if nnz <= copy_below:
-                cv = v.copy()
-                lib.xg_coo_free(pcoo)
-            else:
-                cv = v.view(_View)
-                cv._owner = _CooOwner(lib, pcoo, ctx_obj)
-            return RowSegments(row_beg, row_cnt, None, None, shape, cv16=cv, over=over)
-        views = [np_view(p, nnz, np.int32) for p in (m.col, m.val)]
-        if nnz <= copy_below:
-            cv = [v.copy() for v in views]
-            lib.xg_coo_free(pcoo)
-        else:
-            owner = _CooOwner(lib, pcoo, ctx_obj)
-            cv = []
-            for v in views:
-                w = v.view(_View)
-                w._owner = owner
-                cv.append(w)
-        return RowSegments(row_beg, row_cnt, cv[0], cv[1], shape)
-    has_rows = bool(m.row)
-    row_ptr = np_view(m.row_ptr, shape[0] + 1, np.int64).copy()
-    views = [np_view(p, nnz, np.int32) for p in ((m.row if has_rows else m.col), m.col, m.val)]
-    if nnz <= copy_below:
-        out = [v.copy() for v in views]
-        lib.xg_coo_free(pcoo)
-    else:
-        owner = _CooOwner(lib, pcoo, ctx_obj)
-        out = []
-        for v in views:
-            w = v.view(_View)
-            w._owner = owner
-            out.append(w)
-    row = out[0] if has_rows else LazyRows(row_ptr, nnz)
-    return row, out[1], out[2], shape
+    copy = nnz <= copy_below
+    if not bool(m.row_beg):                   # CSR
+        row_ptr = np_view(m.row_ptr, shape[0] + 1, np.int64).copy()
+        col, val = _take(lib, pcoo, ctx_obj, [np_view(m.col, nnz, np.int32), np_view(m.val, nnz, np.int32)], copy)
+        return LazyRows(row_ptr, nnz), col, val, shape
+    row_beg = np_view(m.row_beg, shape[0], np.int64).copy()
+    row_cnt = np_view(m.row_cnt, shape[0], np.int32).copy()
+    n_over = int(m.n_over)
+    if bool(m.coldelta16):                    # 16-bit entries; the side list holds about one entry per row
+        tiny, idx, oval, ocol = _take(lib, pcoo, ctx_obj, [
+            np_view(m.coldelta16, nnz, np.uint16), np_view(m.over_idx, n_over, np.int64),
+            np_view(m.over_val, n_over, np.int32), np_view(m.over_col, n_over, np.int32)], copy)
+        return RowSegments(row_beg, row_cnt, None, None, shape, over=(idx, oval, ocol), tiny=tiny)
+    if bool(m.colval16):                      # narrow entries
+        over = (np_view(m.over_idx, n_over, np.int64).copy(), np_view(m.over_val, n_over, np.int32).copy())
+        cv, = _take(lib, pcoo, ctx_obj, [np_view(m.colval16, nnz, np.uint32)], copy)
+        return RowSegments(row_beg, row_cnt, None, None, shape, cv16=cv, over=over)
+    col, val = _take(lib, pcoo, ctx_obj, [np_view(m.col, nnz, np.int32), np_view(m.val, nnz, np.int32)], copy)
+    return RowSegments(row_beg, row_cnt, col, val, shape)
 
 
 class Context(object):
@@ -554,7 +535,6 @@ class Context(object):
                 self.lib.xg_destroy(self.h)
                 self.h = None
             raise XgError(rc, msg)
-        self.lib.xg_set_option(self.h, b"coo_rows", 0)      # CSR over PCIe; rows expanded lazily on the host
 
     def _check(self, rc):
         if rc != 0:
@@ -616,26 +596,27 @@ class Context(object):
         self.lib.xg_last_timing(self.h, t)
         return list(t)
 
-    def basefc(self, dreads, gid, beg, end, cell_keys, n_samples, params, segments=False):
-        """(row, col, val, shape) sorted by (row, col); segments=True: a RowSegments (rows in
-        completion order, copied out while the counting is still running); segments="narrow": the
-        same with 32-bit packed entries when there are at most 65536 columns; segments="tiny": 16-bit entries
-        (column delta | small count) + a side list -- a quarter of the bytes, for matrices of small counts."""
+    def _basefc(self, entry, reads, gid, beg, end, cell_keys, n_samples, params, segments):
         gid = np.ascontiguousarray(gid, dtype=np.int32)
         beg = np.ascontiguousarray(beg, dtype=np.int32)
         end = np.ascontiguousarray(end, dtype=np.int32)
         keys = np.ascontiguousarray(cell_keys if cell_keys is not None else [], dtype=np.uint64)
         f = Features(len(gid), as_ptr(gid, c_i32p), as_ptr(beg, c_i32p), as_ptr(end, c_i32p))
         b = Barcodes(len(keys), as_ptr(keys, c_u64p), n_samples)
+        if not segments:
+            layout = XG_LAYOUT_CSR
+        else:
+            layout = {"narrow": XG_LAYOUT_ROWS_NARROW, "tiny": XG_LAYOUT_ROWS_TINY}.get(segments, XG_LAYOUT_ROWS)
         out = C.POINTER(Coo)()
-        self.lib.xg_set_option(self.h, b"row_order", 0 if segments else 1)
-        self.lib.xg_set_option(self.h, b"narrow_rows", {"narrow": 1, "tiny": 2}.get(segments, 0))
-        try:
-            self._check(self.lib.xg_basefc(self.h, dreads.h, C.byref(f), C.byref(b), C.byref(params.c),
-                                           C.byref(out)))
-        finally:
-            self.lib.xg_set_option(self.h, b"row_order", 1)
+        self._check(entry(self.h, reads, C.byref(f), C.byref(b), C.byref(params.c), layout, C.byref(out)))
         return coo_to_numpy(self.lib, out, ctx_obj=self)
+
+    def basefc(self, dreads, gid, beg, end, cell_keys, n_samples, params, segments=False):
+        """(row, col, val, shape) sorted by (row, col); segments=True: a RowSegments (rows in
+        completion order, copied out while the counting is still running); segments="narrow": the
+        same with 32-bit packed entries when there are at most 65536 columns; segments="tiny": 16-bit entries
+        (column delta | small count) + a side list -- a quarter of the bytes, for matrices of small counts."""
+        return self._basefc(self.lib.xg_basefc, dreads.h, gid, beg, end, cell_keys, n_samples, params, segments)
 
     def basefc_write_mtx(self, path, out_row, n_rows_out, n_threads=0):
         """Matrix-Market text of the LAST basefc(..., segments=...) result of this context, formatted on the device
@@ -647,21 +628,8 @@ class Context(object):
 
     def basefc_host(self, host_reads, gid, beg, end, cell_keys, n_samples, params, segments=False):
         """basefc straight from a pinned host batch: H2D streamed under the counting kernels."""
-        gid = np.ascontiguousarray(gid, dtype=np.int32)
-        beg = np.ascontiguousarray(beg, dtype=np.int32)
-        end = np.ascontiguousarray(end, dtype=np.int32)
-        keys = np.ascontiguousarray(cell_keys if cell_keys is not None else [], dtype=np.uint64)
-        f = Features(len(gid), as_ptr(gid, c_i32p), as_ptr(beg, c_i32p), as_ptr(end, c_i32p))
-        b = Barcodes(len(keys), as_ptr(keys, c_u64p), n_samples)
-        out = C.POINTER(Coo)()
-        self.lib.xg_set_option(self.h, b"row_order", 0 if segments else 1)
-        self.lib.xg_set_option(self.h, b"narrow_rows", {"narrow": 1, "tiny": 2}.get(segments, 0))
-        try:
-            self._check(self.lib.xg_basefc_host(self.h, host_reads.ptr, C.byref(f), C.byref(b), C.byref(params.c),
-                                                C.byref(out)))
-        finally:
-            self.lib.xg_set_option(self.h, b"row_order", 1)
-        return coo_to_numpy(self.lib, out, ctx_obj=self)
+        return self._basefc(self.lib.xg_basefc_host, host_reads.ptr, gid, beg, end, cell_keys, n_samples, params,
+                            segments)
 
     def baf_pileup(self, dreads, gid, pos, cell_keys, n_samples, params, reuse_totals=False):
         """reuse_totals: the returned totals array is the context's own buffer, overwritten by the next pileup."""
