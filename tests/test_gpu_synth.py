@@ -433,18 +433,24 @@ def test_basefc_narrow_entries_with_large_counts(gpu_ctx):
     for a, b in zip(seg.to_sorted(), ref):
         assert np.array_equal(a, b)
     p2 = gpu_params(Conf())
-    seg = gpu_ctx.basefc(w.dreads, w.gid, w.beg, w.end, np.arange(1, 70001, dtype=np.uint64) << np.uint64(40), 70000, p2,
-                         segments="narrow")
+    # the batch's 50 barcodes among 70 000 keys: 40 at columns 0, 1000, ..., 39000, then a gap of 6000 (wider than a
+    # 16-bit entry's 4095) and 10 at 45000, 47500, ..., 67500 (beyond 16-bit columns); the other keys match no read
+    keys70k = np.arange(1, 70001, dtype=np.uint64) << np.uint64(40)
+    at = np.concatenate([np.arange(40) * 1000, 45000 + np.arange(10) * 2500])
+    keys70k[at] = w.cell_keys
+    seg = gpu_ctx.basefc(w.dreads, w.gid, w.beg, w.end, keys70k, 70000, p2, segments="narrow")
     assert seg.cv16 is None                                # too many columns for 16 bits
     # the 16-bit layout: counts in the tens of thousands all go through the side list; 70 000 columns are fine
     seg = gpu_ctx.basefc(w.dreads, gid, beg, end, None, 1, p, segments="tiny")
     assert seg.tiny is not None and len(seg.over[0]) >= int((ref[2] > 15).sum())
     for a, b in zip(seg.to_sorted(), ref):
         assert np.array_equal(a, b)
-    keys70k = np.arange(1, 70001, dtype=np.uint64) << np.uint64(40)
+    r50 = [np.array(x) for x in gpu_ctx.basefc(w.dreads, w.gid, w.beg, w.end, w.cell_keys, 50, p2)[:3]]
     r70 = [np.array(x) for x in gpu_ctx.basefc(w.dreads, w.gid, w.beg, w.end, keys70k, 70000, p2)[:3]]
+    assert len(r70[2]) > 1000 and r70[1].max() > 65535
+    assert np.array_equal(r70[0], r50[0]) and np.array_equal(r70[1], at[r50[1]]) and np.array_equal(r70[2], r50[2])
     seg = gpu_ctx.basefc(w.dreads, w.gid, w.beg, w.end, keys70k, 70000, p2, segments="tiny")
-    assert seg.tiny is not None
+    assert seg.tiny is not None and len(seg.over[0]) > int((np.asarray(seg.row_cnt) > 0).sum())    # wide gaps too
     for a, b in zip(seg.to_sorted(), r70):
         assert np.array_equal(a, b)
 

@@ -714,7 +714,12 @@ extern "C" int xg_baf_pileup(xg_ctx *ctx, const xg_dreads *rd, const xg_snps *sn
     st->n_snps = snps->n;
     st->n_cols = cells->n_samples;
     if (n_pairs > 0) {
-        const uint32_t cap = (uint32_t)(2 * n_pairs + 16);
+        const uint64_t cap64 = 2ull * n_pairs + 16ull;         // slots are 32-bit indices
+        if (cap64 > 0xFFFFFFFFull) {
+            xg_baf_state_free(ctx, st);
+            return ctx->fail(XG_E_LIMIT, "(SNP, cell, UMI) table exceeds 2^32 slots");
+        }
+        const uint32_t cap = (uint32_t)cap64;
         XG_GET(tbl, xg_e128, "bf_tbl1", cap);
         XG_GET(min_ord, unsigned long long, "bf_minord", cap);
         XG_GET(pr_slot, uint32_t, "bf_pr_slot", n_pairs);
@@ -876,7 +881,9 @@ static int baf_count_impl(xg_ctx *ctx, xg_baf_state *st, int32_t n_regions, cons
     XG_CUDA(cudaMemcpyAsync(&combos, reg_log_off + n_regions, 8, cudaMemcpyDeviceToHost, ctx->stream));
     XG_CUDA(cudaStreamSynchronize(ctx->stream));
     if (combos >= (1ll << 31)) return ctx->fail(XG_E_LIMIT, "more than 2^31 (region, cell, UMI) candidates");
-    const uint32_t cap = (uint32_t)(2 * combos + 16);
+    const uint64_t cap64 = 2ull * (uint64_t)combos + 16ull;   // slots are 32-bit indices
+    if (cap64 > 0xFFFFFFFFull) return ctx->fail(XG_E_LIMIT, "(region, cell, UMI) table exceeds 2^32 slots");
+    const uint32_t cap = (uint32_t)cap64;
     XG_GET(tbl, xg_e128, "bf_tbl2", cap);
     XG_GET(mask, uint32_t, "bf_mask", cap);
     XG_GET(reg_log, uint32_t, "bf_reg_log", combos + 1);

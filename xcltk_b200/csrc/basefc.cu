@@ -1929,11 +1929,14 @@ static int basefc_epochs(BasefcCall &c, bool rows) {
         return ((size_t)8 << tbl_log2) + ((size_t)2 << tbl_log2) + (size_t)(2 * bm_words + 1) * 4;    // table, counters, bitmap + prefix
     };
     const size_t segs_bytes = segs_smem(FS_TBL_LOG2), big_bytes = segs_smem(FS_BIG_TBL_LOG2);
-    XG_CUDA(cudaFuncSetAttribute(k_basefc_finalize_segs<FS_THREADS, FS_TBL_LOG2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)segs_bytes));
+    // only segment features use these kernels, and only in seg_mode (n_cols <= 2^19) does their bitmap fit: with
+    // more columns the attribute would be refused and the call fail although no segment kernel runs
+    if (c.seg_mode)
+        XG_CUDA(cudaFuncSetAttribute(k_basefc_finalize_segs<FS_THREADS, FS_TBL_LOG2>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)segs_bytes));
     // big CTAs need the large table; with so many cells that it does not fit, big features go the ordinary way
     const bool big_ok = big_bytes + sizeof(FsShared) + 1280 <= 200 * 1024;
-    if (big_ok)
+    if (c.seg_mode && big_ok)
         XG_CUDA(cudaFuncSetAttribute(k_basefc_finalize_segs<FS_BIG_THREADS, FS_BIG_TBL_LOG2>,
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)big_bytes));
     const int segs_ctas_per_sm = std::max(1, std::min(8, (int)(224 * 1024 / (segs_bytes + sizeof(FsShared) + 1280))));
