@@ -338,6 +338,20 @@ int xg_baf_fc(xg_ctx *ctx, const xg_dreads *reads, const xg_snps *snps, const xg
               const xg_params *par, const xg_snp_filter *filt, int32_t n_regions, const int64_t *reg_ptr,
               const int32_t *reg_snp, const uint8_t *hap_of, int32_t no_dup_hap, int64_t *totals,
               uint8_t *keep_out, xg_coo **ad, xg_coo **dp, xg_coo **oth);
+/* SNP-level allele counting: the per-SNP x cell counts of the candidate SNPs themselves (what cellsnp-lite's
+ * cellSNP.tag.{AD,DP,OTH}.mtx hold), with the pileup of plp_snp (baf/fc/core.py:198-247; first read wins per
+ * (SNP, cell, UMI), a None allele included: baf/fc/mcount.py:39-60,109-150) and its filter as in xg_baf_fc.  Each SNP
+ * counts as a region of one SNP with GT 0|1 (baf/fc/core.py:143-194): over the winning UMIs of SNP i in cell c whose
+ * allele is not None,  AD = UMIs whose base is the ALT (base index alt_idx[i]),  DP = UMIs whose base is REF or ALT,
+ * OTH = the others (IUPAC codes and '=' match neither; REF == ALT counts as ALT).  Rows are all snps->n SNPs in
+ * input order -- a SNP removed by the filter has empty rows, keep_out reports it -- columns cells->n_samples
+ * (< 2^24, else XG_E_LIMIT); XG_LAYOUT_CSR.  Works on batches from xg_upload_reads, the device decoder and
+ * xg_map_reads.  xg_last_timing: [0] device span  [1] scan  [2] launches  [4] result D2H  [6] (read, SNP) pairs
+ * [7] winners reduced  [8..10] host milestones (ms since entry: pileup, kernels queued, end)
+ * [14] / [15] SNPs reduced by one warp / by a whole CTA.                                                      */
+int xg_snp_pileup(xg_ctx *ctx, const xg_dreads *reads, const xg_snps *snps, const xg_barcodes *cells,
+                  const xg_params *par, const xg_snp_filter *filt, int64_t *totals /* may be NULL */,
+                  uint8_t *keep_out /* may be NULL */, xg_coo **ad, xg_coo **dp, xg_coo **oth);
 
 /* Synthetic 10x-style records generated directly in HBM (bench / tests; no reference
  * counterpart -- SURVEY.md 8(d) C3 allows device-side generation for kernel-only runs).  */

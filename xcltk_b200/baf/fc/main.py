@@ -50,8 +50,9 @@ def afc_wrapper(sam_fn, barcode_fn, region_fn, phased_snp_fn, out_dir, sam_list_
     return afc_run(conf)
 
 
-def prepare_config(conf):
-    """Validate options, load regions / SNPs; 0 if ok, -1 otherwise (baf/fc/main.py:298-495)."""
+def prepare_samples(conf):
+    """BAM list and columns (baf/fc/main.py:298-357): conf.sam_fn_list, conf.barcodes (sorted) or conf.sample_ids,
+    conf.samples; then the output directory.  0 if ok, -1 otherwise."""
     if conf.sam_fn:
         if conf.sam_list_fn:
             error("should not specify 'sam_fn' and 'sam_list_fn' together.")
@@ -104,6 +105,31 @@ def prepare_config(conf):
         return -1
     if not os.path.isdir(conf.out_dir):
         os.mkdir(conf.out_dir)
+    return 0
+
+
+def prepare_tags(conf):
+    """Cell / UMI tags ('None' / 'Auto') and the default exclude flag (baf/fc/main.py:467-495).  0 if ok, -1
+    otherwise."""
+    if conf.cell_tag and conf.cell_tag.upper() == "NONE":
+        conf.cell_tag = None
+    if (not conf.cell_tag) != (not conf.barcodes):
+        error("should not specify cell_tag or barcodes alone.")
+        return -1
+    if conf.umi_tag:
+        if conf.umi_tag.upper() == "AUTO":
+            conf.umi_tag = None if conf.barcodes is None else conf.defaults.UMI_TAG_BC
+        elif conf.umi_tag.upper() == "NONE":
+            conf.umi_tag = None
+    if conf.excl_flag < 0:
+        conf.excl_flag = conf.defaults.EXCL_FLAG_UMI if conf.use_umi() else conf.defaults.EXCL_FLAG_XUMI
+    return 0
+
+
+def prepare_config(conf):
+    """Validate options, load regions / SNPs; 0 if ok, -1 otherwise (baf/fc/main.py:298-495)."""
+    if prepare_samples(conf) < 0:
+        return -1
     pre = os.path.join(conf.out_dir, conf.out_prefix)
     conf.out_region_fn, conf.out_sample_fn = pre + "region.tsv", pre + "samples.tsv"
     conf.out_ad_fn, conf.out_dp_fn, conf.out_oth_fn = pre + "AD.mtx", pre + "DP.mtx", pre + "OTH.mtx"
@@ -165,21 +191,10 @@ def prepare_config(conf):
         for cell in conf.ref_cells:
             assert cell in conf.samples
 
-    if conf.cell_tag and conf.cell_tag.upper() == "NONE":
-        conf.cell_tag = None
-    if (not conf.cell_tag) != (not conf.barcodes):
-        error("should not specify cell_tag or barcodes alone.")
+    if prepare_tags(conf) < 0:
         return -1
-    if conf.umi_tag:
-        if conf.umi_tag.upper() == "AUTO":
-            conf.umi_tag = None if conf.barcodes is None else conf.defaults.UMI_TAG_BC
-        elif conf.umi_tag.upper() == "NONE":
-            conf.umi_tag = None
-
     with open(conf.out_sample_fn, "w") as fp:
         fp.write("".join(smp + "\n" for smp in conf.samples))
-    if conf.excl_flag < 0:
-        conf.excl_flag = conf.defaults.EXCL_FLAG_UMI if conf.use_umi() else conf.defaults.EXCL_FLAG_XUMI
     return 0
 
 
@@ -213,7 +228,29 @@ def hap_table(snps):
     return hap
 
 
-def _count_shard(conf, ctx, dreads, keyspace, gid_of, max_aln_len, regs, snps):
+def snp_arrays(conf, batch, snps):
+    """Device arguments of a list of SNPs on one batch: contig ids, 0-based positions (fetch(chrom, pos-1, pos); a
+    SNP that can never be fetched gets gid -1), the barcode keys and the read filters."""
+    gid = np.array([batch.gid_of.get(s.chrom, -1) for s in snps], dtype=np.int32)
+    pos0 = np.array([s.pos - 1 for s in snps], dtype=np.int64)
+    bad = (pos0 < 0) | (pos0 >= 2147483647)
+    gid[bad] = -1
+    pos0[bad] = 0
+    cell_keys = None
+    if conf.use_barcodes():
+        cell_keys = np.array([batch.keyspace.encode(b) for b in conf.barcodes], dtype=np.uint64)
+    params = engine.make_params(conf, batch.stats["max_aln_len"], with_include=False)
+    return gid, pos0.astype(np.int32), cell_keys, params
+
+
+def allele_indices(snps):
+    """MCount.base_idx of every SNP's REF and ALT (baf/fc/mcount.py:178)."""
+    n = len(snps)
+    return (np.fromiter((BASE_IDX[s.ref] for s in snps), dtype=np.uint8, count=n),
+            np.fromiter((BASE_IDX[s.alt] for s in snps), dtype=np.uint8, count=n))
+
+
+def _count_shard(conf, batch, regs, snps):
     """Pileup + count of `regs` (whose snp_list entries index `snps`) on one device."""
     local = {}                                   # SNPs of this shard, renumbered
     reg_ptr = np.zeros(len(regs) + 1, dtype=np.int64)
@@ -225,42 +262,33 @@ def _count_shard(conf, ctx, dreads, keyspace, gid_of, max_aln_len, regs, snps):
     sub = [None] * len(local)
     for gi, li in local.items():
         sub[li] = snps[gi]
-    gid = np.array([gid_of.get(s.chrom, -1) for s in sub], dtype=np.int32)
-    pos0 = np.array([s.pos - 1 for s in sub], dtype=np.int64)          # fetch(chrom, pos-1, pos)
-    bad = (pos0 < 0) | (pos0 >= 2147483647)
-    gid[bad] = -1
-    pos0[bad] = 0
-    cell_keys = None
-    if conf.use_barcodes():
-        cell_keys = np.array([keyspace.encode(b) for b in conf.barcodes], dtype=np.uint64)
-    params = engine.make_params(conf, max_aln_len, with_include=False)
+    gid, pos0, cell_keys, params = snp_arrays(conf, batch, sub)
     # pileup -> plp_snp's filter (on the device, IEEE double as Python evaluates it; `snp_filter` above is the same
     # test on the host, kept for the tests) -> region count, one library call
-    n = len(sub)
-    ref_i = np.fromiter((BASE_IDX[s.ref] for s in sub), dtype=np.uint8, count=n)
-    alt_i = np.fromiter((BASE_IDX[s.alt] for s in sub), dtype=np.uint8, count=n)
-    out = ctx.baf_fc(dreads, gid, pos0.astype(np.int32), cell_keys, len(conf.samples), params, ref_i, alt_i,
+    ref_i, alt_i = allele_indices(sub)
+    ctx = batch.ctx
+    out = ctx.baf_fc(batch.dreads, gid, pos0, cell_keys, len(conf.samples), params, ref_i, alt_i,
                      conf.min_count, conf.min_maf, reg_ptr, np.array(reg_snp, dtype=np.int32), hap_table(sub),
                      conf.no_dup_hap)
-    return out, [ctx.timing()]
+    return out, [ctx.timing()], None
 
 
-def count_regions(conf, regs, batch=None):
-    """Device counting; returns three (row, col, val, shape) tuples (AD, DP, OTH), rows index
-    `regs`.  With several GPUs the regions are cut into contiguous genomic chunks (their SNPs
-    follow them; a SNP shared by regions of two chunks is piled up on both), no collective."""
+def count_units(conf, chroms, unit_chrom, unit_beg, unit_end, count, batch=None):
+    """Device counting of independent units (regions, or single SNPs) with one read batch per GPU.
+    unit_chrom / unit_beg / unit_end: contig (None: never fetched) and 0-based [beg, end) of every unit;
+    count(batch, idx) -> ((ad, dp, oth), timings, per_unit) counts the units `idx` on one batch, the rows of its
+    matrices indexing idx, per_unit an array over idx or None.  With several GPUs the units are cut into contiguous
+    genomic chunks, no collective.  Returns the three (row, col, val, shape) tuples in unit order and the
+    [(idx, per_unit)] of the shards."""
     from ... import parallel
-    snps = conf.snp_set.snps
+    n_unit = len(unit_beg)
     n_dev = parallel.n_devices(getattr(conf, "n_gpus", None))
     own = batch is None
     if own:
-        chroms = list(dict.fromkeys([s.chrom for s in snps]))
         threads = engine.n_decode_threads(conf.nproc)
         if n_dev > 1:
             batch = engine.load_reads_sharded(conf.sam_fn_list, chroms, conf.cell_tag, conf.umi_tag, True,
-                                              parallel.device_list(n_dev),
-                                              [r.chrom if r.snp_list else None for r in regs],
-                                              [r.start - 1 for r in regs], [r.end - 1 for r in regs])
+                                              parallel.device_list(n_dev), unit_chrom, unit_beg, unit_end)
             if batch is None:
                 batch = engine.load_reads_multi(conf.sam_fn_list, chroms, conf.cell_tag, conf.umi_tag, True,
                                                 threads, devices=parallel.device_list(n_dev))
@@ -268,48 +296,51 @@ def count_regions(conf, regs, batch=None):
             batch = engine.load_reads(conf.sam_fn_list, chroms, conf.cell_tag, conf.umi_tag, True, threads,
                                       mapped=True)
     try:
-        shape = (len(regs), len(conf.samples))
-        if isinstance(batch, engine.ShardedBatch):
-            shards = batch.shards
+        shape = (n_unit, len(conf.samples))
+        if isinstance(batch, (engine.ShardedBatch, engine.MultiBatch)):
+            if isinstance(batch, engine.ShardedBatch):
+                shards = batch.shards
+            else:
+                gid = np.array([batch.gid_of.get(c, -1) if c is not None else -1 for c in unit_chrom], dtype=np.int32)
+                load, total = parallel.reads_before(gid, np.asarray(unit_beg, dtype=np.int64), batch.runs,
+                                                    batch.pos_of_run)
+                shards = parallel.partition(gid, np.asarray(unit_beg, dtype=np.int64), load, total,
+                                            len(batch.batches))
 
             def one(k):
                 b = batch.batches[k]
                 if b is None or len(shards[k]) == 0:
                     z = np.zeros(0, np.int32)
-                    return ((z, z, z, shape),) * 3, [[0.0] * 16, [0.0] * 16]
-                return _count_shard(conf, b.ctx, b.dreads, b.keyspace, b.gid_of, b.stats["max_aln_len"],
-                                    [regs[i] for i in shards[k]], snps)
+                    return ((z, z, z, shape),) * 3, [[0.0] * 16, [0.0] * 16], None
+                return count(b, shards[k])
             parts = parallel.run_on_devices(len(shards), one)
             out = []
             for w in range(3):
-                r, c, v = parallel.merge_coo([[np.array(x) for x in p[0][w][:3]] for p in parts], shards, len(regs))
+                r, c, v = parallel.merge_coo([[np.array(x) for x in p[0][w][:3]] for p in parts], shards, n_unit)
                 out.append((r, c, v, shape))
             out = tuple(out)
             conf.last_timing = parts[0][1]
-        elif isinstance(batch, engine.MultiBatch):
-            gid = np.array([batch.gid_of.get(r.chrom, -1) if r.snp_list else -1 for r in regs], dtype=np.int32)
-            beg = np.array([r.start - 1 for r in regs], dtype=np.int64)
-            load, total = parallel.reads_before(gid, beg, batch.runs, batch.pos_of_run)
-            shards = parallel.partition(gid, beg, load, total, len(batch.batches))
-
-            def one(k):
-                b = batch.batches[k]
-                return _count_shard(conf, b.ctx, b.dreads, b.keyspace, b.gid_of, b.stats["max_aln_len"],
-                                    [regs[i] for i in shards[k]], snps)
-            parts = parallel.run_on_devices(len(shards), one)
-            out = []
-            for w in range(3):
-                r, c, v = parallel.merge_coo([[np.array(x) for x in p[0][w][:3]] for p in parts], shards, len(regs))
-                out.append((r, c, v, shape))
-            out = tuple(out)
-            conf.last_timing = parts[0][1]
+            per_unit = [(idx, p[2]) for idx, p in zip(shards, parts) if p[2] is not None]
         else:
-            out, conf.last_timing = _count_shard(conf, batch.ctx, batch.dreads, batch.keyspace, batch.gid_of,
-                                                 batch.stats["max_aln_len"], regs, snps)
+            idx = np.arange(n_unit, dtype=np.int64)
+            out, conf.last_timing, pu = count(batch, idx)
+            per_unit = [] if pu is None else [(idx, pu)]
         conf.last_stats = dict(batch.stats)
     finally:
         if own:
             batch.close()
+    return out, per_unit
+
+
+def count_regions(conf, regs, batch=None):
+    """Device counting; returns three (row, col, val, shape) tuples (AD, DP, OTH), rows index
+    `regs`.  With several GPUs the regions are cut into contiguous genomic chunks (their SNPs
+    follow them; a SNP shared by regions of two chunks is piled up on both), no collective."""
+    snps = conf.snp_set.snps
+    chroms = list(dict.fromkeys([s.chrom for s in snps]))
+    out, _ = count_units(conf, chroms, [r.chrom if r.snp_list else None for r in regs], [r.start - 1 for r in regs],
+                         [r.end - 1 for r in regs], lambda b, idx: _count_shard(conf, b, [regs[i] for i in idx], snps),
+                         batch)
     return out
 
 
@@ -386,7 +417,8 @@ def afc_core(conf):
         engine.write_mtx(fn, n_reg, row, col, val, emitted, len(conf.samples), engine.n_decode_threads(conf.nproc))
 
 
-def afc_run(conf):
+def afc_run(conf, core=afc_core):
+    """Runs `core(conf)` with the reference's logging (baf/fc/main.py:262-295); 0, or -1 on ValueError."""
     ret = -1
     cmdline = None
     start_time = time.time()
@@ -395,7 +427,7 @@ def afc_run(conf):
         cmdline = " ".join(conf.argv)
         info("CMD: %s" % cmdline)
     try:
-        ret = afc_core(conf)
+        ret = core(conf)
     except ValueError as e:
         error(str(e))
         error("Running program failed.")

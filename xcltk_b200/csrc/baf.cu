@@ -944,14 +944,39 @@ static __global__ void k_baf_snp_filter(const unsigned long long *tot, const uin
     keep[i] = skip ? 0 : 1;
 }
 
+static int snp_filter_check(xg_ctx *ctx, const xg_snps *snps, const xg_snp_filter *filt, const char *fn) {
+    if (!ctx || !ctx->stream) return ctx ? ctx->fail(XG_E_CUDA, "context has no device") : XG_E_ARG;
+    if (!snps || !filt || !filt->ref_idx || !filt->alt_idx) return ctx->fail(XG_E_ARG, std::string(fn) + ": null argument");
+    for (int32_t i = 0; i < snps->n; i++)
+        if (filt->ref_idx[i] > 4 || filt->alt_idx[i] > 4)
+            return ctx->fail(XG_E_ARG, std::string(fn) + ": allele index out of range");
+    return XG_OK;
+}
+
+// plp_snp's filter on the totals the last xg_baf_pileup left on the device -> d_keep (scratch "bf_keep"), and the
+// allele indices on the device (scratch "bf_ref_i" / "bf_alt_i"); keep_out (may be NULL) receives the filter
+static int snp_filter_launch(xg_ctx *ctx, const xg_snps *snps, const xg_snp_filter *filt, uint8_t *keep_out,
+                             const uint8_t **d_keep_out, const uint8_t **d_ref, const uint8_t **d_alt, const char *fn) {
+    uint8_t *d_keep = (uint8_t *)ctx->get("bf_keep", (size_t)snps->n + 16);
+    if (!d_keep || upload_arr(ctx, filt->ref_idx, (size_t)snps->n, "bf_ref_i", d_ref) ||
+        upload_arr(ctx, filt->alt_idx, (size_t)snps->n, "bf_alt_i", d_alt))
+        return ctx->fail(XG_E_CUDA, std::string(fn) + ": out of device memory");
+    if (snps->n > 0)
+        k_baf_snp_filter<<<(snps->n + 255) / 256, 256, 0, ctx->stream>>>(
+            (const unsigned long long *)ctx->scratch["bf_totals"].p, *d_ref, *d_alt, snps->n, filt->min_count, filt->min_maf,
+            d_keep);
+    if (keep_out && snps->n > 0)          // pageable destination: the copy has landed when the call returns
+        cudaMemcpyAsync(keep_out, d_keep, (size_t)snps->n, cudaMemcpyDeviceToHost, ctx->stream);
+    *d_keep_out = d_keep;
+    return XG_OK;
+}
+
 extern "C" int xg_baf_fc(xg_ctx *ctx, const xg_dreads *rd, const xg_snps *snps, const xg_barcodes *cells,
                          const xg_params *par, const xg_snp_filter *filt, int32_t n_regions, const int64_t *reg_ptr,
                          const int32_t *reg_snp, const uint8_t *hap_of, int32_t no_dup_hap, int64_t *totals,
                          uint8_t *keep_out, xg_coo **ad, xg_coo **dp, xg_coo **oth) {
-    if (!ctx || !ctx->stream) return ctx ? ctx->fail(XG_E_CUDA, "context has no device") : XG_E_ARG;
-    if (!snps || !filt || !filt->ref_idx || !filt->alt_idx) return ctx->fail(XG_E_ARG, "xg_baf_fc: null argument");
-    for (int32_t i = 0; i < snps->n; i++)
-        if (filt->ref_idx[i] > 4 || filt->alt_idx[i] > 4) return ctx->fail(XG_E_ARG, "xg_baf_fc: allele index out of range");
+    int rc = snp_filter_check(ctx, snps, filt, "xg_baf_fc");
+    if (rc) return rc;
     const auto t_call = std::chrono::steady_clock::now();
     auto ms_since = [](std::chrono::steady_clock::time_point a) {
         return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - a).count();
@@ -959,24 +984,16 @@ extern "C" int xg_baf_fc(xg_ctx *ctx, const xg_dreads *rd, const xg_snps *snps, 
     xg_baf_state *st = nullptr;
     XG_CUDA(cudaSetDevice(ctx->device));
     cudaEventRecord(ctx->ev[6], ctx->stream);
-    int rc = xg_baf_pileup(ctx, rd, snps, cells, par, totals, &st);
+    rc = xg_baf_pileup(ctx, rd, snps, cells, par, totals, &st);
     if (rc) return rc;
     double tp[16];
     for (int k = 0; k < 16; k++) tp[k] = ctx->timing[k];
     const double ms_pileup = ms_since(t_call);
-    const uint8_t *d_ref = nullptr, *d_alt = nullptr;
-    uint8_t *d_keep = (uint8_t *)ctx->get("bf_keep", (size_t)snps->n + 16);
-    if (!d_keep || upload_arr(ctx, filt->ref_idx, (size_t)snps->n, "bf_ref_i", &d_ref) ||
-        upload_arr(ctx, filt->alt_idx, (size_t)snps->n, "bf_alt_i", &d_alt)) {
+    const uint8_t *d_ref = nullptr, *d_alt = nullptr, *d_keep = nullptr;
+    if ((rc = snp_filter_launch(ctx, snps, filt, keep_out, &d_keep, &d_ref, &d_alt, "xg_baf_fc"))) {
         xg_baf_state_free(ctx, st);
-        return ctx->fail(XG_E_CUDA, "xg_baf_fc: out of device memory");
+        return rc;
     }
-    if (snps->n > 0)
-        k_baf_snp_filter<<<(snps->n + 255) / 256, 256, 0, ctx->stream>>>(
-            (const unsigned long long *)ctx->scratch["bf_totals"].p, d_ref, d_alt, snps->n, filt->min_count, filt->min_maf,
-            d_keep);
-    if (keep_out && snps->n > 0)          // pageable destination: the copy has landed when the call returns
-        cudaMemcpyAsync(keep_out, d_keep, (size_t)snps->n, cudaMemcpyDeviceToHost, ctx->stream);
     rc = baf_count_impl(ctx, st, n_regions, reg_ptr, reg_snp, hap_of, nullptr, d_keep, no_dup_hap, ad, dp, oth);
     xg_baf_state_free(ctx, st);
     if (rc) return rc;
@@ -1000,5 +1017,305 @@ extern "C" int xg_baf_fc(xg_ctx *ctx, const xg_dreads *rd, const xg_snps *snps, 
     ctx->timing[8] = ms_pileup;
     ctx->timing[9] = ms_pileup + tc9;
     ctx->timing[10] = ms_since(t_call);
+    return XG_OK;
+}
+
+// ---- SNP-level counting (xg_snp_pileup): the winners of the pileup reduced straight into SNP x cell AD / DP / OTH.
+// One SNP is a region of one SNP with GT 0|1 (baf/fc/core.py:143-194 with ref_idx 0, alt_idx 1): a winning UMI whose
+// allele is not None is ALT (its base is the SNP's ALT; checked first, so REF == ALT counts as ALT), REF, or OTH.
+// AD = ALT UMIs, DP = REF + ALT UMIs, OTH = the others; no_dup_hap cannot matter, a UMI has one allele at one SNP.
+#define SNP_WARP_MAX 128      // a SNP with at most this many winners is reduced by one warp, more by the whole CTA
+#define SNP_HIST_COLS 4096    // cells per column range of the CTA path's shared-memory histograms
+#define SNP_BATCH 8           // SNPs a CTA takes from the work counter at a time: one per warp
+
+namespace {
+
+enum { CLS_REF = 0, CLS_ALT = 1, CLS_OTH = 2 };
+
+// winners of kept SNPs with an allele: one count per SNP
+__global__ void k_snp_hist(int64_t n, const uint32_t *pr_snp, const uint32_t *pr_colal, const uint8_t *keep,
+                           int32_t *cnt) {
+    const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n) return;
+    const uint32_t ca = pr_colal[p], snp = pr_snp[p];
+    if (!(ca & 0x80000000u) || ((ca >> 24) & 7u) == CODE_NONE || !keep[snp]) return;
+    atomicAdd(&cnt[snp], 1);
+}
+
+// the same winners, one word each (col << 2 | class) in their SNP's segment [off[snp], off[snp + 1])
+__global__ void k_snp_scatter(int64_t n, const uint32_t *pr_snp, const uint32_t *pr_colal, const uint8_t *keep,
+                              const uint8_t *ref_i, const uint8_t *alt_i, const int64_t *off, int32_t *cur,
+                              uint32_t *words) {
+    const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n) return;
+    const uint32_t ca = pr_colal[p], snp = pr_snp[p], code = (ca >> 24) & 7u;
+    if (!(ca & 0x80000000u) || code == CODE_NONE || !keep[snp]) return;
+    const uint32_t cls = code == alt_i[snp] ? CLS_ALT : code == ref_i[snp] ? CLS_REF : CLS_OTH;
+    words[off[snp] + atomicAdd(&cur[snp], 1)] = (ca & 0xFFFFFFu) << 2 | cls;
+}
+
+__device__ __forceinline__ void snp_emit(int wh, int32_t v, uint32_t col, int64_t o, int32_t *st_col, int32_t *st_val,
+                                         int64_t st_stride) {
+    st_col[(size_t)wh * st_stride + o] = (int32_t)col;
+    st_val[(size_t)wh * st_stride + o] = v;
+}
+
+// Rows of the SNPs, in column order.  A SNP's rows go to the staging areas at its own word segment (a row has at most
+// as many entries as the SNP has winners), so no cursor is needed: seg_base = off[snp] in all three matrices.
+//   warp path (n <= SNP_WARP_MAX): the words are rank-sorted in shared memory; the first word of a column run counts
+//     the run's classes and emits the column's entries, placed by ballots;
+//   CTA path: three histograms (REF / ALT / OTH) over a range of SNP_HIST_COLS cells + a bitmap of touched cells,
+//     one range after another; the set bits walked in order give the entries (as k_baf_finalize).
+__global__ void __launch_bounds__(256) k_snp_finalize(const int64_t *off, const uint32_t *words, int32_t n_snps,
+                                                      int32_t n_cols, int32_t hist_cols, unsigned int *work,
+                                                      unsigned long long *paths /* [2] */, int64_t *seg_base,
+                                                      int32_t *seg_nnz, int32_t *st_col, int32_t *st_val,
+                                                      int64_t st_stride) {
+    extern __shared__ uint32_t smem[];
+    uint32_t *hist = smem;                                   // [3][hist_cols]
+    uint32_t *bitmap = smem + 3 * (size_t)hist_cols;         // (hist_cols + 31) / 32
+    __shared__ uint32_t s_words[SNP_BATCH][2 * SNP_WARP_MAX];
+    __shared__ int warp_tot[3][8];
+    __shared__ int s_first;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const unsigned lt = (1u << lane) - 1u;
+    const int nwm = (hist_cols + 31) >> 5;
+    for (int c = threadIdx.x; c < 3 * hist_cols; c += blockDim.x) hist[c] = 0;
+    for (int c = threadIdx.x; c < nwm; c += blockDim.x) bitmap[c] = 0;
+    unsigned long long n_warp = 0, n_cta = 0;
+    while (true) {
+        __syncthreads();
+        if (threadIdx.x == 0) s_first = (int)atomicAdd(work, (unsigned)SNP_BATCH);
+        __syncthreads();
+        const int first = s_first;
+        if (first >= n_snps) break;
+        // ---- warp path: SNP first + w
+        const int s = first + w;
+        if (s < n_snps) {
+            const int64_t beg = off[s];
+            const int n = (int)min(off[s + 1] - beg, (int64_t)SNP_WARP_MAX + 1);
+            if (n > 0 && n <= SNP_WARP_MAX) {
+                uint32_t *sw = s_words[w], *ss = sw + SNP_WARP_MAX;
+                for (int i = lane; i < n; i += 32) sw[i] = words[beg + i];
+                __syncwarp();
+                for (int i = lane; i < n; i += 32) {             // rank sort; equal words keep their order
+                    const uint32_t x = sw[i];
+                    int r = 0;
+                    for (int j = 0; j < n; j++) {
+                        const uint32_t y = sw[j];
+                        r += (y < x) || (y == x && j < i);
+                    }
+                    ss[r] = x;
+                }
+                __syncwarp();
+                int o[3] = {0, 0, 0};
+                for (int i0 = 0; i0 < n; i0 += 32) {
+                    const int i = i0 + lane;
+                    const uint32_t col = i < n ? ss[i] >> 2 : 0u;
+                    const bool start = i < n && (i == 0 || (ss[i - 1] >> 2) != col);
+                    int cr = 0, ca = 0, co = 0;
+                    if (start)
+                        for (int j = i; j < n && (ss[j] >> 2) == col; j++) {
+                            const uint32_t cls = ss[j] & 3u;
+                            cr += cls == CLS_REF;
+                            ca += cls == CLS_ALT;
+                            co += cls == CLS_OTH;
+                        }
+                    const int v[3] = {ca, cr + ca, co};                  // AD, DP, OTH
+#pragma unroll
+                    for (int wh = 0; wh < 3; wh++) {
+                        const unsigned m = __ballot_sync(0xffffffffu, v[wh] > 0);
+                        if (v[wh] > 0) snp_emit(wh, v[wh], col, beg + o[wh] + __popc(m & lt), st_col, st_val, st_stride);
+                        o[wh] += __popc(m);
+                    }
+                }
+                if (lane == 0) {
+#pragma unroll
+                    for (int wh = 0; wh < 3; wh++) {
+                        seg_base[(size_t)wh * n_snps + s] = beg;
+                        seg_nnz[(size_t)wh * n_snps + s] = o[wh];
+                    }
+                    n_warp++;
+                }
+            }
+        }
+        // ---- CTA path: the batch's SNPs with more winners, one after the other (the test is uniform over the CTA)
+        for (int k = 0; k < SNP_BATCH && first + k < n_snps; k++) {
+            const int sc = first + k;
+            const int64_t beg = off[sc], n = off[sc + 1] - beg;
+            if (n <= SNP_WARP_MAX) continue;
+            int o[3] = {0, 0, 0};
+            for (int c_lo = 0; c_lo < n_cols; c_lo += hist_cols) {
+                const int nc = min(hist_cols, n_cols - c_lo), nw = (nc + 31) >> 5;
+                for (int64_t i = threadIdx.x; i < n; i += blockDim.x) {
+                    const uint32_t x = words[beg + i], col = (x >> 2) - (uint32_t)c_lo;
+                    if (col >= (uint32_t)nc) continue;
+                    atomicAdd(&hist[(x & 3u) * hist_cols + col], 1u);
+                    atomicOr(&bitmap[col >> 5], 1u << (col & 31));
+                }
+                __syncthreads();
+                for (int k0 = 0; k0 < nw; k0 += blockDim.x) {          // ordered walk over the bitmap
+                    const int kw = k0 + threadIdx.x;
+                    const uint32_t bits = kw < nw ? bitmap[kw] : 0u;
+                    int cnt[3] = {0, 0, 0};
+                    for (uint32_t bb = bits; bb; bb &= bb - 1) {
+                        const int c = (kw << 5) + __ffs(bb) - 1;
+                        const uint32_t r = hist[CLS_REF * hist_cols + c], a = hist[CLS_ALT * hist_cols + c];
+                        cnt[0] += a != 0;
+                        cnt[1] += (r + a) != 0;
+                        cnt[2] += hist[CLS_OTH * hist_cols + c] != 0;
+                    }
+                    int incl[3], before[3] = {0, 0, 0}, tot[3] = {0, 0, 0};
+#pragma unroll
+                    for (int wh = 0; wh < 3; wh++) {
+                        incl[wh] = cnt[wh];
+                        for (int d = 1; d < 32; d <<= 1) {
+                            const int y = __shfl_up_sync(0xffffffffu, incl[wh], d);
+                            if (lane >= d) incl[wh] += y;
+                        }
+                        if (lane == 31) warp_tot[wh][w] = incl[wh];
+                    }
+                    __syncthreads();
+#pragma unroll
+                    for (int wh = 0; wh < 3; wh++)
+                        for (int q = 0; q < 8; q++) {
+                            const int x = warp_tot[wh][q];
+                            if (q < w) before[wh] += x;
+                            tot[wh] += x;
+                        }
+                    int64_t e[3];
+#pragma unroll
+                    for (int wh = 0; wh < 3; wh++) e[wh] = beg + o[wh] + before[wh] + (incl[wh] - cnt[wh]);
+                    for (uint32_t bb = bits; bb; bb &= bb - 1) {
+                        const int c = (kw << 5) + __ffs(bb) - 1;
+                        const uint32_t r = hist[CLS_REF * hist_cols + c], a = hist[CLS_ALT * hist_cols + c],
+                                       t = hist[CLS_OTH * hist_cols + c], col = (uint32_t)(c_lo + c);
+                        if (a) snp_emit(0, (int32_t)a, col, e[0]++, st_col, st_val, st_stride);
+                        if (r + a) snp_emit(1, (int32_t)(r + a), col, e[1]++, st_col, st_val, st_stride);
+                        if (t) snp_emit(2, (int32_t)t, col, e[2]++, st_col, st_val, st_stride);
+                    }
+#pragma unroll
+                    for (int wh = 0; wh < 3; wh++) o[wh] += tot[wh];
+                    __syncthreads();                          // warp_tot is rewritten by the next chunk
+                }
+                for (int kw = threadIdx.x; kw < nw; kw += blockDim.x) {   // clear what this range touched
+                    for (uint32_t bb = bitmap[kw]; bb; bb &= bb - 1) {
+                        const int c = (kw << 5) + __ffs(bb) - 1;
+                        hist[c] = 0;
+                        hist[hist_cols + c] = 0;
+                        hist[2 * hist_cols + c] = 0;
+                    }
+                    bitmap[kw] = 0;
+                }
+                __syncthreads();
+            }
+            if (threadIdx.x == 0) {
+#pragma unroll
+                for (int wh = 0; wh < 3; wh++) {
+                    seg_base[(size_t)wh * n_snps + sc] = beg;
+                    seg_nnz[(size_t)wh * n_snps + sc] = o[wh];
+                }
+                n_cta++;
+            }
+        }
+    }
+    if (n_warp) atomicAdd(&paths[0], n_warp);
+    if (n_cta) atomicAdd(&paths[1], n_cta);
+}
+
+}  // namespace
+
+extern "C" int xg_snp_pileup(xg_ctx *ctx, const xg_dreads *rd, const xg_snps *snps, const xg_barcodes *cells,
+                             const xg_params *par, const xg_snp_filter *filt, int64_t *totals, uint8_t *keep_out,
+                             xg_coo **ad, xg_coo **dp, xg_coo **oth) {
+    int rc = snp_filter_check(ctx, snps, filt, "xg_snp_pileup");
+    if (rc) return rc;
+    if (!ad || !dp || !oth) return ctx->fail(XG_E_ARG, "xg_snp_pileup: null argument");
+    if (cells && cells->n_samples >= (1 << 24))       // col << 2 | class must fit 32 bits
+        return ctx->fail(XG_E_LIMIT, "xg_snp_pileup: more than 2^24 columns");
+    const auto t_call = std::chrono::steady_clock::now();
+    auto ms_since = [](std::chrono::steady_clock::time_point a) {
+        return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - a).count();
+    };
+    xg_baf_state *st = nullptr;
+    XG_CUDA(cudaSetDevice(ctx->device));
+    cudaEventRecord(ctx->ev[6], ctx->stream);
+    if ((rc = xg_baf_pileup(ctx, rd, snps, cells, par, totals, &st))) return rc;
+    const double tp2 = ctx->timing[2], ms_pileup = ms_since(t_call);
+    const int64_t n_pairs = st->n_pairs;
+    const int32_t n_snps = snps->n, n_cols = st->n_cols;
+    const uint8_t *d_ref = nullptr, *d_alt = nullptr, *d_keep = nullptr;
+    // one free of the state on every path out; the scratch buffers below do not depend on it
+    struct StateGuard {
+        xg_ctx *c;
+        xg_baf_state *s;
+        ~StateGuard() { xg_baf_state_free(c, s); }
+    } guard{ctx, st};
+    if ((rc = snp_filter_launch(ctx, snps, filt, keep_out, &d_keep, &d_ref, &d_alt, "xg_snp_pileup"))) return rc;
+    int launches = 1;
+    // capacities: the winners of one SNP never exceed the batch's pairs (< 2^31, checked by the pileup)
+    const size_t cap = (size_t)n_pairs + 1;
+    XG_GET(cnt, int32_t, "sp_cnt", (size_t)n_snps + 1);
+    XG_GET(cur, int32_t, "sp_cur", (size_t)n_snps + 1);
+    XG_GET(off, int64_t, "sp_off", (size_t)n_snps + 2);
+    XG_GET(words, uint32_t, "sp_words", cap);
+    XG_GET(work, unsigned int, "sp_work", 4);
+    XG_GET(paths, unsigned long long, "sp_paths", 2);
+    XG_GET(seg_base, int64_t, "sp_seg_base", 3 * (size_t)n_snps + 1);
+    XG_GET(seg_nnz, int32_t, "sp_seg_nnz", 3 * (size_t)n_snps + 1);
+    XG_GET(st_col, int32_t, "sp_st_col", 3 * cap);
+    XG_GET(st_val, int32_t, "sp_st_val", 3 * cap);
+    XG_CUDA(cudaMemsetAsync(cnt, 0, sizeof(int32_t) * ((size_t)n_snps + 1), ctx->stream));
+    XG_CUDA(cudaMemsetAsync(cur, 0, sizeof(int32_t) * ((size_t)n_snps + 1), ctx->stream));
+    XG_CUDA(cudaMemsetAsync(work, 0, 16, ctx->stream));
+    XG_CUDA(cudaMemsetAsync(paths, 0, 16, ctx->stream));
+    XG_CUDA(cudaMemsetAsync(seg_base, 0, sizeof(int64_t) * (3 * (size_t)n_snps + 1), ctx->stream));
+    XG_CUDA(cudaMemsetAsync(seg_nnz, 0, sizeof(int32_t) * (3 * (size_t)n_snps + 1), ctx->stream));
+    const unsigned grid = (unsigned)((n_pairs + 255) / 256);
+    if (n_pairs > 0) {
+        k_snp_hist<<<grid, 256, 0, ctx->stream>>>(n_pairs, st->pr_snp, st->pr_colal, d_keep, cnt);
+        launches++;
+    }
+    k_exclusive_scan<<<1, 1024, 0, ctx->stream>>>(cnt, off, n_snps);
+    launches++;
+    if (n_pairs > 0 && n_snps > 0) {
+        k_snp_scatter<<<grid, 256, 0, ctx->stream>>>(n_pairs, st->pr_snp, st->pr_colal, d_keep, d_ref, d_alt, off, cur,
+                                                     words);
+        const int32_t hist_cols = std::min(n_cols, SNP_HIST_COLS);
+        const size_t smem = (size_t)hist_cols * 12 + (size_t)((hist_cols + 31) / 32) * 4;
+        XG_CUDA(cudaFuncSetAttribute(k_snp_finalize, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        const int per_sm = std::max(1, std::min(8, (int)(200 * 1024 / (smem + 8 * 1024 + 1024))));
+        const int n_batches = (n_snps + SNP_BATCH - 1) / SNP_BATCH;
+        k_snp_finalize<<<std::min(n_batches, 148 * per_sm), 256, smem, ctx->stream>>>(
+            off, words, n_snps, n_cols, hist_cols, work, paths, seg_base, seg_nnz, st_col, st_val, (int64_t)cap);
+        launches += 2;
+    }
+    XG_CUDA(cudaGetLastError());
+    const double ms_kernels = ms_since(t_call);
+    xg_coo **outs[3] = {ad, dp, oth};
+    if ((rc = xg_staging_to_coo3(ctx, "sp3", n_snps, n_cols, seg_base, seg_nnz, st_col, st_val, (int64_t)cap, outs,
+                                 &launches)))
+        return rc;
+    // the stream is idle now: the winner count and the path counters cost one short copy
+    long long stats[3] = {0, 0, 0};
+    XG_CUDA(cudaMemcpyAsync(&stats[0], off + n_snps, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    XG_CUDA(cudaMemcpyAsync(&stats[1], paths, 16, cudaMemcpyDeviceToHost, ctx->stream));
+    XG_CUDA(cudaStreamSynchronize(ctx->stream));
+    float t_all = 0, t_scan = 0;
+    cudaEventElapsedTime(&t_all, ctx->ev[6], ctx->ev[3]);
+    cudaEventElapsedTime(&t_scan, ctx->ev[1], ctx->ev[2]);
+    const double t_d2h = ctx->timing[4];       // the pileup's totals (if copied out) + the results
+    for (double &t : ctx->timing) t = 0;
+    ctx->timing[0] = t_all;
+    ctx->timing[1] = t_scan;
+    ctx->timing[2] = tp2 + launches;
+    ctx->timing[4] = t_d2h;
+    ctx->timing[6] = (double)n_pairs;
+    ctx->timing[7] = (double)stats[0];
+    ctx->timing[8] = ms_pileup;
+    ctx->timing[9] = ms_kernels;
+    ctx->timing[10] = ms_since(t_call);
+    ctx->timing[14] = (double)stats[1];
+    ctx->timing[15] = (double)stats[2];
     return XG_OK;
 }

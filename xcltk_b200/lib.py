@@ -149,6 +149,9 @@ SYMBOLS = {
     "xg_baf_fc": (C.c_int, [_P, _P, C.POINTER(Snps), C.POINTER(Barcodes), C.POINTER(Params), C.POINTER(SnpFilter),
                             C.c_int32, c_i64p, c_i32p, c_u8p, C.c_int32, c_i64p, c_u8p,
                             C.POINTER(C.POINTER(Coo)), C.POINTER(C.POINTER(Coo)), C.POINTER(C.POINTER(Coo))]),
+    "xg_snp_pileup": (C.c_int, [_P, _P, C.POINTER(Snps), C.POINTER(Barcodes), C.POINTER(Params), C.POINTER(SnpFilter),
+                                c_i64p, c_u8p, C.POINTER(C.POINTER(Coo)), C.POINTER(C.POINTER(Coo)),
+                                C.POINTER(C.POINTER(Coo))]),
     "xg_synth_reads": (C.c_int, [_P, C.POINTER(SynthParams), C.POINTER(_P), c_u64p]),
     "xg_synth_read_index": (C.c_int64, [C.POINTER(SynthParams), C.c_int32, C.c_int32]),
     "xg_write_bam": (C.c_int, [C.c_char_p, C.POINTER(Reads), C.c_int32, C.POINTER(C.c_char_p), c_i64p, _P,
@@ -688,6 +691,35 @@ class Context(object):
                                        as_ptr(totals, c_i64p) if want_totals else None,
                                        as_ptr(keep, c_u8p) if want_keep else None,
                                        C.byref(ad), C.byref(dp), C.byref(oth)))
+        out = tuple(coo_to_numpy(self.lib, m, ctx_obj=self) for m in (ad, dp, oth))
+        if want_totals:
+            out += (totals,)
+        if want_keep:
+            out += (keep,)
+        return out
+
+    def snp_pileup(self, dreads, gid, pos, cell_keys, n_samples, params, ref_i, alt_i, min_count, min_maf,
+                   want_totals=False, want_keep=False):
+        """SNP x cell AD / DP / OTH of the SNPs themselves (xg_snp_pileup): pileup, the SNP filter on the device, each
+        SNP counted as a region of one SNP with GT 0|1.  Rows are all input SNPs (a filtered SNP has empty rows).
+        Returns (ad, dp, oth[, totals][, keep]) as baf_fc does."""
+        gid = np.ascontiguousarray(gid, dtype=np.int32)
+        pos = np.ascontiguousarray(pos, dtype=np.int32)
+        keys = np.ascontiguousarray(cell_keys if cell_keys is not None else [], dtype=np.uint64)
+        ref_i = np.ascontiguousarray(ref_i, dtype=np.uint8)
+        alt_i = np.ascontiguousarray(alt_i, dtype=np.uint8)
+        if len(pos) != len(gid) or len(ref_i) != len(gid) or len(alt_i) != len(gid):
+            raise ValueError("snp_pileup: per-SNP arrays of different lengths")
+        s = Snps(len(gid), as_ptr(gid, c_i32p), as_ptr(pos, c_i32p))
+        b = Barcodes(len(keys), as_ptr(keys, c_u64p), n_samples)
+        f = SnpFilter(as_ptr(ref_i, c_u8p), as_ptr(alt_i, c_u8p), float(min_count), float(min_maf))
+        totals = np.zeros((len(gid), 5), dtype=np.int64) if want_totals else None
+        keep = np.zeros(len(gid), dtype=np.uint8) if want_keep else None
+        ad, dp, oth = C.POINTER(Coo)(), C.POINTER(Coo)(), C.POINTER(Coo)()
+        self._check(self.lib.xg_snp_pileup(self.h, dreads.h, C.byref(s), C.byref(b), C.byref(params.c), C.byref(f),
+                                           as_ptr(totals, c_i64p) if want_totals else None,
+                                           as_ptr(keep, c_u8p) if want_keep else None,
+                                           C.byref(ad), C.byref(dp), C.byref(oth)))
         out = tuple(coo_to_numpy(self.lib, m, ctx_obj=self) for m in (ad, dp, oth))
         if want_totals:
             out += (totals,)

@@ -16,8 +16,9 @@ Commands:
      basefc           Basic feature counting (GPU).
 
   -- BAF calculation
+     pileup           SNP-level allele counting at candidate SNPs (GPU): cellSNP.* output.
      (feature-level allele counting is a Python API: xcltk_b200.baf.fc.main.afc_wrapper;
-      the `baf` pipeline around it -- cellsnp-lite, Eagle2 -- stays in the reference)
+      the `baf` pipeline around it -- genotyping, Eagle2 -- stays in the reference)
 
   -- Others
      -h, --help       Print this message and exit.
@@ -33,6 +34,11 @@ def _run_basefc(argv):
     return fc_main(argv) or 0
 
 
+def _run_pileup(argv):
+    from .baf.pileup import pileup_main
+    return pileup_main(argv) or 0
+
+
 def main(argv=None):
     argv = list(sys.argv if argv is None else argv)
     command = argv[1] if len(argv) > 1 else "--help"
@@ -44,6 +50,8 @@ def main(argv=None):
         sys.exit(0)
     if command == "basefc":
         sys.exit(_run_basefc(argv))
+    if command == "pileup":
+        sys.exit(_run_pileup(argv))
     if command in _ELSEWHERE:
         sys.stderr.write("Error: command '%s' is outside the scope of xcltk_b200; use the reference.\n" % command)
     else:
