@@ -400,6 +400,9 @@ int xg_write_bam(const char *path, const xg_reads *reads, int32_t n_gid, const c
  * [13] bytes copied host -> device (xg_basefc_host); [14] / [15] features counted in segments / in sets.
  * xg_baf_*: [8..10] host milestones of the call (ms since entry).                                   */
 void xg_last_timing(xg_ctx *ctx, double out[16]);
+/* Route counters of the segment finalize in the last xg_basefc / xg_basefc_host call: [0..3] ordinary CTAs,
+ * [4..7] big CTAs, each {heavy features, careful column ranges, fast ranges that overflowed, sub-partition doublings}. */
+int xg_basefc_finalize_stats(xg_ctx *ctx, int64_t out[8]);
 
 const char *xg_version(void);
 

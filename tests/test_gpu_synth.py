@@ -141,17 +141,22 @@ def test_basefc_feature_rows_are_independent(gpu_ctx, fc_batch):
         assert got.get(k, []) == full.get(orig, [])
 
 
-def test_basefc_many_cells_multi_pass_histogram(gpu_ctx):
-    """More cells than the shared-memory histogram holds (> 40 960): column-range passes."""
+def test_basefc_many_cells_multi_pass_histogram(gpu_ctx, monkeypatch):
+    """100 000 cells: in segments (pair words fit up to 2^19 cells), and with a set per feature (XG_SEG_MODE=0), whose
+    finalize reads each row in column-range passes because the cells do not fit its histogram (> 40 960)."""
     from oracle import oracle
     from xcltk_b200 import workload
     w = workload.make_basefc_workload(gpu_ctx, 300000, 100000, 2000, seed=4, chroms={"20", "21", "22"})
     conf = Conf()
-    row, col, val, _ = gpu_ctx.basefc(w.dreads, w.gid, w.beg, w.end, w.cell_keys, 100000, gpu_params(conf))
     host = w.dreads.download()
     o = oracle.basefc(host, w.gid, w.beg, w.end, w.cell_keys, 100000, oracle.params(conf), 4)
-    assert col.max() > 40960
-    assert np.array_equal(row, o[0]) and np.array_equal(col, o[1]) and np.array_equal(val, o[2])
+    for seg_mode in ("1", "0"):
+        monkeypatch.setenv("XG_SEG_MODE", seg_mode)
+        row, col, val, _ = gpu_ctx.basefc(w.dreads, w.gid, w.beg, w.end, w.cell_keys, 100000, gpu_params(conf))
+        t = gpu_ctx.timing()
+        assert (t[14] > 0, t[15] > 0) == ((True, False) if seg_mode == "1" else (False, True))
+        assert col.max() > 40960
+        assert np.array_equal(row, o[0]) and np.array_equal(col, o[1]) and np.array_equal(val, o[2])
 
 
 def test_basefc_bins_large_windows(gpu_ctx):

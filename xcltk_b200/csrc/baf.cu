@@ -599,13 +599,11 @@ extern "C" int xg_baf_pileup(xg_ctx *ctx, const xg_dreads *rd, const xg_snps *sn
     // SNPs sorted by (gid, pos); pos < 0 (1-based pos <= 0) can never be fetched.  The sorted
     // table depends on the SNP list only: it is kept on the device while the caller passes
     // the same list (hash of the arrays).
-    uint64_t sh = 1469598103934665603ull;
-    auto mixh = [&](const void *p, size_t n) { xg_mix_bytes(sh, p, n); };
-    mixh(&n_gid, sizeof n_gid);
-    mixh(&snps->n, sizeof snps->n);
-    mixh(snps->gid, sizeof(int32_t) * (size_t)snps->n);
-    mixh(snps->pos, sizeof(int32_t) * (size_t)snps->n);
-    const bool snp_cached = ctx->bf_snp_valid && ctx->bf_snp_hash == sh;
+    const size_t sb = sizeof(int32_t) * (size_t)snps->n;
+    const std::initializer_list<xg_input_key::Span> in = {
+        {&n_gid, sizeof n_gid}, {&snps->n, sizeof snps->n}, {snps->gid, sb}, {snps->pos, sb}};
+    const uint64_t sh = xg_input_key::hash_of(in);
+    const bool snp_cached = ctx->bf_snp_valid && ctx->bf_snp_key.matches(sh, in);
     if (!snp_cached) {
         ctx->bf_snp_valid = false;
         std::vector<int32_t> ord;
@@ -629,7 +627,7 @@ extern "C" int xg_baf_pileup(xg_ctx *ctx, const xg_dreads *rd, const xg_snps *sn
         if ((rc0 = upload_arr(ctx, spos.data(), spos.size(), "bf_spos", &dummy))) return rc0;
         if ((rc0 = upload_arr(ctx, sidx.data(), sidx.size(), "bf_sidx", &dummy))) return rc0;
         XG_CUDA(cudaStreamSynchronize(ctx->stream));
-        ctx->bf_snp_hash = sh;
+        ctx->bf_snp_key.assign(sh, in);
         ctx->bf_snp_sorted = (int64_t)ord.size();
         ctx->bf_snp_valid = true;
     }
@@ -809,13 +807,12 @@ static int baf_count_impl(xg_ctx *ctx, xg_baf_state *st, int32_t n_regions, cons
     const int32_t n_cols = st->n_cols, n_snps = st->n_snps;
     // invert region -> SNP lists (cached on the device while the caller passes the same lists)
     const int64_t n_mem = reg_ptr[n_regions];
-    uint64_t sh = 1469598103934665603ull;
-    auto mixh = [&](const void *p, size_t n) { xg_mix_bytes(sh, p, n); };
-    mixh(&n_snps, sizeof n_snps);
-    mixh(&n_regions, sizeof n_regions);
-    mixh(reg_ptr, sizeof(int64_t) * ((size_t)n_regions + 1));
-    mixh(reg_snp, sizeof(int32_t) * (size_t)n_mem);
-    const bool sr_cached = ctx->bf_sr_valid && ctx->bf_sr_hash == sh;
+    const std::initializer_list<xg_input_key::Span> in = {{&n_snps, sizeof n_snps},
+                                                          {&n_regions, sizeof n_regions},
+                                                          {reg_ptr, sizeof(int64_t) * ((size_t)n_regions + 1)},
+                                                          {reg_snp, sizeof(int32_t) * (size_t)n_mem}};
+    const uint64_t sh = xg_input_key::hash_of(in);
+    const bool sr_cached = ctx->bf_sr_valid && ctx->bf_sr_key.matches(sh, in);
     if (!sr_cached) {
         ctx->bf_sr_valid = false;
         std::vector<int64_t> sr_ptr((size_t)n_snps + 1, 0);
@@ -836,7 +833,7 @@ static int baf_count_impl(xg_ctx *ctx, xg_baf_state *st, int32_t n_regions, cons
         if ((rc0 = upload_arr(ctx, sr_ptr.data(), sr_ptr.size(), "bf_sr_ptr", &d64))) return rc0;
         if ((rc0 = upload_arr(ctx, sr.data(), sr.size(), "bf_sr", &d32))) return rc0;
         XG_CUDA(cudaStreamSynchronize(ctx->stream));
-        ctx->bf_sr_hash = sh;
+        ctx->bf_sr_key.assign(sh, in);
         ctx->bf_sr_valid = true;
     }
 

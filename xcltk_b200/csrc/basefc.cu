@@ -392,7 +392,7 @@ struct __align__(16) FeatDesc {
 // same one) and the host-side working arrays of a call, reused so that they are not paged in anew every time.
 struct FeatCache {
     bool valid = false;
-    uint64_t hash = 0;
+    xg_input_key key;
     FeatIndexHost ix;
     EpochPlan plan;
     std::vector<unsigned long long> cand;
@@ -1142,6 +1142,7 @@ __global__ void __launch_bounds__(256) k_zero_segments(uint8_t *pool, const uint
 #define FS_RANGES 1024                // column ranges of a heavy feature (counters live in the idle table)
 #define FS_TBL_LOG2 12                // ordinary CTAs: 4096-slot table (FS_TBL)
 #define FS_BIG_TBL_LOG2 14            // big CTAs: 16384 slots -- a quarter of the ranges, each a barrier and a round trip
+#define FS_STATS 8                    // route counters of the two instantiations (xg_basefc_finalize_stats)
 static_assert((1 << FS_TBL_LOG2) == FS_TBL, "table size");
 
 __device__ __forceinline__ uint64_t pair_hash(unsigned long long pw) {
@@ -1218,13 +1219,15 @@ template <int THREADS, int TBL_LOG2>
 __global__ void __maxnreg__(48) k_basefc_finalize_segs(
     const uint8_t *pool, const FeatDesc *fdesc, const uint32_t *seg_cur, const int32_t *sf_row,
     const int32_t *fin_feat, int32_t n_fin, int32_t n_cols, unsigned int *work, unsigned long long *cursor,
-    int64_t *seg_base, int32_t *seg_nnz, int32_t *st_col, int32_t *st_val) {
+    int64_t *seg_base, int32_t *seg_nnz, int32_t *st_col, int32_t *st_val, unsigned long long *stats) {
     extern __shared__ __align__(16) uint8_t fin_smem[];
     // table slots; words a table pass should hold (40 % load: the light / heavy limit); cells of a range on the fast
     // path = one counter bank; the counters (a light feature uses both banks as one)
     constexpr uint32_t TBL = 1u << TBL_LOG2, CAP = TBL * 2 / 5, RCELLS = TBL / 4, CNT = 2 * RCELLS;
     constexpr uint32_t LIGHT = CAP < FS_REG * THREADS ? CAP : FS_REG * THREADS;     // words a CTA keeps in registers
     static_assert(LIGHT >= SEG_PART_WORDS, "a feature without a scratch half must be light");
+    // xg_basefc_finalize_stats: heavy features, careful ranges, fast-range overflows, sub-partition doublings
+    if (THREADS == FS_BIG_THREADS) stats += FS_STATS / 2;
     const int bm_words = (n_cols + 31) >> 5;
     unsigned long long *tbl = reinterpret_cast<unsigned long long *>(fin_smem);      // TBL
     uint32_t *cnt = reinterpret_cast<uint32_t *>(tbl + TBL);                       // CNT rank counters
@@ -1256,6 +1259,7 @@ __global__ void __maxnreg__(48) k_basefc_finalize_segs(
         uint32_t n_rng = 1;
         uint32_t *rc = reinterpret_cast<uint32_t *>(tbl);             // the table is idle: counters, then cursors
         if (!light) {
+            if (threadIdx.x == 0) atomicAdd(&stats[0], 1ull);
             while (wshift < TBL_LOG2 - 2 && ((uint64_t)n << (wshift + 1)) <= (uint64_t)(CAP * 3 / 4) * (uint64_t)n_cols) wshift++;
             while (((n_cols - 1) >> wshift) + 1 > FS_RANGES) wshift++;      // very many cells: wider ranges, rank windows
             n_rng = (uint32_t)((n_cols - 1) >> wshift) + 1;
@@ -1448,11 +1452,15 @@ __global__ void __maxnreg__(48) k_basefc_finalize_segs(
                 // 96 probes were not enough (never with a sane hash): forget the attempt, take the careful path
                 __syncthreads();
                 for (uint32_t r = threadIdx.x; r < RCELLS; r += THREADS) cb[r] = 0;
-                if (threadIdx.x == 0) F.ovf_b[bank] = 0;
+                if (threadIdx.x == 0) {
+                    F.ovf_b[bank] = 0;
+                    atomicAdd(&stats[2], 1ull);
+                }
                 slow = true;
             }
             // ---- careful path: [clear table] sync [insert] sync per hash sub-partition, rank windows of CAP cells
             __syncthreads();                 // both banks are idle from here on
+            if (threadIdx.x == 0) atomicAdd(&stats[1], 1ull);
             for (uint32_t win = 0; win < nz_r; win += CAP) {
                 uint32_t n_sub = (m + CAP - 1) / CAP;
                 while (true) {
@@ -1485,7 +1493,10 @@ __global__ void __maxnreg__(48) k_basefc_finalize_segs(
                     // a pass overflowed the table: forget the window's counts, sweep again with finer sub-partitions
                     __syncthreads();
                     for (uint32_t c = threadIdx.x; c < CAP; c += THREADS) cnt[c] = 0;
-                    if (threadIdx.x == 0) F.ovf_s = 0;
+                    if (threadIdx.x == 0) {
+                        F.ovf_s = 0;
+                        atomicAdd(&stats[3], 1ull);
+                    }
                     n_sub *= 2;
                 }
                 // the window's counts; the counters go back to zero as they are read
@@ -1663,6 +1674,7 @@ struct BasefcCall {
     unsigned long long *cursor = nullptr;
     unsigned int *fin_work = nullptr;
     uint32_t *seg_cur = nullptr;
+    unsigned long long *fs_stats = nullptr;   // route counters of the segment finalize (xg_basefc_finalize_stats)
     unsigned long long *h_cur = nullptr;    // rows layouts: the staging cursor after every epoch (mapped host memory)
     int64_t h2d_bytes = 0;
     double ms_index = 0, ms_windows = 0, ms_plan = 0, ms_upload = 0;
@@ -1678,13 +1690,10 @@ static int basefc_windows(BasefcCall &c, const xg_features *feats, int32_t n_gid
     auto t_ph = std::chrono::steady_clock::now();
     // the interval index depends on the features only: reuse it (host copy and the uploaded
     // device arrays, which live in named scratch buffers) while the caller passes the same set
-    uint64_t fh = 1469598103934665603ull;
-    auto mixh = [&](const void *p, size_t n) { xg_mix_bytes(fh, p, n); };
-    mixh(&n_gid, sizeof n_gid);
-    mixh(&feats->n, sizeof feats->n);
-    mixh(feats->gid, sizeof(int32_t) * (size_t)feats->n);
-    mixh(feats->beg, sizeof(int32_t) * (size_t)feats->n);
-    mixh(feats->end, sizeof(int32_t) * (size_t)feats->n);
+    const size_t fb = sizeof(int32_t) * (size_t)feats->n;
+    const std::initializer_list<xg_input_key::Span> in = {
+        {&n_gid, sizeof n_gid}, {&feats->n, sizeof feats->n}, {feats->gid, fb}, {feats->beg, fb}, {feats->end, fb}};
+    const uint64_t fh = xg_input_key::hash_of(in);
     FeatCache *fc = (FeatCache *)ctx->fx_cache;
     if (!fc) {
         fc = new FeatCache();
@@ -1692,13 +1701,13 @@ static int basefc_windows(BasefcCall &c, const xg_features *feats, int32_t n_gid
         ctx->fx_cache_free = [](void *p) { delete (FeatCache *)p; };
     }
     c.fc = fc;
-    const bool index_cached = fc->valid && fc->hash == fh;
+    const bool index_cached = fc->valid && fc->key.matches(fh, in);
     int rc = XG_OK;
     if (!index_cached) {
         fc->valid = false;
         fc->ix = FeatIndexHost();
         if ((rc = build_feat_index(ctx, feats, n_gid, fc->ix))) return rc;
-        fc->hash = fh;
+        fc->key.assign(fh, in);
     }
     const FeatIndexHost &ix = fc->ix;
     const size_t m = c.m = ix.sf_beg.size();
@@ -2037,7 +2046,7 @@ static int basefc_epochs(BasefcCall &c, bool rows) {
             k_basefc_finalize_segs<FS_BIG_THREADS, FS_BIG_TBL_LOG2><<<std::min(n_big, 148), FS_BIG_THREADS, big_bytes,
                                                                      ctx->big_stream>>>(
                 P.pool, P.fdesc, c.seg_cur, c.d_sf_row, c.d_fin_big + pl.fin_big_ptr[(size_t)e], n_big, n_cols,
-                big_work + e, c.cursor, c.seg_base, c.seg_nnz, c.st_col, c.st_val);
+                big_work + e, c.cursor, c.seg_base, c.seg_nnz, c.st_col, c.st_val, c.fs_stats);
             c.launches++;
             XG_DBG("k_basefc_finalize_segs<big>");
             cudaEventRecord(c.ev(4, e), ctx->big_stream);
@@ -2046,7 +2055,7 @@ static int basefc_epochs(BasefcCall &c, bool rows) {
             const int grid = std::min(n_fin, 148 * segs_ctas_per_sm);
             k_basefc_finalize_segs<FS_THREADS, FS_TBL_LOG2><<<grid, FS_THREADS, segs_bytes, st>>>(
                 P.pool, P.fdesc, c.seg_cur, c.d_sf_row, c.d_fin_feat + pl.fin_ptr[(size_t)e], n_fin, n_cols,
-                c.fin_work + e, c.cursor, c.seg_base, c.seg_nnz, c.st_col, c.st_val);
+                c.fin_work + e, c.cursor, c.seg_base, c.seg_nnz, c.st_col, c.st_val, c.fs_stats);
             c.launches++;
             XG_DBG("k_basefc_finalize_segs");
         }
@@ -2315,6 +2324,10 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
         for (auto &r : rd->h_runs)
             if (r.bam_idx >= c.n_cols) return ctx->fail(XG_E_ARG, "more BAMs than sample columns");
     const auto t_call = std::chrono::steady_clock::now();
+    c.fs_stats = (unsigned long long *)ctx->get("fx_fs_stats", sizeof(unsigned long long) * FS_STATS);
+    if (!c.fs_stats) return XG_E_CUDA;
+    // a call redone with sets keeps the counts of its first attempt, whose segments were reduced
+    if (!force_sets) XG_CUDA(cudaMemsetAsync(c.fs_stats, 0, sizeof(unsigned long long) * FS_STATS, ctx->stream));
     int rc = XG_OK;
     if ((rc = basefc_windows(c, feats, n_gid)) || (rc = basefc_plan(c, cells, par, force_sets)) ||
         (rc = basefc_epochs(c, layout != XG_LAYOUT_CSR)))
@@ -2538,5 +2551,20 @@ extern "C" int xg_basefc_write_mtx_device(xg_ctx *ctx, const char *path, int32_t
         cudaGetLastError();
         return ctx->fail(XG_E_IO, std::string("short write on '") + path + "'");
     }
+    return XG_OK;
+}
+
+extern "C" int xg_basefc_finalize_stats(xg_ctx *ctx, int64_t out[8]) {
+    if (!ctx || !ctx->stream) return ctx ? ctx->fail(XG_E_CUDA, "context has no device") : XG_E_ARG;
+    if (!out) return ctx->fail(XG_E_ARG, "xg_basefc_finalize_stats: null argument");
+    XG_CUDA(cudaSetDevice(ctx->device));
+    static_assert(FS_STATS == 8, "xg_basefc_finalize_stats reports 8 counters");
+    unsigned long long h[FS_STATS] = {};
+    auto it = ctx->scratch.find("fx_fs_stats");
+    if (it != ctx->scratch.end() && it->second.p) {
+        XG_CUDA(cudaStreamSynchronize(ctx->stream));
+        XG_CUDA(cudaMemcpy(h, it->second.p, sizeof h, cudaMemcpyDeviceToHost));
+    }
+    for (int k = 0; k < FS_STATS; k++) out[k] = (int64_t)h[k];
     return XG_OK;
 }

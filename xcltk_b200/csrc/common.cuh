@@ -5,6 +5,7 @@
 
 #include <cstdint>
 #include <cstdio>
+#include <initializer_list>
 #include <map>
 #include <string>
 #include <vector>
@@ -66,6 +67,38 @@ static inline void xg_mix_bytes(uint64_t &h, const void *p, size_t n) {
     h = (h ^ (uint64_t)n) * 1099511628211ull;
     h ^= h >> 32;
 }
+
+// The input a device-side cache was built from (the features, SNPs, regions or barcodes of the last call).  The hash
+// is the quick test; inputs with equal hashes are easy to build (every step of xg_mix_bytes can be inverted), so a hit
+// also compares the bytes, of which the key keeps a copy.
+struct xg_input_key {
+    struct Span {
+        const void *p;
+        size_t n;
+    };
+    uint64_t hash = 0;
+    std::vector<uint8_t> bytes;
+    static uint64_t hash_of(std::initializer_list<Span> in) {
+        uint64_t h = 1469598103934665603ull;
+        for (const Span &s : in) xg_mix_bytes(h, s.p, s.n);
+        return h;
+    }
+    bool matches(uint64_t h, std::initializer_list<Span> in) const {
+        if (h != hash) return false;
+        size_t at = 0;
+        for (const Span &s : in) {
+            if (s.n > bytes.size() - at || (s.n && memcmp(bytes.data() + at, s.p, s.n) != 0)) return false;
+            at += s.n;
+        }
+        return at == bytes.size();
+    }
+    void assign(uint64_t h, std::initializer_list<Span> in) {
+        hash = h;
+        bytes.clear();
+        for (const Span &s : in)
+            if (s.n) bytes.insert(bytes.end(), (const uint8_t *)s.p, (const uint8_t *)s.p + s.n);
+    }
+};
 
 struct xg_ctx {
     int device = 0;
@@ -196,14 +229,14 @@ struct xg_ctx {
     }
     // cache of the last sorted SNP table of xg_baf_pileup (device arrays in scratch "bf_*")
     bool bf_snp_valid = false;
-    uint64_t bf_snp_hash = 0;
+    xg_input_key bf_snp_key;
     int64_t bf_snp_sorted = 0;
     bool bf_sr_valid = false;              // ... and of the inverted region -> SNP lists of xg_baf_count
-    uint64_t bf_sr_hash = 0;
+    xg_input_key bf_sr_key;
     // the two most recent barcode tables (basefc and baf alternate with different cell lists): scratch "bc_slots0/1"
     struct BcCache {
         bool valid = false;
-        uint64_t hash = 0;
+        xg_input_key key;
         uint64_t used = 0;
         const void *slots = nullptr;
         uint32_t mask = 0, shift = 0;

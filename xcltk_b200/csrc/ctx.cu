@@ -340,6 +340,8 @@ int xg_make_tile_pmax(xg_ctx *ctx, xg_dreads *d) {
 // Replaces the dict lookup `smp in self.cell_cnt` (rdr/fc/mcount.py:119-127).
 int xg_build_barcode_table(xg_ctx *ctx, const xg_barcodes *cells, BarcodeTable *out) {
     // the table depends on the key list only: it stays on the device while the caller passes the same list
+    const std::initializer_list<xg_input_key::Span> in = {{&cells->n, sizeof cells->n},
+                                                          {cells->keys, sizeof(uint64_t) * (size_t)cells->n}};
     uint64_t h = 1469598103934665603ull ^ (uint64_t)cells->n;
     for (int32_t i = 0; i < cells->n; i++) {
         h = (h ^ cells->keys[i]) * 1099511628211ull;
@@ -347,7 +349,7 @@ int xg_build_barcode_table(xg_ctx *ctx, const xg_barcodes *cells, BarcodeTable *
     }
     for (int k = 0; k < 2; k++) {
         xg_ctx::BcCache &c = ctx->bc_cache[k];
-        if (c.valid && c.hash == h) {
+        if (c.valid && c.key.matches(h, in)) {
             c.used = ++ctx->bc_clock;
             out->slots = (const ulonglong2 *)c.slots;
             out->mask = c.mask;
@@ -386,7 +388,7 @@ int xg_build_barcode_table(xg_ctx *ctx, const xg_barcodes *cells, BarcodeTable *
     ctx->bc_cache[slot].slots = dt;
     ctx->bc_cache[slot].mask = out->mask;
     ctx->bc_cache[slot].shift = out->shift;
-    ctx->bc_cache[slot].hash = h;
+    ctx->bc_cache[slot].key.assign(h, in);
     ctx->bc_cache[slot].used = ++ctx->bc_clock;
     ctx->bc_cache[slot].valid = true;
     return XG_OK;

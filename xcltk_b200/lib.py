@@ -164,6 +164,7 @@ SYMBOLS = {
     "xg_free_array": (None, [_P]),
     "xg_bam_block_probe": (C.c_int, [C.c_char_p, C.c_int64, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "xg_last_timing": (None, [_P, C.POINTER(C.c_double)]),
+    "xg_basefc_finalize_stats": (C.c_int, [_P, c_i64p]),
     "xg_version": (C.c_char_p, []),
 }
 
@@ -598,6 +599,14 @@ class Context(object):
         t = (C.c_double * 16)()
         self.lib.xg_last_timing(self.h, t)
         return list(t)
+
+    def basefc_finalize_stats(self):
+        """Route counters of the segment finalize in the last basefc call (xg_basefc_finalize_stats):
+        {"ordinary" / "big": {"heavy", "careful", "fast_overflow", "doubled"}}."""
+        out = np.zeros(8, dtype=np.int64)
+        self._check(self.lib.xg_basefc_finalize_stats(self.h, as_ptr(out, c_i64p)))
+        names = ("heavy", "careful", "fast_overflow", "doubled")
+        return {cta: dict(zip(names, out[k:k + 4].tolist())) for cta, k in (("ordinary", 0), ("big", 4))}
 
     def _basefc(self, entry, reads, gid, beg, end, cell_keys, n_samples, params, segments):
         gid = np.ascontiguousarray(gid, dtype=np.int32)
