@@ -353,6 +353,38 @@ int xg_snp_pileup(xg_ctx *ctx, const xg_dreads *reads, const xg_snps *snps, cons
                   const xg_params *par, const xg_snp_filter *filt, int64_t *totals /* may be NULL */,
                   uint8_t *keep_out /* may be NULL */, xg_coo **ad, xg_coo **dp, xg_coo **oth);
 
+/* SNP discovery (cellsnp-lite's mode without a candidate list; the reference has no such mode): every 0-based
+ * position p in [beg, end) of every target (targets->n entries {gid, beg, end}; gid < 0 or end <= beg: skipped;
+ * targets of one contig must not overlap, else XG_E_ARG) is a possible site.  Its totals are exactly plp_snp's for a
+ * SNP at p (baf/fc/core.py:198-247), i.e. what xg_baf_pileup writes: check_read, a listed cell (or the BAM's column in
+ * sample mode), a UMI key, the first read per (cell, UMI) in file order wins even when its allele is None, and the
+ * winners with an allele count into A / C / G / T / N.  REF is the A..T bucket with the largest count, ALT the one
+ * with the second largest (ties to the lower index in A < C < G < T; N is never REF or ALT).  A site is kept iff
+ * ALT >= 1, sum >= min_count and ALT >= sum * min_maf (plp_snp's filter, baf/fc/core.py:238-246, in IEEE double).
+ * The reads' aligned bases are first counted per position without the UMI collapse; positions whose raw counts
+ * cannot pass (raw sum < min_count, or fewer than two A..T buckets with max(1, min_count * min_maf) bases) are
+ * dropped, the others go through xg_baf_pileup (in slices when one slice exceeds its limits) and the filter.
+ * *out: the kept sites in target order, then by position, with their totals (n x 5: A C G T N) and the allele
+ * indices (0..3 = A C G T); library-owned host memory, release with xg_sites_free.
+ * xg_last_timing: [0] device span  [1] raw scan  [2] launches  [3] exact stage  [5] windows with reads
+ * [6] positions scanned (the positions of those windows)  [7] raw candidates  [11] pileup slices
+ * [12] host ms of the call  [13] (read, window) entries  [14] kept sites.
+ * xg_set_option(ctx, "discover_slice", n): at most n candidates per pileup slice (0: the default, 2^22).        */
+typedef struct {
+    double min_count, min_maf;
+} xg_discover_filter;
+typedef struct {
+    int64_t n;
+    const int32_t *gid;
+    const int32_t *pos;        /* 0-based */
+    const uint8_t *ref;
+    const uint8_t *alt;
+    const int64_t *totals;     /* n x 5 */
+} xg_sites;
+int xg_snp_discover(xg_ctx *ctx, const xg_dreads *reads, const xg_features *targets, const xg_barcodes *cells,
+                    const xg_params *par, const xg_discover_filter *filter, xg_sites **out);
+void xg_sites_free(xg_sites *sites);
+
 /* Synthetic 10x-style records generated directly in HBM (bench / tests; no reference
  * counterpart -- SURVEY.md 8(d) C3 allows device-side generation for kernel-only runs).  */
 typedef struct {
@@ -378,6 +410,11 @@ typedef struct {
      * hold one genomic chunk of ONE library                                                   */
     int64_t first_read;
     int64_t total_reads;
+    /* pseudo_ref != 0: aligned bases away from the SNP table are a seeded pseudo-reference base of (gid, pos), each
+     * replaced by one of the other three bases with probability ref_error (so that SNP discovery has a background
+     * to find sites in); 0: pseudo-random bases, as without these fields                                       */
+    int32_t pseudo_ref;
+    double ref_error;
 } xg_synth_params;
 int xg_synth_reads(xg_ctx *ctx, const xg_synth_params *p, xg_dreads **out, uint64_t *barcode_keys);
 /* Index of the first read at or after (gid, pos) in the library of p->n_reads reads (host only). */

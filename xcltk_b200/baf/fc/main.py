@@ -273,13 +273,11 @@ def _count_shard(conf, batch, regs, snps):
     return out, [ctx.timing()], None
 
 
-def count_units(conf, chroms, unit_chrom, unit_beg, unit_end, count, batch=None):
-    """Device counting of independent units (regions, or single SNPs) with one read batch per GPU.
-    unit_chrom / unit_beg / unit_end: contig (None: never fetched) and 0-based [beg, end) of every unit;
-    count(batch, idx) -> ((ad, dp, oth), timings, per_unit) counts the units `idx` on one batch, the rows of its
-    matrices indexing idx, per_unit an array over idx or None.  With several GPUs the units are cut into contiguous
-    genomic chunks, no collective.  Returns the three (row, col, val, shape) tuples in unit order and the
-    [(idx, per_unit)] of the shards."""
+def shard_units(conf, chroms, unit_chrom, unit_beg, unit_end, run, batch=None):
+    """Device work on independent units (regions, single SNPs, genomic windows) with one read batch per GPU.
+    unit_chrom / unit_beg / unit_end: contig (None: never fetched) and 0-based [beg, end) of every unit; run(batch,
+    idx) works on the units `idx` of one batch.  With several GPUs the units are cut into contiguous genomic chunks,
+    no collective.  Returns ([(idx, run(batch, idx), or None for a chunk without reads or units)], sharded)."""
     from ... import parallel
     n_unit = len(unit_beg)
     n_dev = parallel.n_devices(getattr(conf, "n_gpus", None))
@@ -296,7 +294,6 @@ def count_units(conf, chroms, unit_chrom, unit_beg, unit_end, count, batch=None)
             batch = engine.load_reads(conf.sam_fn_list, chroms, conf.cell_tag, conf.umi_tag, True, threads,
                                       mapped=True)
     try:
-        shape = (n_unit, len(conf.samples))
         if isinstance(batch, (engine.ShardedBatch, engine.MultiBatch)):
             if isinstance(batch, engine.ShardedBatch):
                 shards = batch.shards
@@ -310,26 +307,41 @@ def count_units(conf, chroms, unit_chrom, unit_beg, unit_end, count, batch=None)
             def one(k):
                 b = batch.batches[k]
                 if b is None or len(shards[k]) == 0:
-                    z = np.zeros(0, np.int32)
-                    return ((z, z, z, shape),) * 3, [[0.0] * 16, [0.0] * 16], None
-                return count(b, shards[k])
-            parts = parallel.run_on_devices(len(shards), one)
-            out = []
-            for w in range(3):
-                r, c, v = parallel.merge_coo([[np.array(x) for x in p[0][w][:3]] for p in parts], shards, n_unit)
-                out.append((r, c, v, shape))
-            out = tuple(out)
-            conf.last_timing = parts[0][1]
-            per_unit = [(idx, p[2]) for idx, p in zip(shards, parts) if p[2] is not None]
+                    return None
+                return run(b, shards[k])
+            res = list(zip(shards, parallel.run_on_devices(len(shards), one))), True
         else:
             idx = np.arange(n_unit, dtype=np.int64)
-            out, conf.last_timing, pu = count(batch, idx)
-            per_unit = [] if pu is None else [(idx, pu)]
+            res = [(idx, run(batch, idx))], False
         conf.last_stats = dict(batch.stats)
     finally:
         if own:
             batch.close()
-    return out, per_unit
+    return res
+
+
+def count_units(conf, chroms, unit_chrom, unit_beg, unit_end, count, batch=None):
+    """Device counting of independent units (regions, or single SNPs) with one read batch per GPU (shard_units).
+    count(batch, idx) -> ((ad, dp, oth), timings, per_unit) counts the units `idx` on one batch, the rows of its
+    matrices indexing idx, per_unit an array over idx or None.  Returns the three (row, col, val, shape) tuples in
+    unit order and the [(idx, per_unit)] of the shards."""
+    from ... import parallel
+    n_unit = len(unit_beg)
+    shape = (n_unit, len(conf.samples))
+    res, sharded = shard_units(conf, chroms, unit_chrom, unit_beg, unit_end, count, batch)
+    if not sharded:
+        idx, (out, conf.last_timing, pu) = res[0]
+        return out, ([] if pu is None else [(idx, pu)])
+    z = np.zeros(0, np.int32)
+    shards = [idx for idx, _ in res]
+    parts = [p if p is not None else (((z, z, z, shape),) * 3, [[0.0] * 16, [0.0] * 16], None) for _, p in res]
+    out = []
+    for w in range(3):
+        r, c, v = parallel.merge_coo([[np.array(x) for x in p[0][w][:3]] for p in parts], shards, n_unit)
+        out.append((r, c, v, shape))
+    conf.last_timing = parts[0][1]
+    per_unit = [(idx, p[2]) for idx, p in zip(shards, parts) if p[2] is not None]
+    return tuple(out), per_unit
 
 
 def count_regions(conf, regs, batch=None):

@@ -105,7 +105,8 @@ struct xg_ctx {
     cudaStream_t stream = nullptr;
     cudaStream_t copy_stream = nullptr;    // xg_basefc_host: H2D of the next epoch
     cudaStream_t d2h_stream = nullptr;     // basefc rows layouts: result rows copied out while later epochs run
-    int64_t fx_nnz_hint = 0;               // nnz of the last basefc call (sizes the pinned result up front)
+    int64_t fx_nnz_hint = 0;
+    int64_t discover_slice = 0;            // xg_snp_discover: candidates per pileup slice (0: the default)               // nnz of the last basefc call (sizes the pinned result up front)
     // the rows of the last basefc call with a rows layout are still in the staging area (scratch "fx_st_col" /
     // "fx_st_val", places in "fx_seg_base" / "fx_seg_nnz") until the next call: xg_basefc_write_mtx_device formats them
     bool fx_res_valid = false;

@@ -82,6 +82,11 @@ int xg_set_option(xg_ctx *ctx, const char *name, int64_t value) {
         ctx->stream = st;
         return XG_OK;
     }
+    if (std::string(name) == "discover_slice") {
+        if (value < 0) return ctx->fail(XG_E_ARG, "discover_slice must be >= 0");
+        ctx->discover_slice = value;
+        return XG_OK;
+    }
     return ctx->fail(XG_E_ARG, std::string("unknown option '") + name + "'");
 }
 

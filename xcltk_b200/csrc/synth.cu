@@ -31,6 +31,8 @@ struct SynthDev {
     const int32_t *snp_pos;
     const uint8_t *snp_ref, *snp_alt, *snp_ref_hap;
     int32_t n_gid;
+    int32_t pseudo_ref;              // bases of aligned query positions follow a pseudo-reference ...
+    uint32_t ref_err_ppm;            // ... except this many per million, which get another base
     // outputs
     int2 *pos_end;
     uint32_t *fmq, *cig_off, *cigar, *seq_off, *seq;
@@ -213,6 +215,35 @@ __global__ void __launch_bounds__(1024) k_synth_fill(const __grid_constant__ Syn
             uint32_t word = 0;
             for (int b = 0; b < 8; b++) word |= (1u << ((hb >> (2 * b)) & 3u)) << (4 * b);
             sq[wd] = word;
+        }
+        // pseudo-reference: an aligned base at (gid, p) is the library's base there, or with probability
+        // ref_err_ppm / 10^6 one of the other three; the SNP table below overrides its positions
+        if (P.pseudo_ref) {
+            int32_t p = pos, qi = 0;
+            for (int k = 0; k < (cp.n ? cp.n : 1); k++) {
+                uint32_t op = 0;
+                int32_t l = cp.rlen;
+                if (cp.n) {
+                    op = cp.w[k] & 15u;
+                    l = (int32_t)(cp.w[k] >> 4);
+                }
+                if (op == 0) {
+                    for (int32_t t = 0; t < l; t++) {
+                        const int32_t q = qi + t;
+                        uint32_t base = (uint32_t)hsh(P.seed, ((uint64_t)(uint32_t)gid << 32) | (uint32_t)(p + t), 10) & 3u;
+                        const uint64_t he = hsh(P.seed, gi * 4096 + (uint64_t)q, 11);
+                        if (he % 1000000u < P.ref_err_ppm) base = (base + 1u + (uint32_t)((he >> 32) % 3u)) & 3u;
+                        const uint32_t byte = (uint32_t)q >> 1, shift = 8 * (byte & 3u) + ((q & 1) ? 0u : 4u);
+                        sq[byte >> 2] = (sq[byte >> 2] & ~(15u << shift)) | ((1u << base) << shift);
+                    }
+                    p += l;
+                    qi += l;
+                } else if (op == 2 || op == 3) {
+                    p += l;
+                } else if (op == 1 || op == 4) {
+                    qi += l;
+                }
+            }
         }
         // haplotype-consistent bases at SNPs covered by aligned blocks
         if (P.n_snps > 0 && gid < P.n_gid) {
@@ -451,6 +482,8 @@ extern "C" int xg_synth_reads(xg_ctx *ctx, const xg_synth_params *sp, xg_dreads 
     P.snp_alt = d_snp_alt;
     P.snp_ref_hap = d_snp_rh;
     P.n_gid = n_gid;
+    P.pseudo_ref = sp->pseudo_ref;
+    P.ref_err_ppm = (uint32_t)std::min(1e6, std::max(0.0, sp->ref_error * 1e6 + 0.5));
     P.pos_end = d->pos_end;
     P.fmq = d->fmq;
     P.cig_off = d->cig_off;

@@ -91,7 +91,17 @@ class SynthParams(C.Structure):
                 ("n_spans", C.c_int32), ("span_gid", c_i32p), ("span_beg", c_i32p), ("span_end", c_i32p),
                 ("n_snps", C.c_int32), ("snp_gid", c_i32p), ("snp_pos", c_i32p),
                 ("snp_ref", c_u8p), ("snp_alt", c_u8p), ("snp_ref_hap", c_u8p),
-                ("first_read", C.c_int64), ("total_reads", C.c_int64)]
+                ("first_read", C.c_int64), ("total_reads", C.c_int64),
+                ("pseudo_ref", C.c_int32), ("ref_error", C.c_double)]
+
+
+class DiscoverFilter(C.Structure):
+    _fields_ = [("min_count", C.c_double), ("min_maf", C.c_double)]
+
+
+class Sites(C.Structure):
+    _fields_ = [("n", C.c_int64), ("gid", c_i32p), ("pos", c_i32p), ("ref", c_u8p), ("alt", c_u8p),
+                ("totals", c_i64p)]
 
 
 # every symbol include/xcltk_b200.h declares: name -> (restype, argtypes)
@@ -152,6 +162,9 @@ SYMBOLS = {
     "xg_snp_pileup": (C.c_int, [_P, _P, C.POINTER(Snps), C.POINTER(Barcodes), C.POINTER(Params), C.POINTER(SnpFilter),
                                 c_i64p, c_u8p, C.POINTER(C.POINTER(Coo)), C.POINTER(C.POINTER(Coo)),
                                 C.POINTER(C.POINTER(Coo))]),
+    "xg_snp_discover": (C.c_int, [_P, _P, C.POINTER(Features), C.POINTER(Barcodes), C.POINTER(Params),
+                                  C.POINTER(DiscoverFilter), C.POINTER(C.POINTER(Sites))]),
+    "xg_sites_free": (None, [C.POINTER(Sites)]),
     "xg_synth_reads": (C.c_int, [_P, C.POINTER(SynthParams), C.POINTER(_P), c_u64p]),
     "xg_synth_read_index": (C.c_int64, [C.POINTER(SynthParams), C.c_int32, C.c_int32]),
     "xg_write_bam": (C.c_int, [C.c_char_p, C.POINTER(Reads), C.c_int32, C.POINTER(C.c_char_p), c_i64p, _P,
@@ -736,9 +749,40 @@ class Context(object):
             out += (keep,)
         return out
 
+    def snp_discover(self, dreads, gid, beg, end, cell_keys, n_samples, params, min_count, min_maf):
+        """SNP discovery on the targets [beg, end) of contigs gid (xg_snp_discover).  Returns a dict of numpy arrays
+        over the kept sites in target order, then by position: gid, pos (0-based), ref, alt (0..3 = A C G T) and
+        totals (n x 5, A C G T N).  timing() then holds the stage times and the counts of the two stages."""
+        gid = np.ascontiguousarray(gid, dtype=np.int32)
+        beg = np.ascontiguousarray(beg, dtype=np.int32)
+        end = np.ascontiguousarray(end, dtype=np.int32)
+        if len(beg) != len(gid) or len(end) != len(gid):
+            raise ValueError("snp_discover: target arrays of different lengths")
+        keys = np.ascontiguousarray(cell_keys if cell_keys is not None else [], dtype=np.uint64)
+        t = Features(len(gid), as_ptr(gid, c_i32p), as_ptr(beg, c_i32p), as_ptr(end, c_i32p))
+        b = Barcodes(len(keys), as_ptr(keys, c_u64p), n_samples)
+        f = DiscoverFilter(float(min_count), float(min_maf))
+        out = C.POINTER(Sites)()
+        self._check(self.lib.xg_snp_discover(self.h, dreads.h, C.byref(t), C.byref(b), C.byref(params.c), C.byref(f),
+                                             C.byref(out)))
+        try:
+            s = out.contents
+            n = int(s.n)
+            res = {"gid": np_view(s.gid, n, np.int32).copy(), "pos": np_view(s.pos, n, np.int32).copy(),
+                   "ref": np_view(s.ref, n, np.uint8).copy(), "alt": np_view(s.alt, n, np.uint8).copy(),
+                   "totals": np_view(s.totals, 5 * n, np.int64).copy().reshape(n, 5)}
+        finally:
+            self.lib.xg_sites_free(out)
+        return res
+
+    def set_option(self, name, value):
+        self._check(self.lib.xg_set_option(self.h, name.encode(), int(value)))
+
     def synth_reads(self, n_reads, n_cells, span_gid, span_beg, span_end, seed=7, read_len=91,
-                    want_seq=False, snps=None, first_read=0, total_reads=0):
-        """total_reads > 0: only reads [first_read, first_read + n_reads) of a library of total_reads."""
+                    want_seq=False, snps=None, first_read=0, total_reads=0, ref_error=None):
+        """total_reads > 0: only reads [first_read, first_read + n_reads) of a library of total_reads.
+        ref_error not None: aligned bases away from `snps` follow a seeded pseudo-reference, each replaced by another
+        base with probability ref_error."""
         sg = np.ascontiguousarray(span_gid, dtype=np.int32)
         sb = np.ascontiguousarray(span_beg, dtype=np.int32)
         se = np.ascontiguousarray(span_end, dtype=np.int32)
@@ -746,6 +790,8 @@ class Context(object):
         p.n_reads, p.n_cells, p.read_len, p.want_seq, p.seed = n_reads, n_cells, read_len, int(want_seq), seed
         p.n_spans, p.span_gid, p.span_beg, p.span_end = len(sg), as_ptr(sg, c_i32p), as_ptr(sb, c_i32p), as_ptr(se, c_i32p)
         p.first_read, p.total_reads = int(first_read), int(total_reads)
+        if ref_error is not None:
+            p.pseudo_ref, p.ref_error = 1, float(ref_error)
         keep = [sg, sb, se]
         if snps is not None:
             arrs = [np.ascontiguousarray(snps[0], dtype=np.int32), np.ascontiguousarray(snps[1], dtype=np.int32)] + \

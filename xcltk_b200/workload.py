@@ -178,8 +178,10 @@ def make_basefc_workload(ctx, n_reads, n_cells, n_features=33472, seed=7, chroms
     return w
 
 
-def make_baf_workload(ctx, n_reads, n_cells, n_snps=200000, seed=7, chroms=None, part=None, snp_seed=None):
+def make_baf_workload(ctx, n_reads, n_cells, n_snps=200000, seed=7, chroms=None, part=None, snp_seed=None,
+                      ref_error=None):
     """Config 2: chr1-22 reads, 5k cells, 200k phased het SNPs inside gene spans.
+    ref_error not None: the bases away from the SNPs follow a pseudo-reference with this error rate (SNP discovery).
     part = (rank, world): the regions of that genomic chunk (w.feat_index: their rows in the whole matrices),
     the whole SNP table, and the reads that can overlap the chunk's regions."""
     w = Workload()
@@ -205,16 +207,18 @@ def make_baf_workload(ctx, n_reads, n_cells, n_snps=200000, seed=7, chroms=None,
     snps = (w.snp_gid, w.snp_pos, w.snp_ref, w.snp_alt, w.snp_ref_hap)
     if part is None:
         w.feat_index = np.arange(len(w.gid))
-        w.dreads, w.cell_keys = ctx.synth_reads(n_reads, n_cells, sg, sb, se, seed=seed, want_seq=True, snps=snps)
+        w.dreads, w.cell_keys = ctx.synth_reads(n_reads, n_cells, sg, sb, se, seed=seed, want_seq=True, snps=snps,
+                                                ref_error=ref_error)
         w.n_reads = n_reads
     else:
         idx, i0, n_loc = genomic_chunk(ctx, n_reads, seed, sg, sb, se, w.gid, w.beg, w.end, part)
         w.feat_index, w.first_read = idx, i0
         w.gid, w.beg, w.end = w.gid[idx], w.beg[idx], w.end[idx]
         w.dreads, w.cell_keys = ctx.synth_reads(max(1, n_loc), n_cells, sg, sb, se, seed=seed, want_seq=True,
-                                                snps=snps, first_read=i0, total_reads=n_reads)
+                                                snps=snps, first_read=i0, total_reads=n_reads, ref_error=ref_error)
         w.n_reads = n_loc
     w.n_cells = n_cells
+    w.contigs = auto
     w.params = engine.make_params(Conf(), 91, with_include=False)
     # region -> SNP lists (start0 <= pos0 < end0), hap table
     order = np.lexsort((w.snp_pos, w.snp_gid))

@@ -16,7 +16,8 @@ Commands:
      basefc           Basic feature counting (GPU).
 
   -- BAF calculation
-     pileup           SNP-level allele counting at candidate SNPs (GPU): cellSNP.* output.
+     pileup           SNP-level allele counting at candidate SNPs, or at sites discovered from the
+                      reads when no -P is given (GPU): cellSNP.* output.
      (feature-level allele counting is a Python API: xcltk_b200.baf.fc.main.afc_wrapper;
       the `baf` pipeline around it -- genotyping, Eagle2 -- stays in the reference)
 
