@@ -318,3 +318,189 @@ int orc_snp_discover(const xg_reads *r, int32_t n_tg, const int32_t *tg_gid, con
     if (err) orc_sites_free(out);
     return err;
 }
+
+/* ============================== raw scan mirror ===========================================
+ * orc_disc_raw: the counters the device's raw scan (k_disc_route / k_disc_hist) reports, restated per read on the
+ * CPU so that a test can compare them exactly -- timing()[5] covered windows, [6] positions scanned, [13] (read,
+ * window) entries, [7] raw candidates.  Separate from orc_snp_discover on purpose: that oracle defines the sites
+ * without any pre-filter; this one pins what the pre-filter looks at, so that over-counting (a read routed twice,
+ * a histogram left over from a CTA's previous window) and under-counting show even where no site changes.
+ *
+ * The contract it follows (discover.cu):
+ *   a read counts   check_read's flags, a stored SEQ, a UMI key that is neither none nor empty, a listed cell in
+ *                   barcode mode, aligned length >= min_len
+ *   a read enters   its [pos, end) meets a live target of its contig (live: 0 <= gid < 1 + the largest gid of a
+ *                   run, beg >= 0, end > beg); an unmapped read has end = pos + 1 but all its blocks are walked
+ *   windows         DISC_W positions from each live target's beg, numbered in caller order; a read adds one entry
+ *                   per distinct window its aligned (M / = / X) blocks touch
+ *   counters        covered = windows with an entry; scanned = their lengths inside their targets; a position of a
+ *                   covered window is a candidate iff raw A+C+G+T+N >= t_sum and the second largest of A..T >= t_alt,
+ *                   the raw count being the entering reads with an aligned base there (code 1/2/4/8 A/C/G/T, else N)
+ *   thresholds      t_sum = ceil(min_count), t_alt = max(1, ceil(min_count * min_maf)) with the product in double
+ * out[4] = {covered windows, positions scanned, entries, raw candidates}.  Returns 0, -1 (out of memory) or -2
+ * (overlapping live targets of one contig, or reads without sequences: the device rejects both). */
+#define ORC_DISC_W 2048
+
+static uint64_t orc_ceil_count(double v) {
+    if (!(v > 0)) return 0;
+    if (v >= 1e18) return 1000000000000000000ull;
+    uint64_t c = (uint64_t)v;
+    return (double)c < v ? c + 1 : c;
+}
+
+typedef struct {
+    int32_t beg, end, win0;
+} orc_tg;
+
+static int orc_tg_cmp(const void *a, const void *b) {
+    const orc_tg *x = (const orc_tg *)a, *y = (const orc_tg *)b;
+    return x->beg < y->beg ? -1 : x->beg > y->beg;
+}
+
+int orc_disc_raw(const xg_reads *r, int32_t n_tg, const int32_t *tg_gid, const int32_t *tg_beg, const int32_t *tg_end,
+                 int32_t n_bc, const uint64_t *bc_keys, const orc_params *c, double min_count, double min_maf,
+                 int64_t *out) {
+    memset(out, 0, 4 * sizeof(int64_t));
+    if (!r->seq_off || !r->seq) return -2;
+    int32_t n_gid = 0;
+    for (int32_t k = 0; k < r->n_runs; k++)
+        if (r->runs[k].gid + 1 > n_gid) n_gid = r->runs[k].gid + 1;
+    /* live targets: windows in caller order, then per contig sorted by beg */
+    int64_t n_win = 0;
+    int32_t *cnt = (int32_t *)calloc((size_t)n_gid + 1, 4);
+    orc_tg *all = (orc_tg *)malloc(((size_t)n_tg + 1) * sizeof(orc_tg));
+    int32_t *gof = (int32_t *)calloc((size_t)n_gid + 2, 4);
+    if (!cnt || !all || !gof) {
+        free(cnt), free(all), free(gof);
+        return -1;
+    }
+    for (int32_t t = 0; t < n_tg; t++) {
+        int32_t g = tg_gid[t], b = tg_beg[t], e = tg_end[t];
+        if (!(g >= 0 && g < n_gid && b >= 0 && e > b)) continue;
+        cnt[g]++;
+        n_win += ((int64_t)e - b + ORC_DISC_W - 1) / ORC_DISC_W;
+    }
+    for (int32_t g = 0; g < n_gid; g++) gof[g + 1] = gof[g] + cnt[g];
+    memset(cnt, 0, (size_t)n_gid * 4);
+    int64_t w_at = 0;
+    for (int32_t t = 0; t < n_tg; t++) {
+        int32_t g = tg_gid[t], b = tg_beg[t], e = tg_end[t];
+        if (!(g >= 0 && g < n_gid && b >= 0 && e > b)) continue;
+        orc_tg *x = &all[gof[g] + cnt[g]++];
+        x->beg = b;
+        x->end = e;
+        x->win0 = (int32_t)w_at;
+        w_at += ((int64_t)e - b + ORC_DISC_W - 1) / ORC_DISC_W;
+    }
+    int err = 0;
+    for (int32_t g = 0; g < n_gid; g++) {
+        qsort(all + gof[g], (size_t)(gof[g + 1] - gof[g]), sizeof(orc_tg), orc_tg_cmp);
+        for (int32_t k = gof[g] + 1; k < gof[g + 1]; k++)
+            if (all[k - 1].end > all[k].beg) err = -2;
+    }
+    int64_t *entries = (int64_t *)calloc((size_t)n_win + 1, 8);
+    uint32_t **hist = (uint32_t **)calloc((size_t)n_win + 1, sizeof(uint32_t *));
+    int32_t *wbeg = (int32_t *)malloc(((size_t)n_win + 1) * 4), *wlen = (int32_t *)malloc(((size_t)n_win + 1) * 4);
+    bc_dict bc;
+    memset(&bc, 0, sizeof(bc));
+    if (!entries || !hist || !wbeg || !wlen || (c->use_cell_tag && bc_build(&bc, n_bc, bc_keys))) err = err ? err : -1;
+    for (int32_t k = 0; k < gof[n_gid] && !err; k++)
+        for (int32_t w = 0; (int64_t)all[k].beg + (int64_t)w * ORC_DISC_W < all[k].end; w++) {
+            int32_t s = all[k].beg + w * ORC_DISC_W;
+            wbeg[all[k].win0 + w] = s;
+            wlen[all[k].win0 + w] = (all[k].end - s < ORC_DISC_W) ? all[k].end - s : ORC_DISC_W;
+        }
+    for (int32_t k = 0; k < r->n_runs && !err; k++) {
+        const xg_run *run = &r->runs[k];
+        int32_t g = run->gid;
+        if (g < 0 || g >= n_gid || gof[g] == gof[g + 1]) continue;
+        const orc_tg *T = all + gof[g];
+        int32_t nt = gof[g + 1] - gof[g];
+        for (int64_t i = run->rec_beg; i < run->rec_end && !err; i++) {
+            int32_t pos = r->pos_end[2 * i], rend = r->pos_end[2 * i + 1];
+            int32_t t0 = 0;
+            while (t0 < nt && T[t0].end <= pos) t0++;
+            if (t0 >= nt || T[t0].beg >= rend) continue;                 /* meets no live target */
+            if (check_read_head(r, i, c) < 0 || r->seq_off[i] == 0xFFFFFFFFu) continue;
+            uint64_t umi = r->keys[2 * i + 1];
+            if (umi == XG_KEY_NONE || umi == XG_KEY_EMPTY) continue;
+            if (c->use_cell_tag && bc_get(&bc, r->keys[2 * i]) < 0) continue;
+            const uint32_t *wd;
+            uint32_t one, nops = rd_cigar(r, i, &wd, &one);
+            int32_t aln = 0;
+            for (uint32_t q = 0; q < nops; q++) {
+                uint32_t op = wd[q] & 15u;
+                if (op == 0 || op == 7 || op == 8) aln += (int32_t)(wd[q] >> 4);
+            }
+            if (aln < c->min_len) continue;
+            const uint8_t *seq = (const uint8_t *)(r->seq + r->seq_off[i]);
+            int32_t rp = pos, qp = 0;
+            int64_t last = -1;
+            for (uint32_t q = 0; q < nops && !err; q++) {
+                uint32_t op = wd[q] & 15u;
+                int32_t l = (int32_t)(wd[q] >> 4);
+                if (op == 0 || op == 7 || op == 8) {
+                    for (int32_t p = rp; p < rp + l; p++) {             /* every aligned base, one at a time */
+                        int32_t t = t0;
+                        while (t < nt && T[t].end <= p) t++;
+                        if (t >= nt || T[t].beg > p) continue;
+                        int64_t w = T[t].win0 + (p - T[t].beg) / ORC_DISC_W;
+                        if (w != last) {
+                            entries[w]++;
+                            last = w;
+                        }
+                        if (!hist[w] && !(hist[w] = (uint32_t *)calloc(5 * ORC_DISC_W, 4))) {
+                            err = -1;
+                            break;
+                        }
+                        int32_t qi = qp + (p - rp);
+                        uint8_t b = seq[qi >> 1], nib = (qi & 1) ? (b & 15) : (b >> 4);
+                        int bk = nib == 1 ? 0 : nib == 2 ? 1 : nib == 4 ? 2 : nib == 8 ? 3 : 4;
+                        hist[w][bk * ORC_DISC_W + (p - wbeg[w])]++;
+                    }
+                    rp += l;
+                    qp += l;
+                } else if (op == 2 || op == 3) {
+                    rp += l;
+                } else if (op == 1 || op == 4) {
+                    qp += l;
+                }
+            }
+        }
+    }
+    uint64_t t_sum = orc_ceil_count(min_count);
+    double prod = (min_count > 0 && min_maf > 0) ? min_count * min_maf : 0.0;
+    uint64_t t_alt = orc_ceil_count(prod);
+    if (t_alt < 1) t_alt = 1;
+    for (int64_t w = 0; w < n_win && !err; w++) {
+        if (!entries[w]) continue;
+        out[0]++;
+        out[1] += wlen[w];
+        out[2] += entries[w];
+        for (int32_t b = 0; b < wlen[w]; b++) {
+            uint64_t v[5], sum = 0;
+            for (int k = 0; k < 5; k++) sum += v[k] = hist[w][k * ORC_DISC_W + b];
+            uint64_t m1 = 0, m2 = 0;                                      /* largest and second largest of A..T */
+            for (int k = 0; k < 4; k++) {
+                if (v[k] > m1) {
+                    m2 = m1;
+                    m1 = v[k];
+                } else if (v[k] > m2) {
+                    m2 = v[k];
+                }
+            }
+            out[3] += sum >= t_sum && m2 >= t_alt;
+        }
+    }
+    for (int64_t w = 0; hist && w < n_win; w++) free(hist[w]);
+    free(hist);
+    free(entries);
+    free(wbeg);
+    free(wlen);
+    free(cnt);
+    free(all);
+    free(gof);
+    free(bc.keys);
+    free(bc.cols);
+    return err;
+}

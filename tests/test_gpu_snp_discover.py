@@ -190,7 +190,7 @@ def test_empty_batch_and_target_without_reads(gpu_ctx):
 
 def test_synthetic_3m_pseudo_reference(gpu_ctx):
     """3M device-synthesised reads over a pseudo-reference with 0.1 % errors and 300 planted SNPs: every planted
-    SNP with enough depth is found, and the site set equals the oracle's."""
+    SNP with enough depth is found, the site set equals the oracle's and the raw counters equal orc_disc_raw's."""
     from oracle import oracle
     rng = np.random.RandomState(9)
     span = (np.array([0], np.int32), np.array([0], np.int32), np.array([2000000], np.int32))
@@ -211,6 +211,9 @@ def test_synthetic_3m_pseudo_reference(gpu_ctx):
     exp = discover_oracle.orc_snp_discover(host, [0], [0], [2000000], bk, oracle.params(conf), 20, 0.1)
     for k in ("gid", "pos", "ref", "alt", "totals"):
         assert np.array_equal(got[k], exp[k]), k
+    # the raw scan's covered windows, positions scanned, entries and candidates equal their mirror's
+    raw = discover_oracle.orc_disc_raw(host, [0], [0], [2000000], bk, oracle.params(conf), 20, 0.1)
+    assert discover_oracle.raw_counters(t) == raw and raw[0] == -(-2000000 // W)
     found = set(got["pos"].tolist())
     assert t[7] < t[6] / 100 and t[14] <= t[7]        # the pre-filter pruned the background
     deep = [p for p in sp.tolist() if p in found]

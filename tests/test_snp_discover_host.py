@@ -191,3 +191,148 @@ def test_ctypes_mirrors_match_the_header(tmp_path):
         assert int(got[cname]) == C.sizeof(py), cname
         for f, _t in py._fields_:
             assert int(got["%s.%s" % (cname, f)]) == getattr(py, f).offset, (cname, f)
+
+
+# ---- the raw-scan mirror (orc_disc_raw) against a plain per-read loop -------------------------------------------
+W = 2048                   # DISC_W of discover.cu
+
+
+def py_disc_raw(reads, tg, ck, conf, min_count, min_maf):
+    """The raw scan's counters restated read by read with sets and dicts: (covered windows, positions scanned,
+    (read, window) entries, raw candidates)."""
+    import math
+    a = reads._arrays
+    pe, fmq, keys = a["pos_end"].reshape(-1, 2), a["fmq"], a["keys"].reshape(-1, 2)
+    cig_off, cigar, seq_off, seq = a["cig_off"], a["cigar"], a["seq_off"], a["seq"].view(np.uint8)
+    none, empty = 0xFFFFFFFFFFFFFFFF, 0
+    n_gid = max(r[1] for r in reads.runs) + 1
+    live, n_win = [], 0                                  # (gid, beg, end, first window) in caller order
+    for g, b, e in zip(*tg):
+        if 0 <= g < n_gid and b >= 0 and e > b:
+            live.append((g, b, e, n_win))
+            n_win += -(-(e - b) // W)
+    listed = set(int(k) for k in ck) if conf.use_barcodes() else None
+    entries, hist = {}, {}
+    for _bam, gid, rb, re_ in reads.runs:
+        mine = [t for t in live if t[0] == gid]
+        for i in range(rb, re_):
+            pos, end = int(pe[i, 0]), int(pe[i, 1])
+            if not any(b < end and pos < e for _g, b, e, _w in mine):
+                continue
+            flag, mapq = int(fmq[i]) & 0xFFFF, (int(fmq[i]) >> 16) & 0xFF
+            if mapq < conf.min_mapq or (conf.excl_flag and flag & conf.excl_flag):
+                continue
+            if (conf.incl_flag and not flag & conf.incl_flag) or (conf.no_orphan and flag & 1 and not flag & 2):
+                continue
+            cell, umi = int(keys[i, 0]), int(keys[i, 1])
+            if seq_off[i] == 0xFFFFFFFF or umi in (none, empty) or (listed is not None and cell not in listed):
+                continue
+            n_ops = int(fmq[i]) >> 24
+            if n_ops == 0:
+                ops = [(0, end - pos)]
+            else:
+                o = int(cig_off[i])
+                k = int(cigar[o - 1]) if n_ops == 255 else n_ops
+                ops = [(int(w) & 15, int(w) >> 4) for w in cigar[o:o + k]]
+            if sum(l for op, l in ops if op in (0, 7, 8)) < conf.min_len:
+                continue
+            wins, rp, qp = set(), pos, 0
+            for op, l in ops:
+                if op in (0, 7, 8):
+                    for j in range(l):
+                        p, q = rp + j, qp + j
+                        for _g, b, e, w0 in mine:
+                            if b <= p < e:
+                                w = w0 + (p - b) // W
+                                wins.add(w)
+                                byte = int(seq[4 * int(seq_off[i]) + (q >> 1)])
+                                nib = byte & 15 if q & 1 else byte >> 4
+                                c = hist.setdefault((w, p), [0] * 5)
+                                c[{1: 0, 2: 1, 4: 2, 8: 3}.get(nib, 4)] += 1
+                    rp += l
+                    qp += l
+                elif op in (2, 3):
+                    rp += l
+                elif op in (1, 4):
+                    qp += l
+            for w in wins:
+                entries[w] = entries.get(w, 0) + 1
+    t_sum = math.ceil(min_count) if min_count > 0 else 0
+    t_alt = max(1, math.ceil(min_count * min_maf)) if min_count > 0 and min_maf > 0 else 1
+    scanned = 0
+    for _g, b, e, w0 in live:
+        for w in range(w0, w0 + -(-(e - b) // W)):
+            if w in entries:
+                s = b + (w - w0) * W
+                scanned += min(e, s + W) - s
+    cand = sum(1 for c in hist.values() if sum(c) >= t_sum and sorted(c[:4])[2] >= t_alt)
+    return len(entries), scanned, sum(entries.values()), cand
+
+
+def mixed_batch(seed, n, contig_len):
+    """Random exotic CIGARs on two contigs with every filter's failing values mixed in: flags (unmapped, orphan,
+    duplicate), low mapq, short reads, unlisted / missing cells, none / empty UMIs, records without SEQ.  Unmapped
+    reads end at pos + 1 but keep their CIGAR."""
+    from test_gpu_baf_edges import exotic, random_codes
+    from recsets import query_len
+    rng = np.random.RandomState(seed)
+    ops = [exotic(rng) for _ in range(n)]
+    gid = (rng.rand(n) < 0.4).astype(np.int64)
+    pos = rng.randint(0, contig_len, size=n)
+    order = np.lexsort((pos, gid))
+    gid, pos, ops = gid[order], pos[order], [ops[k] for k in order]
+    ln = rng.randint(1, 120, size=n)
+    seq = [None if rng.rand() < 0.03 else random_codes(rng, query_len(o) if o else int(l)) for o, l in zip(ops, ln)]
+    ck = cell_keys(12)
+    cell = np.concatenate([ck, cell_keys(3, salt=100), [0xFFFFFFFFFFFFFFFF]])[rng.randint(0, 16, size=n)]
+    umi = umi_keys(200)[rng.randint(0, 200, size=n)]
+    umi[rng.rand(n) < 0.03] = 0xFFFFFFFFFFFFFFFF
+    umi[rng.rand(n) < 0.03] = 0
+    flag = rng.choice([0, 0, 0, 4, 1, 3, 1024, 16], size=n).astype(np.uint32)
+    mapq = rng.choice([60, 20, 19, 0], size=n).astype(np.uint32)
+    h = int((gid == 0).sum())
+    reads = build(pos, cell.astype(np.uint64), umi, [(0, 0, 0, h), (0, 1, h, n)], end=pos + ln, ops=ops, seq=seq,
+                  flag=flag, mapq=mapq)
+    un = np.nonzero(flag & 4)[0]
+    reads.pos_end[un, 1] = reads.pos_end[un, 0] + 1
+    return reads, ck
+
+
+MIRROR_TARGETS = [
+    ([0], [0], [9000]),
+    ([1, -1, 0, 0, 5, 0, 1], [4000, 0, 3071, 1000, 0, 7000, 0], [9000, 50, 7000, 3071, 100, 6000, 4000]),
+    ([0, 0, 1, 0], [2047, 2049, 1, 8191], [2048, 4097, 2, 8200]),
+]
+
+
+@pytest.mark.parametrize("tg", range(len(MIRROR_TARGETS)))
+def test_raw_scan_mirror_against_a_per_read_loop(tg):
+    """orc_disc_raw (C) equals a per-read Python restatement on the CIGAR panel with the 301-op read, and on a
+    mixed batch of exotic CIGARs and failing filters; targets starting mid-window, of length 1, adjacent, on two
+    contigs out of order, and skipped (gid -1, gid past the last contig, end <= beg)."""
+    from oracle import oracle
+    from recsets import CIGAR_PANEL, cigar_panel
+    from test_gpu_baf_edges import WIDE
+    tgt = tuple(np.array(x, np.int32) for x in MIRROR_TARGETS[tg])
+    conf = Conf()
+    panel, pck = cigar_panel(CIGAR_PANEL + [WIDE])
+    mixed, mck = mixed_batch(4, 700, 9000)
+    seen = []
+    for reads, ck, mc, maf in ((panel, pck, 0, 0.0), (panel, pck, 2, 0.5), (mixed, mck, 0, 0.0),
+                               (mixed, mck, 3, 0.1), (mixed, mck, 2.5, 0.4)):
+        for c in (conf, type("C", (Conf,), {"min_mapq": 20, "min_len": 30, "excl_flag": 1024, "no_orphan": True,
+                                             "incl_flag": 0})()):
+            got = discover_oracle.orc_disc_raw(reads, *tgt, ck, oracle.params(c), mc, maf)
+            assert got == py_disc_raw(reads, tgt, ck, c, mc, maf), (mc, maf)
+            seen.append(got)
+    assert all(s[2] >= s[0] > 0 and s[3] > 0 for s in seen[4:])
+
+
+def test_raw_scan_mirror_rejects_what_the_device_rejects():
+    from oracle import oracle
+    reads, ck = column("AACC")
+    with pytest.raises(ValueError):          # [0, 50) and [40, 60) overlap
+        discover_oracle.orc_disc_raw(reads, [0, 0], [0, 40], [50, 60], ck, oracle.params(Conf()), 0, 0.0)
+    bare = build(np.zeros(2, np.int64), ck[0], umi_keys(2), [(0, 0, 0, 2)], end=np.full(2, 20))
+    with pytest.raises(ValueError):
+        discover_oracle.orc_disc_raw(bare, [0], [0], [50], ck, oracle.params(Conf()), 0, 0.0)
