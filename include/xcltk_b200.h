@@ -433,7 +433,8 @@ int xg_write_bam(const char *path, const xg_reads *reads, int32_t n_gid, const c
  * [0] device span of the call  [1] sum of the dominant counting kernel's launches
  * [2] kernel launches          [3] span of the epoch loop + gather (basefc)
  * [4] result D2H               [5] epochs (basefc)   [6] pool bytes / pairs   [7] staging entries
- * [8..11] host phases of xg_basefc (ms): index build, windows, plan, uploads; [12] whole call;
+ * [8..11] host phases of xg_basefc (ms): index build; windows and epoch plan (device kernels) until the plan's
+ * summary is back; allocation of the pool and the staging area; uploads (filters, barcode table); [12] whole call;
  * [13] bytes copied host -> device (xg_basefc_host); [14] / [15] features counted in segments / in sets.
  * xg_baf_*: [8..10] host milestones of the call (ms since entry).                                   */
 void xg_last_timing(xg_ctx *ctx, double out[16]);

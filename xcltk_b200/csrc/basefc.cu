@@ -209,159 +209,10 @@ __global__ void __launch_bounds__(256) k_feature_windows(const WinJob *jobs, int
 // cap > 0: a set (slots, cursor, log); cap == 0: a segment of log_cap 8-byte pair words
 #define SEG_TBL_SLOTS 4096                         // dedup table of the finalize CTAs (64-bit words)
 #define SEG_PART_WORDS (SEG_TBL_SLOTS * 2 / 5)     // a segment with more words is split by hash first
-static inline uint64_t plan_blk_bytes(uint32_t cap, uint32_t log_cap) {
+__host__ __device__ __forceinline__ uint64_t plan_blk_bytes(uint32_t cap, uint32_t log_cap) {
     // a segment that may have to be split carries a scratch half of the same size
     if (!cap) return ((((uint64_t)log_cap * 8) + 15) & ~15ull) * (log_cap > SEG_PART_WORDS ? 2 : 1);
     return (uint64_t)cap * 16 + 16 + ((((uint64_t)log_cap * 4) + 15) & ~15ull);
-}
-
-struct EpochPlan {
-    int32_t n_epochs = 0, epoch_tiles = 0;
-    std::vector<uint64_t> blk_off;      // per sorted feature: byte offset of its block
-    std::vector<uint32_t> tbl_cap;      // slots of its set (0 = segment feature, or never active)
-    std::vector<uint32_t> log_cap;      // candidate reads: entries of its log / pair words of its segment
-    uint64_t pool_bytes = 0;
-    std::vector<int32_t> zero_ptr, fin_ptr, fin_set_ptr, fin_big_ptr;    // per epoch ranges
-    std::vector<uint64_t> zseg_off, zseg_pre;
-    std::vector<int32_t> fin_feat, fin_set, fin_big;  // features ending in the epoch: segments / sets / big segments
-    int64_t staging_cap = 0;
-    int64_t n_seg_feat = 0, n_set_feat = 0;
-    // planner scratch
-    std::vector<int32_t> first_e, last_e, start_ptr, end_ptr, starts, ends, sc, ec;
-    std::vector<uint8_t> bucket_of;
-    std::vector<uint64_t> epoch_bytes;
-    // The plan object lives in the context and is reused from call to call: vectors of this size are mmap'ed
-    // afresh by every allocation, and the page faults of a new plan cost more than computing it.
-    void reset() {
-        n_epochs = epoch_tiles = 0;
-        pool_bytes = 0;
-        staging_cap = n_seg_feat = n_set_feat = 0;
-        for (auto *v : {&zero_ptr, &fin_ptr, &fin_set_ptr, &fin_big_ptr, &fin_feat, &fin_set, &fin_big}) v->clear();
-        zseg_off.clear();
-        zseg_pre.clear();
-    }
-};
-
-// seg_max: features with at most this many candidate reads collect pair words in a segment
-// (0: every feature keeps a set)
-// seg_big: a segment feature with more candidate reads is reduced by a CTA of FS_BIG_THREADS threads
-int make_plan(xg_ctx *ctx, const std::vector<unsigned long long> &cand, const std::vector<int32_t> &tlo,
-              const std::vector<int32_t> &thi, int32_t n_tiles, int32_t n_cols, int32_t epoch_tiles,
-              uint64_t seg_max, uint64_t seg_big, EpochPlan &pl) {
-    // The planner sits on the critical path of every call (the GPU waits for it): flat arrays and counting sorts,
-    // O(features), no per-epoch containers, no sort, no free list.
-    const size_t m = cand.size();
-    pl.epoch_tiles = epoch_tiles;
-    pl.n_epochs = std::max(1, (n_tiles + epoch_tiles - 1) / epoch_tiles);
-    const size_t ne = (size_t)pl.n_epochs;
-    pl.blk_off.assign(m, 0);
-    pl.tbl_cap.assign(m, 0);
-    pl.log_cap.assign(m, 0);
-    // first / last epoch of every active feature; features per first epoch and per (last epoch, log2 bucket)
-    std::vector<int32_t> &first_e = pl.first_e, &last_e = pl.last_e, &start_ptr = pl.start_ptr, &end_ptr = pl.end_ptr;
-    std::vector<uint8_t> &bucket_of = pl.bucket_of;
-    first_e.resize(m);
-    last_e.resize(m);
-    bucket_of.resize(m);
-    start_ptr.assign(ne + 1, 0);
-    end_ptr.assign(ne * 33 + 1, 0);
-    for (size_t j = 0; j < m; j++) {
-        const unsigned long long c = cand[j];
-        if (c == 0) {
-            first_e[j] = -1;
-            continue;
-        }
-        const unsigned long long cap = c + c / 4 + 8;
-        if (cap >= (1ull << 32)) return ctx->fail(XG_E_LIMIT, "feature window exceeds 2^32 reads");
-        if (c <= seg_max) {
-            pl.n_seg_feat++;
-        } else {
-            pl.tbl_cap[j] = (uint32_t)cap;
-            pl.n_set_feat++;
-        }
-        pl.log_cap[j] = (uint32_t)c;
-        pl.staging_cap += (int64_t)std::min<unsigned long long>(c, (unsigned long long)n_cols);
-        const int32_t fe = tlo[j] / epoch_tiles, le = (thi[j] - 1) / epoch_tiles;
-        first_e[j] = fe;
-        last_e[j] = le;
-        const int bk = std::min(63 - __builtin_clzll(c), 32);            // floor(log2(c)), c >= 1
-        bucket_of[j] = (uint8_t)bk;
-        start_ptr[(size_t)fe + 1]++;
-        end_ptr[(size_t)le * 33 + (size_t)(32 - bk) + 1]++;               // heavy buckets first within an epoch
-    }
-    for (size_t e = 0; e < ne; e++) start_ptr[e + 1] += start_ptr[e];
-    for (size_t k = 0; k < ne * 33; k++) end_ptr[k + 1] += end_ptr[k];
-    std::vector<int32_t> &starts = pl.starts, &ends = pl.ends;
-    starts.resize((size_t)start_ptr[ne]);
-    ends.resize((size_t)end_ptr[ne * 33]);
-    {
-        std::vector<int32_t> &sc = pl.sc, &ec = pl.ec;
-        sc.assign(start_ptr.begin(), start_ptr.end() - 1);
-        ec.assign(end_ptr.begin(), end_ptr.end() - 1);
-        for (size_t j = 0; j < m; j++) {
-            if (first_e[j] < 0) continue;
-            starts[(size_t)sc[(size_t)first_e[j]]++] = (int32_t)j;
-            ends[(size_t)ec[(size_t)last_e[j] * 33 + (size_t)(32 - bucket_of[j])]++] = (int32_t)j;
-        }
-    }
-    // Pool layout.  A block is needed from its feature's first epoch to the finalize of its last one, and
-    // zero(e) / count(e) are ordered after finalize(e-2): a feature that lives in one or two epochs takes its
-    // block from the arena of its first epoch -- three arenas in rotation, each as large as the busiest
-    // epoch -- and the few that live longer get a place of their own behind the arenas.
-    std::vector<uint64_t> &epoch_bytes = pl.epoch_bytes;
-    epoch_bytes.assign(ne, 0);
-    uint64_t long_bytes = 0;
-    for (size_t e = 0; e < ne; e++)
-        for (int32_t k = start_ptr[e]; k < start_ptr[e + 1]; k++) {
-            const size_t j = (size_t)starts[(size_t)k];
-            const uint64_t need = plan_blk_bytes(pl.tbl_cap[j], pl.log_cap[j]);
-            if (last_e[j] <= (int32_t)e + 1) {
-                pl.blk_off[j] = epoch_bytes[e];                     // offset inside the arena, for now
-                epoch_bytes[e] += need;
-            } else {
-                pl.blk_off[j] = long_bytes;
-                long_bytes += need;
-            }
-        }
-    uint64_t arena = 0;
-    for (uint64_t bts : epoch_bytes) arena = std::max(arena, bts);
-    arena = (arena + 255) & ~255ull;
-    const int n_arenas = std::min(3, pl.n_epochs);
-    pl.pool_bytes = arena * (uint64_t)n_arenas + long_bytes;
-    pl.zero_ptr.assign(ne + 1, 0);
-    pl.fin_ptr.assign(ne + 1, 0);
-    pl.fin_set_ptr.assign(ne + 1, 0);
-    pl.fin_big_ptr.assign(ne + 1, 0);
-    pl.fin_feat.reserve(ends.size());
-    for (size_t e = 0; e < ne; e++) {
-        uint64_t pre = 0;
-        for (int32_t k = start_ptr[e]; k < start_ptr[e + 1]; k++) {
-            const size_t j = (size_t)starts[(size_t)k];
-            const uint64_t off = pl.blk_off[j] + (last_e[j] <= (int32_t)e + 1 ? arena * (uint64_t)(e % (size_t)n_arenas)
-                                                                              : arena * (uint64_t)n_arenas);
-            pl.blk_off[j] = off;
-            if (pl.tbl_cap[j]) {                 // a set is zeroed before its first epoch; a segment only has a cursor
-                pl.zseg_off.push_back(off);
-                pl.zseg_pre.push_back(pre);
-                pre += (uint64_t)pl.tbl_cap[j] * 16 + 16;           // set + cursor
-            } else if (off / 16 >= 0xFFFFFFFFull) {
-                return ctx->fail(XG_E_LIMIT, "segment pool exceeds 64 GiB; use smaller epochs (XG_EPOCH_TILES)");
-            }
-        }
-        pl.zseg_pre.push_back(pre);      // terminator of the epoch: total bytes
-        pl.zseg_off.push_back(0);
-        pl.zero_ptr[e + 1] = (int32_t)pl.zseg_off.size();
-        // finalize order: heavy rows first (`ends` is bucketed by power of two), so that the persistent CTAs end
-        // closer together
-        for (int32_t k = end_ptr[e * 33]; k < end_ptr[(e + 1) * 33]; k++) {
-            const int32_t j = ends[(size_t)k];
-            (pl.tbl_cap[(size_t)j] ? pl.fin_set : cand[(size_t)j] > seg_big ? pl.fin_big : pl.fin_feat).push_back(j);
-        }
-        pl.fin_ptr[e + 1] = (int32_t)pl.fin_feat.size();
-        pl.fin_set_ptr[e + 1] = (int32_t)pl.fin_set.size();
-        pl.fin_big_ptr[e + 1] = (int32_t)pl.fin_big.size();
-    }
-    return XG_OK;
 }
 
 // ---- the counting kernel ------------------------------------------------------------------
@@ -388,17 +239,209 @@ struct __align__(16) FeatDesc {
     uint32_t cap, log_cap;
 };
 
+// ---- the epoch planner (device) ---------------------------------------------------------------
+// From every sorted feature's candidate reads and tile window (k_feature_windows) the planner decides, without a
+// round trip to the host: set or segment (big or not), the feature's block in the pool, and the per-epoch lists
+// of features to zero and to finalize.  Lists are counting sorts over one histogram of keys
+//   [kind k][last epoch e][32 - floor(log2 candidates)]   kind 0 segments, 1 sets, 2 big segments
+//   [first epoch e]                                       sets to zero before their first epoch
+// so that the finalize list of (k, e) is one range of a single array, heaviest rows first (the persistent finalize
+// CTAs end closer together); order inside a key is whatever the atomics made it.  Blocks: a feature that lives in
+// one or two epochs takes its block from the arena of its first epoch -- three arenas in rotation, each as large
+// as the busiest epoch, since zero(e) / count(e) are ordered after finalize(e-2) -- and the few that live longer
+// get a place of their own behind the arenas.  The host reads the summary only.
+#define PLAN_KEYS 33                               // log2 buckets of an epoch
+#define PLAN_SCAN_THREADS 1024
+struct PlanSummary {
+    unsigned long long pool_bytes, staging_cap;    // staging_cap = sum of min(candidates, columns)
+    unsigned long long n_seg_feat, n_set_feat, n_big_feat;
+    unsigned int err;                              // bit 0: a window of >= 2^32 reads; bit 1: segment pool >= 64 GiB
+    unsigned int pad;
+};
+struct PlanAcc {                                   // the planner's state of a call, zeroed before it starts
+    PlanSummary sum;
+    unsigned long long long_bytes, arena;
+};
+
+// atomicAdd(p, v) of the lanes with `on`, one atomic per distinct address of the warp; returns what a plain
+// atomicAdd would have returned in some order of the lanes.  Whole warp.
+template <class T>
+__device__ __forceinline__ T warp_add(bool on, T *p, T v) {
+    const unsigned act = __ballot_sync(0xffffffffu, on);
+    if (!on) return 0;
+    const unsigned peers = __match_any_sync(act, (unsigned long long)p);
+    const int lane = threadIdx.x & 31, leader = __ffs(peers) - 1;
+    T pre = 0, tot = 0;
+    for (unsigned q = peers; q; q &= q - 1) {
+        const int l = __ffs(q) - 1;
+        const T x = __shfl_sync(peers, v, l);
+        if (l < lane) pre += x;
+        tot += x;
+    }
+    T base = 0;
+    if (lane == leader) base = atomicAdd(p, tot);
+    return __shfl_sync(peers, base, leader) + pre;
+}
+
+// What the plan's rules make of one feature.
+struct PlanFeat {
+    bool on, set;                 // has candidates (and fits); keeps a set
+    uint32_t cap, log_cap;        // FeatDesc
+    int32_t fe, le;               // first / last epoch
+    int64_t fin_key;              // histogram key of its finalize
+};
+__device__ __forceinline__ PlanFeat plan_feat(unsigned long long c, int32_t tlo, int32_t thi, int32_t epoch_tiles,
+                                              int32_t n_epochs, uint64_t seg_max, uint64_t seg_big) {
+    PlanFeat f;
+    const unsigned long long cap = c + c / 4 + 8;
+    f.on = c != 0 && cap < (1ull << 32);
+    f.set = f.on && c > seg_max;
+    f.cap = f.set ? (uint32_t)cap : 0u;
+    f.log_cap = f.on ? (uint32_t)c : 0u;
+    f.fe = f.on ? tlo / epoch_tiles : 0;
+    f.le = f.on ? (thi - 1) / epoch_tiles : 0;
+    const int bk = f.on ? min(63 - __clzll((long long)c), 32) : 0;
+    const int kind = f.set ? 1 : c > seg_big ? 2 : 0;
+    f.fin_key = ((int64_t)kind * n_epochs + f.le) * PLAN_KEYS + (32 - bk);
+    return f;
+}
+
+// per feature: classify, count into the histogram, take a block of its first epoch's arena or of the long region
+__global__ void __launch_bounds__(256) k_plan_features(const unsigned long long *cand, const int32_t *tlo,
+                                                       const int32_t *thi, int32_t m, int32_t n_cols,
+                                                       int32_t epoch_tiles, int32_t n_epochs, uint64_t seg_max,
+                                                       uint64_t seg_big, PlanAcc *acc,
+                                                       unsigned long long *epoch_bytes, int32_t *hist,
+                                                       FeatDesc *fdesc, uint32_t *segoff16) {
+    const int32_t j = blockIdx.x * blockDim.x + threadIdx.x;         // no early exit: warp_add takes whole warps
+    const unsigned long long c = j < m ? cand[j] : 0ull;
+    const PlanFeat f = plan_feat(c, j < m ? tlo[j] : 0, j < m ? thi[j] : 0, epoch_tiles, n_epochs, seg_max, seg_big);
+    if (c != 0 && !f.on) atomicOr(&acc->sum.err, 1u);
+    typedef unsigned long long u64;
+    warp_add<u64>(f.on, &acc->sum.staging_cap, c < (u64)n_cols ? c : (u64)n_cols);
+    warp_add<u64>(f.on && !f.set, &acc->sum.n_seg_feat, 1ull);
+    warp_add<u64>(f.set, &acc->sum.n_set_feat, 1ull);
+    warp_add<u64>(f.on && !f.set && c > seg_big, &acc->sum.n_big_feat, 1ull);
+    warp_add<int32_t>(f.on, &hist[f.fin_key], 1);
+    warp_add<int32_t>(f.set, &hist[(int64_t)3 * n_epochs * PLAN_KEYS + f.fe], 1);
+    const u64 need = f.on ? plan_blk_bytes(f.cap, f.log_cap) : 0ull;
+    // offset inside the arena or the long region, for now
+    const u64 at = warp_add<u64>(f.on, f.le <= f.fe + 1 ? &epoch_bytes[f.fe] : &acc->long_bytes, need);
+    if (j < m) {
+        fdesc[j] = FeatDesc{at, f.cap, f.log_cap};
+        segoff16[j] = NO_SEG;
+    }
+}
+
+// Exclusive prefix sums over [0, n) in one CTA of PLAN_SCAN_THREADS threads: store(i, sum of load(0 .. i-1)).
+// Returns the total to every thread.
+template <class T, class Load, class Store>
+__device__ T cta_scan(int64_t n, Load load, Store store) {
+    __shared__ T wsum[PLAN_SCAN_THREADS / 32];
+    __shared__ T carry_s;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    T carry = 0;
+    for (int64_t b = 0; b < n; b += PLAN_SCAN_THREADS) {
+        const int64_t i = b + threadIdx.x;
+        const T v = i < n ? load(i) : (T)0;
+        T s = v;
+        for (int d = 1; d < 32; d <<= 1) {
+            const T y = __shfl_up_sync(0xffffffffu, s, d);
+            if (lane >= d) s += y;
+        }
+        if (lane == 31) wsum[w] = s;
+        __syncthreads();
+        if (w == 0) {
+            T t = wsum[lane];
+            for (int d = 1; d < 32; d <<= 1) {
+                const T y = __shfl_up_sync(0xffffffffu, t, d);
+                if (lane >= d) t += y;
+            }
+            wsum[lane] = t;
+        }
+        __syncthreads();
+        const T before = carry + (w ? wsum[w - 1] : (T)0) + s - v;
+        if (i < n) store(i, before);
+        if (threadIdx.x == PLAN_SCAN_THREADS - 1) carry_s = before + v;
+        __syncthreads();
+        carry = carry_s;
+        __syncthreads();
+    }
+    return carry;
+}
+
+// one CTA: the arena size and the pool's; the histogram becomes the lists' offsets (hist[n_hist] = total), and
+// a copy of them the scatter cursors
+__global__ void __launch_bounds__(PLAN_SCAN_THREADS) k_plan_offsets(PlanAcc *acc, const unsigned long long *epoch_bytes,
+                                                                    int32_t n_epochs, int32_t *hist, int64_t n_hist,
+                                                                    int32_t *cur) {
+    __shared__ unsigned long long wmax[PLAN_SCAN_THREADS / 32];
+    unsigned long long mx = 0;
+    for (int32_t e = threadIdx.x; e < n_epochs; e += PLAN_SCAN_THREADS) mx = max(mx, epoch_bytes[e]);
+    for (int d = 16; d > 0; d >>= 1) mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, d));
+    if ((threadIdx.x & 31) == 0) wmax[threadIdx.x >> 5] = mx;
+    __syncthreads();
+    const int32_t total = cta_scan<int32_t>(
+        n_hist, [&](int64_t i) { return hist[i]; },
+        [&](int64_t i, int32_t v) {
+            hist[i] = v;
+            cur[i] = v;
+        });
+    if (threadIdx.x == 0) {
+        hist[n_hist] = total;
+        for (int k = 0; k < PLAN_SCAN_THREADS / 32; k++) mx = max(mx, wmax[k]);
+        const unsigned long long arena = (mx + 255) & ~255ull;
+        acc->arena = arena;
+        acc->sum.pool_bytes = arena * (unsigned long long)min(3, n_epochs) + acc->long_bytes;
+    }
+}
+
+// per feature: its final block offset, and its places in the finalize list and (a set) in the zero list
+__global__ void __launch_bounds__(256) k_plan_place(const unsigned long long *cand, const int32_t *tlo,
+                                                    const int32_t *thi, int32_t m, int32_t epoch_tiles,
+                                                    int32_t n_epochs, uint64_t seg_max, uint64_t seg_big,
+                                                    PlanAcc *acc, int32_t *cur, int32_t *list, FeatDesc *fdesc,
+                                                    uint32_t *segoff16) {
+    const int32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    const PlanFeat f = plan_feat(j < m ? cand[j] : 0ull, j < m ? tlo[j] : 0, j < m ? thi[j] : 0, epoch_tiles,
+                                 n_epochs, seg_max, seg_big);
+    if (f.on) {
+        const unsigned long long arena = acc->arena;
+        const int n_arenas = min(3, n_epochs);
+        const unsigned long long off =
+            fdesc[j].blk_off + arena * (unsigned long long)(f.le <= f.fe + 1 ? f.fe % n_arenas : n_arenas);
+        fdesc[j].blk_off = off;
+        if (!f.set) {
+            if (off / 16 >= 0xFFFFFFFFull) atomicOr(&acc->sum.err, 2u);
+            segoff16[j] = (uint32_t)(off / 16);
+        }
+    }
+    const int32_t pf = warp_add<int32_t>(f.on, &cur[f.fin_key], 1);
+    if (f.on) list[pf] = j;
+    const int32_t pz = warp_add<int32_t>(f.set, &cur[(int64_t)3 * n_epochs * PLAN_KEYS + f.fe], 1);
+    if (f.set) list[pz] = j;
+}
+
+// one CTA: byte prefix of the zero list (set + cursor of each), so that k_zero_segments spreads an epoch's bytes
+// evenly over its CTAs
+__global__ void __launch_bounds__(PLAN_SCAN_THREADS) k_plan_zero_prefix(const int32_t *zero_lo, const int32_t *zero_hi,
+                                                                        const int32_t *list, const FeatDesc *fdesc,
+                                                                        unsigned long long *zpre) {
+    const int32_t z0 = *zero_lo, z1 = *zero_hi;
+    const unsigned long long total = cta_scan<unsigned long long>(
+        z1 - z0, [&](int64_t i) { return (unsigned long long)fdesc[list[z0 + i]].cap * 16 + 16; },
+        [&](int64_t i, unsigned long long v) { zpre[z0 + i] = v; });
+    if (threadIdx.x == 0) zpre[z1] = total;
+}
+
 // What a context keeps between calls: the interval index of the last feature set (valid while the caller passes the
-// same one) and the host-side working arrays of a call, reused so that they are not paged in anew every time.
+// same one), the window jobs of the last call and the pinned slot the plan's summary comes back to.
 struct FeatCache {
     bool valid = false;
     xg_input_key key;
     FeatIndexHost ix;
-    EpochPlan plan;
-    std::vector<unsigned long long> cand;
-    std::vector<int32_t> tlo, thi;
-    std::vector<FeatDesc> fdesc;
-    std::vector<uint32_t> segoff16;
+    std::vector<WinJob> jobs;
+    PlanSummary *h_sum = nullptr;
 };
 
 // Everything the counting kernel needs to know about a tile, in one 64-byte line that the CTA
@@ -1094,24 +1137,35 @@ __global__ void k_snapshot_cursor(const unsigned long long *cursor, unsigned lon
     __threadfence_system();
 }
 
-// Zero the sets of the features that become active in this epoch.  The segments are laid
-// end to end in a virtual byte space (pre[] = exclusive prefix, pre[n_seg] = total).
+// Zero the sets of the features that become active in this epoch: the zero list's entries [*lo, *hi), laid end to
+// end in a virtual byte space (pre = byte prefix of the list, k_plan_zero_prefix).  CTAs stride over its chunks.
 #define ZERO_CHUNK 16384
-__global__ void __launch_bounds__(256) k_zero_segments(uint8_t *pool, const uint64_t *off,
-                                                       const uint64_t *pre, int32_t n_seg) {
-    const uint64_t total = pre[n_seg];
-    const uint64_t c0 = (uint64_t)blockIdx.x * ZERO_CHUNK;
-    int32_t lo = 0, hi = n_seg;          // last segment with pre <= c0
-    while (hi - lo > 1) {
-        int32_t mid = (lo + hi) >> 1;
-        if (pre[mid] <= c0) lo = mid; else hi = mid;
-    }
-    int32_t s = lo;
+__global__ void __launch_bounds__(256) k_zero_segments(uint8_t *pool, const FeatDesc *fdesc, const int32_t *list,
+                                                       const unsigned long long *pre, const int32_t *lo_p,
+                                                       const int32_t *hi_p) {
+    const int32_t lo = *lo_p, hi = *hi_p;
+    if (hi <= lo) return;
+    const uint64_t base = pre[lo], total = pre[hi] - base;
     const uint4 z = make_uint4(0, 0, 0, 0);
-    for (uint64_t p = c0 + (uint64_t)threadIdx.x * 16; p < c0 + ZERO_CHUNK && p < total;
-         p += (uint64_t)blockDim.x * 16) {
-        while (p >= pre[s + 1]) s++;
-        *(uint4 *)(pool + off[s] + (p - pre[s])) = z;
+    for (uint64_t c0 = (uint64_t)blockIdx.x * ZERO_CHUNK; c0 < total; c0 += (uint64_t)gridDim.x * ZERO_CHUNK) {
+        int32_t a = lo, b = hi;          // last entry with pre <= c0
+        while (b - a > 1) {
+            int32_t mid = (a + b) >> 1;
+            if (pre[mid] - base <= c0) a = mid; else b = mid;
+        }
+        int32_t s = a;
+        uint64_t s_beg = pre[s] - base, s_end = pre[s + 1] - base;
+        uint8_t *blk = pool + fdesc[list[s]].blk_off;
+        for (uint64_t p = c0 + (uint64_t)threadIdx.x * 16; p < c0 + ZERO_CHUNK && p < total;
+             p += (uint64_t)blockDim.x * 16) {
+            while (p >= s_end) {
+                s++;
+                s_beg = s_end;
+                s_end = pre[s + 1] - base;
+                blk = pool + fdesc[list[s]].blk_off;
+            }
+            *(uint4 *)(blk + (p - s_beg)) = z;
+        }
     }
 }
 
@@ -1218,9 +1272,13 @@ __device__ __forceinline__ bool fs_insert_range(unsigned long long *tbl, unsigne
 template <int THREADS, int TBL_LOG2>
 __global__ void __maxnreg__(48) k_basefc_finalize_segs(
     const uint8_t *pool, const FeatDesc *fdesc, const uint32_t *seg_cur, const int32_t *sf_row,
-    const int32_t *fin_feat, int32_t n_fin, int32_t n_cols, unsigned int *work, unsigned long long *cursor,
-    int64_t *seg_base, int32_t *seg_nnz, int32_t *st_col, int32_t *st_val, unsigned long long *stats) {
+    const int32_t *fin_list, const int32_t *fin_lo, const int32_t *fin_hi, int32_t n_cols, unsigned int *work,
+    unsigned long long *cursor, int64_t *seg_base, int32_t *seg_nnz, int32_t *st_col, int32_t *st_val,
+    unsigned long long *stats) {
     extern __shared__ __align__(16) uint8_t fin_smem[];
+    // the epoch's features: a range of the plan's finalize list (surplus CTAs of the fixed grid leave at once)
+    const int32_t *fin_feat = fin_list + *fin_lo;
+    const int32_t n_fin = *fin_hi - *fin_lo;
     // table slots; words a table pass should hold (40 % load: the light / heavy limit); cells of a range on the fast
     // path = one counter bank; the counters (a light feature uses both banks as one)
     constexpr uint32_t TBL = 1u << TBL_LOG2, CAP = TBL * 2 / 5, RCELLS = TBL / 4, CNT = 2 * RCELLS;
@@ -1525,10 +1583,12 @@ __global__ void __maxnreg__(48) k_basefc_finalize_segs(
 #define FIN_WARPS (FIN_THREADS / 32)
 
 __global__ void __launch_bounds__(FIN_THREADS) k_basefc_finalize_sets(
-    const uint8_t *pool, const FeatDesc *fdesc, const int32_t *sf_row, const int32_t *fin_feat, int32_t n_fin,
-    int32_t n_cols, int32_t hist_cols, unsigned int *work, unsigned long long *cursor, int64_t *seg_base,
-    int32_t *seg_nnz, int32_t *st_col, int32_t *st_val) {
+    const uint8_t *pool, const FeatDesc *fdesc, const int32_t *sf_row, const int32_t *fin_list,
+    const int32_t *fin_lo, const int32_t *fin_hi, int32_t n_cols, int32_t hist_cols, unsigned int *work,
+    unsigned long long *cursor, int64_t *seg_base, int32_t *seg_nnz, int32_t *st_col, int32_t *st_val) {
     extern __shared__ __align__(16) uint8_t fin_smem[];
+    const int32_t *fin_feat = fin_list + *fin_lo;      // the epoch's features (as in k_basefc_finalize_segs)
+    const int32_t n_fin = *fin_hi - *fin_lo;
     uint32_t *hist = reinterpret_cast<uint32_t *>(fin_smem);                          // hist_cols
     uint32_t *bitmap = hist + hist_cols;                                              // (hist_cols + 31) / 32
     __shared__ int warp_tot[FIN_WARPS];
@@ -1651,7 +1711,7 @@ static double ms_since(std::chrono::steady_clock::time_point a) {
     return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - a).count();
 }
 
-// One basefc call: what its phases (windows -> plan -> epochs -> result) hand on to one another.
+// One basefc call: what its phases (params -> windows -> plan -> epochs -> result) hand on to one another.
 struct BasefcCall {
     xg_ctx *ctx = nullptr;
     const xg_dreads *rd = nullptr;
@@ -1661,14 +1721,19 @@ struct BasefcCall {
     int32_t n_rows = 0, n_cols = 0;
     bool dbg_sync = false;
     int launches = 0;
-    FeatCache *fc = nullptr;          // interval index, windows and epoch plan (kept by the context)
+    FeatCache *fc = nullptr;          // interval index and window jobs (kept by the context)
     size_t m = 0;                     // sorted features of the interval index
     BasefcDev P;
     const int32_t *d_sf_row = nullptr;
     TileDesc *d_tdesc = nullptr;
+    const unsigned long long *d_cand = nullptr;     // per sorted feature: candidate reads, first / end tile
+    const int32_t *d_tlo = nullptr, *d_thi = nullptr;
     bool seg_mode = false;
-    const int32_t *d_fin_feat = nullptr, *d_fin_set = nullptr, *d_fin_big = nullptr;
-    const uint64_t *d_zoff = nullptr, *d_zpre = nullptr;
+    int32_t n_epochs = 0, epoch_tiles = 0;
+    PlanSummary plan;                 // the part of the device plan the host needs
+    const int32_t *d_off = nullptr;   // the plan's list offsets (k_plan_offsets)
+    const int32_t *d_list = nullptr;  // finalize lists, then the zero list
+    const unsigned long long *d_zpre = nullptr;
     int64_t *seg_base = nullptr;      // staging area: first entry and entries of every row, the entries
     int32_t *seg_nnz = nullptr, *st_col = nullptr, *st_val = nullptr;
     unsigned long long *cursor = nullptr;
@@ -1677,11 +1742,45 @@ struct BasefcCall {
     unsigned long long *fs_stats = nullptr;   // route counters of the segment finalize (xg_basefc_finalize_stats)
     unsigned long long *h_cur = nullptr;    // rows layouts: the staging cursor after every epoch (mapped host memory)
     int64_t h2d_bytes = 0;
-    double ms_index = 0, ms_windows = 0, ms_plan = 0, ms_upload = 0;
+    double ms_index = 0, ms_windows = 0, ms_alloc = 0, ms_upload = 0;
     // per-epoch events: 0 count start, 1 count end, 2 epoch end, 3 H2D, 4 big finalize end
     cudaEvent_t ev(int kind, int32_t e) const { return ctx->ev_pool[(size_t)5 * e + kind]; }
-    cudaEvent_t ev_init() const { return ctx->ev_pool[(size_t)5 * fc->plan.n_epochs]; }
+    cudaEvent_t ev_init() const { return ctx->ev_pool[(size_t)5 * n_epochs]; }
+    // offsets of the finalize list of kind k (0 segments, 1 sets, 2 big segments) / of the zero list, epoch e
+    const int32_t *fin_off(int k, int32_t e) const { return d_off + ((int64_t)k * n_epochs + e) * PLAN_KEYS; }
+    const int32_t *zero_off(int32_t e) const { return d_off + (int64_t)3 * n_epochs * PLAN_KEYS + e; }
 };
+
+// The filters of the call and the cell-barcode table on the device.
+static int basefc_params(BasefcCall &c, const xg_barcodes *cells, const xg_params *par) {
+    xg_ctx *ctx = c.ctx;
+    BasefcDev &P = c.P;
+    auto t_ph = std::chrono::steady_clock::now();
+    if (par->min_incl_tab) {
+        if (par->min_incl_tab_len <= c.rd->max_aln_len)
+            return ctx->fail(XG_E_ARG, "min_incl_tab shorter than max aligned length + 1");
+        XG_GET(d_incl, int32_t, "fx_incl_tab", par->min_incl_tab_len + 1);
+        // the caller's table outlives the call, which ends in a synchronisation
+        XG_CUDA(cudaMemcpyAsync(d_incl, par->min_incl_tab, sizeof(int32_t) * (size_t)par->min_incl_tab_len,
+                                cudaMemcpyHostToDevice, ctx->stream));
+        P.incl_tab = d_incl;
+        P.incl_tab_len = par->min_incl_tab_len;
+    }
+    P.incl_len = par->min_incl_len;
+    P.col_bits = 1;
+    while ((1 << P.col_bits) < c.n_cols) P.col_bits++;
+    P.fp.min_mapq = par->min_mapq;
+    P.fp.min_len = par->min_len;
+    P.fp.incl_flag = par->incl_flag;
+    P.fp.excl_flag = par->excl_flag;
+    P.fp.no_orphan = par->no_orphan;
+    P.fp.use_cell_tag = par->use_cell_tag;
+    P.fp.need_umi_tag = par->need_umi_tag;
+    int rc = XG_OK;
+    if (par->use_cell_tag && (rc = xg_build_barcode_table(ctx, cells, &P.bc))) return rc;
+    c.ms_upload = ms_since(t_ph);
+    return XG_OK;
+}
 
 // Interval index of the features (host) and every feature's tile window and exact candidate count (device).
 static int basefc_windows(BasefcCall &c, const xg_features *feats, int32_t n_gid) {
@@ -1701,6 +1800,8 @@ static int basefc_windows(BasefcCall &c, const xg_features *feats, int32_t n_gid
         ctx->fx_cache_free = [](void *p) { delete (FeatCache *)p; };
     }
     c.fc = fc;
+    if (!fc->h_sum && !(fc->h_sum = (PlanSummary *)ctx->pinned_get(sizeof(PlanSummary))))
+        return ctx->fail(XG_E_NOMEM, "out of pinned host memory");
     const bool index_cached = fc->valid && fc->key.matches(fh, in);
     int rc = XG_OK;
     if (!index_cached) {
@@ -1752,22 +1853,15 @@ static int basefc_windows(BasefcCall &c, const xg_features *feats, int32_t n_gid
     P.stab_off = (const int32_t *)ctx->scratch["fx_stab_off"].p;
     P.stab4 = (const int4 *)ctx->scratch["fx_stab4"].p;
     P.fb = (const int32_t *)ctx->scratch["fx_fb"].p;
-    // feature windows on the device: one job per run whose contig has features
-    std::vector<WinJob> jobs;
+    // feature windows on the device: one job per stretch of tiles of a run whose contig has features
+    std::vector<WinJob> &jobs = fc->jobs;      // kept: the copy may still read it when this function returns
+    jobs.clear();
     int64_t n_warps = 0;
-    {
-        size_t t = 0;
-        const size_t nt = rd->h_tiles.size();
-        while (t < nt) {
-            const int32_t r = rd->h_tiles[t].run;
-            size_t e = t;
-            while (e < nt && rd->h_tiles[e].run == r) e++;
-            const int32_t g = rd->h_runs[(size_t)r].gid;
-            if (g >= 0 && g < n_gid && ix.sf_goff[(size_t)g + 1] > ix.sf_goff[(size_t)g]) {
-                jobs.push_back(WinJob{ix.sf_goff[(size_t)g], ix.sf_goff[(size_t)g + 1], (int32_t)t, (int32_t)e, n_warps});
-                n_warps += ix.sf_goff[(size_t)g + 1] - ix.sf_goff[(size_t)g];
-            }
-            t = e;
+    for (const int3 &rt : rd->h_run_tiles) {
+        const int32_t g = rd->h_runs[(size_t)rt.x].gid;
+        if (g >= 0 && g < n_gid && ix.sf_goff[(size_t)g + 1] > ix.sf_goff[(size_t)g]) {
+            jobs.push_back(WinJob{ix.sf_goff[(size_t)g], ix.sf_goff[(size_t)g + 1], rt.y, rt.z, n_warps});
+            n_warps += ix.sf_goff[(size_t)g + 1] - ix.sf_goff[(size_t)g];
         }
     }
     const WinJob *d_jobs = nullptr;
@@ -1777,15 +1871,13 @@ static int basefc_windows(BasefcCall &c, const xg_features *feats, int32_t n_gid
     XG_GET(d_thi, int32_t, "fx_thi", m + 1);
     XG_GET(d_tdesc, TileDesc, "fx_tdesc", rd->n_tiles + 1);
     P.tdesc = c.d_tdesc = d_tdesc;
+    c.d_cand = d_cand;
+    c.d_tlo = d_tlo;
+    c.d_thi = d_thi;
     cudaEventRecord(ctx->ev[0], ctx->stream);
     XG_CUDA(cudaMemsetAsync(d_cand, 0, sizeof(unsigned long long) * (m + 1), ctx->stream));
     XG_CUDA(cudaMemsetAsync(d_tlo, 0x7f, sizeof(int32_t) * (m + 1), ctx->stream));
     XG_CUDA(cudaMemsetAsync(d_thi, 0xff, sizeof(int32_t) * (m + 1), ctx->stream));
-    std::vector<unsigned long long> &cand = fc->cand;
-    std::vector<int32_t> &tlo = fc->tlo, &thi = fc->thi;
-    cand.assign(m, 0);
-    tlo.assign(m, INT32_MAX);
-    thi.assign(m, -1);
     if (n_warps > 0) {
         k_feature_windows<<<(unsigned)((n_warps + 7) / 8), 256, 0, ctx->stream>>>(
             d_jobs, (int32_t)jobs.size(), n_warps, rd->tiles, rd->tile_pmax, rd->pos_end, c.src ? 0 : 1, d_sf_beg,
@@ -1801,26 +1893,20 @@ static int basefc_windows(BasefcCall &c, const xg_features *feats, int32_t n_gid
         c.launches++;
         XG_DBG("k_tile_desc");
     }
-    if (m) {
-        XG_CUDA(cudaMemcpyAsync(cand.data(), d_cand, sizeof(unsigned long long) * m, cudaMemcpyDeviceToHost, ctx->stream));
-        XG_CUDA(cudaMemcpyAsync(tlo.data(), d_tlo, sizeof(int32_t) * m, cudaMemcpyDeviceToHost, ctx->stream));
-        XG_CUDA(cudaMemcpyAsync(thi.data(), d_thi, sizeof(int32_t) * m, cudaMemcpyDeviceToHost, ctx->stream));
-    }
-    XG_CUDA(cudaStreamSynchronize(ctx->stream));
     c.ms_windows = ms_since(t_ph);
     return XG_OK;
 }
 
-// The epoch plan (host) -- pool layout, which features each epoch zeroes and finalizes -- and its upload with the
-// filters and the buffers of the call.
-static int basefc_plan(BasefcCall &c, const xg_barcodes *cells, const xg_params *par, bool force_sets) {
+// The epoch plan, on the device where the windows are (k_plan_*): pool layout, which features each epoch zeroes
+// and finalizes.  Its summary is the call's one wait before the epochs: it sizes the pool and the staging area.
+static int basefc_plan(BasefcCall &c, bool force_sets) {
     xg_ctx *ctx = c.ctx;
     const xg_dreads *rd = c.rd;
     FeatCache *fc = c.fc;
-    const FeatIndexHost &ix = fc->ix;
     const size_t m = c.m;
     const int32_t n_cols = c.n_cols;
     BasefcDev &P = c.P;
+    auto t_ph = std::chrono::steady_clock::now();
     int32_t epoch_tiles = c.src ? 8192 : 65536;     // streaming: finer epochs = finer H2D / kernel overlap
     if (const char *e = getenv(c.src ? "XG_EPOCH_TILES_HOST" : "XG_EPOCH_TILES")) {
         epoch_tiles = std::max(1, atoi(e));
@@ -1829,6 +1915,9 @@ static int basefc_plan(BasefcCall &c, const xg_barcodes *cells, const xg_params 
         const int32_t n_ep = (rd->n_tiles + epoch_tiles - 1) / epoch_tiles;
         epoch_tiles = (rd->n_tiles + n_ep - 1) / n_ep;
     }
+    c.epoch_tiles = epoch_tiles;
+    c.n_epochs = std::max(1, (rd->n_tiles + epoch_tiles - 1) / epoch_tiles);
+    const int32_t ne = c.n_epochs;
     // Pair-word mode: a (cell, UMI) pair is one 64-bit word `umi | cell` (every UMI key of the batch leaves
     // its low 24 bits free: packed strings of up to 13 symbols, interned ids below 2^39), features collect
     // their words in segments.  The kernel verifies the keys it meets; a key that does not fit raises a
@@ -1836,11 +1925,12 @@ static int basefc_plan(BasefcCall &c, const xg_barcodes *cells, const xg_params 
     bool seg_mode = !force_sets && n_cols <= (1 << 19) && rd->umi_compact != 0;      // cell bitmap + ranks in shared memory
     if (const char *e = getenv("XG_SEG_MODE")) seg_mode = seg_mode && atoi(e) != 0;
     c.seg_mode = seg_mode;
-    uint64_t seg_max = 1ull << 22;             // heavier features keep a set in global memory
+    P.seg_mode = seg_mode ? 1 : 0;
+    // seg_max: features with at most this many candidate reads collect pair words in a segment (0: every feature
+    // keeps a set); heavier features keep a set in global memory
+    uint64_t seg_max = 1ull << 22;
     if (const char *e = getenv("XG_SEG_MAX")) seg_max = (uint64_t)atoll(e);
-    EpochPlan &pl = fc->plan;
-    pl.reset();
-    auto t_ph = std::chrono::steady_clock::now();
+    if (!seg_mode) seg_max = 0;
     // The reduction of a feature is one CTA's work and its passes are bound by the loads that CTA keeps in flight:
     // the few features with very many reads (a long tail in expression data) would be the critical path of their
     // epoch.  They get CTAs of 1024 threads, launched beside the ordinary ones.
@@ -1848,63 +1938,65 @@ static int basefc_plan(BasefcCall &c, const xg_barcodes *cells, const xg_params 
     if (const char *e = getenv("XG_SEG_BIG")) seg_big = (uint64_t)atoll(e);
     if (((size_t)10 << FS_BIG_TBL_LOG2) + (size_t)(2 * ((n_cols + 31) / 32) + 1) * 4 + sizeof(FsShared) + 1280 > 200 * 1024)
         seg_big = ~0ull;                      // so many cells that the big CTA's shared memory does not fit: no big CTAs
-    int rc = XG_OK;
-    if ((rc = make_plan(ctx, fc->cand, fc->tlo, fc->thi, rd->n_tiles, n_cols, epoch_tiles, seg_mode ? seg_max : 0,
-                        seg_big, pl)))
-        return rc;
-    c.ms_plan = ms_since(t_ph);
-    t_ph = std::chrono::steady_clock::now();
-    std::vector<FeatDesc> &fdesc = fc->fdesc;
-    std::vector<uint32_t> &segoff16 = fc->segoff16;
-    fdesc.resize(m);
-    segoff16.resize(m);
-    for (size_t j = 0; j < m; j++) {
-        fdesc[j] = FeatDesc{pl.blk_off[j], pl.tbl_cap[j], pl.log_cap[j]};
-        segoff16[j] = (!pl.tbl_cap[j] && pl.log_cap[j]) ? (uint32_t)(pl.blk_off[j] / 16) : NO_SEG;
+    // histogram / offsets: [3 kinds][epochs][PLAN_KEYS], then [epochs] of the zero list, then the total
+    const int64_t n_hist = (int64_t)3 * ne * PLAN_KEYS + ne;
+    XG_GET(fdesc, FeatDesc, "fx_fdesc", m + 1);
+    XG_GET(segoff16, uint32_t, "fx_segoff16", m + 1);
+    XG_GET(list, int32_t, "fx_plan_list", 2 * m + 1);
+    XG_GET(zpre, unsigned long long, "fx_plan_zpre", 2 * m + 2);
+    XG_GET(cur, int32_t, "fx_plan_cur", n_hist + 1);
+    const size_t acc_bytes = sizeof(PlanAcc) + sizeof(unsigned long long) * (size_t)ne + sizeof(int32_t) * (size_t)(n_hist + 1);
+    XG_GET(acc_raw, uint8_t, "fx_plan_acc", acc_bytes);
+    PlanAcc *acc = (PlanAcc *)acc_raw;
+    unsigned long long *epoch_bytes = (unsigned long long *)(acc + 1);
+    int32_t *hist = (int32_t *)(epoch_bytes + ne);
+    P.fdesc = fdesc;
+    P.segoff16 = segoff16;
+    c.d_off = hist;
+    c.d_list = list;
+    c.d_zpre = zpre;
+    cudaStream_t st = ctx->stream;
+    XG_CUDA(cudaMemsetAsync(acc_raw, 0, acc_bytes, st));
+    const unsigned plan_grid = (unsigned)((m + 255) / 256);
+    if (m) {
+        k_plan_features<<<plan_grid, 256, 0, st>>>(c.d_cand, c.d_tlo, c.d_thi, (int32_t)m, n_cols, epoch_tiles, ne, seg_max,
+                                                   seg_big, acc, epoch_bytes, hist, fdesc, segoff16);
+        c.launches++;
+        XG_DBG("k_plan_features");
     }
-    if ((rc = upload_vec(ctx, fdesc, "fx_fdesc", &P.fdesc))) return rc;
-    if ((rc = upload_vec(ctx, segoff16, "fx_segoff16", &P.segoff16))) return rc;
-    if (!ix.stab.empty()) {
-        k_patch_stab<<<(unsigned)((ix.stab.size() + 255) / 256), 256, 0, ctx->stream>>>(
-            (int4 *)ctx->scratch["fx_stab4"].p, (int32_t)ix.stab.size(), P.segoff16);
+    k_plan_offsets<<<1, PLAN_SCAN_THREADS, 0, st>>>(acc, epoch_bytes, ne, hist, n_hist, cur);
+    c.launches++;
+    XG_DBG("k_plan_offsets");
+    if (m) {
+        k_plan_place<<<plan_grid, 256, 0, st>>>(c.d_cand, c.d_tlo, c.d_thi, (int32_t)m, epoch_tiles, ne, seg_max, seg_big,
+                                                acc, cur, list, fdesc, segoff16);
+        c.launches++;
+        XG_DBG("k_plan_place");
+    }
+    k_plan_zero_prefix<<<1, PLAN_SCAN_THREADS, 0, st>>>(c.zero_off(0), c.zero_off(ne), list, fdesc, zpre);
+    c.launches++;
+    XG_DBG("k_plan_zero_prefix");
+    const size_t n_stab = fc->ix.stab.size();
+    if (n_stab) {      // the segment offsets of the plan go into the stabbing entries
+        k_patch_stab<<<(unsigned)((n_stab + 255) / 256), 256, 0, st>>>((int4 *)P.stab4, (int32_t)n_stab, segoff16);
         c.launches++;
         XG_DBG("k_patch_stab");
     }
-    if ((rc = upload_vec(ctx, pl.fin_feat, "fx_fin_feat", &c.d_fin_feat))) return rc;
-    if ((rc = upload_vec(ctx, pl.fin_set, "fx_fin_set", &c.d_fin_set))) return rc;
-    if ((rc = upload_vec(ctx, pl.fin_big, "fx_fin_big", &c.d_fin_big))) return rc;
-    if ((rc = upload_vec(ctx, pl.zseg_off, "fx_zseg_off", &c.d_zoff))) return rc;
-    if ((rc = upload_vec(ctx, pl.zseg_pre, "fx_zseg_pre", &c.d_zpre))) return rc;
-    if (par->min_incl_tab) {
-        if (par->min_incl_tab_len <= rd->max_aln_len)
-            return ctx->fail(XG_E_ARG, "min_incl_tab shorter than max aligned length + 1");
-        std::vector<int32_t> t(par->min_incl_tab, par->min_incl_tab + par->min_incl_tab_len);
-        if ((rc = upload_vec(ctx, t, "fx_incl_tab", &P.incl_tab))) return rc;
-        P.incl_tab_len = par->min_incl_tab_len;
-        XG_CUDA(cudaStreamSynchronize(ctx->stream));
-    }
-    P.incl_len = par->min_incl_len;
-    P.seg_mode = seg_mode ? 1 : 0;
-    P.col_bits = 1;
-    while ((1 << P.col_bits) < n_cols) P.col_bits++;
-    P.fp.min_mapq = par->min_mapq;
-    P.fp.min_len = par->min_len;
-    P.fp.incl_flag = par->incl_flag;
-    P.fp.excl_flag = par->excl_flag;
-    P.fp.no_orphan = par->no_orphan;
-    P.fp.use_cell_tag = par->use_cell_tag;
-    P.fp.need_umi_tag = par->need_umi_tag;
-    if (par->use_cell_tag) {
-        if ((rc = xg_build_barcode_table(ctx, cells, &P.bc))) return rc;
-    }
-    XG_GET(pool, uint8_t, "fx_pool", pl.pool_bytes + 16);
+    XG_CUDA(cudaMemcpyAsync(fc->h_sum, &acc->sum, sizeof(PlanSummary), cudaMemcpyDeviceToHost, st));
+    XG_CUDA(cudaStreamSynchronize(st));
+    c.plan = *fc->h_sum;
+    c.ms_windows += ms_since(t_ph);
+    if (c.plan.err & 1u) return ctx->fail(XG_E_LIMIT, "feature window exceeds 2^32 reads");
+    if (c.plan.err & 2u) return ctx->fail(XG_E_LIMIT, "segment pool exceeds 64 GiB; use smaller epochs (XG_EPOCH_TILES)");
+    t_ph = std::chrono::steady_clock::now();
+    XG_GET(pool, uint8_t, "fx_pool", c.plan.pool_bytes + 16);
     XG_GET(seg_base, int64_t, "fx_seg_base", c.n_rows + 1);
     XG_GET(seg_nnz, int32_t, "fx_seg_nnz", c.n_rows + 1);
-    XG_GET(st_col, int32_t, "fx_st_col", pl.staging_cap + 1);
-    XG_GET(st_val, int32_t, "fx_st_val", pl.staging_cap + 1);
+    XG_GET(st_col, int32_t, "fx_st_col", c.plan.staging_cap + 1);
+    XG_GET(st_val, int32_t, "fx_st_val", c.plan.staging_cap + 1);
     XG_GET(cursor, unsigned long long, "fx_cursor", 2);
     // per epoch: work counters of the ordinary finalize, counting, set finalize and big finalize launches; flags
-    XG_GET(fin_work, unsigned int, "fx_fin_work", 4 * (pl.n_epochs + 1) + 4);
+    XG_GET(fin_work, unsigned int, "fx_fin_work", 4 * (ne + 1) + 4);
     XG_GET(seg_cur, uint32_t, "fx_seg_cur", m + 1);
     c.seg_base = seg_base;
     c.seg_nnz = seg_nnz;
@@ -1915,20 +2007,21 @@ static int basefc_plan(BasefcCall &c, const xg_barcodes *cells, const xg_params 
     c.seg_cur = seg_cur;
     P.pool = pool;
     P.seg_cur = seg_cur;
-    P.flags = fin_work + 4 * (pl.n_epochs + 1);
-    XG_CUDA(cudaStreamSynchronize(ctx->stream));   // host vectors above are about to die
-    c.ms_upload = ms_since(t_ph);
+    P.flags = fin_work + 4 * (ne + 1);
+    c.ms_alloc = ms_since(t_ph);
     return XG_OK;
 }
 
 // The epochs on the device: zero(e) -> count(e) -> finalize(e), one after another on the context's stream.  The
 // counting kernel is persistent and fills the GPU by itself; only the big-segment finalize runs beside the
-// ordinary one, and (xg_basefc_host) the copy of the next epoch's records beside the kernels.
+// ordinary one, and (xg_basefc_host) the copy of the next epoch's records beside the kernels.  How many features
+// an epoch zeroes and finalizes is known on the device only: those kernels get a fixed grid and read their
+// epoch's range of the plan's lists.
 static int basefc_epochs(BasefcCall &c, bool rows) {
     xg_ctx *ctx = c.ctx;
     const xg_dreads *rd = c.rd;
-    const EpochPlan &pl = c.fc->plan;
-    const int32_t n_rows = c.n_rows, n_cols = c.n_cols;
+    const PlanSummary &pl = c.plan;
+    const int32_t n_rows = c.n_rows, n_cols = c.n_cols, ne = c.n_epochs;
     const size_t m = c.m;
     BasefcDev &P = c.P;
     // shared memory of the finalize kernels.  Segments: dedup table, rank counters, bitmap over the cells and
@@ -1955,23 +2048,29 @@ static int basefc_epochs(BasefcCall &c, bool rows) {
     XG_CUDA(cudaFuncSetAttribute(k_basefc_finalize_sets, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hist_bytes));
     const int fin_ctas_per_sm = std::max(1, std::min(4, (int)(220 * 1024 / (hist_bytes + 2048))));
     XG_CUDA(cudaFuncSetAttribute(k_basefc_count<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CountSmem)));
+    // fixed grids: the most CTAs that fit the GPU, fewer when the whole call has fewer features of the kind
+    const int64_t n_seg = (int64_t)(pl.n_seg_feat - pl.n_big_feat), n_big = (int64_t)pl.n_big_feat,
+                  n_set = (int64_t)pl.n_set_feat;
+    const int segs_grid = (int)std::min<int64_t>(n_seg, 148 * segs_ctas_per_sm);
+    const int big_grid = (int)std::min<int64_t>(n_big, 148);
+    const int sets_grid = (int)std::min<int64_t>(n_set, 148 * fin_ctas_per_sm);
+    const unsigned zero_grid = 148 * 8;
 
-    if (!pl.fin_big.empty() && !ctx->big_stream)
-        XG_CUDA(cudaStreamCreateWithFlags(&ctx->big_stream, cudaStreamNonBlocking));
+    if (n_big > 0 && !ctx->big_stream) XG_CUDA(cudaStreamCreateWithFlags(&ctx->big_stream, cudaStreamNonBlocking));
     if (c.src && !ctx->copy_stream) XG_CUDA(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-    while ((int32_t)ctx->ev_pool.size() < 5 * pl.n_epochs + 1) {
+    while ((int32_t)ctx->ev_pool.size() < 5 * ne + 1) {
         cudaEvent_t ev;
         XG_CUDA(cudaEventCreate(&ev));
         ctx->ev_pool.push_back(ev);
     }
-    unsigned int *cnt_work = c.fin_work + pl.n_epochs + 1;          // tile counters of the counting launches
-    unsigned int *set_work = c.fin_work + 2 * (pl.n_epochs + 1);    // work counters of the set finalize launches
-    unsigned int *big_work = c.fin_work + 3 * (pl.n_epochs + 1);    // ... of the big-segment finalize launches
+    unsigned int *cnt_work = c.fin_work + ne + 1;          // tile counters of the counting launches
+    unsigned int *set_work = c.fin_work + 2 * (ne + 1);    // work counters of the set finalize launches
+    unsigned int *big_work = c.fin_work + 3 * (ne + 1);    // ... of the big-segment finalize launches
     cudaStream_t st = ctx->stream;
     XG_CUDA(cudaMemsetAsync(c.seg_nnz, 0, sizeof(int32_t) * (size_t)(n_rows + 1), st));
     XG_CUDA(cudaMemsetAsync(c.seg_base, 0, sizeof(int64_t) * (size_t)(n_rows + 1), st));
     XG_CUDA(cudaMemsetAsync(c.cursor, 0, 16, st));
-    XG_CUDA(cudaMemsetAsync(c.fin_work, 0, sizeof(unsigned int) * (size_t)(4 * (pl.n_epochs + 1) + 4), st));
+    XG_CUDA(cudaMemsetAsync(c.fin_work, 0, sizeof(unsigned int) * (size_t)(4 * (ne + 1) + 4), st));
     XG_CUDA(cudaMemsetAsync(c.seg_cur, 0, sizeof(uint32_t) * (m + 1), st));
     c.launches += 6;
     cudaEventRecord(c.ev_init(), st);
@@ -1981,7 +2080,7 @@ static int basefc_epochs(BasefcCall &c, bool rows) {
     unsigned long long *d_cur = nullptr;
     if (rows) {
         if (!ctx->d2h_stream) XG_CUDA(cudaStreamCreateWithFlags(&ctx->d2h_stream, cudaStreamNonBlocking));
-        c.h_cur = (unsigned long long *)ctx->pinned_get(sizeof(unsigned long long) * (size_t)(pl.n_epochs + 1));
+        c.h_cur = (unsigned long long *)ctx->pinned_get(sizeof(unsigned long long) * (size_t)(ne + 1));
         if (!c.h_cur) return ctx->fail(XG_E_NOMEM, "out of pinned host memory");
         if (cudaHostGetDevicePointer((void **)&d_cur, c.h_cur, 0) != cudaSuccess) {
             cudaGetLastError();
@@ -1990,8 +2089,8 @@ static int basefc_epochs(BasefcCall &c, bool rows) {
             return ctx->fail(XG_E_CUDA, "pinned host memory is not mapped for the device");
         }
     }
-    for (int32_t e = 0; e < pl.n_epochs; e++) {
-        const int32_t t0 = e * pl.epoch_tiles, t1 = std::min(rd->n_tiles, t0 + pl.epoch_tiles);
+    for (int32_t e = 0; e < ne; e++) {
+        const int32_t t0 = e * c.epoch_tiles, t1 = std::min(rd->n_tiles, t0 + c.epoch_tiles);
         if (c.src) {      // this epoch's records: host -> HBM on the copy stream
             const xg_reads *src = c.src;
             if (t1 > t0) {
@@ -2012,12 +2111,8 @@ static int basefc_epochs(BasefcCall &c, bool rows) {
             cudaEventRecord(c.ev(3, e), ctx->copy_stream);
             cudaStreamWaitEvent(st, c.ev(3, e), 0);
         }
-        const int32_t z0 = pl.zero_ptr[(size_t)e], z1 = pl.zero_ptr[(size_t)e + 1];
-        const int32_t n_seg = z1 - z0 - 1;
-        if (n_seg > 0) {
-            const uint64_t total = pl.zseg_pre[(size_t)z1 - 1];
-            k_zero_segments<<<(unsigned)((total + ZERO_CHUNK - 1) / ZERO_CHUNK), 256, 0, st>>>(
-                P.pool, c.d_zoff + z0, c.d_zpre + z0, n_seg);
+        if (n_set > 0) {
+            k_zero_segments<<<zero_grid, 256, 0, st>>>(P.pool, P.fdesc, c.d_list, c.d_zpre, c.zero_off(e), c.zero_off(e + 1));
             c.launches++;
             XG_DBG("k_zero_segments");
         }
@@ -2036,33 +2131,27 @@ static int basefc_epochs(BasefcCall &c, bool rows) {
             XG_DBG("k_basefc_count");
         }
         cudaEventRecord(c.ev(1, e), st);
-        const int32_t n_fin = pl.fin_ptr[(size_t)e + 1] - pl.fin_ptr[(size_t)e];
-        const int32_t n_fin_set = pl.fin_set_ptr[(size_t)e + 1] - pl.fin_set_ptr[(size_t)e];
         // big segments first, on a stream of their own: their few large CTAs take their SMs before the ordinary
         // finalize CTAs fill the rest, and both kernels run side by side
-        const int32_t n_big = pl.fin_big_ptr[(size_t)e + 1] - pl.fin_big_ptr[(size_t)e];
         if (n_big > 0) {
             cudaStreamWaitEvent(ctx->big_stream, c.ev(1, e), 0);
-            k_basefc_finalize_segs<FS_BIG_THREADS, FS_BIG_TBL_LOG2><<<std::min(n_big, 148), FS_BIG_THREADS, big_bytes,
-                                                                     ctx->big_stream>>>(
-                P.pool, P.fdesc, c.seg_cur, c.d_sf_row, c.d_fin_big + pl.fin_big_ptr[(size_t)e], n_big, n_cols,
+            k_basefc_finalize_segs<FS_BIG_THREADS, FS_BIG_TBL_LOG2><<<big_grid, FS_BIG_THREADS, big_bytes, ctx->big_stream>>>(
+                P.pool, P.fdesc, c.seg_cur, c.d_sf_row, c.d_list, c.fin_off(2, e), c.fin_off(2, e + 1), n_cols,
                 big_work + e, c.cursor, c.seg_base, c.seg_nnz, c.st_col, c.st_val, c.fs_stats);
             c.launches++;
             XG_DBG("k_basefc_finalize_segs<big>");
             cudaEventRecord(c.ev(4, e), ctx->big_stream);
         }
-        if (n_fin > 0) {
-            const int grid = std::min(n_fin, 148 * segs_ctas_per_sm);
-            k_basefc_finalize_segs<FS_THREADS, FS_TBL_LOG2><<<grid, FS_THREADS, segs_bytes, st>>>(
-                P.pool, P.fdesc, c.seg_cur, c.d_sf_row, c.d_fin_feat + pl.fin_ptr[(size_t)e], n_fin, n_cols,
+        if (n_seg > 0) {
+            k_basefc_finalize_segs<FS_THREADS, FS_TBL_LOG2><<<segs_grid, FS_THREADS, segs_bytes, st>>>(
+                P.pool, P.fdesc, c.seg_cur, c.d_sf_row, c.d_list, c.fin_off(0, e), c.fin_off(0, e + 1), n_cols,
                 c.fin_work + e, c.cursor, c.seg_base, c.seg_nnz, c.st_col, c.st_val, c.fs_stats);
             c.launches++;
             XG_DBG("k_basefc_finalize_segs");
         }
-        if (n_fin_set > 0) {
-            const int grid = std::min(n_fin_set, 148 * fin_ctas_per_sm);
-            k_basefc_finalize_sets<<<grid, FIN_THREADS, hist_bytes, st>>>(
-                P.pool, P.fdesc, c.d_sf_row, c.d_fin_set + pl.fin_set_ptr[(size_t)e], n_fin_set, n_cols, hist_cols,
+        if (n_set > 0) {
+            k_basefc_finalize_sets<<<sets_grid, FIN_THREADS, hist_bytes, st>>>(
+                P.pool, P.fdesc, c.d_sf_row, c.d_list, c.fin_off(1, e), c.fin_off(1, e + 1), n_cols, hist_cols,
                 set_work + e, c.cursor, c.seg_base, c.seg_nnz, c.st_col, c.st_val);
             c.launches++;
             XG_DBG("k_basefc_finalize_sets");
@@ -2083,7 +2172,7 @@ static int basefc_epochs(BasefcCall &c, bool rows) {
 // copies everything at the end.
 static int basefc_collect_rows(BasefcCall &c, int32_t layout, xg_coo **out) {
     xg_ctx *ctx = c.ctx;
-    const EpochPlan &pl = c.fc->plan;
+    const int64_t staging_cap = (int64_t)c.plan.staging_cap;
     const int32_t n_rows = c.n_rows, n_cols = c.n_cols;
     const int32_t *st_col = c.st_col, *st_val = c.st_val;
     const auto t_tail = std::chrono::steady_clock::now();
@@ -2099,7 +2188,7 @@ static int basefc_collect_rows(BasefcCall &c, int32_t layout, xg_coo **out) {
         return ctx->fail(code, msg);
     };
     int64_t cap = ctx->fx_nnz_hint > 0 ? ctx->fx_nnz_hint + ctx->fx_nnz_hint / 8 + 1024 : 0;
-    cap = std::min<int64_t>(cap, pl.staging_cap + 1);
+    cap = std::min<int64_t>(cap, staging_cap + 1);
     // The entry format: narrow entries need 16-bit columns, and a packed format whose side list overflows falls
     // back to plain entries (below) -- the only two places it is chosen.
     int32_t fmt = layout == XG_LAYOUT_ROWS_NARROW && n_cols > 65536 ? XG_LAYOUT_ROWS : layout;
@@ -2111,11 +2200,11 @@ static int basefc_collect_rows(BasefcCall &c, int32_t layout, xg_coo **out) {
     long long *d_over_idx = nullptr;
     int32_t *d_over_val = nullptr, *d_over_col = nullptr;
     unsigned int *d_over_n = nullptr;
-    const size_t row_start_words = (size_t)(pl.staging_cap + 32) / 32 + 1;
+    const size_t row_start_words = (size_t)(staging_cap + 32) / 32 + 1;
     if (narrow || tiny) {
-        if (narrow) d_packed = (uint32_t *)ctx->get("fx_packed", sizeof(uint32_t) * (size_t)(pl.staging_cap + 1));
+        if (narrow) d_packed = (uint32_t *)ctx->get("fx_packed", sizeof(uint32_t) * (size_t)(staging_cap + 1));
         if (tiny) {
-            d_tiny = (uint16_t *)ctx->get("fx_tiny", sizeof(uint16_t) * (size_t)(pl.staging_cap + 2));
+            d_tiny = (uint16_t *)ctx->get("fx_tiny", sizeof(uint16_t) * (size_t)(staging_cap + 2));
             d_row_start = (uint32_t *)ctx->get("fx_row_start", sizeof(uint32_t) * row_start_words);
             d_over_col = (int32_t *)ctx->get("fx_over_col", sizeof(int32_t) * (size_t)OVER_CAP);
         }
@@ -2174,7 +2263,7 @@ static int basefc_collect_rows(BasefcCall &c, int32_t layout, xg_coo **out) {
     if (cap > 0 && !host_buffers(cap)) return give_up(XG_E_NOMEM, "out of pinned host memory for the result");
     int64_t done = 0;            // entries already queued for the host
     bool fits = cap > 0;
-    for (int32_t e = 0; e < pl.n_epochs && fits; e++) {
+    for (int32_t e = 0; e < c.n_epochs && fits; e++) {
         cudaError_t ce = cudaEventSynchronize(c.ev(2, e));
         if (ce != cudaSuccess) return give_up(XG_E_CUDA, std::string("basefc: ") + cudaGetErrorString(ce));
         const int64_t cur = (int64_t)c.h_cur[e];
@@ -2269,11 +2358,10 @@ static int basefc_collect_rows(BasefcCall &c, int32_t layout, xg_coo **out) {
 // xg_last_timing of the call (include/xcltk_b200.h); [4], the result copy, is set by the result phase.
 static void basefc_timing(const BasefcCall &c, std::chrono::steady_clock::time_point t_call) {
     xg_ctx *ctx = c.ctx;
-    const EpochPlan &pl = c.fc->plan;
     float t_all = 0, t_span = 0;
     double t_cnt = 0;
     cudaEventElapsedTime(&t_all, ctx->ev[0], ctx->ev[3]);
-    for (int32_t e = 0; e < pl.n_epochs; e++) {
+    for (int32_t e = 0; e < c.n_epochs; e++) {
         float t = 0;
         cudaEventElapsedTime(&t, c.ev(0, e), c.ev(1, e));
         t_cnt += t;
@@ -2283,17 +2371,17 @@ static void basefc_timing(const BasefcCall &c, std::chrono::steady_clock::time_p
     ctx->timing[1] = t_cnt;      // sum over epochs of the counting kernel
     ctx->timing[2] = c.launches;
     ctx->timing[3] = t_span;     // epochs + scan + gather (no host planning in between)
-    ctx->timing[5] = pl.n_epochs;
-    ctx->timing[6] = (double)pl.pool_bytes;
-    ctx->timing[7] = (double)pl.staging_cap;
+    ctx->timing[5] = c.n_epochs;
+    ctx->timing[6] = (double)c.plan.pool_bytes;
+    ctx->timing[7] = (double)c.plan.staging_cap;
     ctx->timing[8] = c.ms_index;
     ctx->timing[9] = c.ms_windows;
-    ctx->timing[10] = c.ms_plan;
+    ctx->timing[10] = c.ms_alloc;
     ctx->timing[11] = c.ms_upload;
     ctx->timing[12] = ms_since(t_call);
     ctx->timing[13] = (double)c.h2d_bytes;
-    ctx->timing[14] = (double)pl.n_seg_feat;
-    ctx->timing[15] = (double)pl.n_set_feat;
+    ctx->timing[14] = (double)c.plan.n_seg_feat;
+    ctx->timing[15] = (double)c.plan.n_set_feat;
 }
 
 // `src` != nullptr: the records of `rd` are copied from the pinned host batch `src` epoch by epoch (BasefcCall).
@@ -2329,8 +2417,8 @@ static int basefc_run(xg_ctx *ctx, const xg_dreads *rd, const xg_reads *src, con
     // a call redone with sets keeps the counts of its first attempt, whose segments were reduced
     if (!force_sets) XG_CUDA(cudaMemsetAsync(c.fs_stats, 0, sizeof(unsigned long long) * FS_STATS, ctx->stream));
     int rc = XG_OK;
-    if ((rc = basefc_windows(c, feats, n_gid)) || (rc = basefc_plan(c, cells, par, force_sets)) ||
-        (rc = basefc_epochs(c, layout != XG_LAYOUT_CSR)))
+    if ((rc = basefc_params(c, cells, par)) || (rc = basefc_windows(c, feats, n_gid)) ||
+        (rc = basefc_plan(c, force_sets)) || (rc = basefc_epochs(c, layout != XG_LAYOUT_CSR)))
         return rc;
     if (layout != XG_LAYOUT_CSR)
         rc = basefc_collect_rows(c, layout, out);

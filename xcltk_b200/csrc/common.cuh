@@ -36,6 +36,7 @@ struct xg_dreads {
     int32_t *tile_pmax = nullptr;   // device: per run, prefix max of tile.max_end (window planning)
     std::vector<xg_run> h_runs;  // host copies for the planners
     std::vector<xg_tile> h_tiles;
+    std::vector<int3> h_run_tiles;  // maximal stretches of tiles of one run: {run, first tile, end tile}
     double h2d_ms = 0;
     int64_t bytes = 0;
     bool pooled = false;         // buffers came from xg_ctx::dev_get

@@ -326,13 +326,17 @@ xg_dreads *xg_dreads_new(const xg_reads *h) {
 }
 
 // Prefix max (restarting at every run) of the tiles' max_end: with it "first tile whose records
-// can still reach position x" is a binary search.  Built once per batch from the host tile index.
+// can still reach position x" is a binary search.  Built once per batch from the host tile index, with the
+// stretches of tiles of one run (basefc plans one window job per stretch and call).
 int xg_make_tile_pmax(xg_ctx *ctx, xg_dreads *d) {
     size_t nt = d->h_tiles.size();
     std::vector<int32_t> pm(nt);
+    d->h_run_tiles.clear();
     for (size_t t = 0; t < nt; t++) {
         bool first = (t == 0) || d->h_tiles[t - 1].run != d->h_tiles[t].run;
         pm[t] = first ? d->h_tiles[t].max_end : std::max(pm[t - 1], d->h_tiles[t].max_end);
+        if (first) d->h_run_tiles.push_back(make_int3(d->h_tiles[t].run, (int)t, (int)t));
+        d->h_run_tiles.back().z = (int)t + 1;
     }
     if (d->tile_pmax) ctx->dev_put(d->tile_pmax);
     d->tile_pmax = (int32_t *)ctx->dev_get(nt * 4 + 16);
