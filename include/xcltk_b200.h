@@ -188,6 +188,50 @@ int xg_decode_bams_device_range(xg_ctx *ctx, int32_t n_bams, const char *const *
                                 const char *cell_tag, const char *umi_tag, int32_t want_seq, xg_keyspace *ks,
                                 const int64_t *range_lo, const int64_t *range_hi, xg_dreads **out,
                                 int64_t *n_records_seen);
+/* The same for a list of ranges per file: BAM b decodes the ranges r = range_ptr[b] .. range_ptr[b + 1] - 1, ascending
+ * and disjoint.  range_lo[r] is the BGZF virtual offset of the range's first record (block offset << 16 | offset in
+ * the inflated block, as a .bai gives it), range_hi[r] the file offset of the block after the range (or the file's
+ * end); the walk of the range's first block starts at that record.  An empty list decodes nothing of that BAM,
+ * range_ptr = NULL every file whole.  The ranges of a BAM go through one staging / window pipeline one after the
+ * other (the bytes between them are never read); runs and the sort check are stitched across them as across windows.
+ * *n_records_seen counts the records walked, *bytes_read (may be NULL) the compressed bytes read from the files,
+ * headers included.  Records that cross blocks: XG_E_UNSUPPORTED, as for the whole file; so is, when a BAM is read
+ * in ranges, a record that does not parse or is out of order (a range that does not start at a record): the caller
+ * then decodes the whole files on the host, which reports what is wrong with them.  The ranges come from
+ * xg_bam_index_ranges.                                                                                          */
+int xg_decode_bams_device_ranges(xg_ctx *ctx, int32_t n_bams, const char *const *paths,
+                                 const int32_t *const *tid_map, const int32_t *tid_map_len,
+                                 const char *cell_tag, const char *umi_tag, int32_t want_seq, xg_keyspace *ks,
+                                 const int64_t *range_ptr, const int64_t *range_lo, const int64_t *range_hi,
+                                 xg_dreads **out, int64_t *n_records_seen, int64_t *bytes_read);
+
+/* ---- BAM index (.bai, SAMv1 section 5.2) ---------------------------------------------
+ * xg_bam_index_open looks for <bam>.bai, then <bam without .bam>.bai.  Neither there: XG_OK with *out = NULL (the
+ * file is read whole; a .csi is not read).  An index that is there but cannot be trusted returns XG_E_FORMAT with the
+ * reason in xg_host_last_error(): not a BAI or truncated, n_ref differs from the BAM header, an offset beyond the BAM,
+ * older than the BAM.  Release with xg_bam_index_free.                                                          */
+typedef struct xg_bam_index xg_bam_index;
+int xg_bam_index_open(const char *bam_path, xg_bam_index **out);
+void xg_bam_index_free(xg_bam_index *idx);
+int32_t xg_bam_index_n_ref(const xg_bam_index *idx);
+/* The index of contig tid as read (pointers into idx): n_bins bins ascending (the pseudo-bin left out), the chunks of
+ * bin i as (beg, end) virtual-offset pairs chunks[2k], chunks[2k + 1] for k in [bin_ptr[i], bin_ptr[i + 1]), and
+ * the n_intv offsets of the 16 kb linear index.                                                                  */
+int xg_bam_index_ref(const xg_bam_index *idx, int32_t tid, int64_t *n_bins, const uint32_t **bins,
+                     const int64_t **bin_ptr, const uint64_t **chunks, int64_t *n_intv, const uint64_t **linear);
+/* The ranges of the BAM that hold every record overlapping one of the n 0-based half-open intervals
+ * (tid[i], beg[i], end[i]): the chunks htslib's bam_itr_queryi visits (the bins of reg2bins, less the chunks that end
+ * at or before the linear-index offset of the interval's start), merged, then widened to the end of whole BGZF
+ * blocks -- a range ends at the block after its last chunk's end -- and merged again when fewer than
+ * XG_BAM_INDEX_MERGE_GAP bytes lie between them (reading the gap costs less than one more range).  *ranges: 2 *
+ * *n_ranges entries lo, hi, ascending, lo the virtual offset of the range's first record, hi a file offset (release
+ * with xg_free_array); the form xg_decode_bams_device_ranges takes.  Unknown tids and empty intervals add nothing.
+ * XG_E_FORMAT when an offset is not a BGZF block start of the BAM or lies beyond its block (an index of another
+ * file): the caller then reads the file whole.                                                                   */
+#define XG_BAM_INDEX_MERGE_GAP (256 << 10)
+int xg_bam_index_ranges(const xg_bam_index *idx, int64_t n, const int32_t *tid, const int64_t *beg, const int64_t *end,
+                        int64_t **ranges, int64_t *n_ranges);
+
 /* Host helpers for choosing the ranges (what the .bai linear index gives pysam's fetch, computed from the file):
  * offsets of all BGZF blocks (n + 1 entries, the last = file size; release with xg_free_array), the block in which
  * the first record starts (*aligned = 1: exactly at its beginning, as htslib writes), and the (tid, pos) of the

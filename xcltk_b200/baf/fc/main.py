@@ -291,8 +291,8 @@ def shard_units(conf, chroms, unit_chrom, unit_beg, unit_end, run, batch=None):
                 batch = engine.load_reads_multi(conf.sam_fn_list, chroms, conf.cell_tag, conf.umi_tag, True,
                                                 threads, devices=parallel.device_list(n_dev))
         else:
-            batch = engine.load_reads(conf.sam_fn_list, chroms, conf.cell_tag, conf.umi_tag, True, threads,
-                                      mapped=True)
+            batch = engine.load_reads(conf.sam_fn_list, engine.Request(chroms, unit_chrom, unit_beg, unit_end),
+                                      conf.cell_tag, conf.umi_tag, True, threads, mapped=True)
     try:
         if isinstance(batch, (engine.ShardedBatch, engine.MultiBatch)):
             if isinstance(batch, engine.ShardedBatch):

@@ -288,7 +288,7 @@ def usage(fp=sys.stdout, d=None):
         "  --minMAPQ INT           Minimum MAPQ for read filtering [%d]" % d.MIN_MAPQ,
         "  --countORPHAN           If use, do not skip anomalous read pairs.",
         "",
-        "B200 notes: input must be coordinate-sorted BAM (no index needed; SAM/CRAM are not decoded);",
+        "B200 notes: input must be coordinate-sorted BAM (a .bai is used when present; SAM/CRAM are not decoded);",
         "  -p sets the host BGZF/BAM decode threads; counting runs on the GPU (no CPU fallback).",
         "  A UMI is counted once per SNP and cell, with the allele of its first read in file order.",
         "  Without -P, REF and ALT of a site are its two most frequent bases among A, C, G, T (ties in that",

@@ -7,6 +7,7 @@
 // Semantics restated from the SAM/BAM specification (SAMv1 section 4.2) and SURVEY.md A.3.
 // Inflate and field extraction are multi-threaded; nothing here touches the GPU except the
 // (optional) pinned allocator installed by the CUDA translation unit.
+#include <sys/stat.h>
 #include <zlib.h>
 
 #include <algorithm>
@@ -1257,4 +1258,240 @@ extern "C" int xg_bam_block_probe(const char *path, int64_t offset, int32_t *tid
     *tid = (int32_t)rd32(&u[4]);
     *pos = (int32_t)rd32(&u[8]);
     return XG_OK;
+}
+
+// ---- the BAM index (.bai, SAMv1 section 5.2) -------------------------------------------------------------
+// Which blocks hold the records of a set of intervals, the way htslib's bam_itr_queryi finds them: the chunks of the
+// bins that overlap an interval (reg2bins), less those that end before the linear index's offset of the interval's
+// 16 kb window.  The chunks are then widened to whole BGZF blocks and merged, so that the device decoder can stage
+// them: a range starts at the block of its first chunk and ends at the block after its last chunk's end.
+struct xg_bam_index {
+    struct Ref {
+        std::vector<uint32_t> bins;          // ascending
+        std::vector<int64_t> bin_ptr;        // bins.size() + 1 entries into chunks (pairs)
+        std::vector<uint64_t> chunks;        // (beg, end) virtual offsets, per bin as the index lists them
+        std::vector<uint64_t> linear;        // 16 kb windows
+    };
+    std::string bam_path;
+    uint64_t bam_size = 0;
+    std::vector<Ref> refs;
+};
+
+namespace {
+
+constexpr uint32_t BAI_PSEUDO_BIN = 37450;
+
+int bai_fail(const std::string &bai, const std::string &why) {
+    return fail(XG_E_FORMAT, std::string("index '") + bai + "' is not used: " + why);
+}
+
+int bai_parse(const Bytes &f, const std::string &bai, xg_bam_index &idx) {
+    const uint64_t n = f.size();
+    uint64_t o = 0;
+    auto need = [&](uint64_t k) { return o + k <= n; };
+    if (!need(8) || memcmp(f.data(), "BAI\1", 4) != 0) return bai_fail(bai, "not a BAI file");
+    const int32_t n_ref = (int32_t)rd32(&f[4]);
+    o = 8;
+    if (n_ref < 0) return bai_fail(bai, "negative n_ref");
+    idx.refs.resize((size_t)n_ref);
+    for (int32_t t = 0; t < n_ref; t++) {
+        xg_bam_index::Ref &R = idx.refs[(size_t)t];
+        if (!need(4)) return bai_fail(bai, "truncated");
+        const int32_t n_bin = (int32_t)rd32(&f[o]);
+        o += 4;
+        if (n_bin < 0) return bai_fail(bai, "negative n_bin");
+        std::vector<std::pair<uint32_t, std::pair<uint64_t, uint64_t>>> all;     // (bin, chunk); stable by bin below
+        for (int32_t b = 0; b < n_bin; b++) {
+            if (!need(8)) return bai_fail(bai, "truncated");
+            const uint32_t bin = rd32(&f[o]);
+            const int32_t n_chunk = (int32_t)rd32(&f[o + 4]);
+            o += 8;
+            if (n_chunk < 0 || !need(16ull * (uint64_t)n_chunk)) return bai_fail(bai, "truncated");
+            for (int32_t c = 0; c < n_chunk; c++, o += 16) {
+                uint64_t cb, ce;
+                memcpy(&cb, &f[o], 8);
+                memcpy(&ce, &f[o + 8], 8);
+                if (bin == BAI_PSEUDO_BIN) continue;          // (ref_beg, ref_end), (n_mapped, n_unmapped)
+                if (bin > BAI_PSEUDO_BIN) return bai_fail(bai, "bin number out of range");
+                all.push_back({bin, {cb, ce}});
+            }
+        }
+        std::stable_sort(all.begin(), all.end(), [](const auto &x, const auto &y) { return x.first < y.first; });
+        for (const auto &e : all) {
+            if (R.bins.empty() || R.bins.back() != e.first) {
+                R.bins.push_back(e.first);
+                R.bin_ptr.push_back((int64_t)R.chunks.size() / 2);
+            }
+            R.chunks.push_back(e.second.first);
+            R.chunks.push_back(e.second.second);
+        }
+        R.bin_ptr.push_back((int64_t)R.chunks.size() / 2);
+        if (!need(4)) return bai_fail(bai, "truncated");
+        const int32_t n_intv = (int32_t)rd32(&f[o]);
+        o += 4;
+        if (n_intv < 0 || !need(8ull * (uint64_t)n_intv)) return bai_fail(bai, "truncated");
+        R.linear.resize((size_t)n_intv);
+        if (n_intv) memcpy(R.linear.data(), &f[o], 8ull * (uint64_t)n_intv);
+        o += 8ull * (uint64_t)n_intv;
+    }
+    // an optional n_no_coor may follow
+    return XG_OK;
+}
+
+// The BGZF block at file offset `coff`: its total and inflated sizes; false when no block header is there.
+bool block_at(FILE *fp, uint64_t coff, uint32_t *total, uint32_t *isize) {
+    uint8_t h[18], t4[4];
+    if (fseeko(fp, (off_t)coff, SEEK_SET) != 0 || fread(h, 1, 18, fp) != 18) return false;
+    uint32_t hl = 0;
+    if (bgzf_block_header(h, 18, total, &hl) != 0) return false;
+    if (fseeko(fp, (off_t)(coff + *total - 4), SEEK_SET) != 0 || fread(t4, 1, 4, fp) != 4) return false;
+    *isize = rd32(t4);
+    return true;
+}
+
+}  // namespace
+
+extern "C" int xg_bam_index_open(const char *bam_path, xg_bam_index **out) {
+    if (!bam_path || !out) return fail(XG_E_ARG, "xg_bam_index_open: null argument");
+    *out = nullptr;
+    std::string bam(bam_path), bai = bam + ".bai";
+    struct stat st_bai, st_bam;
+    if (stat(bai.c_str(), &st_bai) != 0) {
+        if (bam.size() > 4 && bam.compare(bam.size() - 4, 4, ".bam") == 0) bai = bam.substr(0, bam.size() - 4) + ".bai";
+        if (stat(bai.c_str(), &st_bai) != 0) return XG_OK;     // no index: the caller reads the whole file
+    }
+    if (stat(bam_path, &st_bam) != 0) return fail(XG_E_IO, std::string("cannot open '") + bam + "'");
+    if (st_bai.st_mtime < st_bam.st_mtime) return bai_fail(bai, "it is older than the BAM");
+    std::unique_ptr<xg_bam_index> idx(new (std::nothrow) xg_bam_index());
+    if (!idx) return fail(XG_E_NOMEM, "out of memory");
+    idx->bam_path = bam;
+    idx->bam_size = (uint64_t)st_bam.st_size;
+    {
+        Bytes f;
+        int rc = read_file(bai.c_str(), f);
+        if (rc) return rc;
+        try {
+            rc = bai_parse(f, bai, *idx);
+        } catch (const std::exception &e) {
+            return fail(XG_E_NOMEM, std::string("reading '") + bai + "': " + e.what());
+        }
+        if (rc) return rc;
+    }
+    BamFile bf;
+    int rc = open_bam(bam_path, bf, true);
+    if (rc) return rc;
+    if (bf.h.names.size() != idx->refs.size())
+        return bai_fail(bai, "it lists " + std::to_string(idx->refs.size()) + " contigs, the BAM header " +
+                                 std::to_string(bf.h.names.size()));
+    for (const auto &R : idx->refs) {
+        for (uint64_t v : R.chunks)
+            if ((v >> 16) >= idx->bam_size) return bai_fail(bai, "an offset lies beyond the end of the BAM");
+        for (uint64_t v : R.linear)
+            if ((v >> 16) >= idx->bam_size) return bai_fail(bai, "an offset lies beyond the end of the BAM");
+    }
+    *out = idx.release();
+    return XG_OK;
+}
+
+extern "C" void xg_bam_index_free(xg_bam_index *idx) { delete idx; }
+
+extern "C" int32_t xg_bam_index_n_ref(const xg_bam_index *idx) { return idx ? (int32_t)idx->refs.size() : 0; }
+
+extern "C" int xg_bam_index_ref(const xg_bam_index *idx, int32_t tid, int64_t *n_bins, const uint32_t **bins,
+                                const int64_t **bin_ptr, const uint64_t **chunks, int64_t *n_intv,
+                                const uint64_t **linear) {
+    if (!idx || tid < 0 || tid >= (int32_t)idx->refs.size()) return fail(XG_E_ARG, "xg_bam_index_ref: no such contig");
+    const xg_bam_index::Ref &R = idx->refs[(size_t)tid];
+    *n_bins = (int64_t)R.bins.size();
+    *bins = R.bins.data();
+    *bin_ptr = R.bin_ptr.data();
+    *chunks = R.chunks.data();
+    *n_intv = (int64_t)R.linear.size();
+    *linear = R.linear.data();
+    return XG_OK;
+}
+
+static int bam_index_ranges_impl(const xg_bam_index *idx, int64_t n, const int32_t *tid, const int64_t *beg,
+                                 const int64_t *end, int64_t **ranges, int64_t *n_ranges) {
+    // (tid, bin) -> the smallest linear-index offset among the intervals that visit the bin
+    std::unordered_map<uint64_t, uint64_t> visit;
+    for (int64_t i = 0; i < n; i++) {
+        if (tid[i] < 0 || tid[i] >= (int32_t)idx->refs.size()) continue;
+        const int64_t b = std::max<int64_t>(0, beg[i]), e = std::min<int64_t>(end[i], (int64_t)1 << 29);
+        if (e <= b) continue;
+        const xg_bam_index::Ref &R = idx->refs[(size_t)tid[i]];
+        if (R.bins.empty()) continue;
+        const uint64_t w = (uint64_t)b >> 14;
+        const uint64_t min_off = w < R.linear.size() ? R.linear[w] : 0;
+        const int64_t last = e - 1;
+        const int shifts[6] = {29, 26, 23, 20, 17, 14};
+        const uint32_t firsts[6] = {0, 1, 9, 73, 585, 4681};
+        for (int l = 0; l < 6; l++)
+            for (uint32_t k = firsts[l] + (uint32_t)(b >> shifts[l]); k <= firsts[l] + (uint32_t)(last >> shifts[l]); k++) {
+                if (!std::binary_search(R.bins.begin(), R.bins.end(), k)) continue;
+                const uint64_t key = ((uint64_t)(uint32_t)tid[i] << 32) | k;
+                auto it = visit.find(key);
+                if (it == visit.end()) visit.emplace(key, min_off);
+                else it->second = std::min(it->second, min_off);
+            }
+    }
+    std::vector<std::pair<uint64_t, uint64_t>> ch;
+    for (const auto &kv : visit) {
+        const xg_bam_index::Ref &R = idx->refs[(size_t)(kv.first >> 32)];
+        const size_t j = (size_t)(std::lower_bound(R.bins.begin(), R.bins.end(), (uint32_t)kv.first) - R.bins.begin());
+        for (int64_t c = R.bin_ptr[j]; c < R.bin_ptr[j + 1]; c++) {
+            const uint64_t cb = R.chunks[2 * (size_t)c], ce = R.chunks[2 * (size_t)c + 1];
+            if (ce > kv.second && ce > cb) ch.push_back({cb, ce});
+        }
+    }
+    std::sort(ch.begin(), ch.end());
+    std::vector<std::pair<uint64_t, uint64_t>> vm;              // merged in virtual offsets
+    for (const auto &c : ch) {
+        if (!vm.empty() && c.first <= vm.back().second) vm.back().second = std::max(vm.back().second, c.second);
+        else vm.push_back(c);
+    }
+    std::vector<int64_t> out;
+    FILE *fp = vm.empty() ? nullptr : fopen(idx->bam_path.c_str(), "rb");
+    if (!vm.empty() && !fp) return fail(XG_E_IO, "cannot open '" + idx->bam_path + "'");
+    auto bad = [&](const std::string &why) {
+        fclose(fp);
+        return fail(XG_E_FORMAT, "index of '" + idx->bam_path + "' is not used: " + why);
+    };
+    for (const auto &c : vm) {
+        const uint64_t lo = c.first >> 16, last = c.second >> 16;
+        uint32_t total = 0, isize = 0;
+        uint64_t hi = last;
+        if (c.second & 0xffff) {                                // the last chunk ends inside block `last`
+            if (!block_at(fp, last, &total, &isize)) return bad("offset " + std::to_string(last) + " is not a BGZF block start");
+            hi = last + total;
+        }
+        if (hi > idx->bam_size) return bad("an offset lies beyond the end of the BAM");
+        if (hi <= lo) continue;
+        if (!out.empty() && (int64_t)lo <= out.back() + XG_BAM_INDEX_MERGE_GAP) {     // close enough: read the gap too
+            out.back() = std::max<int64_t>(out.back(), (int64_t)hi);
+            continue;
+        }
+        if (!block_at(fp, lo, &total, &isize)) return bad("offset " + std::to_string(lo) + " is not a BGZF block start");
+        if ((c.first & 0xffff) >= isize) return bad("a record offset lies beyond its block");
+        out.push_back((int64_t)c.first);                        // the virtual offset of the range's first record
+        out.push_back((int64_t)hi);
+    }
+    if (fp) fclose(fp);
+    int64_t *o = (int64_t *)malloc(std::max<size_t>(1, out.size()) * sizeof(int64_t));
+    if (!o) return fail(XG_E_NOMEM, "out of memory");
+    if (!out.empty()) memcpy(o, out.data(), out.size() * sizeof(int64_t));
+    *ranges = o;
+    *n_ranges = (int64_t)out.size() / 2;
+    return XG_OK;
+}
+
+extern "C" int xg_bam_index_ranges(const xg_bam_index *idx, int64_t n, const int32_t *tid, const int64_t *beg,
+                                   const int64_t *end, int64_t **ranges, int64_t *n_ranges) {
+    if (!idx || n < 0 || (n && (!tid || !beg || !end)) || !ranges || !n_ranges)
+        return fail(XG_E_ARG, "xg_bam_index_ranges: bad argument");
+    try {
+        return bam_index_ranges_impl(idx, n, tid, beg, end, ranges, n_ranges);
+    } catch (const std::exception &e) {
+        return fail(XG_E_NOMEM, std::string("xg_bam_index_ranges: ") + e.what());
+    }
 }

@@ -156,6 +156,13 @@ __device__ __forceinline__ RecGeom rec_geom(const uint8_t *r, uint32_t bs, bool 
     return o;
 }
 
+// Where the records of a block start: behind the header, and behind the head of a range's first block that comes
+// before the record the range starts at.
+__device__ __forceinline__ uint32_t walk_start(const BgzfBlockDev &bk, unsigned long long hdr_end) {
+    const uint32_t h = bk.uoff < hdr_end ? (uint32_t)(hdr_end - bk.uoff) : 0u;
+    return h > bk.skip ? h : bk.skip;
+}
+
 // One thread per BGZF block: check that the block holds whole records in coordinate order and
 // size what the kept ones will store.
 __global__ void k_walk(const BgzfBlockDev *blocks, int32_t n_blocks, unsigned long long hdr_end,
@@ -173,7 +180,7 @@ __global__ void k_walk(const BgzfBlockDev *blocks, int32_t n_blocks, unsigned lo
         info[b] = bi;
         return;
     }
-    uint32_t off = bk.uoff < hdr_end ? (uint32_t)(hdr_end - bk.uoff) : 0u;      // offsets within the block
+    uint32_t off = walk_start(bk, hdr_end);                                      // offsets within the block
     const uint32_t end = bk.isize;
     int32_t max_aln = 0, max_span = 0, prev_kept_tid = -2;
     while (off < end) {
@@ -449,7 +456,7 @@ __global__ void __launch_bounds__(EXTRACT_THREADS) k_extract(const ExtractArgs a
         return;
     }
     const BgzfBlockDev bk = a.blocks[b];
-    uint32_t off = bk.uoff < a.hdr_end ? (uint32_t)(a.hdr_end - bk.uoff) : 0u;      // uniform: the next link
+    uint32_t off = walk_start(bk, a.hdr_end);                                      // uniform: the next link
     const uint32_t end = bk.isize;
     unsigned long long g0 = a.rec_base[b], co0 = a.cig_base[b], so0 = a.seq_base[b];
     int32_t prev_tid = -2;                 // contig of the last kept record before this batch
@@ -565,7 +572,7 @@ __global__ void k_keys_gather(const ExtractArgs a, const unsigned long long *req
     if (b >= a.n_blocks) return;
     if (a.hk[b].x == 0) return;
     const BgzfBlockDev bk = a.blocks[b];
-    uint32_t off = bk.uoff < a.hdr_end ? (uint32_t)(a.hdr_end - bk.uoff) : 0u;
+    uint32_t off = walk_start(bk, a.hdr_end);
     const uint32_t end = bk.isize;
     unsigned long long g = a.rec_base[b], ri = req_base[b], so = str_base[b];
     while (off < end) {
@@ -740,6 +747,7 @@ struct Decoder {
     int32_t max_aln = 0, max_span = 0;
     std::vector<RunStart> starts;
     uint64_t comp_all = 0, comp_done = 0;     // compressed bytes of all BAMs / consumed so far (sizes the batch)
+    uint64_t bytes_read = 0;                  // compressed bytes read from the files, headers included
     double t_read = 0, t_stream = 0, t_walk = 0, t_extract = 0, t_alloc = 0;
     int n_windows = 0;
 
@@ -816,6 +824,7 @@ struct BamState {                       // per BAM, across its windows
     int32_t bam_idx, n_ref = 0;
     uint64_t hdr_end = 0;
     unsigned long long last_key = 0;
+    bool seeks = false;                 // read in ranges: a record that does not parse may be a range's wrong start
 };
 
 // The values of the window that do not pack into 63 bits: their strings are gathered on the
@@ -938,12 +947,15 @@ int flush_window(Decoder &D, BamState &B, int32_t nb) {
     int64_t kept = 0, cig = 0, seq = 0, n_all = 0, n_starts = 0;
     for (int32_t b = 0; b < nb; b++) {
         const BlkInfo &bi = h_info[(size_t)b];
-        if (bi.status == 2) return ctx->fail(XG_E_FORMAT, std::string("corrupt BAM record in '") + B.path + "'");
-        if (bi.status == 3) return ctx->fail(XG_E_FORMAT, std::string("'") + B.path + "' is not coordinate sorted");
+        // Read in ranges, a block of a BAM whose records cross blocks may start inside a record and parse as
+        // garbage: the host decoder then reads the whole file and reports what is wrong with it, if anything.
+        const int bad = B.seeks ? XG_E_UNSUPPORTED : XG_E_FORMAT;
+        if (bi.status == 2) return ctx->fail(bad, std::string("corrupt BAM record in '") + B.path + "'");
+        if (bi.status == 3) return ctx->fail(bad, std::string("'") + B.path + "' is not coordinate sorted");
         if (bi.status == 1)
             return ctx->fail(XG_E_UNSUPPORTED, std::string("records of '") + B.path + "' cross BGZF block boundaries");
         if (bi.n_all) {
-            if (bi.first_key < B.last_key) return ctx->fail(XG_E_FORMAT, std::string("'") + B.path + "' is not coordinate sorted");
+            if (bi.first_key < B.last_key) return ctx->fail(bad, std::string("'") + B.path + "' is not coordinate sorted");
             B.last_key = bi.last_key;
         }
         bases[(size_t)b] = (unsigned long long)(D.n_total + kept);
@@ -1026,12 +1038,16 @@ int flush_window(Decoder &D, BamState &B, int32_t nb) {
 }
 
 // Stream one BAM through the window buffers.
-// range_lo / range_hi (range_hi > 0): only the BGZF blocks in [range_lo, range_hi) of the file -- both must be block
-// starts (or the file's end), and the block at range_lo must begin with a record (htslib's layout; the caller takes
-// the offsets from xg_bgzf_block_index / xg_bam_block_probe).  The header is still read from the file's beginning.
+// ranges: ascending, disjoint (lo, hi): lo the virtual offset of the range's first record (its block's file offset
+// << 16 | the record's offset in the inflated block), hi the file offset of the block after the range (or the file's
+// end).  The walk of the range's first block starts at that record; the caller takes lo from the .bai, or a block
+// start that begins with a record from xg_bgzf_block_index / xg_bam_block_probe.  The ranges go through the same
+// chunks and windows one after the other: a window holds the blocks of several ranges back to back, and the bytes
+// between ranges are never read.  The header is read from the file's beginning.
 int decode_bam(Decoder &D, const char *path, int32_t bam_idx, const int32_t *tid_map, int32_t tid_map_len,
-               int64_t range_lo = 0, int64_t range_hi = 0) {
+               const std::vector<std::pair<uint64_t, uint64_t>> &ranges) {
     xg_ctx *ctx = D.ctx;
+    if (ranges.empty()) return XG_OK;
     const int fd = open(path, O_RDONLY);
     struct stat stt;
     if (fd < 0 || fstat(fd, &stt) != 0) {
@@ -1039,12 +1055,13 @@ int decode_bam(Decoder &D, const char *path, int32_t bam_idx, const int32_t *tid
         return ctx->fail(XG_E_IO, std::string("cannot open '") + path + "'");
     }
     const uint64_t fsize = (uint64_t)stt.st_size;
-    const bool ranged = range_hi > 0;
-    if (ranged && (range_lo < 0 || range_lo > range_hi || (uint64_t)range_hi > fsize)) {
-        close(fd);
-        return ctx->fail(XG_E_ARG, "xg_decode_bams_device_range: byte range outside the file");
-    }
-    const uint64_t csize = ranged ? (uint64_t)range_hi : fsize;     // the streaming loop ends here
+    for (size_t r = 0; r < ranges.size(); r++)
+        if ((ranges[r].first >> 16) >= ranges[r].second || ranges[r].second > fsize ||
+            (r && (ranges[r].first >> 16) < ranges[r - 1].second)) {
+            close(fd);
+            return ctx->fail(XG_E_ARG, std::string("xg_decode_bams_device_ranges: the ranges of '") + path +
+                                           "' are not ascending, disjoint and inside the file");
+        }
     const size_t STAGE_BYTES = stage_bytes();
     uint8_t *stage[2] = {(uint8_t *)ctx->pinned_get(STAGE_HEAD + STAGE_BYTES), (uint8_t *)ctx->pinned_get(STAGE_HEAD + STAGE_BYTES)};
     // the chunk's block descriptors travel through pinned memory too: a copy from pageable memory
@@ -1068,11 +1085,11 @@ int decode_bam(Decoder &D, const char *path, int32_t bam_idx, const int32_t *tid
         return finish(XG_E_NOMEM, "out of pinned host memory for the staging buffers");
     cudaEventCreateWithFlags(&done[0], cudaEventDisableTiming);
     cudaEventCreateWithFlags(&done[1], cudaEventDisableTiming);
-    if (csize == 0) return finish(XG_E_FORMAT, std::string("'") + path + "' is not BGZF (empty file)");
     const int n_threads = (int)std::max(1u, std::min(8u, std::thread::hardware_concurrency()));
     BamState B;
     B.path = path;
     B.bam_idx = bam_idx;
+    B.seeks = !(ranges.size() == 1 && ranges[0].first == 0 && ranges[0].second == fsize);
     uint64_t next_off = 0, uoff = 0;
     const uint8_t *prev_data = nullptr;
     size_t prev_len = 0;
@@ -1085,42 +1102,63 @@ int decode_bam(Decoder &D, const char *path, int32_t bam_idx, const int32_t *tid
     size_t win_infl = 0;
     int32_t win_blocks = 0;
     bool win_open = false;
+    uint64_t win_used = 0;                         // compressed bytes the open window holds
     const double t_loop = now_ms();
-    uint64_t c_begin = 0;
-    if (ranged && range_lo > 0) {
-        // the header comes from the file's first blocks (host inflate); the stream then starts at range_lo
-        const size_t len = (size_t)std::min<uint64_t>(STAGE_BYTES, fsize);
-        uint8_t *data = stage[0] + STAGE_HEAD;
-        if (!pread_parallel(fd, data, len, 0, n_threads)) return finish(XG_E_IO, std::string("short read on '") + path + "'");
-        uint64_t off = 0, uo = 0;
-        while (off < len) {
-            uint32_t total = 0, hl = 0;
-            int rc = xg_dec::bgzf_block_header(data + off, len - off, &total, &hl);
-            if (rc != 0 || off + total > len) break;
-            xg_dec::BgzfBlock b;
-            b.coff = off + hl;
-            b.clen = total - hl - 8;
-            memcpy(&b.isize, data + off + total - 4, 4);
-            memcpy(&b.crc, data + off + total - 8, 4);
-            b.uoff = uo;
-            uo += b.isize;
-            hb.push_back(b);
-            off += total;
+    // the blocks that hold header bytes: (file offset, offset in the inflated stream), and where they end
+    std::vector<std::pair<uint64_t, uint64_t>> hdr_blk;
+    uint64_t hdr_cend = 0;
+    auto note_header_blocks = [&] {
+        uint64_t at = 0;
+        for (size_t i = 0; i < hb.size() && hb[i].uoff < hdr.end_off; i++) {
+            hdr_blk.push_back({at, hb[i].uoff});
+            at = hb[i].coff + hb[i].clen + 8;
         }
-        size_t nb = 1;
+        hdr_cend = at;
+    };
+    if ((ranges[0].first >> 16) > 0) {
+        // the header comes from the file's first blocks (host inflate); the stream then starts at the first range
+        size_t len = (size_t)std::min<uint64_t>(std::min<size_t>(STAGE_BYTES, 64u << 10), fsize);    // grows x4
+        uint8_t *data = stage[0] + STAGE_HEAD;
         while (true) {
+            const double t0 = now_ms();
+            if (!pread_parallel(fd, data, len, 0, n_threads)) return finish(XG_E_IO, std::string("short read on '") + path + "'");
+            D.t_read += now_ms() - t0;
+            D.bytes_read += len;
+            hb.clear();
+            uint64_t off = 0, uo = 0;
+            while (off < len) {
+                uint32_t total = 0, hl = 0;
+                int rc = xg_dec::bgzf_block_header(data + off, len - off, &total, &hl);
+                if (rc != 0 || off + total > len) break;
+                xg_dec::BgzfBlock b;
+                b.coff = off + hl;
+                b.clen = total - hl - 8;
+                memcpy(&b.isize, data + off + total - 4, 4);
+                memcpy(&b.crc, data + off + total - 8, 4);
+                b.uoff = uo;
+                uo += b.isize;
+                hb.push_back(b);
+                off += total;
+            }
             if (hb.empty()) return finish(XG_E_FORMAT, std::string("'") + path + "' is not BGZF (bad block header)");
-            const size_t take = std::min(nb, hb.size());
-            xg_dec::Bytes u;
-            int rc = xg_dec::inflate_blocks(data, 0, hb.data(), take, u, 1);
-            if (rc) return finish(rc, xg_host_last_error());
-            rc = xg_dec::parse_header(u, hdr, path);
+            size_t nb = 1;
+            int rc;
+            while (true) {
+                const size_t take = std::min(nb, hb.size());
+                xg_dec::Bytes u;
+                rc = xg_dec::inflate_blocks(data, 0, hb.data(), take, u, 1);
+                if (rc) return finish(rc, xg_host_last_error());
+                rc = xg_dec::parse_header(u, hdr, path);
+                if (rc != XG_E_LIMIT || take >= hb.size()) break;
+                nb *= 2;
+            }
             if (rc == XG_OK) break;
             if (rc != XG_E_LIMIT) return finish(rc, xg_host_last_error());
-            if (take >= hb.size())
+            if (len >= std::min<uint64_t>(STAGE_BYTES, fsize))
                 return finish(XG_E_UNSUPPORTED, std::string("BAM header of '") + path + "' does not end within the first staged chunk");
-            nb *= 2;
+            len = (size_t)std::min<uint64_t>(std::min<uint64_t>(STAGE_BYTES, fsize), 4 * (uint64_t)len);   // read more
         }
+        note_header_blocks();
         hb.clear();
         header_done = true;
         B.hdr_end = hdr.end_off;
@@ -1134,142 +1172,163 @@ int decode_bam(Decoder &D, const char *path, int32_t bam_idx, const int32_t *tid
         }
         cudaMemcpyAsync(D.d_tid_map, tid_map, (size_t)B.n_ref * 4, cudaMemcpyHostToDevice, ctx->stream);
         cudaStreamSynchronize(ctx->stream);          // stage[0] is about to be reused
-        c_begin = next_off = (uint64_t)range_lo;
-        uoff = hdr.end_off;                           // every block of the range lies behind the header
     }
     uint64_t k = 0;
-    for (uint64_t c0 = c_begin; c0 < csize; c0 += STAGE_BYTES, k++) {
-        const int si = (int)(k & 1);
-        const size_t len = (size_t)std::min<uint64_t>(STAGE_BYTES, csize - c0);
-        if (k >= 2) cudaEventSynchronize(done[si]);
-        uint8_t *data = stage[si] + STAGE_HEAD;
-        const size_t carry = (size_t)(c0 - next_off);
-        if (carry) memcpy(data - carry, prev_data + prev_len - carry, carry);
-        const double t0 = now_ms();
-        if (!pread_parallel(fd, data, len, c0, n_threads)) return finish(XG_E_IO, std::string("short read on '") + path + "'");
-        D.t_read += now_ms() - t0;
-        const uint64_t view_beg = next_off, view_end = c0 + len;
-        hb.clear();
-        size_t chunk_infl = 0;
-        while (next_off < view_end) {
-            const uint8_t *p = data - (c0 - next_off);      // next_off >= c0 - carry
-            uint32_t total = 0, hl = 0;
-            int rc = xg_dec::bgzf_block_header(p, view_end - next_off, &total, &hl);
-            if (rc == 0 && next_off + total > view_end) rc = 1;
-            if (rc == 1) {
-                if (view_end == csize) return finish(XG_E_FORMAT, std::string("truncated BGZF block in '") + path + "'");
-                break;
+    for (size_t ri = 0; ri < ranges.size(); ri++) {
+        const uint64_t c_begin = ranges[ri].first >> 16, csize = ranges[ri].second;     // this range's streaming loop
+        const uint32_t skip = (uint32_t)(ranges[ri].first & 0xffff);                     // ... and its first record
+        next_off = c_begin;
+        if (header_done) {
+            // the inflated offset only tells the walk where the header ends: a block behind the header gets any offset
+            // past it, a header block its own
+            if (c_begin < hdr_cend) {
+                auto it = std::find_if(hdr_blk.begin(), hdr_blk.end(),
+                                       [&](const std::pair<uint64_t, uint64_t> &x) { return x.first == c_begin; });
+                if (it == hdr_blk.end())
+                    return finish(XG_E_ARG, std::string("xg_decode_bams_device_ranges: offset ") + std::to_string(c_begin) +
+                                                " of '" + path + "' is not a BGZF block start");
+                uoff = it->second;
+            } else {
+                uoff = std::max<uint64_t>(uoff, hdr.end_off);
             }
-            if (rc < 0) return finish(XG_E_FORMAT, std::string("'") + path + "' is not BGZF (bad block header)");
-            xg_dec::BgzfBlock b;
-            b.coff = next_off + hl;
-            b.clen = total - hl - 8;
-            memcpy(&b.isize, p + total - 4, 4);
-            memcpy(&b.crc, p + total - 8, 4);
-            b.uoff = uoff;
-            if (b.isize > 65536) return finish(XG_E_FORMAT, "BGZF block larger than 64 KiB");
-            uoff += b.isize;
-            chunk_infl += b.isize;
-            hb.push_back(b);
-            next_off += total;
         }
-        if (view_end - next_off > STAGE_HEAD) return finish(XG_E_FORMAT, "BGZF block larger than 64 KiB");
-        if (!header_done) {
-            // the BAM header: inflate leading blocks on the host until it parses
-            size_t nb = 1;
-            while (true) {
-                const size_t take = std::min(nb, hb.size());
-                xg_dec::Bytes u;
-                int rc = xg_dec::inflate_blocks(data, c0, hb.data(), take, u, 1);
-                if (rc) return finish(rc, xg_host_last_error());
-                rc = xg_dec::parse_header(u, hdr, path);
-                if (rc == XG_OK) break;
-                if (rc != XG_E_LIMIT) return finish(rc, xg_host_last_error());
-                if (take >= hb.size())
-                    return finish(view_end == csize ? XG_E_FORMAT : XG_E_UNSUPPORTED,
-                                  std::string("BAM header of '") + path + "' does not end within the first staged chunk");
-                nb *= 2;
-            }
-            header_done = true;
-            B.hdr_end = hdr.end_off;
-            B.n_ref = (int32_t)hdr.names.size();
-            if (tid_map_len < B.n_ref) return finish(XG_E_ARG, "tid_map shorter than the BAM's contig list");
-            if ((size_t)B.n_ref + 1 > D.tid_cap) {
-                ctx->dev_put(D.d_tid_map);
-                D.tid_cap = (size_t)B.n_ref + 1;
-                D.d_tid_map = (int32_t *)ctx->dev_get(D.tid_cap * 4);
-                if (!D.d_tid_map) return finish(XG_E_CUDA, "out of device memory");
-            }
-            cudaMemcpyAsync(D.d_tid_map, tid_map, (size_t)B.n_ref * 4, cudaMemcpyHostToDevice, ctx->stream);
-        }
-        // does the chunk fit the open window?
-        if (win_open && ((size_t)(view_end - win_base) > D.comp_cap || win_infl + chunk_infl + 16 > D.slab_cap ||
-                         (size_t)win_blocks + hb.size() > D.blk_cap)) {
-            int rc = flush_window(D, B, win_blocks);
-            if (rc) return finish(rc, ctx->err);
-            win_open = false;
-        }
-        if (!win_open) {
-            // an empty window takes any chunk: grow the buffers if this one alone is too large
-            if (chunk_infl + 16 > D.slab_cap || hb.size() > D.blk_cap) {
-                cudaStreamSynchronize(ctx->stream);
-                if (chunk_infl + 16 > D.slab_cap) {
-                    ctx->dev_put(D.slab);
-                    D.slab_cap = chunk_infl + chunk_infl / 4 + 16;
-                    D.slab = (uint8_t *)ctx->dev_get(D.slab_cap);
+        if (win_open) win_base = c_begin - win_used;     // the range continues the open window where the last one ended
+        for (uint64_t c0 = c_begin; c0 < csize; c0 += STAGE_BYTES, k++) {
+            const int si = (int)(k & 1);
+            const size_t len = (size_t)std::min<uint64_t>(STAGE_BYTES, csize - c0);
+            if (k >= 2) cudaEventSynchronize(done[si]);
+            uint8_t *data = stage[si] + STAGE_HEAD;
+            const size_t carry = (size_t)(c0 - next_off);
+            if (carry) memcpy(data - carry, prev_data + prev_len - carry, carry);
+            const double t0 = now_ms();
+            if (!pread_parallel(fd, data, len, c0, n_threads)) return finish(XG_E_IO, std::string("short read on '") + path + "'");
+            D.t_read += now_ms() - t0;
+            const uint64_t view_beg = next_off, view_end = c0 + len;
+            hb.clear();
+            size_t chunk_infl = 0;
+            while (next_off < view_end) {
+                const uint8_t *p = data - (c0 - next_off);      // next_off >= c0 - carry
+                uint32_t total = 0, hl = 0;
+                int rc = xg_dec::bgzf_block_header(p, view_end - next_off, &total, &hl);
+                if (rc == 0 && next_off + total > view_end) rc = 1;
+                if (rc == 1) {
+                    if (view_end == csize) return finish(XG_E_FORMAT, std::string("truncated BGZF block in '") + path + "'");
+                    break;
                 }
-                if (hb.size() > D.blk_cap) {
-                    ctx->dev_put(D.blocks);
-                    ctx->dev_put(D.info);
-                    ctx->dev_put(D.bases);
-                    D.blk_cap = hb.size() + hb.size() / 4;
-                    ctx->dev_put(D.hk);
-                    D.blocks = (BgzfBlockDev *)ctx->dev_get((D.blk_cap + 1) * sizeof(BgzfBlockDev));
-                    D.info = (BlkInfo *)ctx->dev_get((D.blk_cap + 1) * sizeof(BlkInfo));
-                    D.bases = (unsigned long long *)ctx->dev_get((3 * D.blk_cap + 1) * 8);
-                    D.hk = (uint2 *)ctx->dev_get((D.blk_cap + 1) * sizeof(uint2));
+                if (rc < 0) return finish(XG_E_FORMAT, std::string("'") + path + "' is not BGZF (bad block header)");
+                xg_dec::BgzfBlock b;
+                b.coff = next_off + hl;
+                b.clen = total - hl - 8;
+                memcpy(&b.isize, p + total - 4, 4);
+                memcpy(&b.crc, p + total - 8, 4);
+                b.uoff = uoff;
+                if (b.isize > 65536) return finish(XG_E_FORMAT, "BGZF block larger than 64 KiB");
+                uoff += b.isize;
+                chunk_infl += b.isize;
+                hb.push_back(b);
+                next_off += total;
+            }
+            if (view_end - next_off > STAGE_HEAD) return finish(XG_E_FORMAT, "BGZF block larger than 64 KiB");
+            if (!header_done) {
+                // the BAM header: inflate leading blocks on the host until it parses
+                size_t nb = 1;
+                while (true) {
+                    const size_t take = std::min(nb, hb.size());
+                    xg_dec::Bytes u;
+                    int rc = xg_dec::inflate_blocks(data, c0, hb.data(), take, u, 1);
+                    if (rc) return finish(rc, xg_host_last_error());
+                    rc = xg_dec::parse_header(u, hdr, path);
+                    if (rc == XG_OK) break;
+                    if (rc != XG_E_LIMIT) return finish(rc, xg_host_last_error());
+                    if (take >= hb.size())
+                        return finish(view_end == csize ? XG_E_FORMAT : XG_E_UNSUPPORTED,
+                                      std::string("BAM header of '") + path + "' does not end within the first staged chunk");
+                    nb *= 2;
                 }
-                if (!D.slab || !D.blocks || !D.info || !D.bases || !D.hk)
-                    return finish(XG_E_UNSUPPORTED, "the inflate window does not fit the device");
+                header_done = true;
+                B.hdr_end = hdr.end_off;
+                B.n_ref = (int32_t)hdr.names.size();
+                if (tid_map_len < B.n_ref) return finish(XG_E_ARG, "tid_map shorter than the BAM's contig list");
+                if ((size_t)B.n_ref + 1 > D.tid_cap) {
+                    ctx->dev_put(D.d_tid_map);
+                    D.tid_cap = (size_t)B.n_ref + 1;
+                    D.d_tid_map = (int32_t *)ctx->dev_get(D.tid_cap * 4);
+                    if (!D.d_tid_map) return finish(XG_E_CUDA, "out of device memory");
+                }
+                cudaMemcpyAsync(D.d_tid_map, tid_map, (size_t)B.n_ref * 4, cudaMemcpyHostToDevice, ctx->stream);
+                note_header_blocks();
             }
-            win_open = true;
-            win_base = view_beg;       // a fresh window starts at the carried bytes of the cut block
-            win_infl = 0;
-            win_blocks = 0;
-            cudaStreamWaitEvent(ctx->copy_stream, D.ev_win, 0);     // the previous window has left the buffers
-        }
-        const uint64_t up_off = win_blocks == 0 && win_infl == 0 && win_base == view_beg ? view_beg : c0;
-        cudaMemcpyAsync(D.comp + (up_off - win_base), data - (c0 - up_off), (size_t)(view_end - up_off),
-                        cudaMemcpyHostToDevice, ctx->copy_stream);
-        dv.resize(hb.size());
-        for (size_t i = 0; i < hb.size(); i++) {
-            dv[i].coff = hb[i].coff - win_base;
-            dv[i].clen = hb[i].clen;
-            dv[i].isize = hb[i].isize;
-            dv[i].uoff = hb[i].uoff;
-            dv[i].uptr = D.slab + win_infl;
-            dv[i].crc = hb[i].crc;
-            dv[i].pad_ = 0;
-            win_infl += hb[i].isize;
-        }
-        if (!dv.empty()) {
-            const BgzfBlockDev *src = dv.data();
-            if (dv.size() * sizeof(BgzfBlockDev) <= DESC_STAGE) {
-                memcpy(desc_stage[si], dv.data(), dv.size() * sizeof(BgzfBlockDev));
-                src = desc_stage[si];
+            // does the chunk fit the open window?
+            if (win_open && ((size_t)(view_end - win_base) > D.comp_cap || win_infl + chunk_infl + 16 > D.slab_cap ||
+                             (size_t)win_blocks + hb.size() > D.blk_cap)) {
+                int rc = flush_window(D, B, win_blocks);
+                if (rc) return finish(rc, ctx->err);
+                win_open = false;
             }
-            cudaMemcpyAsync(D.blocks + win_blocks, src, dv.size() * sizeof(BgzfBlockDev), cudaMemcpyHostToDevice,
-                            ctx->copy_stream);
+            if (!win_open) {
+                // an empty window takes any chunk: grow the buffers if this one alone is too large
+                if (chunk_infl + 16 > D.slab_cap || hb.size() > D.blk_cap) {
+                    cudaStreamSynchronize(ctx->stream);
+                    if (chunk_infl + 16 > D.slab_cap) {
+                        ctx->dev_put(D.slab);
+                        D.slab_cap = chunk_infl + chunk_infl / 4 + 16;
+                        D.slab = (uint8_t *)ctx->dev_get(D.slab_cap);
+                    }
+                    if (hb.size() > D.blk_cap) {
+                        ctx->dev_put(D.blocks);
+                        ctx->dev_put(D.info);
+                        ctx->dev_put(D.bases);
+                        D.blk_cap = hb.size() + hb.size() / 4;
+                        ctx->dev_put(D.hk);
+                        D.blocks = (BgzfBlockDev *)ctx->dev_get((D.blk_cap + 1) * sizeof(BgzfBlockDev));
+                        D.info = (BlkInfo *)ctx->dev_get((D.blk_cap + 1) * sizeof(BlkInfo));
+                        D.bases = (unsigned long long *)ctx->dev_get((3 * D.blk_cap + 1) * 8);
+                        D.hk = (uint2 *)ctx->dev_get((D.blk_cap + 1) * sizeof(uint2));
+                    }
+                    if (!D.slab || !D.blocks || !D.info || !D.bases || !D.hk)
+                        return finish(XG_E_UNSUPPORTED, "the inflate window does not fit the device");
+                }
+                win_open = true;
+                win_base = view_beg;       // a fresh window starts at the carried bytes of the cut block
+                win_infl = 0;
+                win_blocks = 0;
+                cudaStreamWaitEvent(ctx->copy_stream, D.ev_win, 0);     // the previous window has left the buffers
+            }
+            const uint64_t up_off = win_blocks == 0 && win_infl == 0 && win_base == view_beg ? view_beg : c0;
+            cudaMemcpyAsync(D.comp + (up_off - win_base), data - (c0 - up_off), (size_t)(view_end - up_off),
+                            cudaMemcpyHostToDevice, ctx->copy_stream);
+            dv.resize(hb.size());
+            for (size_t i = 0; i < hb.size(); i++) {
+                dv[i].coff = hb[i].coff - win_base;
+                dv[i].clen = hb[i].clen;
+                dv[i].isize = hb[i].isize;
+                dv[i].uoff = hb[i].uoff;
+                dv[i].uptr = D.slab + win_infl;
+                dv[i].crc = hb[i].crc;
+                dv[i].skip = c0 == c_begin && i == 0 ? skip : 0;
+                win_infl += hb[i].isize;
+            }
+            if (!dv.empty()) {
+                const BgzfBlockDev *src = dv.data();
+                if (dv.size() * sizeof(BgzfBlockDev) <= DESC_STAGE) {
+                    memcpy(desc_stage[si], dv.data(), dv.size() * sizeof(BgzfBlockDev));
+                    src = desc_stage[si];
+                }
+                cudaMemcpyAsync(D.blocks + win_blocks, src, dv.size() * sizeof(BgzfBlockDev), cudaMemcpyHostToDevice,
+                                ctx->copy_stream);
+            }
+            cudaEventRecord(done[si], ctx->copy_stream);
+            cudaStream_t ist = (k & 1) && D.ist2 ? D.ist2 : ctx->stream;
+            cudaStreamWaitEvent(ist, done[si], 0);
+            launch_inflate(ist, D.comp, D.blocks + win_blocks, (int32_t)dv.size(), D.cnt + 0);
+            if (ist != ctx->stream) cudaEventRecord(D.ev_i2, ist);
+            win_blocks += (int32_t)hb.size();
+            win_used = view_end - win_base;
+            D.comp_done += len;
+            D.bytes_read += len;
+            prev_data = data;
+            prev_len = len;
         }
-        cudaEventRecord(done[si], ctx->copy_stream);
-        cudaStream_t ist = (k & 1) && D.ist2 ? D.ist2 : ctx->stream;
-        cudaStreamWaitEvent(ist, done[si], 0);
-        launch_inflate(ist, D.comp, D.blocks + win_blocks, (int32_t)dv.size(), D.cnt + 0);
-        if (ist != ctx->stream) cudaEventRecord(D.ev_i2, ist);
-        win_blocks += (int32_t)hb.size();
-        D.comp_done += len;
-        prev_data = data;
-        prev_len = len;
     }
     D.t_stream += now_ms() - t_loop;
     if (win_open) {
@@ -1317,7 +1376,7 @@ int xg_bgzf_inflate_device(xg_ctx *ctx, const char *path, uint8_t *out, int64_t 
         dv[i].uoff = blocks[i].uoff;
         dv[i].uptr = ubuf + blocks[i].uoff;
         dv[i].crc = blocks[i].crc;
-        dv[i].pad_ = 0;
+        dv[i].skip = 0;
     }
     cudaMemcpyAsync(dblk, dv.data(), dv.size() * sizeof(BgzfBlockDev), cudaMemcpyHostToDevice, st);
     cudaMemsetAsync(cnt, 0, 8 * sizeof(int), st);
@@ -1339,19 +1398,49 @@ int xg_bgzf_inflate_device(xg_ctx *ctx, const char *path, uint8_t *out, int64_t 
     return XG_OK;
 }
 
+using RangeList = std::vector<std::pair<uint64_t, uint64_t>>;
+
 static int decode_bams_device_impl(xg_ctx *ctx, int32_t n_bams, const char *const *paths, const int32_t *const *tid_map,
                                    const int32_t *tid_map_len, const char *cell_tag, const char *umi_tag,
                                    int32_t want_seq, xg_keyspace *ks, xg_dreads **out, int64_t *n_records_seen,
-                                   const int64_t *range_lo, const int64_t *range_hi);
+                                   int64_t *bytes_read, const std::vector<RangeList> &ranges);
 
 // no C++ exception crosses the C boundary (host vectors of the block index, the key strings ...)
-int xg_decode_bams_device_range(xg_ctx *ctx, int32_t n_bams, const char *const *paths, const int32_t *const *tid_map,
-                                const int32_t *tid_map_len, const char *cell_tag, const char *umi_tag, int32_t want_seq,
-                                xg_keyspace *ks, const int64_t *range_lo, const int64_t *range_hi, xg_dreads **out,
-                                int64_t *n_records_seen) {
+static int decode_bams_device_guarded(xg_ctx *ctx, int32_t n_bams, const char *const *paths,
+                                      const int32_t *const *tid_map, const int32_t *tid_map_len, const char *cell_tag,
+                                      const char *umi_tag, int32_t want_seq, xg_keyspace *ks,
+                                      const int64_t *range_ptr, const int64_t *range_lo, const int64_t *range_hi,
+                                      bool one_range_each, xg_dreads **out, int64_t *n_records_seen,
+                                      int64_t *bytes_read) {
     try {
+        if (!ctx || !ctx->stream) return ctx ? ctx->fail(XG_E_CUDA, "context has no device") : XG_E_ARG;
+        if (n_bams < 0 || !paths) return ctx->fail(XG_E_ARG, "xg_decode_bams_device: bad argument");
+        std::vector<RangeList> ranges((size_t)n_bams);
+        for (int32_t b = 0; b < n_bams; b++) {
+            struct stat stt;
+            if (!paths[b] || stat(paths[b], &stt) != 0)
+                return ctx->fail(XG_E_IO, std::string("cannot open '") + (paths[b] ? paths[b] : "") + "'");
+            const uint64_t fsize = (uint64_t)stt.st_size;
+            if (fsize == 0) return ctx->fail(XG_E_FORMAT, std::string("'") + paths[b] + "' is not BGZF (empty file)");
+            if (one_range_each && range_hi && range_hi[b] > 0) {        // xg_decode_bams_device_range
+                if (range_lo[b] < 0 || range_lo[b] > range_hi[b] || (uint64_t)range_hi[b] > fsize)
+                    return ctx->fail(XG_E_ARG, "xg_decode_bams_device_range: byte range outside the file");
+                if (range_lo[b] < range_hi[b])
+                    ranges[(size_t)b].push_back({(uint64_t)range_lo[b] << 16, (uint64_t)range_hi[b]});
+            } else if (!one_range_each && range_ptr) {
+                if (range_ptr[b] < 0 || range_ptr[b + 1] < range_ptr[b])
+                    return ctx->fail(XG_E_ARG, "xg_decode_bams_device_ranges: range_ptr is not ascending");
+                for (int64_t r = range_ptr[b]; r < range_ptr[b + 1]; r++) {
+                    if (range_lo[r] < 0 || range_hi[r] < 0)
+                        return ctx->fail(XG_E_ARG, "xg_decode_bams_device_ranges: negative offset");
+                    ranges[(size_t)b].push_back({(uint64_t)range_lo[r], (uint64_t)range_hi[r]});
+                }
+            } else {
+                ranges[(size_t)b].push_back({0, fsize});
+            }
+        }
         return decode_bams_device_impl(ctx, n_bams, paths, tid_map, tid_map_len, cell_tag, umi_tag, want_seq, ks, out,
-                                       n_records_seen, range_lo, range_hi);
+                                       n_records_seen, bytes_read, ranges);
     } catch (const std::exception &e) {
         if (ctx && ctx->stream) {
             cudaStreamSynchronize(ctx->stream);
@@ -1359,27 +1448,37 @@ int xg_decode_bams_device_range(xg_ctx *ctx, int32_t n_bams, const char *const *
         }
         return ctx ? ctx->fail(XG_E_NOMEM, std::string("device decode: ") + e.what()) : XG_E_NOMEM;
     }
+}
+
+int xg_decode_bams_device_ranges(xg_ctx *ctx, int32_t n_bams, const char *const *paths, const int32_t *const *tid_map,
+                                 const int32_t *tid_map_len, const char *cell_tag, const char *umi_tag, int32_t want_seq,
+                                 xg_keyspace *ks, const int64_t *range_ptr, const int64_t *range_lo,
+                                 const int64_t *range_hi, xg_dreads **out, int64_t *n_records_seen, int64_t *bytes_read) {
+    if (range_ptr && (!range_lo || !range_hi))
+        return ctx ? ctx->fail(XG_E_ARG, "xg_decode_bams_device_ranges: null range arrays") : XG_E_ARG;
+    return decode_bams_device_guarded(ctx, n_bams, paths, tid_map, tid_map_len, cell_tag, umi_tag, want_seq, ks, range_ptr,
+                                      range_lo, range_hi, false, out, n_records_seen, bytes_read);
+}
+
+int xg_decode_bams_device_range(xg_ctx *ctx, int32_t n_bams, const char *const *paths, const int32_t *const *tid_map,
+                                const int32_t *tid_map_len, const char *cell_tag, const char *umi_tag, int32_t want_seq,
+                                xg_keyspace *ks, const int64_t *range_lo, const int64_t *range_hi, xg_dreads **out,
+                                int64_t *n_records_seen) {
+    return decode_bams_device_guarded(ctx, n_bams, paths, tid_map, tid_map_len, cell_tag, umi_tag, want_seq, ks, nullptr,
+                                      range_lo, range_hi, true, out, n_records_seen, nullptr);
 }
 
 int xg_decode_bams_device(xg_ctx *ctx, int32_t n_bams, const char *const *paths, const int32_t *const *tid_map,
                           const int32_t *tid_map_len, const char *cell_tag, const char *umi_tag, int32_t want_seq,
                           xg_keyspace *ks, xg_dreads **out, int64_t *n_records_seen) {
-    try {
-        return decode_bams_device_impl(ctx, n_bams, paths, tid_map, tid_map_len, cell_tag, umi_tag, want_seq, ks, out,
-                                       n_records_seen, nullptr, nullptr);
-    } catch (const std::exception &e) {
-        if (ctx && ctx->stream) {
-            cudaStreamSynchronize(ctx->stream);
-            if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
-        }
-        return ctx ? ctx->fail(XG_E_NOMEM, std::string("device decode: ") + e.what()) : XG_E_NOMEM;
-    }
+    return decode_bams_device_guarded(ctx, n_bams, paths, tid_map, tid_map_len, cell_tag, umi_tag, want_seq, ks, nullptr,
+                                      nullptr, nullptr, false, out, n_records_seen, nullptr);
 }
 
 static int decode_bams_device_impl(xg_ctx *ctx, int32_t n_bams, const char *const *paths, const int32_t *const *tid_map,
                                    const int32_t *tid_map_len, const char *cell_tag, const char *umi_tag,
                                    int32_t want_seq, xg_keyspace *ks, xg_dreads **out, int64_t *n_records_seen,
-                                   const int64_t *range_lo, const int64_t *range_hi) {
+                                   int64_t *bytes_read, const std::vector<RangeList> &ranges) {
     if (!ctx || !ctx->stream) return ctx ? ctx->fail(XG_E_CUDA, "context has no device") : XG_E_ARG;
     if (n_bams < 0 || !out) return ctx->fail(XG_E_ARG, "xg_decode_bams_device: bad argument");
     if (cell_tag && strlen(cell_tag) != 2) return ctx->fail(XG_E_ARG, "cell tag must have 2 characters");
@@ -1401,9 +1500,8 @@ static int decode_bams_device_impl(xg_ctx *ctx, int32_t n_bams, const char *cons
     // window buffers: as large as the largest BAM needs, at most XG_DECODE_WINDOW compressed bytes
     uint64_t max_csize = 0;
     for (int32_t b = 0; b < n_bams; b++) {
-        struct stat stt;
-        if (stat(paths[b], &stt) != 0) return ctx->fail(XG_E_IO, std::string("cannot open '") + paths[b] + "'");
-        const uint64_t part = range_hi && range_hi[b] > 0 ? (uint64_t)(range_hi[b] - range_lo[b]) : (uint64_t)stt.st_size;
+        uint64_t part = 0;
+        for (const auto &r : ranges[(size_t)b]) part += r.second > (r.first >> 16) ? r.second - (r.first >> 16) : 0;
         D.comp_all += part;
         max_csize = std::max<uint64_t>(max_csize, part);
     }
@@ -1446,8 +1544,7 @@ static int decode_bams_device_impl(xg_ctx *ctx, int32_t n_bams, const char *cons
     lap("setup");
     std::vector<int64_t> bam_end((size_t)n_bams, 0);
     for (int32_t b = 0; b < n_bams; b++) {
-        int rc = decode_bam(D, paths[b], b, tid_map[b], tid_map_len[b], range_lo ? range_lo[b] : 0,
-                            range_hi ? range_hi[b] : 0);
+        int rc = decode_bam(D, paths[b], b, tid_map[b], tid_map_len[b], ranges[(size_t)b]);
         if (rc) {
             const std::string msg = ctx->err;
             return bail(rc, msg);
@@ -1550,6 +1647,7 @@ static int decode_bams_device_impl(xg_ctx *ctx, int32_t n_bams, const char *cons
     }
     ctx->timing[12] = now_ms() - t_begin;   // whole call
     if (n_records_seen) *n_records_seen = D.n_seen;
+    if (bytes_read) *bytes_read = (int64_t)D.bytes_read;
     *out = d;
     return XG_OK;
 }

@@ -23,7 +23,7 @@ struct BgzfBlockDev {
     unsigned long long uoff;   // offset in the uncompressed stream
     unsigned char *uptr;       // where the block is inflated to (slabs: blocks are contiguous within one)
     unsigned int crc;          // CRC32 of the uncompressed bytes (gzip trailer)
-    unsigned int pad_;
+    unsigned int skip;         // leading bytes the record walk leaves out (the head of a range's first block)
 };
 
 namespace xg_inflate {

@@ -82,11 +82,11 @@ def device_decode_enabled():
     return os.environ.get("XCLTK_B200_DEVICE_DECODE", "1") not in ("0", "", "no", "false")
 
 
-def _device_decode(ctx, sam_fn_list, tid_maps, cell_tag, umi_tag, want_seq, keyspace=None):
+def _device_decode(ctx, sam_fn_list, tid_maps, cell_tag, umi_tag, want_seq, keyspace=None, range_lists=None):
     """(dreads, stats) or None."""
     if not device_decode_enabled():
         return None
-    res = ctx.decode_bams(sam_fn_list, tid_maps, cell_tag, umi_tag, want_seq, keyspace)
+    res = ctx.decode_bams(sam_fn_list, tid_maps, cell_tag, umi_tag, want_seq, keyspace, range_lists=range_lists)
     if res is None:
         logging.getLogger(__name__).info("device decoder declined (%s); decoding on the host.",
                                          getattr(ctx, "decode_fallback_reason", "?"))
@@ -94,7 +94,45 @@ def _device_decode(ctx, sam_fn_list, tid_maps, cell_tag, umi_tag, want_seq, keys
     dreads, seen = res
     i = dreads.info()
     return dreads, {"n_reads": i["n_reads"], "n_records_seen": seen, "max_aln_len": i["max_aln_len"],
-                    "max_span": i["max_span"], "bytes": i["bytes"], "decoder": "device"}
+                    "max_span": i["max_span"], "bytes": i["bytes"], "decoder": "device",
+                    "bytes_read": getattr(dreads, "bytes_read", None), "range_lists": range_lists}
+
+
+def index_ranges(sam_fn_list, gid_of, tid_maps, units):
+    """Per BAM, the BGZF block ranges its .bai gives for the units (contig as in gid_of, or None; 0-based [beg, end)),
+    or None to read the file whole: no index, or one that cannot be trusted (one warning).  A read that overlaps a
+    unit lies in the index chunks of the unit's interval, so the ranges hold every read the counting can use."""
+    unit_chrom, unit_beg, unit_end = units
+    gid = np.array([gid_of.get(c, -1) if c is not None else -1 for c in unit_chrom], dtype=np.int64)
+    beg = np.asarray(unit_beg, dtype=np.int64)
+    end = np.asarray(unit_end, dtype=np.int64)
+    out = []
+    for fn, tmap in zip(sam_fn_list, tid_maps):
+        tid_of_gid = np.full(len(gid_of) + 1, -1, dtype=np.int32)
+        for t, g in enumerate(tmap):
+            if g >= 0:
+                tid_of_gid[g] = t
+        idx = None
+        try:
+            idx = lib.BamIndex.open(fn)
+            out.append(idx.ranges(tid_of_gid[gid], beg, end) if idx is not None else None)
+        except lib.XgError as ex:
+            logging.getLogger(__name__).warning("%s; reading '%s' whole.", ex, fn)
+            out.append(None)
+        finally:
+            if idx is not None:
+                idx.close()
+    return out
+
+
+class Request(list):
+    """The distinct contigs a call counts on -- what the loaders take as `chroms` -- with the call's units: contig
+    (or None: never fetched) and 0-based [beg, end) of every feature / region / SNP / window.  Being a list, it goes
+    wherever a contig list goes; load_reads takes the units from it to seek with the BAM index."""
+
+    def __init__(self, chroms, unit_chrom, unit_beg, unit_end):
+        list.__init__(self, chroms)
+        self.units = (unit_chrom, unit_beg, unit_end)
 
 
 def load_reads(sam_fn_list, chroms, cell_tag, umi_tag, want_seq, n_threads=0, device=0, mapped=False,
@@ -106,6 +144,9 @@ def load_reads(sam_fn_list, chroms, cell_tag, umi_tag, want_seq, n_threads=0, de
     the BAMs are decoded on the host (multi-threaded) and uploaded.
     chroms: distinct (already 'chr'-stripped) contig names the features / SNPs use; reads on
     other contigs can never be fetched by the reference and are dropped at decode time.
+    When `chroms` is a Request, the device decoder reads only the blocks that the .bai of a BAM gives for its
+    units (index_ranges); a BAM without a usable index is read whole.  The batch may then hold fewer reads and a
+    smaller max_aln_len / max_span; every read that overlaps a unit is in it, in file order.
     Host decoder only -- mapped: keep the records in pinned host memory and copy only pos/end
     (baf pileup); host_only: no upload at all, the caller streams the batch with
     Context.basefc_host."""
@@ -113,7 +154,13 @@ def load_reads(sam_fn_list, chroms, cell_tag, umi_tag, want_seq, n_threads=0, de
     ks = lib.KeySpace()
     bam_refs = [lib.bam_references(fn) for fn in sam_fn_list]
     gid_of, tid_maps = build_tid_maps(bam_refs, list(chroms))
-    dev = _device_decode(ctx, sam_fn_list, tid_maps, cell_tag, umi_tag, want_seq, ks)
+    range_lists = None
+    units = getattr(chroms, "units", None)
+    if units is not None and device_decode_enabled():
+        range_lists = index_ranges(sam_fn_list, gid_of, tid_maps, units)
+        if all(r is None for r in range_lists):
+            range_lists = None
+    dev = _device_decode(ctx, sam_fn_list, tid_maps, cell_tag, umi_tag, want_seq, ks, range_lists)
     if dev is not None:
         return ReadBatch(ctx, dev[0], ks, gid_of, dev[1])
     host = lib.decode_bams(sam_fn_list, tid_maps, cell_tag, umi_tag, want_seq, ks, n_threads)

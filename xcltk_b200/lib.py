@@ -172,6 +172,15 @@ SYMBOLS = {
     "xg_decode_bams_device_range": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_char_p), C.POINTER(c_i32p), c_i32p,
                                               C.c_char_p, C.c_char_p, C.c_int32, _P, c_i64p, c_i64p,
                                               C.POINTER(_P), C.POINTER(C.c_int64)]),
+    "xg_decode_bams_device_ranges": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_char_p), C.POINTER(c_i32p), c_i32p,
+                                               C.c_char_p, C.c_char_p, C.c_int32, _P, c_i64p, c_i64p, c_i64p,
+                                               C.POINTER(_P), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "xg_bam_index_open": (C.c_int, [C.c_char_p, C.POINTER(_P)]),
+    "xg_bam_index_free": (None, [_P]),
+    "xg_bam_index_n_ref": (C.c_int32, [_P]),
+    "xg_bam_index_ref": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int64), C.POINTER(c_u32p), C.POINTER(c_i64p),
+                                   C.POINTER(c_u64p), C.POINTER(C.c_int64), C.POINTER(c_u64p)]),
+    "xg_bam_index_ranges": (C.c_int, [_P, C.c_int64, c_i32p, c_i64p, c_i64p, C.POINTER(c_i64p), C.POINTER(C.c_int64)]),
     "xg_bgzf_block_index": (C.c_int, [C.c_char_p, C.POINTER(c_i64p), C.POINTER(C.c_int64), C.POINTER(C.c_int64),
                                       C.POINTER(C.c_int32)]),
     "xg_free_array": (None, [_P]),
@@ -562,13 +571,16 @@ class Context(object):
         self._check(self.lib.xg_upload_reads(self.h, host_reads.ptr, C.byref(d)))
         return DeviceReads(self, d)
 
-    def decode_bams(self, paths, tid_maps, cell_tag, umi_tag, want_seq, keyspace=None, ranges=None):
+    def decode_bams(self, paths, tid_maps, cell_tag, umi_tag, want_seq, keyspace=None, ranges=None, range_lists=None):
         """BGZF inflate + BAM parse on the device (xg_decode_bams_device).  Returns
-        (DeviceReads, n_records_seen), or None when the files need the host decoder.
+        (DeviceReads, n_records_seen), or None when the files need the host decoder; the compressed bytes read from
+        the files are left in the DeviceReads' `bytes_read`.
         keyspace: interns the cell / UMI values that do not pack into 63 bits (query names,
         free-text barcodes); without it such files are left to the host decoder.
         ranges: [(lo, hi)] byte offsets of BGZF block starts per BAM -- only those blocks are decoded
-        (xg_decode_bams_device_range; see bgzf_block_index / bam_block_probe)."""
+        (xg_decode_bams_device_range; see bgzf_block_index / bam_block_probe).
+        range_lists: per BAM a list of ascending, disjoint ranges (virtual offset of the first record, file offset after
+        the last block) as BamIndex.ranges gives them, or None for the whole file (xg_decode_bams_device_ranges)."""
         n = len(paths)
         cpaths = (C.c_char_p * n)(*[p.encode() for p in paths])
         maps = [np.ascontiguousarray(m, dtype=np.int32) for m in tid_maps]
@@ -579,8 +591,19 @@ class Context(object):
         args = (self.h, n, cpaths, cmaps, as_ptr(lens, c_i32p), cell_tag.encode() if cell_tag else None,
                 umi_tag.encode() if umi_tag else None, 1 if want_seq else 0,
                 keyspace.h if keyspace is not None else None)
+        n_read = C.c_int64(-1)
         if ranges is None:
-            rc = self.lib.xg_decode_bams_device(*args, C.byref(d), C.byref(seen))
+            arrs = (None, None, None)                 # every file whole
+            if range_lists is not None:
+                ptr, lo, hi = [0], [], []
+                for p, rl in zip(paths, range_lists):
+                    for a, b in ([(0, os.path.getsize(p))] if rl is None else rl):
+                        lo.append(int(a))
+                        hi.append(int(b))
+                    ptr.append(len(lo))
+                arrs = tuple(np.array(x, dtype=np.int64) for x in (ptr, lo, hi))
+            rc = self.lib.xg_decode_bams_device_ranges(*args, *[None if x is None else as_ptr(x, c_i64p) for x in arrs],
+                                                       C.byref(d), C.byref(seen), C.byref(n_read))
         else:
             lo = np.array([r[0] for r in ranges], dtype=np.int64)
             hi = np.array([r[1] for r in ranges], dtype=np.int64)
@@ -590,7 +613,9 @@ class Context(object):
             self.decode_fallback_reason = self.lib.xg_last_error(self.h).decode()
             return None
         self._check(rc)
-        return DeviceReads(self, d), int(seen.value)
+        dr = DeviceReads(self, d)
+        dr.bytes_read = int(n_read.value) if n_read.value >= 0 else None
+        return dr, int(seen.value)
 
     def bgzf_inflate(self, path):
         """Inflate a BGZF file on the device; returns the bytes (validation of the inflate kernel)."""
@@ -830,6 +855,68 @@ def bgzf_block_index(path):
     off = np.ctypeslib.as_array(p, shape=(n.value + 1,)).copy()
     lib.xg_free_array(C.cast(p, _P))
     return off, int(first.value), bool(al.value)
+
+
+class BamIndex(object):
+    """The .bai of a BAM (xg_bam_index_open): None from `open` when the BAM has no index."""
+
+    def __init__(self, h):
+        self.lib, self.h = load(), h
+
+    @staticmethod
+    def open(bam_path):
+        """BamIndex, or None when there is no .bai; raises XgError (XG_E_FORMAT) when there is one that cannot be
+        trusted."""
+        lib = load()
+        h = _P()
+        rc = lib.xg_bam_index_open(bam_path.encode(), C.byref(h))
+        if rc != 0:
+            raise XgError(rc, lib.xg_host_last_error().decode())
+        return BamIndex(h) if h.value else None
+
+    def n_ref(self):
+        return int(self.lib.xg_bam_index_n_ref(self.h))
+
+    def ref(self, tid):
+        """({bin: [(beg, end) virtual offsets]}, linear index as a uint64 array) of contig tid."""
+        nb, bins, ptr, ch, ni, lin = C.c_int64(0), c_u32p(), c_i64p(), c_u64p(), C.c_int64(0), c_u64p()
+        rc = self.lib.xg_bam_index_ref(self.h, int(tid), C.byref(nb), C.byref(bins), C.byref(ptr), C.byref(ch),
+                                       C.byref(ni), C.byref(lin))
+        if rc != 0:
+            raise XgError(rc, self.lib.xg_host_last_error().decode())
+        n = nb.value
+        b = np_view(bins, n, np.uint32)
+        p = np_view(ptr, n + 1, np.int64) if n else np.zeros(1, np.int64)
+        c = np_view(ch, 2 * int(p[-1]), np.uint64)
+        out = {int(b[i]): [(int(c[2 * k]), int(c[2 * k + 1])) for k in range(int(p[i]), int(p[i + 1]))] for i in range(n)}
+        return out, np_view(lin, ni.value, np.uint64).copy()
+
+    def ranges(self, tid, beg, end):
+        """Ascending, merged [(lo, hi)] ranges holding every record that overlaps one of the 0-based half-open
+        intervals (tid[i], beg[i], end[i]): lo the virtual offset of the range's first record, hi the file offset
+        after its last BGZF block; ranges less than XG_BAM_INDEX_MERGE_GAP apart are merged."""
+        tid = np.ascontiguousarray(tid, dtype=np.int32)
+        beg = np.ascontiguousarray(beg, dtype=np.int64)
+        end = np.ascontiguousarray(end, dtype=np.int64)
+        p, n = c_i64p(), C.c_int64(0)
+        rc = self.lib.xg_bam_index_ranges(self.h, len(tid), as_ptr(tid, c_i32p), as_ptr(beg, c_i64p),
+                                          as_ptr(end, c_i64p), C.byref(p), C.byref(n))
+        if rc != 0:
+            raise XgError(rc, self.lib.xg_host_last_error().decode())
+        out = np.ctypeslib.as_array(p, shape=(max(1, 2 * n.value),))[:2 * n.value].copy()
+        self.lib.xg_free_array(C.cast(p, _P))
+        return [(int(out[2 * i]), int(out[2 * i + 1])) for i in range(n.value)]
+
+    def close(self):
+        if self.h:
+            self.lib.xg_bam_index_free(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 def bam_block_probe(path, offset):

@@ -59,7 +59,7 @@ def usage(fp=sys.stdout, conf=None):
         % d.MIN_INCLUDE,
         "  --countORPHAN           If use, do not skip anomalous read pairs.",
         "",
-        "B200 notes: input must be coordinate-sorted BAM (no index needed; SAM/CRAM are not decoded);",
+        "B200 notes: input must be coordinate-sorted BAM (a .bai is used when present; SAM/CRAM are not decoded);",
         "  -p sets the host BGZF/BAM decode threads; counting runs on the GPU (no CPU fallback).",
         "",
     ]
@@ -275,8 +275,8 @@ def count_features(conf, batch=None):
                 batch = engine.load_reads_multi(conf.sam_fn_list, chroms, conf.cell_tag, conf.umi_tag, False,
                                                 threads, devices=parallel.device_list(n_dev))
         else:
-            batch = engine.load_reads(conf.sam_fn_list, chroms, conf.cell_tag, conf.umi_tag, False, threads,
-                                      host_only=True)
+            req = engine.Request(chroms, [r.chrom for r in regs], [r.start - 1 for r in regs], [r.end - 1 for r in regs])
+            batch = engine.load_reads(conf.sam_fn_list, req, conf.cell_tag, conf.umi_tag, False, threads, host_only=True)
     try:
         gid, beg, end = feature_arrays(regs, batch.gid_of)
         cell_keys = None
