@@ -138,7 +138,7 @@ def test_tile_boundaries(gpu_ctx, n):
 
 
 def test_many_tiny_features_exceed_the_staged_boundary_slice(gpu_ctx):
-    """> 512 boundaries under one tile window: global binary search path."""
+    """Far more than SB_MAX (128) boundaries under one tile window: global binary search path."""
     rng = np.random.RandomState(1)
     ks = lib.KeySpace()
     reads, ck = build_reads(rng, 3000, 60000, mixed, 50, None, ks)
