@@ -223,7 +223,7 @@ __host__ __device__ __forceinline__ uint64_t plan_blk_bytes(uint32_t cap, uint32
 #define STAB_CAP 128     // stabbing-list entries of those boundaries staged in shared memory
 #define CIG_CAP 1024     // CIGAR words of the tile staged in shared memory
 #define WPAIR_CAP 96     // (feature, cell, UMI) pairs a warp stages before it appends them
-#define FILT_BITS 11     // tile-local duplicate filter: 2^FILT_BITS direct-mapped 64-bit entries
+#define FILT_BITS 10     // tile-local duplicate filter: 2^FILT_BITS direct-mapped 64-bit entries, one per index stage
 #define INCL_CAP 256     // include-threshold table entries kept in shared memory
 #define LEGACY_BIT 0x80000000u
 #define NO_SEG 0xFFFFFFFFu
@@ -487,7 +487,8 @@ struct __align__(16) PairEnt {
     uint32_t b;                   // segment: pool offset / 16; set: column
 };
 
-struct IdxStage {                 // the slice of the interval index under one tile (bulk-copied)
+struct IdxStage {                 // the slice of the interval index under one tile (bulk-copied) and its filter
+    unsigned long long filt[1 << FILT_BITS];       // the tile's duplicate filter (written by the warps)
     int4 stab4[STAB_CAP];
     uint32_t cigar[CIG_CAP + 4];
     int32_t bnd[SB_MAX + 4];
@@ -497,15 +498,16 @@ struct IdxStage {                 // the slice of the interval index under one t
 struct CountSmem {
     IdxStage idx[2];
     TileDesc desc[4];
-    unsigned long long filt[1 << FILT_BITS];
     PairEnt pairs[CNT_WARPS][WPAIR_CAP];
     unsigned long long bar_idx[2], bar_desc[4];
+    unsigned long long bar_done[2];                // tile k done (every warp, and its buffers freed): bar_done[k & 1]
     int32_t incl[INCL_CAP];
     int t_ring[4];
     int np[CNT_WARPS];
-    int chunk_ctr[2];             // next chunk of the current / the next tile (warps claim chunks)
-    int t_pend;                   // the elected thread's pipeline state lives here, not in everybody's registers:
-    uint32_t n_issued;            // tile k+3 (counter value on its way); index slices issued so far
+    int chunk_ctr[2];             // next chunk of tile k: chunk_ctr[k & 1] (warps claim chunks)
+    int n_done[2];                // warps done with tile k: n_done[k & 1] (the last one frees the buffers)
+    int t_pend;                   // the elected lane's pipeline state lives here, not in everybody's registers:
+    uint32_t n_issued;            // the tile of the next descriptor to issue; index slices issued so far
 };
 
 // ---- mbarrier / bulk-copy (TMA) primitives
@@ -515,6 +517,9 @@ __device__ __forceinline__ void mbar_init(unsigned long long *bar, uint32_t coun
 }
 __device__ __forceinline__ void mbar_expect_tx(unsigned long long *bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive(unsigned long long *bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 __device__ __forceinline__ void mbar_wait(unsigned long long *bar, uint32_t parity) {
     const uint32_t a = smem_u32(bar);
@@ -733,8 +738,8 @@ __device__ __forceinline__ void flush_warp(const BasefcDev &P, CountSmem &S, int
 }
 
 // include test of one (read, feature) pair; a passing pair that the tile has not seen yet is staged
-__device__ __forceinline__ void emit_pair(const BasefcDev &P, CountSmem &S, int32_t jmin, int w,
-                                          const RecCtx &r, int32_t j, int32_t s0, int32_t e0, uint32_t segoff) {
+__device__ __forceinline__ void emit_pair(const BasefcDev &P, CountSmem &S, unsigned long long *filt, int32_t jmin,
+                                          int w, const RecCtx &r, int32_t j, int32_t s0, int32_t e0, uint32_t segoff) {
     int32_t m;
     if (r.n_ops == 0) {
         int32_t a = max(r.pos, s0), b = min(r.end, e0);
@@ -753,8 +758,8 @@ __device__ __forceinline__ void emit_pair(const BasefcDev &P, CountSmem &S, int3
         if (jl < (1u << (24 - P.col_bits))) {
             const unsigned long long fk = r.umi_c | ((unsigned long long)jl << P.col_bits) | r.col;
             const uint32_t h = ((((uint32_t)fk * 0x85EBCA6Bu) ^ (uint32_t)(fk >> 32)) * 0x9E3779B1u) >> (32 - FILT_BITS);
-            if (S.filt[h] == fk) return;
-            S.filt[h] = fk;
+            if (filt[h] == fk) return;
+            filt[h] = fk;
         }
     }
     const bool seg = segoff != NO_SEG;
@@ -789,7 +794,7 @@ struct TileRegs {
 };
 
 // One record: filters (check_read), the features it overlaps, include test per feature.
-__device__ __forceinline__ void count_record(const BasefcDev &P, CountSmem &S, const TileRegs &T, const IdxStage &X,
+__device__ __forceinline__ void count_record(const BasefcDev &P, CountSmem &S, const TileRegs &T, IdxStage &X,
                                              int w, int2 pe, uint32_t fmq, uint32_t co, uint64_t umi,
                                              int32_t colv) {
     if (umi == XG_KEY_NONE || umi == XG_KEY_EMPTY) return;       // has_tag / `if umi:`
@@ -872,7 +877,7 @@ __device__ __forceinline__ void count_record(const BasefcDev &P, CountSmem &S, c
         }
         for (int32_t s = s0i; s < s1i; s++) {
             const int4 f = (T.stab_staged && s >= T.st_lo) ? X.stab4[s - T.st_lo] : __ldg(&P.stab4[s]);
-            emit_pair(P, S, T.jmin, w, r, f.x, f.y, f.z, (uint32_t)f.w);
+            emit_pair(P, S, X.filt, T.jmin, w, r, f.x, f.y, f.z, (uint32_t)f.w);
         }
     }
     // (2) features beginning at a boundary inside (pos, end); every boundary from `by` on is
@@ -883,16 +888,19 @@ __device__ __forceinline__ void count_record(const BasefcDev &P, CountSmem &S, c
         if (bv >= r.end) break;
         const int32_t j1 = __ldg(&P.fb[kb + 1]);
         for (int32_t j = __ldg(&P.fb[kb]); j < j1; j++)
-            emit_pair(P, S, T.jmin, w, r, j, bv, __ldg(&P.sf_end[j]), __ldg(&P.segoff16[j]));
+            emit_pair(P, S, X.filt, T.jmin, w, r, j, bv, __ldg(&P.sf_end[j]), __ldg(&P.segoff16[j]));
     }
 }
 
-// Persistent CTAs take tiles from a work counter.  One elected thread runs the staging pipeline:
-// tile k+3's index is fetched from the counter, tile k+2's descriptor and tile k+1's slice of the
-// interval index (boundaries, stabbing lists, CIGAR words) are brought into shared memory by bulk
-// copies completing on mbarriers while the warps count tile k.  Inside a tile the warps work
-// on their own: 32-record chunks claimed from a counter, the record loads issued one chunk ahead, pairs
-// staged per warp and appended per warp -- two CTA barriers per tile (the filter is cleared between them).
+// Persistent CTAs take tiles from a work counter.  Inside a tile the warps work on their own: 32-record chunks
+// claimed from a counter, the record loads issued one chunk ahead, pairs staged per warp and appended per warp.
+// There is no CTA barrier: the state of a tile is double-buffered -- its chunk counter by the tile's parity, its
+// index stage and duplicate filter by the parity of the live tiles counted so far -- and a warp that runs out of
+// chunks in tile k goes on to tile k+1 as soon as tile k-1 has freed its buffers: warps are at most one tile apart.
+// A warp arrives on tile k's "done" mbarrier when it has flushed its pairs of the tile; the last of them first
+// clears the tile's filter and chunk counter for their next user and moves the staging pipeline on (elected lane: tile k+4's index fetched from the counter, tile k+3's descriptor and
+// tile k+2's slice of the interval index -- boundaries, stabbing lists, CIGAR words -- brought into shared memory by
+// bulk copies completing on mbarriers), then arrives: the phase completes only when the buffers are free.
 template <int MIN_CTAS>
 __global__ void __launch_bounds__(CNT_THREADS, MIN_CTAS) k_basefc_count(const __grid_constant__ BasefcDev P) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
@@ -903,16 +911,19 @@ __global__ void __launch_bounds__(CNT_THREADS, MIN_CTAS) k_basefc_count(const __
     if (threadIdx.x == 0) {
         for (int k = 0; k < 2; k++) mbar_init(&S.bar_idx[k], 1);
         for (int k = 0; k < 4; k++) mbar_init(&S.bar_desc[k], 1);
+        for (int k = 0; k < 2; k++) mbar_init(&S.bar_done[k], CNT_WARPS);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (threadIdx.x < CNT_WARPS) S.np[threadIdx.x] = 0;
-    if (threadIdx.x < 2) S.chunk_ctr[threadIdx.x] = 0;
+    if (threadIdx.x < 2) S.chunk_ctr[threadIdx.x] = S.n_done[threadIdx.x] = 0;
+    if (P.seg_mode)                  // both filters start empty; afterwards the last user of a stage clears it
+        for (int q = threadIdx.x; q < 2 << FILT_BITS; q += CNT_THREADS) S.idx[q >> FILT_BITS].filt[q & ((1 << FILT_BITS) - 1)] = 0;
     if (P.incl_tab)
         for (int k = threadIdx.x; k < INCL_CAP && k < P.incl_tab_len; k += CNT_THREADS) S.incl[k] = __ldg(&P.incl_tab[k]);
-    __syncthreads();
 
-    // ---- elected thread: state of the staging pipeline
-    // S.t_pend: tile k+3; S.n_issued: index slices issued so far (buffer = n & 1, parity = (n >> 1) & 1)
+    // ---- elected lane: state of the staging pipeline
+    // S.t_pend: the tile of the next descriptor to issue; S.n_issued: index slices issued so far (buffer = n & 1,
+    // parity = (n >> 1) & 1)
     auto fetch_tile = [&]() -> int {
         const unsigned int v = atomicAdd(P.work, 1u);
         return v < (unsigned int)n_launch ? P.tile0 + (int)v : -1;
@@ -924,7 +935,11 @@ __global__ void __launch_bounds__(CNT_THREADS, MIN_CTAS) k_basefc_count(const __
         mbar_expect_tx(&S.bar_desc[k & 3], (uint32_t)sizeof(TileDesc));
         bulk_g2s(&S.desc[k & 3], &P.tdesc[t], (uint32_t)sizeof(TileDesc), &S.bar_desc[k & 3]);
     };
-    auto issue_idx = [&](const TileDesc &d) {     // the slice of the index under tile d -> next buffer
+    auto issue_idx = [&](int k) {                 // the slice of the index under tile k (if live) -> next buffer
+        if (S.t_ring[k & 3] < 0) return;
+        mbar_wait(&S.bar_desc[k & 3], (uint32_t)(k >> 2) & 1u);
+        const TileDesc &d = S.desc[k & 3];
+        if (d.bx < 0) return;
         IdxStage &X = S.idx[S.n_issued & 1];
         unsigned long long *bar = &S.bar_idx[S.n_issued & 1];
         S.n_issued++;
@@ -946,140 +961,154 @@ __global__ void __launch_bounds__(CNT_THREADS, MIN_CTAS) k_basefc_count(const __
     };
     if (threadIdx.x == 0) {
         S.n_issued = 0;
-        const int t0 = fetch_tile(), t1 = fetch_tile();
-        issue_desc(0, t0);
-        issue_desc(1, t1);
+        for (int k = 0; k < 3; k++) issue_desc(k, fetch_tile());
         S.t_pend = fetch_tile();
-        if (t0 >= 0) {
-            mbar_wait(&S.bar_desc[0], 0);
-            if (S.desc[0].bx >= 0) issue_idx(S.desc[0]);
-        }
+        issue_idx(0);
+        issue_idx(1);
     }
+    __syncthreads();                 // the only CTA barrier: initial state and the pipeline's first stages
+
     uint32_t n_used = 0;             // index slices consumed so far (every thread counts alike)
+    // Warp done with tile k (its pairs flushed).  The last warp of the tile frees the tile's buffers -- nobody touches
+    // its filter, chunk counter or index stage any more -- before it arrives.
+    auto tile_done = [&](int k) {
+        const int s = k & 1;
+        __syncwarp();
+        int last = 0;
+        if (lane == 0) {
+            __threadfence_block();
+            last = atomicAdd(&S.n_done[s], 1) == CNT_WARPS - 1;
+            __threadfence_block();
+        }
+        if (__shfl_sync(0xffffffffu, last, 0)) {
+            __syncwarp();
+            if (S.desc[k & 3].bx >= 0 && P.seg_mode) {     // a live tile's filter is its stage's: (n_used - 1) & 1
+                uint4 *f4 = reinterpret_cast<uint4 *>(S.idx[(n_used - 1) & 1].filt);
+                for (int q = lane; q < (1 << FILT_BITS) / 2; q += 32) f4[q] = make_uint4(0, 0, 0, 0);
+            }
+            if (lane == 0) {
+                S.chunk_ctr[s] = 0;
+                S.n_done[s] = 0;
+                const int t = S.t_pend;
+                S.t_pend = t >= 0 ? fetch_tile() : -1;
+                issue_desc(k + 3, t);
+                issue_idx(k + 2);
+            }
+            __syncwarp();
+        }
+        if (lane == 0) mbar_arrive(&S.bar_done[s]);
+    };
+    // tile k's parity is free once tile k-2 is done with it
+    auto wait_parity = [&](int k) {
+        if (k >= 2) mbar_wait(&S.bar_done[k & 1], (uint32_t)((k - 2) >> 1) & 1u);
+    };
+
     // A warp that runs out of chunks in tile k claims its first chunk of tile k+1 and issues that chunk's record
-    // loads BEFORE it waits for the others at the tile's end: the loads' DRAM latency passes under the barrier
-    // instead of after it.
+    // loads before it flushes its pairs of tile k: the loads' DRAM latency passes under the flush.
     int pre_c = -1;
     int2 pe_n = make_int2(0, 0);
     uint32_t fq_n = 0, co_n = 0;
     ulonglong2 ky_n = make_ulonglong2(XG_KEY_NONE, XG_KEY_NONE);
 
     for (int k = 0;; k++) {
-        __syncthreads();             // A: every warp is done with tile k-1
-        const int t = S.t_ring[k & 3];
-        if (t < 0) break;
+        if (S.t_ring[k & 3] < 0) break;
+        wait_parity(k);
         mbar_wait(&S.bar_desc[k & 3], (uint32_t)(k >> 2) & 1u);
-        const TileDesc &td = S.desc[k & 3];          // stays put until tile k+2 is done with
-        const bool live = td.bx >= 0;
-        if (live && P.seg_mode) {    // clear the duplicate filter
-            uint4 *f4 = reinterpret_cast<uint4 *>(S.filt);
-            const uint4 z = make_uint4(0, 0, 0, 0);
-            for (int q = threadIdx.x; q < (1 << FILT_BITS) / 2; q += CNT_THREADS) f4[q] = z;
-        }
-        if (threadIdx.x == 0) S.chunk_ctr[(k + 1) & 1] = 0;       // tile k-1 was its last user; tile k+1's claims come after B
-        __syncthreads();             // B: filter cleared, everybody has read the descriptor
-        if (threadIdx.x == 0) {      // pipeline: descriptor of tile k+2, index slice of tile k+1
-            const int t2 = S.t_pend;
-            S.t_pend = t2 >= 0 ? fetch_tile() : -1;
-            issue_desc(k + 2, t2);
-            if (S.t_ring[(k + 1) & 3] >= 0) {
-                mbar_wait(&S.bar_desc[(k + 1) & 3], (uint32_t)((k + 1) >> 2) & 1u);
-                if (S.desc[(k + 1) & 3].bx >= 0) {
-                    // tile k+1 takes the buffer after tile k's; tile k's own slice was issued earlier
-                    issue_idx(S.desc[(k + 1) & 3]);
+        const TileDesc &td = S.desc[k & 3];          // stays put until tile k+1 is done with
+        if (td.bx >= 0) {                  // no feature under a dead tile's window: its records are never read
+            IdxStage &X = S.idx[n_used & 1];
+            mbar_wait(&S.bar_idx[n_used & 1], (n_used >> 1) & 1u);
+            n_used++;
+
+            TileRegs T;
+            T.bx = td.bx;
+            T.by = td.by;
+            T.b0 = td.b0;
+            T.td = &td;
+            T.st_lo = td.st_lo;
+            T.jmin = td.jmin;
+            T.c_al = td.c_lo & ~3u;
+            T.staged = T.by - (T.bx & ~3) <= SB_MAX;
+            T.stab_staged = T.staged && td.st_n <= STAB_CAP;
+            T.cig_staged = td.c_hi - T.c_al <= CIG_CAP;
+            const int64_t rec_beg = td.rec_beg;
+            const int32_t n_rec = td.n_rec, tile_col = td.col;
+            const int n_chunks = (n_rec + CHUNK - 1) / CHUNK;
+
+            // ---- the warp's chunks, claimed from the tile's counter one ahead: the records of the next
+            // chunk are on their way (coalesced 8 / 4 / 4 / 16-byte loads) while this one is counted.  (A third
+            // stage that also kept the next chunk's barcode slot in flight was measured slower: the registers
+            // it needs spill.)
+            auto claim = [&]() -> int {
+                int c = 0;
+                if (lane == 0) c = atomicAdd(&S.chunk_ctr[k & 1], 1);
+                return __shfl_sync(0xffffffffu, c, 0);
+            };
+            auto load_from = [&](int64_t beg, int32_t n, int c) {
+                const int r = c * CHUNK + lane;
+                ky_n = make_ulonglong2(XG_KEY_NONE, XG_KEY_NONE);            // an absent UMI drops the record
+                if (r < n) {
+                    const int64_t i = beg + r;
+                    pe_n = __ldcs(&P.pos_end[i]);                             // streamed once: evict-first
+                    fq_n = __ldcs(&P.fmq[i]);
+                    co_n = __ldcs(&P.cig_off[i]);
+                    ky_n = __ldcs(&P.keys[i]);
                 }
+            };
+            auto load_chunk = [&](int c) { load_from(rec_beg, n_rec, c); };
+            int c = pre_c;
+            if (c < 0) {             // nothing claimed at the end of the previous tile
+                c = claim();
+                if (c < n_chunks) load_chunk(c);
             }
-        }
-        if (!live) continue;         // no feature under this tile's window: its records are never read
-        const IdxStage &X = S.idx[n_used & 1];
-        mbar_wait(&S.bar_idx[n_used & 1], (n_used >> 1) & 1u);
-        n_used++;
-
-        TileRegs T;
-        T.bx = td.bx;
-        T.by = td.by;
-        T.b0 = td.b0;
-        T.td = &td;
-        T.st_lo = td.st_lo;
-        T.jmin = td.jmin;
-        T.c_al = td.c_lo & ~3u;
-        T.staged = T.by - (T.bx & ~3) <= SB_MAX;
-        T.stab_staged = T.staged && td.st_n <= STAB_CAP;
-        T.cig_staged = td.c_hi - T.c_al <= CIG_CAP;
-        const int64_t rec_beg = td.rec_beg;
-        const int32_t n_rec = td.n_rec, tile_col = td.col;
-        const int n_chunks = (n_rec + CHUNK - 1) / CHUNK;
-
-        // ---- the warp's chunks, claimed from the tile's counter one ahead: the records of the next
-        // chunk are on their way (coalesced 8 / 4 / 4 / 16-byte loads) while this one is counted.  (A third
-        // stage that also kept the next chunk's barcode slot in flight was measured slower: the registers
-        // it needs spill.)
-        auto claim = [&]() -> int {
-            int c = 0;
-            if (lane == 0) c = atomicAdd(&S.chunk_ctr[k & 1], 1);
-            return __shfl_sync(0xffffffffu, c, 0);
-        };
-        auto load_from = [&](int64_t beg, int32_t n, int c) {
-            const int r = c * CHUNK + lane;
-            ky_n = make_ulonglong2(XG_KEY_NONE, XG_KEY_NONE);            // an absent UMI drops the record
-            if (r < n) {
-                const int64_t i = beg + r;
-                pe_n = __ldcs(&P.pos_end[i]);                             // streamed once: evict-first
-                fq_n = __ldcs(&P.fmq[i]);
-                co_n = __ldcs(&P.cig_off[i]);
-                ky_n = __ldcs(&P.keys[i]);
-            }
-        };
-        auto load_chunk = [&](int c) { load_from(rec_beg, n_rec, c); };
-        int c = pre_c;
-        if (c < 0) {                 // nothing claimed at the end of the previous tile
-            c = claim();
-            if (c < n_chunks) load_chunk(c);
-        }
-        pre_c = -1;
-        while (c < n_chunks) {
-            const int2 pe = pe_n;
-            const uint32_t fq = fq_n, co = co_n;
-            const ulonglong2 ky = ky_n;
-            const int cn = claim();
-            if (cn < n_chunks) load_chunk(cn);
-            // cell lookup
-            int32_t colv = tile_col;
-            if (P.fp.use_cell_tag) {
-                colv = -1;
-                if (ky.x != XG_KEY_NONE) {
-                    uint32_t sl = barcode_home(ky.x, P.bc.shift);
-                    while (true) {
-                        const ulonglong2 e = __ldg(&P.bc.slots[sl]);
-                        if (e.x == ky.x) {
-                            colv = (int32_t)e.y;
-                            break;
+            pre_c = -1;
+            while (c < n_chunks) {
+                const int2 pe = pe_n;
+                const uint32_t fq = fq_n, co = co_n;
+                const ulonglong2 ky = ky_n;
+                const int cn = claim();
+                if (cn < n_chunks) load_chunk(cn);
+                // cell lookup
+                int32_t colv = tile_col;
+                if (P.fp.use_cell_tag) {
+                    colv = -1;
+                    if (ky.x != XG_KEY_NONE) {
+                        uint32_t sl = barcode_home(ky.x, P.bc.shift);
+                        while (true) {
+                            const ulonglong2 e = __ldg(&P.bc.slots[sl]);
+                            if (e.x == ky.x) {
+                                colv = (int32_t)e.y;
+                                break;
+                            }
+                            if (e.x == XG_KEY_NONE) break;
+                            sl = (sl + 1) & P.bc.mask;
                         }
-                        if (e.x == XG_KEY_NONE) break;
-                        sl = (sl + 1) & P.bc.mask;
                     }
                 }
+                count_record(P, S, T, X, w, pe, fq, co, ky.y, colv);
+                __syncwarp();
+                // Append the staged pairs when the stage is more than half full (32 at a time keep the lanes
+                // busy).  The decision is lane 0's: a lane reading the counter for itself could see it already
+                // raised by lanes that went on to the next record, and part ways with them.
+                if (__shfl_sync(0xffffffffu, S.np[w], 0) > WPAIR_CAP / 2) flush_warp(P, S, w, lane);
+                c = cn;
             }
-            count_record(P, S, T, X, w, pe, fq, co, ky.y, colv);
-            __syncwarp();
-            // Append the staged pairs when the stage is more than half full (32 at a time keep the lanes
-            // busy).  The decision is lane 0's: a lane reading the counter for itself could see it already
-            // raised by lanes that went on to the next record, and part ways with them.
-            if (__shfl_sync(0xffffffffu, S.np[w], 0) > WPAIR_CAP / 2) flush_warp(P, S, w, lane);
-            c = cn;
-        }
-        flush_warp(P, S, w, lane);
-        // the first chunk of the next tile (its descriptor arrived two tiles ago; its counter was reset before B)
-        if (S.t_ring[(k + 1) & 3] >= 0) {
-            mbar_wait(&S.bar_desc[(k + 1) & 3], (uint32_t)((k + 1) >> 2) & 1u);
-            const TileDesc &nd = S.desc[(k + 1) & 3];
-            if (nd.bx >= 0) {
-                int cx = 0;
-                if (lane == 0) cx = atomicAdd(&S.chunk_ctr[(k + 1) & 1], 1);
-                pre_c = __shfl_sync(0xffffffffu, cx, 0);
-                if (pre_c * CHUNK < nd.n_rec) load_from(nd.rec_beg, nd.n_rec, pre_c);
+            // the first chunk of the next tile (its descriptor arrived two tiles ago; its parity's counter is reset
+            // once tile k-1 is done)
+            if (S.t_ring[(k + 1) & 3] >= 0) {
+                wait_parity(k + 1);
+                mbar_wait(&S.bar_desc[(k + 1) & 3], (uint32_t)((k + 1) >> 2) & 1u);
+                const TileDesc &nd = S.desc[(k + 1) & 3];
+                if (nd.bx >= 0) {
+                    int cx = 0;
+                    if (lane == 0) cx = atomicAdd(&S.chunk_ctr[(k + 1) & 1], 1);
+                    pre_c = __shfl_sync(0xffffffffu, cx, 0);
+                    if (pre_c * CHUNK < nd.n_rec) load_from(nd.rec_beg, nd.n_rec, pre_c);
+                }
             }
+            flush_warp(P, S, w, lane);
         }
+        tile_done(k);
     }
 }
 
