@@ -429,6 +429,39 @@ int xg_snp_discover(xg_ctx *ctx, const xg_dreads *reads, const xg_features *targ
                     const xg_params *par, const xg_discover_filter *filter, xg_sites **out);
 void xg_sites_free(xg_sites *sites);
 
+/* Local phasing of long regions (the pre-step of `xcltk baf`; xcltk/baf/fc/phasing.py:13-78 over
+ * xcltk/baf/localphase.py:14-243, as xcltk_b200/baf/fc/phasing.py:reg_local_phasing and baf/localphase.py compute it
+ * region by region on the host).  Per region, one CTA: the SNPs with no depth leave the region's list (keep_out), the
+ * counts are oriented by ref_idx (1: DP - AD), then up to 50 rounds of {cells with aggregated BAF in [0.45, 0.55]
+ * leave; two-component EM (min 10, max 1000 iterations, convergence 1e-3) with the posteriors smoothed by the
+ * row-normalised kernel exp(-(x_j - x_i)^2 / 20000^2); flip = Z1 >= Z0; re-orient} until a round after the fifth
+ * flips all or none.  A round in which the live cells give some SNP no depth makes the reference's EM all NaN: it
+ * flips nothing.  No live cell left: the region failed (status 0), nothing flips.  Otherwise (status 1) the final
+ * flips are inverted when more than half flip, written to flip_out and applied to ref_idx (in/out, 0 / 1 per SNP).
+ * Status 2: as 1, but some flip (|Z1 - Z0| < 1e-6) or convergence test (|dll - 1e-3| < 1e-9 max(1, |ll|)) was a
+ * tie that the reference's own rounding decides; the caller re-decides the region and reruns the later waves.
+ * Regions arrive in wave order (wave_ptr): regions of one wave share no SNP, and a region reads ref_idx as the
+ * earlier waves left it; the waves run in order on the context's stream without a host synchronisation.
+ * Entries are the (SNP slot, cell) pairs with DP > 0 of each region, given SNP-major (slot_ent_ptr: per slot, local
+ * cell id, AD = UMIs with ALT, DP = UMIs with REF or ALT) and cell-major (cell_ent_ptr: per local cell, local SNP
+ * index in the region's list) -- the same entries of region r in both.  FP64, fixed summation order: the same
+ * input gives the same bytes.  xg_last_timing: [0] device span  [1] EM kernels  [2] waves  [3] regions
+ * [4] inner EM iterations  [5] longest region (ms, one CTA)  [6] its share of [1]  [7] entries  [8] status-2
+ * regions  [12] host ms.                                                                                        */
+typedef struct {
+    int32_t n_regions, n_waves;
+    const int32_t *wave_ptr;        /* n_waves + 1: regions of wave w are [wave_ptr[w], wave_ptr[w + 1])     */
+    const int64_t *reg_snp_ptr;     /* n_regions + 1: SNP slots of region r                                 */
+    const int32_t *reg_snp;         /* per slot: SNP index (< n_snps), the region's order (sorted by position) */
+    const int64_t *slot_ent_ptr;    /* slots + 1: SNP-major entries of each slot                             */
+    const int32_t *sm_cell, *sm_ad, *sm_dp;
+    const int64_t *reg_cell_ptr;    /* n_regions + 1: local cells of region r                               */
+    const int64_t *cell_ent_ptr;    /* cells + 1: cell-major entries of each local cell                      */
+    const int32_t *cm_snp, *cm_ad, *cm_dp;
+} xg_phase_regions;
+int xg_local_phase(xg_ctx *ctx, int32_t n_snps, const int32_t *snp_pos, uint8_t *ref_idx, const xg_phase_regions *regs,
+                   uint8_t *keep_out /* per slot */, uint8_t *flip_out /* per slot */, int8_t *status_out /* per region */);
+
 /* Synthetic 10x-style records generated directly in HBM (bench / tests; no reference
  * counterpart -- SURVEY.md 8(d) C3 allows device-side generation for kernel-only runs).  */
 typedef struct {

@@ -30,7 +30,7 @@ class Config(object):
         ("sample_id_fn", "sample_id_file", "%s"), ("region_fn", "region_file", "%s"),
         ("snp_fn", "snp_file", "%s"), ("out_dir", "out_dir", "%s"), ("debug", "debug_level", "%d"), None,
         ("cellsnp_dir", "cellsnp_dir", "%s"), ("ref_cell_fn", "ref_cell_fn", "%s"),
-        ("cell_tag", "cell_tag", "%s"), ("umi_tag", "umi_tag", "%s"),
+        ("phase_from_reads", "phase_from_reads", "%s"), ("cell_tag", "cell_tag", "%s"), ("umi_tag", "umi_tag", "%s"),
         ("nproc", "number_of_processes", "%d"), ("min_count", "min_count", "%d"),
         ("min_maf", "min_maf", "%f"), ("output_all_reg", "output_all_reg", "%s"),
         ("no_dup_hap", "no_dup_hap", "%s"), None,
@@ -56,6 +56,7 @@ class Config(object):
         self.region_fn = self.snp_fn = self.out_dir = None
         self.debug = d.DEBUG
         self.cellsnp_dir = self.ref_cell_fn = None
+        self.phase_from_reads = False      # local phasing from the call's own reads instead of cellsnp_dir
         self.cell_tag, self.umi_tag = d.CELL_TAG, d.UMI_TAG
         self.nproc = d.NPROC
         self.min_count, self.min_maf = d.MIN_COUNT, d.MIN_MAF
@@ -99,7 +100,7 @@ class Config(object):
         return self.cell_tag is not None
 
     def use_local_phasing(self):
-        return self.cellsnp_dir is not None
+        return self.cellsnp_dir is not None or self.phase_from_reads
 
     def use_umi(self):
         return self.umi_tag is not None

@@ -20,7 +20,7 @@ from ...utils.zfile import zopen
 from ...utils.csp_io import load_data as csp_load_data
 from ...utils.grange import format_chrom
 from .config import Config
-from .phasing import reg_local_phasing
+from .phasing import csr_from_coo, is_long_region, local_phasing_device, reg_local_phasing
 from .utils import load_region_from_txt, load_snp_from_tsv, load_snp_from_vcf
 
 BASES = "ACGTN"
@@ -31,8 +31,10 @@ def afc_wrapper(sam_fn, barcode_fn, region_fn, phased_snp_fn, out_dir, sam_list_
                 sample_ids=None, sample_id_fn=None, debug_level=0, ncores=1, cellsnp_dir=None,
                 ref_cell_fn=None, cell_tag="CB", umi_tag="UB", min_count=1, min_maf=0,
                 output_all_reg=False, no_dup_hap=True, min_mapq=20, min_len=30, incl_flag=0,
-                excl_flag=None, no_orphan=True):
-    """Python API, signature of baf/fc/main.py:32-47."""
+                excl_flag=None, no_orphan=True, phase_from_reads=False):
+    """Python API, signature of baf/fc/main.py:32-47.  phase_from_reads: phase the long regions locally from this
+    call's own reads (SNP x cell counts of every SNP of those regions, as `pileup_wrapper` with its default filter
+    writes them), without a cellsnp-lite directory; not together with cellsnp_dir."""
     conf = Config()
     conf.sam_fn, conf.sam_list_fn = sam_fn, sam_list_fn
     conf.barcode_fn, conf.region_fn, conf.snp_fn = barcode_fn, region_fn, phased_snp_fn
@@ -47,6 +49,7 @@ def afc_wrapper(sam_fn, barcode_fn, region_fn, phased_snp_fn, out_dir, sam_list_
     conf.incl_flag = incl_flag
     conf.excl_flag = -1 if excl_flag is None else excl_flag
     conf.no_orphan = no_orphan
+    conf.phase_from_reads = bool(phase_from_reads)
     return afc_run(conf)
 
 
@@ -128,6 +131,9 @@ def prepare_tags(conf):
 
 def prepare_config(conf):
     """Validate options, load regions / SNPs; 0 if ok, -1 otherwise (baf/fc/main.py:298-495)."""
+    if conf.phase_from_reads and conf.cellsnp_dir is not None:
+        error("should not specify 'phase_from_reads' and 'cellsnp_dir' together.")
+        return -1
     if prepare_samples(conf) < 0:
         return -1
     pre = os.path.join(conf.out_dir, conf.out_prefix)
@@ -273,6 +279,23 @@ def _count_shard(conf, batch, regs, snps):
     return out, [ctx.timing()], None
 
 
+def load_unit_batch(conf, chroms, unit_chrom, unit_beg, unit_end):
+    """The reads of the units (contig or None, 0-based [beg, end)) with sequences, one batch per GPU: a
+    ShardedBatch / MultiBatch with several GPUs, else one ReadBatch.  The caller closes it."""
+    from ... import parallel
+    n_dev = parallel.n_devices(getattr(conf, "n_gpus", None))
+    threads = engine.n_decode_threads(conf.nproc)
+    if n_dev > 1:
+        batch = engine.load_reads_sharded(conf.sam_fn_list, chroms, conf.cell_tag, conf.umi_tag, True,
+                                          parallel.device_list(n_dev), unit_chrom, unit_beg, unit_end)
+        if batch is None:
+            batch = engine.load_reads_multi(conf.sam_fn_list, chroms, conf.cell_tag, conf.umi_tag, True,
+                                            threads, devices=parallel.device_list(n_dev))
+        return batch
+    return engine.load_reads(conf.sam_fn_list, engine.Request(chroms, unit_chrom, unit_beg, unit_end),
+                             conf.cell_tag, conf.umi_tag, True, threads, mapped=True)
+
+
 def shard_units(conf, chroms, unit_chrom, unit_beg, unit_end, run, batch=None):
     """Device work on independent units (regions, single SNPs, genomic windows) with one read batch per GPU.
     unit_chrom / unit_beg / unit_end: contig (None: never fetched) and 0-based [beg, end) of every unit; run(batch,
@@ -280,19 +303,9 @@ def shard_units(conf, chroms, unit_chrom, unit_beg, unit_end, run, batch=None):
     no collective.  Returns ([(idx, run(batch, idx), or None for a chunk without reads or units)], sharded)."""
     from ... import parallel
     n_unit = len(unit_beg)
-    n_dev = parallel.n_devices(getattr(conf, "n_gpus", None))
     own = batch is None
     if own:
-        threads = engine.n_decode_threads(conf.nproc)
-        if n_dev > 1:
-            batch = engine.load_reads_sharded(conf.sam_fn_list, chroms, conf.cell_tag, conf.umi_tag, True,
-                                              parallel.device_list(n_dev), unit_chrom, unit_beg, unit_end)
-            if batch is None:
-                batch = engine.load_reads_multi(conf.sam_fn_list, chroms, conf.cell_tag, conf.umi_tag, True,
-                                                threads, devices=parallel.device_list(n_dev))
-        else:
-            batch = engine.load_reads(conf.sam_fn_list, engine.Request(chroms, unit_chrom, unit_beg, unit_end),
-                                      conf.cell_tag, conf.umi_tag, True, threads, mapped=True)
+        batch = load_unit_batch(conf, chroms, unit_chrom, unit_beg, unit_end)
     try:
         if isinstance(batch, (engine.ShardedBatch, engine.MultiBatch)):
             if isinstance(batch, engine.ShardedBatch):
@@ -356,6 +369,70 @@ def count_regions(conf, regs, batch=None):
     return out
 
 
+def _phase_pileup_shard(conf, batch, regs, is_long, idx):
+    """SNP x cell AD / DP of the SNPs of the long regions among `idx` on one batch (xg_snp_pileup, filter (0, 0)):
+    (SNP ids, AD (row, col, val), DP (row, col, val)) with rows = SNP ids."""
+    ids = list(dict.fromkeys(s.index for i in idx if is_long[i] for s in regs[i].snp_list))
+    if not ids:
+        return None
+    sub = [conf.snp_set.snps[i] for i in ids]
+    gid, pos0, cell_keys, params = snp_arrays(conf, batch, sub)
+    ref_i, alt_i = allele_indices(sub)
+    ad, dp, _oth = batch.ctx.snp_pileup(batch.dreads, gid, pos0, cell_keys, len(conf.samples), params, ref_i, alt_i,
+                                        0, 0.0)
+    ids = np.asarray(ids, dtype=np.int64)
+    return ids, [(ids[np.asarray(m[0], dtype=np.int64)], np.asarray(m[1]), np.asarray(m[2])) for m in (ad, dp)]
+
+
+def phase_from_reads(conf, regs, batch):
+    """Local phasing of the long regions of `regs` from the reads of `batch` (loaded with `regs` as units): the
+    pileup of their SNPs on every shard (a SNP of two shards is piled up on both; the copy of the first shard is
+    kept), then the EM of all of them on one device, so that the waves stay global.  Returns the counters of
+    afc_core's two log lines."""
+    snps = conf.snp_set.snps
+    chroms = list(dict.fromkeys([s.chrom for s in snps]))
+    is_long = [is_long_region(conf, reg) for reg in regs]
+    long_regs = [reg for reg, x in zip(regs, is_long) if x]
+    n_rlp, n_rlp_failed, n_slp, n_slp_flipped = len(long_regs), 0, 0, 0
+    if long_regs:
+        res, _sharded = shard_units(conf, chroms, [r.chrom if r.snp_list else None for r in regs],
+                                    [r.start - 1 for r in regs], [r.end - 1 for r in regs],
+                                    lambda b, idx: _phase_pileup_shard(conf, b, regs, is_long, idx), batch)
+        seen = np.zeros(len(snps), dtype=bool)
+        parts = ([], [])
+        for _idx, p in res:
+            if p is None:
+                continue
+            ids, mats = p
+            mine = np.zeros(len(snps), dtype=bool)
+            mine[ids[~seen[ids]]] = True
+            seen[ids] = True
+            for w in range(2):
+                r, c, v = mats[w]
+                take = mine[r]
+                parts[w].append((r[take], c[take], v[take]))
+        ad, dp = ([np.concatenate([x[k] for x in parts[w]] + [np.zeros(0, np.int64)]) for k in range(3)]
+                  for w in range(2))
+        cell_mask = np.ones(len(conf.samples), dtype=bool)
+        if conf.ref_cells is not None:
+            cell_mask = ~np.isin(np.asarray(conf.samples, dtype=str), np.asarray(conf.ref_cells, dtype=str))
+        csr = csr_from_coo(len(snps), ad, dp, cell_mask)
+        flips, conf.last_phase_timing = local_phasing_device(engine.get_context(0), long_regs, snps, csr,
+                                                             len(conf.samples))
+        for reg, flip in zip(long_regs, flips):
+            if flip is None:
+                n_rlp_failed += 1
+                if conf.debug > 1:
+                    debug("region '%s': local phasing failed." % reg.name)
+            else:
+                if conf.debug > 1:
+                    debug("region '%s': #SNPs - total=%d; flipped=%d" % (reg.name, len(reg.snp_list), np.sum(flip)))
+                n_slp_flipped += np.sum(flip)
+            n_slp += len(reg.snp_list)
+    conf.ref_cells = None
+    return n_rlp, n_rlp_failed, n_slp, n_slp_flipped
+
+
 def afc_core(conf):
     if prepare_config(conf) < 0:
         raise ValueError("errcode -2")
@@ -374,11 +451,25 @@ def afc_core(conf):
     info("#regions: total=%d; with_snps=%d." % (len(conf.reg_list), len(with_snps)))
     if not conf.output_all_reg:
         conf.reg_list = with_snps
-    # local phasing inside long regions (baf/fc/main.py:107-149): host numpy EM on the cellsnp-lite counts; it
-    # may drop unexpressed SNPs from a region's list and swap the haplotype indices of (shared) SNP objects.
-    # The device gets the lists and haplotype tables as they are afterwards.
+    # local phasing inside long regions (baf/fc/main.py:107-149): host numpy EM on the cellsnp-lite counts, or, with
+    # phase_from_reads, the device EM on the counts of this call's reads (phase_from_reads); it may drop unexpressed
+    # SNPs from a region's list and swap the haplotype indices of (shared) SNP objects.  The device gets the lists
+    # and haplotype tables as they are afterwards.
     n_rlp = n_rlp_failed = n_slp = n_slp_flipped = 0
-    if conf.use_local_phasing():
+    batch = None
+    if conf.phase_from_reads:
+        if conf.reg_list:
+            # one decode for both steps: the regions are the units of the batch, as count_regions would load it
+            snps = conf.snp_set.snps
+            batch = load_unit_batch(conf, list(dict.fromkeys([s.chrom for s in snps])),
+                                    [r.chrom if r.snp_list else None for r in conf.reg_list],
+                                    [r.start - 1 for r in conf.reg_list], [r.end - 1 for r in conf.reg_list])
+            try:
+                n_rlp, n_rlp_failed, n_slp, n_slp_flipped = phase_from_reads(conf, conf.reg_list, batch)
+            except BaseException:
+                batch.close()
+                raise
+    elif conf.use_local_phasing():
         data = conf.snp_adata
         if conf.ref_cells is not None:
             data = data.subset_cells(~np.isin(data.cells.astype(str), np.asarray(conf.ref_cells, dtype=str)))
@@ -409,11 +500,14 @@ def afc_core(conf):
     info("#SNPs: local_phasing=%d; local_phasing_flipped=%d." % (n_slp, n_slp_flipped))
 
     regs = conf.reg_list
-    if len(regs) == 0:
-        # the reference divides by the worker count min(nproc, 0) here (main.py:152-158)
-        raise ZeroDivisionError("integer division or modulo by zero")
-
-    (ad, dp, oth) = count_regions(conf, regs)
+    try:
+        if len(regs) == 0:
+            # the reference divides by the worker count min(nproc, 0) here (main.py:152-158)
+            raise ZeroDivisionError("integer division or modulo by zero")
+        (ad, dp, oth) = count_regions(conf, regs, batch=batch)
+    finally:
+        if batch is not None:
+            batch.close()
 
     # emit (baf/fc/core.py:70-122): a region with SNPs gets a row iff it has a DP or OTH
     # entry, or output_all_reg; SNP-less regions only with output_all_reg.

@@ -15,7 +15,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.environ.get("XG_LIBDIR") or os.path.join(HERE, "_lib")    # XG_LIBDIR: side builds for debugging
 LIB = os.path.join(LIBDIR, "libxcltk_b200.so")
 
-CU = ["ctx.cu", "basefc.cu", "baf.cu", "discover.cu", "synth.cu", "gpu_decode.cu"]
+CU = ["ctx.cu", "basefc.cu", "baf.cu", "discover.cu", "synth.cu", "gpu_decode.cu", "phase.cu"]
 CPP = ["decode.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "--expt-relaxed-constexpr", "-Xcompiler", "-fPIC,-O3,-Wall", "-Xptxas", "-v"]

@@ -104,6 +104,13 @@ class Sites(C.Structure):
                 ("totals", c_i64p)]
 
 
+class PhaseRegions(C.Structure):
+    _fields_ = [("n_regions", C.c_int32), ("n_waves", C.c_int32), ("wave_ptr", c_i32p), ("reg_snp_ptr", c_i64p),
+                ("reg_snp", c_i32p), ("slot_ent_ptr", c_i64p), ("sm_cell", c_i32p), ("sm_ad", c_i32p),
+                ("sm_dp", c_i32p), ("reg_cell_ptr", c_i64p), ("cell_ent_ptr", c_i64p), ("cm_snp", c_i32p),
+                ("cm_ad", c_i32p), ("cm_dp", c_i32p)]
+
+
 # every symbol include/xcltk_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 SYMBOLS = {
@@ -165,6 +172,8 @@ SYMBOLS = {
     "xg_snp_discover": (C.c_int, [_P, _P, C.POINTER(Features), C.POINTER(Barcodes), C.POINTER(Params),
                                   C.POINTER(DiscoverFilter), C.POINTER(C.POINTER(Sites))]),
     "xg_sites_free": (None, [C.POINTER(Sites)]),
+    "xg_local_phase": (C.c_int, [_P, C.c_int32, c_i32p, c_u8p, C.POINTER(PhaseRegions), c_u8p, c_u8p,
+                                 C.POINTER(C.c_int8)]),
     "xg_synth_reads": (C.c_int, [_P, C.POINTER(SynthParams), C.POINTER(_P), c_u64p]),
     "xg_synth_read_index": (C.c_int64, [C.POINTER(SynthParams), C.c_int32, C.c_int32]),
     "xg_write_bam": (C.c_int, [C.c_char_p, C.POINTER(Reads), C.c_int32, C.POINTER(C.c_char_p), c_i64p, _P,
@@ -799,6 +808,39 @@ class Context(object):
         finally:
             self.lib.xg_sites_free(out)
         return res
+
+    def local_phase(self, snp_pos, ref_idx, layout):
+        """Local phasing of the regions of `layout` on the device (xg_local_phase).  snp_pos: 1-based position per
+        SNP; ref_idx: 0 / 1 per SNP, updated in place with the flips.  layout: dict of the xg_phase_regions arrays
+        (wave_ptr, reg_snp_ptr, reg_snp, slot_ent_ptr, sm_cell, sm_ad, sm_dp, reg_cell_ptr, cell_ent_ptr, cm_snp,
+        cm_ad, cm_dp; baf/fc/phasing.py:phase_layout builds it).  Returns (keep, flip, status): uint8 per slot,
+        uint8 per slot, int8 per region (1 phased, 0 failed).  timing() then holds the EM statistics."""
+        pos = np.ascontiguousarray(snp_pos, dtype=np.int32)
+        if not isinstance(ref_idx, np.ndarray) or ref_idx.dtype != np.uint8 or not ref_idx.flags.c_contiguous:
+            raise ValueError("local_phase: ref_idx must be a contiguous uint8 array (updated in place)")
+        if len(ref_idx) != len(pos):
+            raise ValueError("local_phase: snp_pos and ref_idx of different lengths")
+        i32 = ("wave_ptr", "reg_snp", "sm_cell", "sm_ad", "sm_dp", "cm_snp", "cm_ad", "cm_dp")
+        a = {k: np.ascontiguousarray(layout[k], dtype=np.int32 if k in i32 else np.int64)
+             for k in i32 + ("reg_snp_ptr", "slot_ent_ptr", "reg_cell_ptr", "cell_ent_ptr")}
+        n_reg, n_slot = len(a["reg_snp_ptr"]) - 1, len(a["reg_snp"])
+        if n_reg < 0 or len(a["reg_cell_ptr"]) != n_reg + 1 or len(a["slot_ent_ptr"]) != n_slot + 1:
+            raise ValueError("local_phase: inconsistent region arrays")
+        n_ent = len(a["sm_cell"])
+        if any(len(a[k]) != n_ent for k in ("sm_ad", "sm_dp", "cm_snp", "cm_ad", "cm_dp")):
+            raise ValueError("local_phase: entry arrays of different lengths")
+        if a["slot_ent_ptr"][-1] != n_ent or a["cell_ent_ptr"][-1] != n_ent:
+            raise ValueError("local_phase: entry offsets do not end at the number of entries")
+        r = PhaseRegions(n_reg, len(a["wave_ptr"]) - 1, *[as_ptr(a[k], c_i32p if k in i32 else c_i64p) for k in (
+            "wave_ptr", "reg_snp_ptr", "reg_snp", "slot_ent_ptr", "sm_cell", "sm_ad", "sm_dp", "reg_cell_ptr",
+            "cell_ent_ptr", "cm_snp", "cm_ad", "cm_dp")])
+        keep = np.zeros(max(n_slot, 1), dtype=np.uint8)
+        flip = np.zeros(max(n_slot, 1), dtype=np.uint8)
+        status = np.zeros(max(n_reg, 1), dtype=np.int8)
+        self._check(self.lib.xg_local_phase(self.h, len(pos), as_ptr(pos, c_i32p), as_ptr(ref_idx, c_u8p), C.byref(r),
+                                            as_ptr(keep, c_u8p), as_ptr(flip, c_u8p),
+                                            as_ptr(status, C.POINTER(C.c_int8))))
+        return keep[:n_slot], flip[:n_slot], status[:n_reg]
 
     def set_option(self, name, value):
         self._check(self.lib.xg_set_option(self.h, name.encode(), int(value)))
