@@ -342,6 +342,26 @@ int xg_basefc_host(xg_ctx *ctx, const xg_reads *host, const xg_features *feats,
  * writers above (out_row[r]: 1-based output row of input row r, 0 = not emitted; n_rows_in = rows of that call). */
 int xg_basefc_write_mtx_device(xg_ctx *ctx, const char *path, int32_t n_rows_in, const int32_t *out_row,
                                int32_t n_rows_out, int32_t n_threads);
+/* Read-assignment summary of basefc (what htseq-count's special counters and featureCounts' .summary report; the
+ * reference has no counterpart).  It counts RECORDS, not UMIs: a record is in range iff it overlaps some feature that
+ * fetch() would query (gid >= 0, beg >= 0, end > beg) with sam.fetch's rule pos < end && bam_endpos > beg
+ * (utils/sam.py:85-118); records in range of no feature are not counted (the reference never sees them).  Row: the
+ * column of the record's cell key if that key is listed, else row n_samples ("__no_cell": tag missing or barcode not
+ * listed); sample-ID mode: the BAM's column (row n_samples stays 0).  Fate: the first that applies, in check_read's
+ * order (rdr/fc/core.py:46-62) --
+ *   0 mapq < min_mapq   1 excl_flag hit, incl_flag missed or orphan   2 need_umi_tag and the UMI tag missing or
+ *   empty (such a record never reaches the matrix)   3 aligned length < min_len   then the include test
+ *   (rdr/fc/core.py:160-165, as xg_basefc applies it) for every feature the record overlaps:
+ *   4 fails for all   5 passes for exactly one   6 passes for two or more (counted once in each, SURVEY.md A.1 R9).
+ * out: (n_samples + 1) x 7 counters, row-major.  own: NULL, or the half-open range [(own[0], own[1]), (own[2],
+ * own[3])) of record start keys (gid, pos) that the call counts (one library split between GPUs: every record is
+ * counted by the GPU whose cut holds its start).  Works on batches from xg_upload_reads, the device decoder and
+ * xg_map_reads (flags, keys and CIGAR are read for the records in range only); XG_E_ARG when keys are not 16-byte,
+ * pos_end not 8-byte or the other record arrays not 4-byte aligned.  Uses the interval index of the
+ * context's last xg_basefc call when the features are the same; never touches the staging area that
+ * xg_basefc_write_mtx_device formats.  xg_last_timing: [0] / [1] the kernel (ms)  [2] launches  [12] host ms. */
+int xg_basefc_summary(xg_ctx *ctx, const xg_dreads *reads, const xg_features *feats, const xg_barcodes *cells,
+                      const xg_params *par, const int32_t *own, int64_t *out);
 
 /* baf phase 1: replaces plp_snp() up to mcnt.stat() (baf/fc/core.py:198-237; first-read-wins
  * per (SNP, cell, UMI): baf/fc/mcount.py:109-127; allele: :39-60 + utils/sam.py:4-40).

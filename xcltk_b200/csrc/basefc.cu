@@ -1811,13 +1811,10 @@ static int basefc_params(BasefcCall &c, const xg_barcodes *cells, const xg_param
     return XG_OK;
 }
 
-// Interval index of the features (host) and every feature's tile window and exact candidate count (device).
-static int basefc_windows(BasefcCall &c, const xg_features *feats, int32_t n_gid) {
-    xg_ctx *ctx = c.ctx;
-    const xg_dreads *rd = c.rd;
-    auto t_ph = std::chrono::steady_clock::now();
-    // the interval index depends on the features only: reuse it (host copy and the uploaded
-    // device arrays, which live in named scratch buffers) while the caller passes the same set
+// The context's interval index of `feats` (FeatCache).  It depends on the features only: it is rebuilt only when the
+// caller passes another set (host copy in the cache; device arrays in the named scratch buffers "fx_*", uploaded by
+// feat_index_upload).  *cached: the index was the last call's.
+static int feat_index(xg_ctx *ctx, const xg_features *feats, int32_t n_gid, FeatCache **out, bool *cached) {
     const size_t fb = sizeof(int32_t) * (size_t)feats->n;
     const std::initializer_list<xg_input_key::Span> in = {
         {&n_gid, sizeof n_gid}, {&feats->n, sizeof feats->n}, {feats->gid, fb}, {feats->beg, fb}, {feats->end, fb}};
@@ -1828,17 +1825,55 @@ static int basefc_windows(BasefcCall &c, const xg_features *feats, int32_t n_gid
         ctx->fx_cache = fc;
         ctx->fx_cache_free = [](void *p) { delete (FeatCache *)p; };
     }
+    *out = fc;
+    *cached = fc->valid && fc->key.matches(fh, in);
+    if (!*cached) {
+        fc->valid = false;
+        fc->ix = FeatIndexHost();
+        int rc = build_feat_index(ctx, feats, n_gid, fc->ix);
+        if (rc) return rc;
+        fc->key.assign(fh, in);
+    }
+    return XG_OK;
+}
+
+// The index's device arrays (stabbing entries with their segment offsets zeroed); the cache is valid afterwards.
+static int feat_index_upload(xg_ctx *ctx, FeatCache *fc) {
+    const FeatIndexHost &ix = fc->ix;
+    std::vector<int4> stab4(ix.stab.size());
+    for (size_t k = 0; k < ix.stab.size(); k++) {
+        const int32_t j = ix.stab[k];
+        stab4[k] = make_int4(j, ix.sf_beg[(size_t)j], ix.sf_end[(size_t)j], 0);
+    }
+    const int4 *d_stab4 = nullptr;
+    const int32_t *d = nullptr;
+    int rc = XG_OK;
+    if ((rc = upload_vec(ctx, ix.sf_goff, "fx_sf_goff", &d))) return rc;
+    if ((rc = upload_vec(ctx, ix.sf_beg, "fx_sf_beg", &d))) return rc;
+    if ((rc = upload_vec(ctx, ix.sf_end, "fx_sf_end", &d))) return rc;
+    if ((rc = upload_vec(ctx, ix.sf_row, "fx_sf_row", &d))) return rc;
+    if ((rc = upload_vec(ctx, ix.bnd_goff, "fx_bnd_goff", &d))) return rc;
+    if ((rc = upload_vec(ctx, ix.bnd, "fx_bnd", &d))) return rc;
+    if ((rc = upload_vec(ctx, ix.stab_off, "fx_stab_off", &d))) return rc;
+    if ((rc = upload_vec(ctx, stab4, "fx_stab4", &d_stab4))) return rc;
+    if ((rc = upload_vec(ctx, ix.fb, "fx_fb", &d))) return rc;
+    XG_CUDA(cudaStreamSynchronize(ctx->stream));
+    fc->valid = true;
+    return XG_OK;
+}
+
+// Interval index of the features (host) and every feature's tile window and exact candidate count (device).
+static int basefc_windows(BasefcCall &c, const xg_features *feats, int32_t n_gid) {
+    xg_ctx *ctx = c.ctx;
+    const xg_dreads *rd = c.rd;
+    auto t_ph = std::chrono::steady_clock::now();
+    FeatCache *fc = nullptr;
+    bool index_cached = false;
+    int rc = feat_index(ctx, feats, n_gid, &fc, &index_cached);
+    if (rc) return rc;
     c.fc = fc;
     if (!fc->h_sum && !(fc->h_sum = (PlanSummary *)ctx->pinned_get(sizeof(PlanSummary))))
         return ctx->fail(XG_E_NOMEM, "out of pinned host memory");
-    const bool index_cached = fc->valid && fc->key.matches(fh, in);
-    int rc = XG_OK;
-    if (!index_cached) {
-        fc->valid = false;
-        fc->ix = FeatIndexHost();
-        if ((rc = build_feat_index(ctx, feats, n_gid, fc->ix))) return rc;
-        fc->key.assign(fh, in);
-    }
     const FeatIndexHost &ix = fc->ix;
     const size_t m = c.m = ix.sf_beg.size();
     c.ms_index = ms_since(t_ph);
@@ -1852,26 +1887,7 @@ static int basefc_windows(BasefcCall &c, const xg_features *feats, int32_t n_gid
     if (((uintptr_t)rd->pos_end | (uintptr_t)rd->fmq | (uintptr_t)rd->cig_off | (uintptr_t)rd->keys |
          (uintptr_t)rd->cigar) & 15)
         return ctx->fail(XG_E_ARG, "xg_basefc: record arrays must be 16-byte aligned");
-    if (!index_cached) {
-        std::vector<int4> stab4(ix.stab.size());
-        for (size_t k = 0; k < ix.stab.size(); k++) {
-            const int32_t j = ix.stab[k];
-            stab4[k] = make_int4(j, ix.sf_beg[(size_t)j], ix.sf_end[(size_t)j], 0);
-        }
-        const int4 *d_stab4 = nullptr;
-        const int32_t *d = nullptr;
-        if ((rc = upload_vec(ctx, ix.sf_goff, "fx_sf_goff", &d))) return rc;
-        if ((rc = upload_vec(ctx, ix.sf_beg, "fx_sf_beg", &d))) return rc;
-        if ((rc = upload_vec(ctx, ix.sf_end, "fx_sf_end", &d))) return rc;
-        if ((rc = upload_vec(ctx, ix.sf_row, "fx_sf_row", &d))) return rc;
-        if ((rc = upload_vec(ctx, ix.bnd_goff, "fx_bnd_goff", &d))) return rc;
-        if ((rc = upload_vec(ctx, ix.bnd, "fx_bnd", &d))) return rc;
-        if ((rc = upload_vec(ctx, ix.stab_off, "fx_stab_off", &d))) return rc;
-        if ((rc = upload_vec(ctx, stab4, "fx_stab4", &d_stab4))) return rc;
-        if ((rc = upload_vec(ctx, ix.fb, "fx_fb", &d))) return rc;
-        XG_CUDA(cudaStreamSynchronize(ctx->stream));
-        fc->valid = true;
-    }
+    if (!index_cached && (rc = feat_index_upload(ctx, fc))) return rc;
     // the named scratch buffers keep their addresses between calls
     const int32_t *d_sf_goff = (const int32_t *)ctx->scratch["fx_sf_goff"].p;
     const int32_t *d_sf_beg = (const int32_t *)ctx->scratch["fx_sf_beg"].p;
@@ -2683,5 +2699,245 @@ extern "C" int xg_basefc_finalize_stats(xg_ctx *ctx, int64_t out[8]) {
         XG_CUDA(cudaMemcpy(h, it->second.p, sizeof h, cudaMemcpyDeviceToHost));
     }
     for (int k = 0; k < FS_STATS; k++) out[k] = (int64_t)h[k];
+    return XG_OK;
+}
+
+// ---- read-assignment summary (xg_basefc_summary) -----------------------------------------------------------------
+// One CTA per tile, a thread per record.  Phase 1 reads pos / end only (coalesced) and finds, through the interval
+// index of the features, whether the record overlaps one: the features covering `pos` (the stabbing list of its
+// segment) or beginning in (pos, end).  Only the records in range go on to their flags, keys and CIGAR: their fate is
+// the first of check_read's tests (rdr/fc/core.py:46-62) that fails, else how many features pass the include test
+// (rdr/fc/core.py:160-165, as k_basefc_count applies it), counted up to two.  The warp adds its counts per counter
+// (match_any on the address) before the global atomics.
+namespace {
+#define SUM_FATES 7
+#define SUM_THREADS 256
+
+struct SummaryDev {
+    const int2 *pos_end;
+    const uint32_t *fmq, *cig_off, *cigar;
+    const ulonglong2 *keys;
+    const xg_tile *tiles;
+    const xg_run *runs;
+    const int32_t *bnd_goff, *bnd, *stab_off, *fb, *sf_end;
+    const int4 *stab4;            // {sorted feature, beg, end, -}
+    int32_t n_gid, n_samples;
+    int32_t own_g0, own_p0, own_g1, own_p1;   // records with (gid, pos) in [(g0, p0), (g1, p1))
+    BarcodeTable bc;
+    FilterParams fp;
+    const int32_t *incl_tab;
+    int32_t incl_tab_len, incl_len;
+    unsigned long long *out;      // (n_samples + 1) x SUM_FATES
+};
+
+// m of the include test for feature [s0, e0) (emit_pair)
+__device__ __forceinline__ int32_t summary_m(const uint32_t *cig, uint32_t n_ops, int32_t pos, int32_t end, int32_t aln,
+                                             int32_t s0, int32_t e0) {
+    if (n_ops == 0) {
+        const int32_t a = max(pos, s0), b = min(end, e0);
+        return b > a ? b - a : 0;
+    }
+    if (s0 <= pos && end <= e0) return aln;
+    return included_len(cig, n_ops, pos, s0, e0);
+}
+
+__global__ void __launch_bounds__(SUM_THREADS) k_basefc_summary(const __grid_constant__ SummaryDev P) {
+    __shared__ int32_t s_win[2];  // the tile's window of boundaries [lo, hi) for the search of every record
+    const xg_tile tl = P.tiles[blockIdx.x];
+    const int32_t gid = P.runs[tl.run].gid;
+    if (gid < 0 || gid >= P.n_gid) return;
+    const int32_t b0 = P.bnd_goff[gid], b1 = P.bnd_goff[gid + 1];
+    if (b0 == b1) return;                                     // a contig without features
+    if (gid < P.own_g0 || gid > P.own_g1 || (gid == P.own_g1 && tl.first_pos >= P.own_p1)) return;
+    if (threadIdx.x == 0) {
+        // every record's pos is >= first_pos: its first boundary > pos is >= the first one > first_pos, and (when
+        // pos < max_end) <= the first one >= max_end
+        int32_t lo = b0, hi = b1;
+        while (lo < hi) {
+            const int32_t mid = (lo + hi) >> 1;
+            if (P.bnd[mid] <= tl.first_pos) lo = mid + 1; else hi = mid;
+        }
+        int32_t a = lo;
+        hi = b1;
+        while (a < hi) {
+            const int32_t mid = (a + hi) >> 1;
+            if (P.bnd[mid] < tl.max_end) a = mid + 1; else hi = mid;
+        }
+        s_win[0] = lo;
+        s_win[1] = a;
+    }
+    __syncthreads();
+    const int32_t w_lo = s_win[0], w_hi = s_win[1];
+    const int32_t col_tile = P.runs[tl.run].bam_idx;
+    for (int32_t base = 0; base < tl.n_rec; base += SUM_THREADS) {    // the same trip count for every thread
+        const int32_t k = base + (int32_t)threadIdx.x;
+        bool on = false;
+        int32_t row = 0, fate = 0;
+        if (k < tl.n_rec) {
+            const int64_t i = tl.rec_beg + k;
+            const int2 pe = __ldcs(&P.pos_end[i]);
+            const bool own = (gid > P.own_g0 || (gid == P.own_g0 && pe.x >= P.own_p0)) &&
+                             (gid < P.own_g1 || (gid == P.own_g1 && pe.x < P.own_p1));
+            int32_t ub = w_hi, s0i = 0, s1i = 0;
+            if (own) {
+                int32_t lo = w_lo, hi = pe.x < tl.max_end ? w_hi : b1;
+                while (lo < hi) {                             // first boundary > pos
+                    const int32_t mid = (lo + hi) >> 1;
+                    if (__ldg(&P.bnd[mid]) <= pe.x) lo = mid + 1; else hi = mid;
+                }
+                ub = lo;
+                if (ub > b0) {
+                    s0i = __ldg(&P.stab_off[ub - 1]);
+                    s1i = __ldg(&P.stab_off[ub]);
+                }
+                // phase 1: in range iff some feature overlaps [pos, end) (pos < f.end && end > f.beg)
+                for (int32_t s = s0i; s < s1i && !on; s++) {
+                    const int4 f = __ldg(&P.stab4[s]);
+                    on = pe.x < f.z && pe.y > f.y;
+                }
+                for (int32_t kb = ub; kb < b1 && !on; kb++) {  // features beginning at a boundary in (pos, end)
+                    if (__ldg(&P.bnd[kb]) >= pe.y) break;
+                    on = __ldg(&P.fb[kb + 1]) > __ldg(&P.fb[kb]);
+                }
+            }
+            if (on) {
+                const uint32_t fmq = P.fmq[i];
+                if (P.fp.use_cell_tag) {
+                    const uint64_t ck = P.keys[i].x;
+                    const int32_t c = ck == XG_KEY_NONE ? -1 : barcode_lookup(P.bc, ck);
+                    row = c < 0 ? P.n_samples : c;
+                } else {
+                    row = col_tile;
+                }
+                if ((int32_t)((fmq >> 16) & 0xffu) < P.fp.min_mapq) {
+                    fate = 0;
+                } else if (!read_passes_flags(P.fp, fmq)) {           // the mapq test passed: a flag test failed
+                    fate = 1;
+                } else if (P.fp.need_umi_tag && (P.keys[i].y == XG_KEY_NONE || P.keys[i].y == XG_KEY_EMPTY)) {
+                    fate = 2;
+                } else {
+                    uint32_t n_ops = fmq >> 24;
+                    const uint32_t *cig = nullptr;
+                    int32_t aln;
+                    if (n_ops == 0) {
+                        aln = pe.y - pe.x;
+                    } else {
+                        const uint32_t co = P.cig_off[i];
+                        cig = P.cigar + co;
+                        if (n_ops == 255) n_ops = cig[-1];
+                        aln = 0;
+                        for (uint32_t q = 0; q < n_ops; q++) {
+                            const uint32_t cw = cig[q];
+                            if (cig_aligned(cw & 15u)) aln += (int32_t)(cw >> 4);
+                        }
+                    }
+                    if (aln < P.fp.min_len) {
+                        fate = 3;
+                    } else {
+                        const int32_t need =
+                            P.incl_tab ? __ldg(&P.incl_tab[min(aln, P.incl_tab_len - 1)]) : P.incl_len;
+                        int n_pass = 0;
+                        for (int32_t s = s0i; s < s1i && n_pass < 2; s++) {
+                            const int4 f = __ldg(&P.stab4[s]);
+                            if (pe.x < f.z && pe.y > f.y)
+                                n_pass += summary_m(cig, n_ops, pe.x, pe.y, aln, f.y, f.z) >= need;
+                        }
+                        for (int32_t kb = ub; kb < b1 && n_pass < 2; kb++) {
+                            const int32_t bv = __ldg(&P.bnd[kb]);
+                            if (bv >= pe.y) break;
+                            const int32_t j1 = __ldg(&P.fb[kb + 1]);
+                            for (int32_t j = __ldg(&P.fb[kb]); j < j1 && n_pass < 2; j++)
+                                n_pass += summary_m(cig, n_ops, pe.x, pe.y, aln, bv, __ldg(&P.sf_end[j])) >= need;
+                        }
+                        fate = 4 + n_pass;
+                    }
+                }
+            }
+        }
+        warp_add<unsigned long long>(on, &P.out[(int64_t)row * SUM_FATES + fate], 1ull);
+    }
+}
+}  // namespace
+
+extern "C" int xg_basefc_summary(xg_ctx *ctx, const xg_dreads *rd, const xg_features *feats, const xg_barcodes *cells,
+                                 const xg_params *par, const int32_t *own, int64_t *out) {
+    if (!ctx || !ctx->stream) return ctx ? ctx->fail(XG_E_CUDA, "context has no device") : XG_E_ARG;
+    if (!rd || !feats || !cells || !par || !out) return ctx->fail(XG_E_ARG, "xg_basefc_summary: null argument");
+    if (feats->n < 0 || cells->n_samples <= 0) return ctx->fail(XG_E_ARG, "xg_basefc_summary: empty sample list");
+    if (par->use_cell_tag && cells->n != cells->n_samples)
+        return ctx->fail(XG_E_ARG, "xg_basefc_summary: barcode mode needs one key per column");
+    if (par->min_incl_tab && par->min_incl_tab_len <= rd->max_aln_len)
+        return ctx->fail(XG_E_ARG, "min_incl_tab shorter than max aligned length + 1");
+    // the kernel's loads: keys as 16-byte pairs, pos / end as 8-byte pairs, the rest as 32-bit words
+    if (((uintptr_t)rd->keys & 15) | ((uintptr_t)rd->pos_end & 7) |
+        (((uintptr_t)rd->fmq | (uintptr_t)rd->cig_off | (uintptr_t)rd->cigar) & 3))
+        return ctx->fail(XG_E_ARG, "xg_basefc_summary: record arrays are not aligned to their element pairs / words");
+    XG_CUDA(cudaSetDevice(ctx->device));
+    int32_t n_gid = 0;
+    for (auto &r : rd->h_runs) n_gid = std::max(n_gid, r.gid + 1);
+    if (!par->use_cell_tag)
+        for (auto &r : rd->h_runs)
+            if (r.bam_idx >= cells->n_samples) return ctx->fail(XG_E_ARG, "more BAMs than sample columns");
+    for (double &t : ctx->timing) t = 0;
+    const auto t_call = std::chrono::steady_clock::now();
+    FeatCache *fc = nullptr;
+    bool cached = false;
+    int rc = feat_index(ctx, feats, n_gid, &fc, &cached);
+    if (!rc && !cached) rc = feat_index_upload(ctx, fc);
+    if (rc) return rc;
+    SummaryDev P;
+    memset(&P, 0, sizeof(P));
+    P.pos_end = rd->pos_end;
+    P.fmq = rd->fmq;
+    P.cig_off = rd->cig_off;
+    P.cigar = rd->cigar;
+    P.keys = rd->keys;
+    P.tiles = rd->tiles;
+    P.runs = rd->runs;
+    P.bnd_goff = (const int32_t *)ctx->scratch["fx_bnd_goff"].p;
+    P.bnd = (const int32_t *)ctx->scratch["fx_bnd"].p;
+    P.stab_off = (const int32_t *)ctx->scratch["fx_stab_off"].p;
+    P.fb = (const int32_t *)ctx->scratch["fx_fb"].p;
+    P.sf_end = (const int32_t *)ctx->scratch["fx_sf_end"].p;
+    P.stab4 = (const int4 *)ctx->scratch["fx_stab4"].p;
+    P.n_gid = n_gid;
+    P.n_samples = cells->n_samples;
+    P.own_g0 = own ? own[0] : INT32_MIN;
+    P.own_p0 = own ? own[1] : INT32_MIN;
+    P.own_g1 = own ? own[2] : INT32_MAX;
+    P.own_p1 = own ? own[3] : INT32_MAX;
+    P.fp.min_mapq = par->min_mapq;
+    P.fp.min_len = par->min_len;
+    P.fp.incl_flag = par->incl_flag;
+    P.fp.excl_flag = par->excl_flag;
+    P.fp.no_orphan = par->no_orphan;
+    P.fp.use_cell_tag = par->use_cell_tag;
+    P.fp.need_umi_tag = par->need_umi_tag;
+    P.incl_len = par->min_incl_len;
+    if (par->min_incl_tab) {
+        XG_GET(d_incl, int32_t, "sm_incl_tab", par->min_incl_tab_len + 1);
+        XG_CUDA(cudaMemcpyAsync(d_incl, par->min_incl_tab, sizeof(int32_t) * (size_t)par->min_incl_tab_len,
+                                cudaMemcpyHostToDevice, ctx->stream));
+        P.incl_tab = d_incl;
+        P.incl_tab_len = par->min_incl_tab_len;
+    }
+    if (par->use_cell_tag && (rc = xg_build_barcode_table(ctx, cells, &P.bc))) return rc;
+    const size_t n_out = ((size_t)cells->n_samples + 1) * SUM_FATES;
+    XG_GET(d_out, unsigned long long, "sm_out", n_out);
+    P.out = d_out;
+    XG_CUDA(cudaMemsetAsync(d_out, 0, sizeof(unsigned long long) * n_out, ctx->stream));
+    cudaEventRecord(ctx->ev[0], ctx->stream);
+    if (rd->n_tiles > 0 && n_gid > 0) k_basefc_summary<<<(unsigned)rd->n_tiles, SUM_THREADS, 0, ctx->stream>>>(P);
+    XG_CUDA(cudaGetLastError());
+    cudaEventRecord(ctx->ev[1], ctx->stream);
+    static_assert(sizeof(unsigned long long) == sizeof(int64_t), "counters are 64-bit");
+    XG_CUDA(cudaMemcpyAsync(out, d_out, sizeof(int64_t) * n_out, cudaMemcpyDeviceToHost, ctx->stream));
+    XG_CUDA(cudaStreamSynchronize(ctx->stream));
+    float t_k = 0;
+    cudaEventElapsedTime(&t_k, ctx->ev[0], ctx->ev[1]);
+    ctx->timing[0] = t_k;
+    ctx->timing[1] = t_k;
+    ctx->timing[2] = rd->n_tiles > 0 && n_gid > 0 ? 1 : 0;
+    ctx->timing[12] = ms_since(t_call);
     return XG_OK;
 }

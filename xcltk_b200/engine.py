@@ -335,7 +335,9 @@ def load_reads_sharded(sam_fn_list, chroms, cell_tag, umi_tag, want_seq, devices
             per_bam = []
             for b in range(len(sam_fn_list)):
                 off, first = index[b]
-                i_lo = max(first, first_block_with(b, lo_key, True) - 1)
+                # the block before the first one that begins at or after lo_key: records with key == lo_key may sit
+                # at the end of that block (a run of equal starts crosses block boundaries), and none in earlier ones
+                i_lo = max(first, first_block_with(b, lo_key, False) - 1)
                 i_hi = first_block_with(b, hi_key, False)
                 per_bam.append((int(off[i_lo]), int(off[max(i_lo, i_hi)])))
             ranges.append(per_bam)
@@ -369,7 +371,9 @@ def load_reads_sharded(sam_fn_list, chroms, cell_tag, umi_tag, want_seq, devices
              "max_aln_len": max([b.stats["max_aln_len"] for b in live] or [0]),
              "max_span": max([b.stats["max_span"] for b in live] or [0]),
              "bytes": sum(b.stats["bytes"] for b in live), "decoder": "device, sharded",
-             "byte_ranges": ranges, "halo_bp": span}
+             "byte_ranges": ranges, "halo_bp": span,
+             # chunk k holds the records whose start (tid, pos) lies in [cuts[k], cuts[k + 1]); tid_map: tid -> gid
+             "cuts": cuts, "tid_map": list(tid_maps[0])}
     return ShardedBatch(batches, shards, ks, gid_of, stats)
 
 

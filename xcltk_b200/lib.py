@@ -26,6 +26,9 @@ c_u8p = C.POINTER(C.c_uint8)
 
 XG_E_UNSUPPORTED = -7
 
+# columns of xg_basefc_summary's table (include/xcltk_b200.h), in its order
+SUMMARY_FATES = ("mapq", "flag", "no_umi", "short", "not_included", "one_feature", "multi_feature")
+
 # result layouts of xg_basefc (include/xcltk_b200.h), by Context.basefc's `segments`
 XG_LAYOUT_CSR, XG_LAYOUT_ROWS, XG_LAYOUT_ROWS_NARROW, XG_LAYOUT_ROWS_TINY = 0, 1, 2, 3
 
@@ -163,6 +166,8 @@ SYMBOLS = {
                                C.POINTER(C.POINTER(Coo))]),
     "xg_baf_state_free": (None, [_P, _P]),
     "xg_basefc_write_mtx_device": (C.c_int, [_P, C.c_char_p, C.c_int32, c_i32p, C.c_int32, C.c_int32]),
+    "xg_basefc_summary": (C.c_int, [_P, _P, C.POINTER(Features), C.POINTER(Barcodes), C.POINTER(Params), c_i32p,
+                                    c_i64p]),
     "xg_baf_fc": (C.c_int, [_P, _P, C.POINTER(Snps), C.POINTER(Barcodes), C.POINTER(Params), C.POINTER(SnpFilter),
                             C.c_int32, c_i64p, c_i32p, c_u8p, C.c_int32, c_i64p, c_u8p,
                             C.POINTER(C.POINTER(Coo)), C.POINTER(C.POINTER(Coo)), C.POINTER(C.POINTER(Coo))]),
@@ -684,6 +689,23 @@ class Context(object):
         out_row = np.ascontiguousarray(out_row, dtype=np.int32)
         self._check(self.lib.xg_basefc_write_mtx_device(self.h, path.encode(), len(out_row), as_ptr(out_row, c_i32p),
                                                         int(n_rows_out), int(n_threads)))
+
+    def basefc_summary(self, dreads, gid, beg, end, cell_keys, n_samples, params, own=None):
+        """Read-assignment summary (xg_basefc_summary): an (n_samples + 1, 7) int64 array, the records in range of a
+        feature per column (last row: cell tag missing or not listed) and fate (SUMMARY_FATES).  own: None, or
+        (gid_lo, pos_lo, gid_hi, pos_hi) -- only records whose (gid, pos) lies in [lo, hi) are counted."""
+        gid = np.ascontiguousarray(gid, dtype=np.int32)
+        beg = np.ascontiguousarray(beg, dtype=np.int32)
+        end = np.ascontiguousarray(end, dtype=np.int32)
+        keys = np.ascontiguousarray(cell_keys if cell_keys is not None else [], dtype=np.uint64)
+        f = Features(len(gid), as_ptr(gid, c_i32p), as_ptr(beg, c_i32p), as_ptr(end, c_i32p))
+        b = Barcodes(len(keys), as_ptr(keys, c_u64p), n_samples)
+        own_arr = None if own is None else np.ascontiguousarray(own, dtype=np.int32)
+        out = np.zeros((n_samples + 1, len(SUMMARY_FATES)), dtype=np.int64)
+        self._check(self.lib.xg_basefc_summary(self.h, dreads.h, C.byref(f), C.byref(b), C.byref(params.c),
+                                               None if own_arr is None else as_ptr(own_arr, c_i32p),
+                                               as_ptr(out, c_i64p)))
+        return out
 
     def basefc_host(self, host_reads, gid, beg, end, cell_keys, n_samples, params, segments=False):
         """basefc straight from a pinned host batch: H2D streamed under the counting kernels."""

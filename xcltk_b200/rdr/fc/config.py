@@ -56,6 +56,9 @@ class Config(object):
         # B200 additions (not in the reference): GPUs to shard over, host decode threads
         self.n_gpus = None
         self.devices = None
+        # --summary: also write summary.tsv (the table is left in summary_table)
+        self.summary = False
+        self.summary_table = None
 
     def show(self, fp=None, prefix=""):
         fp = fp or sys.stderr

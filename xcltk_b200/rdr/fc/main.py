@@ -48,6 +48,8 @@ def usage(fp=sys.stdout, conf=None):
         "      --cellTAG STR      Tag for cell barcodes, set to None when using sample IDs [%s]" % d.CELL_TAG,
         "      --UMItag STR       Tag for UMI, set to None when reads only [%s]" % d.UMI_TAG,
         "  -D, --debug INT        Used by developer for debugging [%d]" % d.DEBUG,
+        "      --summary          Also write summary.tsv: per cell, the records overlapping a feature by the filter",
+        "                         that dropped them or the number of features they passed.",
         "",
         "Read filtering:",
         "  --inclFLAG INT          Required flags: skip reads with all mask bits unset [%d]" % d.INCL_FLAG,
@@ -68,7 +70,7 @@ def usage(fp=sys.stdout, conf=None):
 
 _LONG = ["sam=", "samList=", "barcode=", "region=", "sampleList=", "sampleIDs=", "outdir=", "help",
          "ncores=", "cellTAG=", "UMItag=", "debug=", "inclFLAG=", "exclFLAG=", "minLEN=", "minMAPQ=",
-         "minINCLUDE=", "countORPHAN"]
+         "minINCLUDE=", "countORPHAN", "summary"]
 
 
 def fc_main(argv, conf=None):
@@ -104,6 +106,8 @@ def fc_main(argv, conf=None):
             sys.exit(0)
         elif op == "--countorphan":
             conf.no_orphan = False
+        elif op == "--summary":
+            conf.summary = True
         elif op in setters:
             attr, conv = setters[op]
             setattr(conf, attr, conv(val))
@@ -116,9 +120,10 @@ def fc_main(argv, conf=None):
 def fc_wrapper(sam_fn, barcode_fn, region_fn, out_dir, sam_list_fn=None, sample_ids=None,
                sample_id_fn=None, debug_level=0, ncores=1, cell_tag="CB", umi_tag="UB",
                output_all_reg=True, min_mapq=20, min_len=30, min_include=0.9, incl_flag=0,
-               excl_flag=None, no_orphan=True):
+               excl_flag=None, no_orphan=True, summary=False):
     """Python API, signature of rdr/fc/main.py:142-156.  As in the reference, a caller-supplied
-    `excl_flag` is ignored (main.py:177-178 only handles None): the default applies."""
+    `excl_flag` is ignored (main.py:177-178 only handles None): the default applies.
+    summary (not in the reference): also write summary.tsv (write_summary)."""
     conf = Config()
     conf.sam_fn, conf.sam_list_fn = sam_fn, sam_list_fn
     conf.barcode_fn, conf.region_fn = barcode_fn, region_fn
@@ -128,6 +133,7 @@ def fc_wrapper(sam_fn, barcode_fn, region_fn, out_dir, sam_list_fn=None, sample_
     conf.nproc, conf.output_all_reg = ncores, output_all_reg
     conf.min_mapq, conf.min_len, conf.min_include = min_mapq, min_len, min_include
     conf.incl_flag, conf.no_orphan = incl_flag, no_orphan
+    conf.summary = summary
     if excl_flag is None:
         conf.excl_flag = -1
     return fc_run(conf)
@@ -297,6 +303,8 @@ def count_features(conf, batch=None):
             row, col, val = parallel.merge_coo([p[:3] for p in parts], shards, len(regs))
             conf.last_timing = next((p[3] for p in parts if p[3] is not None), [0.0] * 16)
             conf.shard_sizes = [len(s) for s in shards]
+            if getattr(conf, "summary", False):
+                conf.summary_table = count_summary(conf, batch, gid, beg, end, cell_keys)
         elif isinstance(batch, engine.MultiBatch):
             load, total = parallel.reads_before(gid, beg, batch.runs, batch.pos_of_run)
             shards = parallel.partition(gid, beg, load, total, len(batch.batches))
@@ -310,6 +318,8 @@ def count_features(conf, batch=None):
             row, col, val = parallel.merge_coo([p[:3] for p in parts], shards, len(regs))
             conf.last_timing = parts[0][3]
             conf.shard_sizes = [len(s) for s in shards]
+            if getattr(conf, "summary", False):
+                conf.summary_table = count_summary(conf, batch, gid, beg, end, cell_keys)
         else:
             params = engine.make_params(conf, batch.stats["max_aln_len"], with_include=True)
             # fc_core: rows as completed, packed -- 16 bits per entry for the UMI counts of barcoded data (small numbers),
@@ -322,6 +332,8 @@ def count_features(conf, batch=None):
                 res = batch.ctx.basefc(batch.dreads, gid, beg, end, cell_keys, len(conf.samples), params,
                                        segments=seg)
             conf.last_timing = batch.ctx.timing()
+            if getattr(conf, "summary", False):      # after the counting: it reuses the context's feature index
+                conf.summary_table = count_summary(conf, batch, gid, beg, end, cell_keys)
             if seg:
                 conf.last_stats = dict(batch.stats)
                 conf.last_ctx = batch.ctx            # its staging area still holds the rows (device-side MTX text)
@@ -332,6 +344,71 @@ def count_features(conf, batch=None):
         if own:
             batch.close()
     return row, col, val
+
+
+SUMMARY_NO_CELL = "__no_cell"
+
+
+def own_ranges(lo, hi, tid_map):
+    """The `own` ranges of Context.basefc_summary, (gid_lo, pos_lo, gid_hi, pos_hi) each, that hold exactly the records
+    whose start (tid, pos) lies in the cut [lo, hi) of a library split by load_reads_sharded (cut keys are BAM tids,
+    record keys gids): one range per stretch of contigs whose gids follow one another in the BAM's order."""
+    neg = -(1 << 31)
+    out = []
+    for t in range(max(lo[0], 0), min(hi[0], len(tid_map) - 1) + 1):
+        g = int(tid_map[t])
+        if g < 0:
+            continue
+        start = (g, int(lo[1]) if t == lo[0] else neg)
+        stop = (g, int(hi[1])) if t == hi[0] else (g + 1, neg)
+        if out and out[-1][1] == start:
+            out[-1] = (out[-1][0], stop)
+        else:
+            out.append((start, stop))
+    return [(a[0], a[1], b[0], b[1]) for a, b in out]
+
+
+def count_summary(conf, batch, gid, beg, end, cell_keys):
+    """The read-assignment summary of the batch (Context.basefc_summary): (len(conf.samples) + 1, 7) int64 counts of
+    the records in range of some feature, per column (last row: no listed cell) and fate (lib.SUMMARY_FATES)."""
+    from ... import parallel
+    n = len(conf.samples)
+
+    def one(b, own=None):
+        params = engine.make_params(conf, b.stats["max_aln_len"], with_include=True)
+        if b.dreads is not None:
+            return b.ctx.basefc_summary(b.dreads, gid, beg, end, cell_keys, n, params, own)
+        # the pinned host batch that basefc_host streamed: mapped zero-copy rather than copied again -- only pos / end
+        # cross PCIe in bulk, flags, keys and CIGAR only for the records in range of a feature
+        dr = b.ctx.map_reads(b.host)
+        try:
+            return b.ctx.basefc_summary(dr, gid, beg, end, cell_keys, n, params, own)
+        finally:
+            dr.close()
+    if isinstance(batch, engine.ShardedBatch):
+        # every shard counts the records that start in its own cut, against all features
+        cuts, tid_map = batch.stats["cuts"], batch.stats["tid_map"]
+
+        def shard(k):
+            b, tot = batch.batches[k], np.zeros((n + 1, len(lib.SUMMARY_FATES)), dtype=np.int64)
+            if b is not None:
+                for own in own_ranges(cuts[k], cuts[k + 1], tid_map):
+                    tot += one(b, own)
+            return tot
+        return np.sum(parallel.run_on_devices(len(batch.batches), shard), axis=0)
+    if isinstance(batch, engine.MultiBatch):
+        return one(batch.batches[0])     # every GPU holds the whole library
+    return one(batch)
+
+
+def write_summary(path, samples, table):
+    """summary.tsv: a header, one row per sample in the order of barcodes.tsv, then the __no_cell row; `total` is the
+    sum of the seven fates.  Decimal integers, tab-separated, lines ending in '\n'."""
+    lines = ["\t".join(("cell", "total") + lib.SUMMARY_FATES)]
+    for name, r in zip(list(samples) + [SUMMARY_NO_CELL], np.asarray(table, dtype=np.int64).tolist()):
+        lines.append("\t".join([name, str(sum(r))] + [str(v) for v in r]))
+    with open(path, "w") as fp:
+        fp.write("\n".join(lines) + "\n")
 
 
 def fc_core(conf):
@@ -373,6 +450,11 @@ def fc_core(conf):
                          engine.n_decode_threads(conf.nproc))
     info("[GPU] %d reads counted in %.2f ms of kernels." % (
         conf.last_stats["n_reads"], conf.last_timing[0]))
+    if conf.summary:
+        write_summary(os.path.join(conf.out_dir, conf.out_prefix + "summary.tsv"), conf.samples, conf.summary_table)
+        tot = np.asarray(conf.summary_table).sum(axis=0)
+        info("[summary] %d records overlap a feature: %s." % (
+            int(tot.sum()), ", ".join("%s %d" % (k, int(v)) for k, v in zip(lib.SUMMARY_FATES, tot))))
 
 
 def fc_run(conf):
