@@ -23,8 +23,10 @@ static inline unsigned __reduce_or_sync(unsigned, unsigned v) { return v; }
 static inline int __popc(unsigned v) { return __builtin_popcount(v); }
 using std::min;
 #include "../xcltk_b200/csrc/inflate.cuh"
+// harness FILE [-r]: every block against zlib; with -r also each block's inflate_group<1> return code
 int main(int argc, char **argv) {
     FILE *fp = fopen(argv[1], "rb");
+    const bool print_rc = argc > 2 && !strcmp(argv[2], "-r");
     std::vector<uint8_t> f;
     uint8_t tmp[65536];
     size_t n;
@@ -43,6 +45,7 @@ int main(int argc, char **argv) {
         zs.next_in = &f[off + 12 + xlen]; zs.avail_in = clen; zs.next_out = exp.data(); zs.avail_out = isize;
         inflate(&zs, Z_FINISH); inflateEnd(&zs);
         int r = isize ? xg_inflate::inflate_group<1>(g, &f[off + 12 + xlen], clen, got.data(), isize) : 0;
+        if (print_rc) printf("block %d: rc %d\n", bi, r);
         // the lane-parallel CRC's arithmetic: 32 chunk CRCs combined must give the block's CRC32
         {
             const unsigned chunk = (isize + 31u) / 32u;

@@ -200,6 +200,37 @@ def test_packed_key_examples():
     assert ks.n_interned() == 2
 
 
+def limit_keys():
+    """values at the 63-bit packing limit (3 bits per base or '-', 7 per digit): 20 / 21 / 22 bases, 17 / 18 bases
+    + "-1", 8 / 9 / 10 digits, 14 bases + 3 digits (the last digit takes bits 56 -> 63) and neighbours"""
+    b = "ACGTN-ACGTACGTACGTACGTAC"
+    return [b[:20], b[:21], b[:22], b[:17] + "-1", b[:18] + "-1", "12345678", "123456789", "1234567890",
+            "ACGTACGTACGTAC" + "12" + "3", "ACGTACGTACGTAC" + "1234", "ACGTACGTACGTACGTAC7", "ACGTACGTACGTACGTACG7"]
+
+
+def packs(s):
+    return sum(7 if c.isdigit() else 3 for c in s) <= 63
+
+
+def test_limit_keys_pack_where_expected(tmp_path):
+    """63 bits pack, 64 do not (bit 63 marks an interned key); the host decoder gives a record the key the keyspace
+    gives its string, as CB, as UB and as query name"""
+    ks = lib.KeySpace()
+    assert sum(packs(s) for s in limit_keys()) == 7
+    for s in limit_keys():
+        assert (ks.encode(s) >> 63 == 0) == packs(s), s
+    keys = limit_keys()
+    recs = [(keys[i], 0, 0, 100 + i, 30, [(0, 10)], "ACGTACGTAC", [("CB", "Z", keys[i]), ("UB", "Z", keys[-1 - i])])
+            for i in range(len(keys))]
+    p = _write(tmp_path, recs, refs=(("chr1", 100000),))
+    for umi_tag, col_of in (("UB", lambda i: keys[-1 - i]), (None, lambda i: keys[i])):
+        hr, ks = decode([p], umi_tag=umi_tag)
+        assert hr.n == len(keys)
+        for i in range(len(keys)):
+            assert int(hr.keys[i, 0]) == ks.encode(keys[i]) and int(hr.keys[i, 1]) == ks.encode(col_of(i)), (i, umi_tag)
+        hr.close()
+
+
 BCH869 = os.path.join(GOLD, "bch869_smartseq", "BCH869.output.bam")     # copied from the reference's merge_smartseq/
 
 

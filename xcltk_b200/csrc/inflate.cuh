@@ -260,10 +260,11 @@ __device__ int inflate_group(GroupSmem &g, const uint8_t *in, uint32_t n_in, uin
         for (int k = (int)lane; k < (1 << DB); k += S) g.dlut[k] = 0;
         __syncwarp(gmask);
         if (lane == 0) {
+            // an incomplete code is legal only as one code of one bit (RFC 1951 3.2.7; zlib's inflate_table)
             int e1 = build_table(g, g.lens, hlit, g.lut, LB, g.lsym, g.lcount, 0);
-            if (type == 2 && (e1 < 0 || (e1 > 0 && hlit - g.lcount[0] != 1))) err = -11;
+            if (type == 2 && (e1 < 0 || (e1 > 0 && (hlit - g.lcount[0] != 1 || g.lcount[1] != 1)))) err = -11;
             int e2 = build_table(g, g.lens + hlit, hdist, g.dlut, DB, g.dsym, g.dcount, 1);
-            if (type == 2 && (e2 < 0 || (e2 > 0 && hdist - g.dcount[0] != 1))) err = -12;   // fixed distance code: 30 of 32
+            if (type == 2 && (e2 < 0 || (e2 > 0 && (hdist - g.dcount[0] != 1 || g.dcount[1] != 1)))) err = -12;   // fixed distance code: 30 of 32
         }
         err = __shfl_sync(gmask, err, 0, S);
         if (err) return err;
